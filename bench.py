@@ -75,7 +75,38 @@ def parse():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--e2e-skip", default="", help="tuning only: comma list of gen,reset,d2h left out of the e2e pass (its number is then not an e2e number)")
     ap.add_argument("--no-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computed (a fixed, seeded sample of at most "
+                         f"{DUMP_ROBOTS} robots per rank) to DIR/<name>.npy")
     return ap.parse_args()
+
+
+DUMP_ROBOTS = 32768  # ~56 MB for the full tick: cost + vehicle, IMU and arm state words as float64
+
+
+def dump_outputs(out_dir, n_rank, lo, rank, world, parts):
+    """Write a seeded sample of this rank's robots to out_dir/<name>.npy.  parts: [(robots, cost, {name: (state, words)})], one
+    per batch of `robots` consecutive robots (a chunk), holding device tensors.  State blocks are SoA ([words/4, robots, 4]); each
+    sampled robot's words are written as float64 (every uint32 word is exact there).  The sample depends only on the robot count,
+    so two builds run with the same arguments dump the same robots."""
+    import torch
+
+    m = min(DUMP_ROBOTS, n_rank)
+    pick = np.sort(np.random.default_rng(0x5EED).choice(n_rank, m, replace=False))
+    out, base = {"robot": [], "cost": []}, 0
+    for robots, cost, states in parts:
+        idx = pick[(pick >= base) & (pick < base + robots)] - base
+        it = torch.from_numpy(idx).to(cost.device)
+        out["robot"].append((idx + base + lo).astype(np.float64))
+        out["cost"].append(cost[it].cpu().numpy().astype(np.float32))
+        for name, (st, words) in states.items():
+            w = st.view(words // 4, robots, 4)[:, it].permute(1, 0, 2).reshape(len(idx), words)
+            out.setdefault(name, []).append(w.cpu().numpy().view(np.uint32).astype(np.float64))
+        base += robots
+    os.makedirs(out_dir, exist_ok=True)
+    sfx = f"_rank{rank}" if world > 1 else ""
+    for name, arrs in out.items():
+        np.save(os.path.join(out_dir, f"{name}{sfx}.npy"), np.concatenate(arrs))
 
 
 def workload_name(a):
@@ -530,6 +561,8 @@ def run_ours(a):
     ms = sharding.max_over_ranks(ms_local, dev)
     value = world * n * T * K / (ms * 1e-3)
     launches = K
+    if a.dump_outputs:  # before the e2e passes below reset and rerun the vehicles
+        dump_outputs(a.dump_outputs, n, first, rank, world, [(n, cost_d, {"vehicle_state": (vb.state, layout.VS_WORDS)})])
 
     ffma_tflops, issue_tflops, sm_count = fp32_probes(lib, local_rank, dev, stream)
     hbm_peak, hbm_src = hbm_peak_measured()
@@ -837,6 +870,11 @@ def run_ours_full(a):
     ms = sharding.max_over_ranks(ms_local, dev)
     value = a.total * T * K / (ms * 1e-3)
     launches = K * n_chunks * 6  # mode_init, push, yaw snapshot, IMU update, arm update, vehicle rollout
+    if a.dump_outputs:  # before the roofline and e2e passes below run chunk 0 again
+        dump_outputs(a.dump_outputs, n_rank, lo, rank, world,
+                     [(n, ch["cost"], {"vehicle_state": (ch["rb"].vehicle.state, layout.VS_WORDS),
+                                       "imu_state": (ch["rb"].imu.state, layout.IS_WORDS),
+                                       "arm_state": (ch["rb"].arm.state, layout.AS_WORDS)}) for ch in chunks])
 
     # ---- roofline of the dominant kernel: its share of the timed region, and timed alone -----------------------------
     ffma_tflops, issue_tflops, sm_count = fp32_probes(lib, local_rank, dev, stream)
@@ -1022,6 +1060,8 @@ def main():
     _JSON_FD = os.dup(1)
     os.dup2(2, 1)
     if a.impl == "reference":
+        if a.dump_outputs:
+            raise SystemExit("--dump-outputs writes what the GPU path computed: use it with --impl ours")
         run_reference(a)
     elif a.workload == "full":
         run_ours_full(a)

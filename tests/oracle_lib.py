@@ -6,6 +6,8 @@
              where /root/reference exists; the prebuilt .so travels to the GPU box)
 """
 import ctypes as C
+import hashlib
+import json
 import os
 import subprocess
 
@@ -62,6 +64,50 @@ def port():
             getattr(lib, nm).restype = C.c_float
         _cache["port"] = lib
     return _cache["port"]
+
+
+REF_DIGESTS = os.path.join(ROOT, "tests", "golden", "ref_digests.json")
+
+
+def digest(out):
+    """SHA-256 over every array in a (nested) result: dtype, shape and bytes."""
+    h = hashlib.sha256()
+
+    def walk(x):
+        if isinstance(x, (list, tuple)):
+            for y in x:
+                walk(y)
+        elif isinstance(x, dict):
+            for k in sorted(x):
+                h.update(k.encode())
+                walk(x[k])
+        elif x is not None:
+            a = np.ascontiguousarray(x)
+            h.update(f"{a.dtype.str}{a.shape}".encode())
+            h.update(a.tobytes())
+
+    walk(out)
+    return h.hexdigest()
+
+
+def reference_result(key, run, *libs):
+    """What the compiled reference returns for one test case: run("ref") where oracle/_ref has every library in `libs`,
+    run("port") elsewhere.  Either way the result must match the SHA-256 recorded under `key` in tests/golden/ref_digests.json,
+    so a checkout without the reference still holds the port (and the GPU tests built on it) to the reference's answer.
+    With ROBOTICK_RECORD_REF_DIGESTS=1 a missing key is recorded instead, noting which implementation produced it."""
+    kind = "ref" if all(os.path.exists(os.path.join(ORACLE, "_ref", name)) for name in libs) else "port"
+    out = run(kind)
+    with open(REF_DIGESTS) as f:
+        table = json.load(f)
+    d = digest(out)
+    if key not in table and os.environ.get("ROBOTICK_RECORD_REF_DIGESTS") == "1":
+        table[key] = {"sha256": d, "from": kind}
+        with open(REF_DIGESTS, "w") as f:
+            json.dump(table, f, indent=1, sort_keys=True)
+            f.write("\n")
+    assert key in table, f"no recorded reference result for {key!r} in {REF_DIGESTS}"
+    assert d == table[key]["sha256"], f"{key}: the {kind} result differs from the recorded reference result"
+    return out
 
 
 def have_ref(name="libref_vdt.so"):

@@ -12,7 +12,6 @@ import oracle_lib as ol
 from roboken_fmskf_robot_controller_b200 import _cabi, layout, streams
 
 GOLD = os.path.join(os.path.dirname(__file__), "golden")
-needs_ref = pytest.mark.skipif(not ol.have_ref("libref_arm.so"), reason="oracle/_ref not built and no /root/reference")
 
 
 def fresh(n):
@@ -90,21 +89,23 @@ def random_arm_states(n, seed, mg_any_branch=False):
     return layout.aos_to_soa(a)
 
 
-@needs_ref
 def test_debug_sequences_port_equals_ref():
     """POS_CMD_SEQ_DEBUG_0/1/2 (AD_mode_positioning_seq_debug_data.cpp:5-64): bring-up, push all
     three, run 600 ticks (the three sequences take 110 + 100 + 300 cycles + transitions)."""
-    r = ol.ref("libref_arm.so")
-    imgs = []
+    imgs = [img.copy() for img in np.load(os.path.join(GOLD, "arm_golden.npz"))["seq_a"][:3]]  # DEBUG_0/1/2 as the reference defines them
+    if ol.have_ref("libref_arm.so"):
+        r = ol.ref("libref_arm.so")
+        for w in range(3):
+            q = _cabi.AdtPosCmdSeq()
+            assert r.ref_adt_debug_seq(w, q) == (1 if w == 2 else 0)  # get_poscmdseq_debug() returns DEBUG_2
+            img = ol.seq_struct_to_image(q)
+            img[0] = 1
+            np.testing.assert_array_equal(img, imgs[w])
     for w in range(3):
-        q = _cabi.AdtPosCmdSeq()
-        assert r.ref_adt_debug_seq(w, q) == (1 if w == 2 else 0)  # get_poscmdseq_debug() returns DEBUG_2
-        img = ol.seq_struct_to_image(q)
-        img[0] = 10 + w
-        imgs.append(img)
+        imgs[w][0] = 10 + w
     script = [("init",)] + [("push", im[None, :], None) for im in imgs] + [("status", [10]), ("update", 150), ("status", [10]),
                                                                              ("status", [11]), ("update", 450), ("status", [12])]
-    a, b = run_script("ref", 1, script), run_script("port", 1, script)
+    a, b = ol.reference_result("arm_debug_sequences", lambda kind: run_script(kind, 1, script), "libref_arm.so"), run_script("port", 1, script)
     assert_same(a, b)
     tr = a[2][-4]  # the 450-tick trace
     assert tr[-1, 11, 0] == layout.ASTATE_STANDBY
@@ -112,7 +113,6 @@ def test_debug_sequences_port_equals_ref():
     np.testing.assert_array_equal(tr[-1, 0:5, 0].view(np.float32), np.float32([0, 120, -60, 0, 45]))
 
 
-@needs_ref
 @pytest.mark.parametrize("seed", [1, 2])
 def test_random_sequences_port_equals_ref(seed):
     n = 96
@@ -121,10 +121,9 @@ def test_random_sequences_port_equals_ref(seed):
     valid = (np.arange(n) % 3 != 0).astype(np.uint8)
     script = [("init",), ("push", s1, None), ("update", 37), ("push", s2, valid), ("status", np.full(n, 1)),
               ("update", 500), ("status", np.full(n, 2)), ("status", np.full(n, 7))]
-    assert_same(run_script("ref", n, script), run_script("port", n, script))
+    assert_same(ol.reference_result(f"arm_random_sequences_{seed}", lambda kind: run_script(kind, n, script), "libref_arm.so"), run_script("port", n, script))
 
 
-@needs_ref
 def test_ring_overflow_and_id0_port_equals_ref():
     """Five pushes into the 4-slot ring (the 4th/5th are dropped while the first is executing),
     id 0 before the first move (isModeFirstCall), status for ids in every ring position."""
@@ -136,10 +135,9 @@ def test_ring_overflow_and_id0_port_equals_ref():
         script += [("push", seqs[k], None)] + [("status", np.full(n, j)) for j in range(6)]
     script += [("update", 900)] + [("status", np.full(n, j)) for j in range(6)]
     script += [("push", seqs[5], None), ("update", 5)] + [("status", np.full(n, j)) for j in range(6)]
-    assert_same(run_script("ref", n, script), run_script("port", n, script))
+    assert_same(ol.reference_result("arm_ring_overflow", lambda kind: run_script(kind, n, script), "libref_arm.so"), run_script("port", n, script))
 
 
-@needs_ref
 def test_random_states_port_equals_ref():
     n = 400
     st0 = random_arm_states(n, seed=4)
@@ -149,10 +147,10 @@ def test_random_states_port_equals_ref():
         taos[:, s * 260 : (s + 1) * 260] = streams.arm_sequences(n, seed=20 + s, seq_id=s + 1, max_len=5)
     tab[:] = layout.aos_to_soa(taos)
     script = [("update", 3), ("status", np.full(n, 2)), ("update", 120)]
-    assert_same(run_script("ref", n, script, st0, tab), run_script("port", n, script, st0, tab))
+    assert_same(ol.reference_result("arm_random_states", lambda kind: run_script(kind, n, script, st0, tab), "libref_arm.so"),
+                run_script("port", n, script, st0, tab))
 
 
-@needs_ref
 def test_mg_torque_control_branches_port_equals_ref():
     """JointMgServo::update, all four branches (AD_joint_mg_servo.cpp:50-73): torque on->off edge
     (PI_D reset), not initialised + torque on (torque control), position control, torque off
@@ -165,7 +163,7 @@ def test_mg_torque_control_branches_port_equals_ref():
         taos[:, s * 260 : (s + 1) * 260] = streams.arm_sequences(n, seed=30 + s, seq_id=s + 1, max_len=4)
     tab = layout.aos_to_soa(taos)
     script = [("update", 1), ("update", 2), ("update", 60)]
-    a, b = run_script("ref", n, script, st0, tab), run_script("port", n, script, st0, tab)
+    a, b = ol.reference_result("arm_mg_branches", lambda kind: run_script(kind, n, script, st0, tab), "libref_arm.so"), run_script("port", n, script, st0, tab)
     assert_same(a, b)
     fl = (layout.soa_to_aos(st0, n, layout.AS_WORDS)[:, layout.AS_JFLAGS] >> 4) & 0xF
     assert len(np.unique(fl)) == 16  # every flag combination of the MG joint occurred
@@ -173,7 +171,6 @@ def test_mg_torque_control_branches_port_equals_ref():
     assert set(np.unique(tr[0, 5, :] * 0 + (layout.soa_to_aos(a[2][1], n, layout.AS_WORDS)[:, layout.AS_MG_TX] & 0xFF))) >= {0xA1, 0xA4}
 
 
-@needs_ref
 def test_extreme_waypoints_port_equals_ref():
     """dt going backwards (u32 wrap -> huge count), dt == previous (count clamps to 1), angles past
     the ICS range (+-180 deg: degPos100 rejects; > +-135 deg: setPos rejects) and a len-0 sequence."""
@@ -181,7 +178,7 @@ def test_extreme_waypoints_port_equals_ref():
           (45, (100, -100, 100, -100, 100))]
     img = np.stack([streams.arm_seq_image(3, wp), streams.arm_seq_image(4, []), streams.arm_seq_image(5, wp[:2])])
     script = [("init",), ("push", img, None), ("update", 40), ("status", [3, 4, 5]), ("update", 40)]
-    assert_same(run_script("ref", 3, script), run_script("port", 3, script))
+    assert_same(ol.reference_result("arm_extreme_waypoints", lambda kind: run_script(kind, 3, script), "libref_arm.so"), run_script("port", 3, script))
 
 
 def test_port_matches_golden():

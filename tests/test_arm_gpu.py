@@ -150,12 +150,11 @@ def test_arm_mg_velocity_division_domains_vs_port():
     assert_same(gpu_script(len(mags), script), run_script("port", len(mags), script))
 
 
-@pytest.mark.skipif(not ol.have_ref("libref_arm.so"), reason="oracle/_ref/libref_arm.so not present")
 def test_arm_vs_compiled_reference():
     n = 64
     s1 = streams.arm_sequences(n, seed=77, seq_id=5, max_len=10)
     script = [("init",), ("push", s1, None), ("update", 250), ("status", np.full(n, 5))]
-    assert_same(gpu_script(n, script), run_script("ref", n, script))
+    assert_same(gpu_script(n, script), ol.reference_result("arm_gpu", lambda kind: run_script(kind, n, script), "libref_arm.so"))
 
 
 def test_arm_full_size_c4():

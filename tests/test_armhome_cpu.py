@@ -9,7 +9,6 @@ import pytest
 import oracle_lib as ol
 from roboken_fmskf_robot_controller_b200 import _cabi, layout
 
-needs_ref = pytest.mark.skipif(not ol.have_ref("libref_arm.so"), reason="oracle/_ref/libref_arm.so not available")
 GOLD = os.path.join(os.path.dirname(__file__), "golden", "armhome_golden.npz")
 PREV_JOINTS = (layout.AJ_P1, layout.AJ_DFL, layout.AJ_DFR, layout.AJ_P3)
 
@@ -56,14 +55,13 @@ def run(kind, mode, s0, n, K, now, chunks=None):
     return st, hs, tr
 
 
-@needs_ref
 @pytest.mark.parametrize("mode", [_cabi.RK_ADH_MODE_INIT, _cabi.RK_ADH_MODE_INIT_POS_MOVE])
 @pytest.mark.parametrize("fb", [False, True])
 def test_homing_port_equals_ref(mode, fb):
     n, K = 48, 1500
     s0 = start_states(n, seed=10 * mode + fb)
     now = feedback(n, K, seed=3) if fb else None
-    a, b = run("port", mode, s0, n, K, now), run("ref", mode, s0, n, K, now)
+    a, b = run("port", mode, s0, n, K, now), ol.reference_result(f"armhome_{mode}_{int(fb)}", lambda kind: run(kind, mode, s0, n, K, now), "libref_arm.so")
     for x, y, nm in zip(a, b, ("state", "mode block", "trace")):
         np.testing.assert_array_equal(x, y, err_msg=nm)
     final = layout.soa_to_aos(a[1], n, layout.HS_WORDS)[:, layout.HS_STATE]
@@ -71,15 +69,14 @@ def test_homing_port_equals_ref(mode, fb):
     assert ((final & 0xFF) == done).all() and (final & layout.AS_FSM_IS_COMP).all()  # every arm reached COMPLETED
 
 
-@needs_ref
 def test_homing_from_power_on_known_sequence():
     """All-zero arm through INIT: 1 + 101 + 501 + 1 cycles of the fixed phases, then the ramp to the init pose
     (slowest axis J2: 0 -> -90 deg at 30 deg/s = 300 cycles; J1 sits at its mechanical end, 150 deg, after the reset and
     needs 17), COMPLETED afterwards; MG in torque control until MOVE_INIT_POS."""
     n, K = 2, 1200
     s0 = start_states(n, 0, zero=True)
-    for kind in ("port", "ref"):
-        st, hs, tr = run(kind, _cabi.RK_ADH_MODE_INIT, s0, n, K, None)
+    for st, hs, tr in (run("port", _cabi.RK_ADH_MODE_INIT, s0, n, K, None),
+                       ol.reference_result("armhome_power_on", lambda kind: run(kind, _cabi.RK_ADH_MODE_INIT, s0, n, K, None), "libref_arm.so")):
         states = tr[:, 11, 0]
         first = {s: int(np.argmax(states == s)) for s in (1, 2, 3, 4, 5)}
         assert first[1] == 0 and first[2] == 101 and first[3] == 101 + 501 and first[4] == 101 + 501 + 1

@@ -7,7 +7,6 @@ import oracle_lib as ol
 from roboken_fmskf_robot_controller_b200 import layout
 from test_arm_cpu import random_arm_states
 
-needs_ref = pytest.mark.skipif(not ol.have_ref("libref_arm.so"), reason="oracle/_ref not built and no /root/reference")
 
 
 def pos_cmds(n, seed, cid):
@@ -65,13 +64,13 @@ def bringup_state(n, seed):
     return st
 
 
-@needs_ref
 @pytest.mark.parametrize("seed", [1, 2])
 def test_positioning_mode_port_equals_ref(seed):
     n = 64
     st0 = bringup_state(n, seed)
     sc = pos_script(n, seed)
-    a, b = run_pos_script("ref", n, sc, st0), run_pos_script("port", n, sc, st0)
+    a = ol.reference_result(f"armpos_{seed}", lambda kind: run_pos_script(kind, n, sc, st0), "libref_arm.so")
+    b = run_pos_script("port", n, sc, st0)
     assert len(a[2]) == len(b[2])
     for x, y in zip(a[2], b[2]):
         np.testing.assert_array_equal(x, y)

@@ -43,11 +43,11 @@ def test_positioning_mode_vs_port(n, seed):
         np.testing.assert_array_equal(x, y, err_msg=f"output {k}")
 
 
-@pytest.mark.skipif(not ol.have_ref("libref_arm.so"), reason="oracle/_ref/libref_arm.so not present")
 def test_positioning_mode_vs_compiled_reference():
     n = 48
     st0 = bringup_state(n, 9)
     sc = pos_script(n, 9)
-    got, exp = gpu_pos_script(n, sc, st0), run_pos_script("ref", n, sc, st0)[2]
+    got = gpu_pos_script(n, sc, st0)
+    exp = ol.reference_result("armpos_gpu", lambda kind: run_pos_script(kind, n, sc, st0), "libref_arm.so")[2]
     for k, (x, y) in enumerate(zip(got, exp)):
         np.testing.assert_array_equal(x, y, err_msg=f"output {k}")

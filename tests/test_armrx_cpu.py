@@ -7,7 +7,6 @@ import pytest
 import oracle_lib as ol
 from roboken_fmskf_robot_controller_b200 import layout
 
-HAVE_REF = ol.have_ref("libref_arm.so")
 
 
 def rx_cases(n, seed, mg_upper_zero=True):
@@ -45,13 +44,12 @@ def run(kind, state, n, frames, cmdid):
     return st, curs
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="oracle/_ref not built")
 @pytest.mark.parametrize("seed", [1, 2, 3])
 def test_port_equals_reference_rx(seed):
     n = 4000
     state, frames, cmdid = rx_cases(n, seed)
     pst, pcur = run("port", state, n, frames, cmdid)
-    rst, rcur = run("ref", state, n, frames, cmdid)
+    rst, rcur = ol.reference_result(f"armrx_{seed}", lambda kind: run(kind, state, n, frames, cmdid), "libref_arm.so")
     np.testing.assert_array_equal(pst, rst)
     for a, b in zip(pcur, rcur):
         np.testing.assert_array_equal(a.view(np.uint32), b.view(np.uint32))

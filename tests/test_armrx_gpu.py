@@ -49,12 +49,11 @@ def test_rx_vs_port(n, seed, upper_zero):
         np.testing.assert_array_equal(a.view(np.uint32), b.view(np.uint32))
 
 
-@pytest.mark.skipif(not ol.have_ref("libref_arm.so"), reason="oracle/_ref not present")
 def test_rx_vs_compiled_reference():
     n = 4096
     state, frames, cmdid = rx_cases(n, 21, mg_upper_zero=True)
     gst, gcur = gpu_rx(state, n, frames, cmdid)
-    rst, rcur = host_rx("ref", state, n, frames, cmdid)
+    rst, rcur = ol.reference_result("armrx_gpu", lambda kind: host_rx(kind, state, n, frames, cmdid), "libref_arm.so")
     np.testing.assert_array_equal(gst, rst)
     for a, b in zip(gcur, rcur):
         np.testing.assert_array_equal(a.view(np.uint32), b.view(np.uint32))

@@ -38,22 +38,22 @@ def test_ref_appendix_d():
     _appendix_d(ol.imu_ref)
 
 
-@needs_ref
 def test_port_equals_ref_random_streams():
     n, K = 96, 40
     regs, have = streams.imu_samples(n, K, seed=5, drop_every=7)
     have[0] = 1
-    a, b = np.zeros(layout.IS_WORDS * n, dtype=np.uint32), np.zeros(layout.IS_WORDS * n, dtype=np.uint32)
-    oa = ol.imu_port(a, n, regs, have, want_out=True, do_init=True)
-    ob = ol.imu_ref(b, n, regs, have, want_out=True, do_init=True)
-    np.testing.assert_array_equal(oa, ob)
-    np.testing.assert_array_equal(a, b)
-    # continue from that state without init
     regs2, have2 = streams.imu_samples(n, K, seed=6, drop_every=5)
-    oa = ol.imu_port(a, n, regs2, have2, want_out=True)
-    ob = ol.imu_ref(b, n, regs2, have2, want_out=True)
-    np.testing.assert_array_equal(oa, ob)
-    np.testing.assert_array_equal(a, b)
+
+    def run(kind):
+        fn = ol.imu_port if kind == "port" else ol.imu_ref
+        st = np.zeros(layout.IS_WORDS * n, dtype=np.uint32)
+        o1 = fn(st, n, regs, have, want_out=True, do_init=True)
+        s1 = st.copy()
+        o2 = fn(st, n, regs2, have2, want_out=True)  # continue from that state without init
+        return o1, s1, o2, st
+
+    for x, y in zip(run("port"), ol.reference_result("imu_random_streams", run, "libref_imu.so")):
+        np.testing.assert_array_equal(x, y)
 
 
 def test_golden_imu():

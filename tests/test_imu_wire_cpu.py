@@ -9,7 +9,6 @@ import pytest
 import oracle_lib as ol
 from roboken_fmskf_robot_controller_b200 import layout, streams
 
-needs_ref = pytest.mark.skipif(not ol.have_ref("libref_imu.so"), reason="oracle/_ref/libref_imu.so not available")
 GOLD = os.path.join(os.path.dirname(__file__), "golden", "imu_wire_golden.npz")
 
 
@@ -17,6 +16,17 @@ def parser_sreg(parser_soa, n):
     """The 16 tracked sReg words of every IMU out of the RK_IP_* block: int16 [n, 16]."""
     a = layout.soa_to_aos(parser_soa, n, layout.IP_WORDS)[:, layout.IP_SREG : layout.IP_SREG + 8]
     return np.ascontiguousarray(a).view(np.int16).reshape(n, 16)
+
+
+def wire_run(kind, n, cells, nbytes):
+    """Raw bytes into the IMU from power-on (update 0 is init()): (out, state, sReg int16 [n, 16]), port or compiled reference."""
+    st = np.zeros(layout.IS_WORDS * n, dtype=np.uint32)
+    if kind == "ref":
+        out, sreg = ol.imu_bytes_ref(st, n, cells, nbytes, want_out=True)
+        return out, st, sreg
+    ps = np.zeros(layout.IP_WORDS * n, dtype=np.uint32)
+    out = ol.imu_bytes_port(st, ps, n, cells, nbytes, want_out=True, do_init=True)
+    return out, st, parser_sreg(ps, n)
 
 
 def test_wit_frame_checksum():
@@ -41,7 +51,6 @@ def test_clean_wire_equals_register_path():
     np.testing.assert_array_equal(yaw, (ang_yaw * streams.DEG2RAD).astype(np.float32))
 
 
-@needs_ref
 @pytest.mark.parametrize("n,K,ncells,seed,full", [(64, 24, 4, 1, False), (48, 40, 1, 2, False), (32, 10, 16, 3, False),
                                                    (40, 64, 1, 4, True), (24, 12, 3, 5, True)])
 def test_port_equals_ref_fuzzed_wire(n, K, ncells, seed, full):
@@ -50,8 +59,7 @@ def test_port_equals_ref_fuzzed_wire(n, K, ncells, seed, full):
         nbytes = None
     a, pa = np.zeros(layout.IS_WORDS * n, dtype=np.uint32), np.zeros(layout.IP_WORDS * n, dtype=np.uint32)
     oa = ol.imu_bytes_port(a, pa, n, cells, nbytes, want_out=True, do_init=True)
-    b = np.zeros(layout.IS_WORDS * n, dtype=np.uint32)
-    ob, sreg = ol.imu_bytes_ref(b, n, cells, nbytes, want_out=True)
+    ob, b, sreg = ol.reference_result(f"imu_wire_fuzz_{seed}", lambda kind: wire_run(kind, n, cells, nbytes), "libref_imu.so")
     np.testing.assert_array_equal(oa, ob)
     np.testing.assert_array_equal(a, b)
     np.testing.assert_array_equal(parser_sreg(pa, n), sreg)
@@ -60,7 +68,6 @@ def test_port_equals_ref_fuzzed_wire(n, K, ncells, seed, full):
     assert 0 < err.sum() < n
 
 
-@needs_ref
 def test_port_chunked_equals_ref_one_pass():
     """Parser state carried across calls (window, fill count, read index, sReg) == one uninterrupted replay."""
     n, K, ncells = 40, 30, 2
@@ -71,8 +78,7 @@ def test_port_chunked_equals_ref_one_pass():
         outs.append(ol.imu_bytes_port(a, pa, n, np.ascontiguousarray(cells[k0:k1]), np.ascontiguousarray(nbytes[k0:k1]),
                                       want_out=True, do_init=(k0 == 0)))
         k0 = k1
-    b = np.zeros(layout.IS_WORDS * n, dtype=np.uint32)
-    ob, sreg = ol.imu_bytes_ref(b, n, cells, nbytes, want_out=True)
+    ob, b, sreg = ol.reference_result("imu_wire_one_pass", lambda kind: wire_run(kind, n, cells, nbytes), "libref_imu.so")
     np.testing.assert_array_equal(np.concatenate(outs), ob)
     np.testing.assert_array_equal(a, b)
     np.testing.assert_array_equal(parser_sreg(pa, n), sreg)
@@ -122,14 +128,12 @@ def late_quaternion_wire(n, K, seed):
     return cells, nb, late
 
 
-@pytest.mark.skipif(not ol.have_ref("libref_imu.so"), reason="oracle/_ref not built")
 def test_init_waits_for_a_late_first_quaternion_frame_like_the_reference():
     """ADVICE r1: init() must not latch q_init (or publish) before its first quaternion frame.  Port == the compiled
     reference, whose blocking init() is fed the following update slots while it spins."""
     n, K = 64, 12
     cells, nb, late = late_quaternion_wire(n, K, 77)
-    st_r = np.zeros(layout.IS_WORDS * n, dtype=np.uint32)
-    out_r, sreg_r = ol.imu_bytes_ref(st_r, n, cells, nb, want_out=True)
+    out_r, st_r, sreg_r = ol.reference_result("imu_wire_late_quaternion", lambda kind: wire_run(kind, n, cells, nb), "libref_imu.so")
     st_p, ps_p = np.zeros(layout.IS_WORDS * n, dtype=np.uint32), np.zeros(layout.IP_WORDS * n, dtype=np.uint32)
     out_p = ol.imu_bytes_port(st_p, ps_p, n, cells, nb, want_out=True, do_init=True)
     np.testing.assert_array_equal(out_p, out_r)

@@ -51,69 +51,66 @@ def test_port_reproduces_survey_appendix_d():
     _check_appendix_d(tr, pos_libm=False)
 
 
-@needs_ref
 def test_port_equals_ref_c1_trace():
-    s_ref, t_ref = _run("ref", wl.c1_inputs())
+    s_ref, t_ref = ol.reference_result("vdt_c1", lambda kind: _run(kind, wl.c1_inputs()), "libref_vdt.so")
     s_port, t_port = _run("port", wl.c1_inputs())
     np.testing.assert_array_equal(t_port, t_ref)
     np.testing.assert_array_equal(s_port, s_ref)
 
 
-@needs_ref
 @pytest.mark.parametrize("seed", [0x5EED, 7])
 def test_port_equals_ref_plant_rollout(seed):
     inp = wl.plant_inputs(48, 2000, seed=seed)
-    s_ref, t_ref = _run("ref", inp)
+    s_ref, t_ref = ol.reference_result(f"vdt_plant_{seed}", lambda kind: _run(kind, inp), "libref_vdt.so")
     s_port, t_port = _run("port", inp)
     np.testing.assert_array_equal(t_port, t_ref)
     np.testing.assert_array_equal(s_port, s_ref)
 
 
-@needs_ref
 def test_port_equals_ref_stream_rollout():
     from roboken_fmskf_robot_controller_b200 import streams
 
     inp = wl.plant_inputs(32, 600, seed=11)
     fr = streams.vehicle_frames(32, 600, seed=11)
-    s_ref, t_ref = _run("ref", inp, sensor=_cabi.RK_SENSOR_STREAM, frames=fr)
+    s_ref, t_ref = ol.reference_result("vdt_stream", lambda kind: _run(kind, inp, sensor=_cabi.RK_SENSOR_STREAM, frames=fr),
+                                       "libref_vdt.so")
     s_port, t_port = _run("port", inp, sensor=_cabi.RK_SENSOR_STREAM, frames=fr)
     np.testing.assert_array_equal(t_port, t_ref)
     np.testing.assert_array_equal(s_port, s_ref)
 
 
-@needs_ref
 def test_port_equals_ref_from_random_states():
     n = 512
     st0 = layout.aos_to_soa(wl.random_states(n, seed=3))
     inp = wl.plant_inputs(n, 40, seed=5, seg_len=8, yaw_period=4)
-    s_ref, t_ref = _run("ref", inp, state=st0)
+    s_ref, t_ref = ol.reference_result("vdt_random_states", lambda kind: _run(kind, inp, state=st0), "libref_vdt.so")
     s_port, t_port = _run("port", inp, state=st0)
     np.testing.assert_array_equal(t_port, t_ref)
     np.testing.assert_array_equal(s_port, s_ref)
     # hold mode (no frames) as well
-    s_ref, t_ref = _run("ref", inp, sensor=_cabi.RK_SENSOR_HOLD, state=st0)
+    s_ref, t_ref = ol.reference_result("vdt_random_states_hold", lambda kind: _run(kind, inp, sensor=_cabi.RK_SENSOR_HOLD, state=st0),
+                                       "libref_vdt.so")
     s_port, t_port = _run("port", inp, sensor=_cabi.RK_SENSOR_HOLD, state=st0)
     np.testing.assert_array_equal(t_port, t_ref)
     np.testing.assert_array_equal(s_port, s_ref)
 
 
-@needs_ref
 def test_mymath_known_answers():
-    r = ol.ref()
+    xs = np.concatenate([np.linspace(-50, 50, 4001), [0.0, 6.2831855, 6.283185, -6.2831855, 360.0, -360.0, 720.5]]).astype(np.float32)
+
+    def values(kind):
+        lib, pre = (ol.ref(), "ref_") if kind == "ref" else (ol.port(), "orc_")
+        fn = {nm: getattr(lib, pre + nm) for nm in ("atan2f", "atanf", "normalize_rad_0to2pi", "normalize_deg_0to360")}
+        sin, cos = (lib.ref_sinf, lib.ref_cosf) if kind == "ref" else (lib.orc_sin, lib.orc_cos)
+        known = [fn["atan2f"](1, 1), fn["atanf"](0.5), fn["atan2f"](-1, -2), fn["normalize_rad_0to2pi"](-0.5),
+                 fn["normalize_rad_0to2pi"](7), fn["normalize_deg_0to360"](-190)]
+        return [np.float32(known)] + [np.float32([f(x) for x in xs]) for f in (fn["normalize_rad_0to2pi"], fn["normalize_deg_0to360"], sin, cos)]
+
+    r = ol.reference_result("mymath", values, "libref_vdt.so")
     # SURVEY.md Appendix D
-    assert np.float32(r.ref_atan2f(1, 1)) == np.float32(0.785398185)
-    assert np.float32(r.ref_atanf(0.5)) == np.float32(0.463646978)
-    assert np.float32(r.ref_atan2f(-1, -2)) == np.float32(-2.67794585)
-    assert np.float32(r.ref_normalize_rad_0to2pi(-0.5)) == np.float32(5.78318548)
-    assert np.float32(r.ref_normalize_rad_0to2pi(7)) == np.float32(0.716814518)
-    assert np.float32(r.ref_normalize_deg_0to360(-190)) == np.float32(170)
-    p = ol.port()
-    xs = np.concatenate([np.linspace(-50, 50, 4001), [0.0, 6.2831855, 6.283185, -6.2831855, 360.0, -360.0, 720.5]])
-    for x in xs.astype(np.float32):
-        assert np.float32(p.orc_normalize_rad_0to2pi(x)).tobytes() == np.float32(r.ref_normalize_rad_0to2pi(x)).tobytes()
-        assert np.float32(p.orc_normalize_deg_0to360(x)).tobytes() == np.float32(r.ref_normalize_deg_0to360(x)).tobytes()
-        assert np.float32(p.orc_sin(x)).tobytes() == np.float32(r.ref_sinf(x)).tobytes()
-        assert np.float32(p.orc_cos(x)).tobytes() == np.float32(r.ref_cosf(x)).tobytes()
+    np.testing.assert_array_equal(r[0], np.float32([0.785398185, 0.463646978, -2.67794585, 5.78318548, 0.716814518, 170]))
+    for got, exp in zip(values("port"), r):
+        np.testing.assert_array_equal(got.view(np.uint32), exp.view(np.uint32))
 
 
 def test_sin_table_accuracy():

@@ -35,56 +35,60 @@ def special_values():
     return v
 
 
-@needs_ref
+def reference_tables(kind):
+    """The arctangent tables of util_mymath.cpp as the compiled reference holds them; the port's are the generated ones."""
+    if kind == "port":
+        return generated_tables()
+    rt, rd, rw = np.zeros(700, dtype=np.float32), np.zeros(27, dtype=np.float32), np.zeros(26, dtype=np.float32)
+    nt = ol.ref("libref_rm.so").ref_rm_atan_tables(rt.ctypes.data, rd.ctypes.data, rw.ctypes.data)
+    return [rt[:nt], rd, rw]
+
+
 def test_generated_atan_tables_equal_the_reference_arrays():
     t, d, w = generated_tables()
-    r = ol.ref("libref_rm.so")
-    rt, rd, rw = np.zeros(700, dtype=np.float32), np.zeros(27, dtype=np.float32), np.zeros(26, dtype=np.float32)
-    nt = r.ref_rm_atan_tables(rt.ctypes.data, rd.ctypes.data, rw.ctypes.data)
-    assert nt == 625 and len(t) == 625 and len(d) == 27 and len(w) == 26
-    np.testing.assert_array_equal(t.view(np.uint32), rt[:625].view(np.uint32))
+    rt, rd, rw = ol.reference_result("rm_atan_tables", reference_tables, "libref_rm.so")
+    assert len(rt) == 625 and len(t) == 625 and len(d) == 27 and len(w) == 26
+    np.testing.assert_array_equal(t.view(np.uint32), rt.view(np.uint32))
     np.testing.assert_array_equal(d.view(np.uint32), rd.view(np.uint32))
     np.testing.assert_array_equal(w.view(np.uint32), rw.view(np.uint32))
 
 
-@needs_ref
 def test_atan_port_equals_ref():
-    r, p = ol.ref("libref_rm.so"), ol.port()
+    p = ol.port()
     rng = np.random.default_rng(4)
     xs = np.concatenate([special_values(), generated_tables()[1], np.nextafter(generated_tables()[1], np.float32(np.inf)),
                          (rng.standard_normal(4000) * 3).astype(np.float32), np.exp(rng.uniform(-20, 20, 4000)).astype(np.float32)])
-    for x in xs:
-        a, b = np.float32(p.orc_atanf(float(x))), np.float32(r.ref_rm_atanf(float(x)))
-        assert a.view(np.uint32) == b.view(np.uint32), (x, a, b)
     ys = rng.permutation(xs)
-    for y, x in zip(ys, xs):
-        a, b = np.float32(p.orc_atan2f(float(y), float(x))), np.float32(r.ref_rm_atan2f(float(y), float(x)))
-        assert a.view(np.uint32) == b.view(np.uint32), (y, x, a, b)
+
+    def values(kind):
+        atanf, atan2f = (p.orc_atanf, p.orc_atan2f) if kind == "port" else (ol.ref("libref_rm.so").ref_rm_atanf, ol.ref("libref_rm.so").ref_rm_atan2f)
+        return np.float32([atanf(float(x)) for x in xs]), np.float32([atan2f(float(y), float(x)) for y, x in zip(ys, xs)])
+
+    for a, b in zip(values("port"), ol.reference_result("rm_atan", values, "libref_rm.so")):
+        np.testing.assert_array_equal(a.view(np.uint32), b.view(np.uint32))
     assert np.float32(p.orc_atan2f(1, 1)) == np.float32(0.785398185)  # SURVEY Appendix D probes
     assert np.float32(p.orc_atanf(0.5)) == np.float32(0.463646978)
     assert np.float32(p.orc_atan2f(-1, -2)) == np.float32(-2.67794585)
 
 
-@needs_ref
 @pytest.mark.parametrize("n,K,seed", [(96, 700, 1), (257, 320, 2)])
 def test_guard_port_equals_ref(n, K, seed):
     inp = streams.rm_inputs(n, K, seed=seed)
-    a, b = np.zeros(layout.RS_WORDS * n, dtype=np.uint32), np.zeros(layout.RS_WORDS * n, dtype=np.uint32)
-    ca, aa = ol.rm_guard("port", a, n, inp)
-    cb, ab = ol.rm_guard("ref", b, n, inp)
-    np.testing.assert_array_equal(ca, cb)
-    np.testing.assert_array_equal(aa, ab)
-    np.testing.assert_array_equal(a, b)
-    seen = np.bitwise_or.reduce(aa.reshape(-1))
-    assert seen == 0x10F0F  # every abort bit the block can raise was raised
-    # continue from that state, other parameters
     p = _cabi.RmtParams(17, 333, 55)
     inp2 = streams.rm_inputs(n, 120, seed=seed + 10)
-    ca, aa = ol.rm_guard("port", a, n, inp2, params=p)
-    cb, ab = ol.rm_guard("ref", b, n, inp2, params=p)
-    np.testing.assert_array_equal(ca, cb)
-    np.testing.assert_array_equal(aa, ab)
-    np.testing.assert_array_equal(a, b)
+
+    def run(kind):
+        st = np.zeros(layout.RS_WORDS * n, dtype=np.uint32)
+        c1, a1 = ol.rm_guard(kind, st, n, inp)
+        s1 = st.copy()
+        c2, a2 = ol.rm_guard(kind, st, n, inp2, params=p)  # continue from that state, other parameters
+        return c1, a1, s1, c2, a2, st
+
+    got = run("port")
+    for x, y in zip(got, ol.reference_result(f"rm_guard_{seed}", run, "libref_rm.so")):
+        np.testing.assert_array_equal(x, y)
+    seen = np.bitwise_or.reduce(got[1].reshape(-1))
+    assert seen == 0x10F0F  # every abort bit the block can raise was raised
 
 
 def record(kind=0, a=0, b=0, c=0, x=0.0, y=0.0, z=0.0, floor=(1,) * 8):

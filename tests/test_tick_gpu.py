@@ -72,11 +72,11 @@ def test_full_tick_vs_port(n, steps, seed):
     compare(gpu_full(n, steps, 10, *inp), oracle_full("port", n, steps, 10, *inp))
 
 
-@pytest.mark.skipif(not (ol.have_ref("libref_arm.so") and ol.have_ref("libref_imu.so")), reason="oracle/_ref not present")
 def test_full_tick_vs_compiled_reference():
     n, steps = 64, 600
     inp = make_inputs(n, steps, 10, 44)
-    compare(gpu_full(n, steps, 10, *inp), oracle_full("ref", n, steps, 10, *inp))
+    exp = ol.reference_result("full_tick_gpu", lambda kind: oracle_full(kind, n, steps, 10, *inp), "libref_vdt.so", "libref_imu.so", "libref_arm.so")
+    compare(gpu_full(n, steps, 10, *inp), exp)
 
 
 def test_full_tick_cost_and_slice_invariance():

@@ -7,7 +7,6 @@ import pytest
 import oracle_lib as ol
 from roboken_fmskf_robot_controller_b200 import _cabi, layout, streams
 
-needs_ref = pytest.mark.skipif(not ol.have_ref("libref_vdt_task.so"), reason="oracle/_ref not built and no /root/reference")
 
 
 def task_inputs(n, steps, seed, seg_len=50, yaw_period=10):
@@ -29,17 +28,15 @@ def run(kind, inp, trace=True):
     return st, ro.trace
 
 
-@needs_ref
 @pytest.mark.parametrize("seed,seg_len", [(1, 50), (2, 30), (3, 200)])
 def test_port_equals_reference_task(seed, seg_len):
     inp = task_inputs(40, 1200, seed, seg_len=seg_len)
-    s_ref, t_ref = run("ref", inp)
+    s_ref, t_ref = ol.reference_result(f"vdt_task_{seed}", lambda kind: run(kind, inp), "libref_vdt_task.so")
     s_port, t_port = run("port", inp)
     np.testing.assert_array_equal(t_port, t_ref)
     np.testing.assert_array_equal(s_port, s_ref)
 
 
-@needs_ref
 def test_every_direction_and_limiter():
     """All REQ_MOVE_DIR codes (0..10 + two undefined) x speeds {default, in range, over the limit}, time 300 ms:
     after the countdown fires every vehicle is commanded to stop."""
@@ -56,7 +53,7 @@ def test_every_direction_and_limiter():
             k += 1
     yaw_deg = np.zeros((1, n), dtype=np.float32)
     inp = dict(n=n, steps=700, cmd=cmd, seg_len=1000, yaw=yaw_deg.copy(), yaw_deg=yaw_deg, yaw_period=1000)
-    s_ref, t_ref = run("ref", inp)
+    s_ref, t_ref = ol.reference_result("vdt_task_directions", lambda kind: run(kind, inp), "libref_vdt_task.so")
     s_port, t_port = run("port", inp)
     np.testing.assert_array_equal(t_port, t_ref)
     np.testing.assert_array_equal(s_port, s_ref)

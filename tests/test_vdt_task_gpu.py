@@ -26,11 +26,10 @@ def test_task_layer_vs_port(n, steps, seed, seg_len):
     assert_same(st, pst, "task-layer state vs port")
 
 
-@pytest.mark.skipif(not ol.have_ref("libref_vdt_task.so"), reason="oracle/_ref/libref_vdt_task.so not present")
 def test_task_layer_vs_reference_task():
     inp = task_inputs(96, 1500, 7, seg_len=70)
     st, tr = gpu_task(inp)
-    rst, rtr = run("ref", inp)
+    rst, rtr = ol.reference_result("vdt_task_gpu", lambda kind: run(kind, inp), "libref_vdt_task.so")
     assert_same(tr, rtr, "task-layer trace vs the compiled VDT task")
     assert_same(st, rst, "task-layer state vs the compiled VDT task")
 

@@ -70,12 +70,12 @@ def port_run(inp, sensor=_cabi.RK_SENSOR_PLANT, frames=None, state=None, trace=T
     return st, ro.trace
 
 
-def ref_run(inp, sensor=_cabi.RK_SENSOR_PLANT, frames=None, state=None):
+def host_run(kind, inp, sensor=_cabi.RK_SENSOR_PLANT, frames=None, state=None):
     n = inp["n"]
     st = np.zeros(layout.VS_WORDS * n, dtype=np.uint32) if state is None else state.copy()
     ro = ol.HostRollout(n, inp["steps"], sensor, inp.get("cmd"), inp.get("seg_len", 0), inp.get("yaw"),
                         inp.get("yaw_period", 0), frames=frames, trace=True)
-    ol.run_ref(st, n, ro)
+    (ol.run_ref if kind == "ref" else ol.run_port)(st, n, ro)
     return st, ro.trace
 
 
@@ -101,11 +101,10 @@ def test_c1_trace_bit_exact_vs_port_and_golden():
         assert tuple(tr[step, 9:13, 0].view(np.int32)) == cur
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(ol.ORACLE, "_ref", "libref_vdt.so")), reason="no prebuilt oracle/_ref")
 def test_plant_rollout_bit_exact_vs_compiled_reference():
     inp = wl.plant_inputs(64, 1500, seed=3)
     st, tr = gpu_run(inp)
-    rst, rtr = ref_run(inp)
+    rst, rtr = ol.reference_result("vdt_gpu_plant", lambda kind: host_run(kind, inp), "libref_vdt.so")
     assert_same(tr, rtr, "plant trace vs compiled reference")
     assert_same(st, rst, "plant state vs compiled reference")
 

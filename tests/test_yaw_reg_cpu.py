@@ -2,13 +2,11 @@
 port and the compiled vehicle reference agree on it, both agree with the float stream computed on the host, and that
 float stream IS what the compiled IMU reference (IMU_IF_WT901C::updateData -> getYawDate) reports for the register."""
 import numpy as np
-import pytest
 
 import oracle_lib as ol
 import workloads as wl
 from roboken_fmskf_robot_controller_b200 import _cabi, layout, streams
 
-needs_ref = pytest.mark.skipif(not (ol.have_ref("libref_vdt.so") and ol.have_ref("libref_imu.so")), reason="oracle/_ref not available")
 
 
 def rollout(kind, n, steps, inp, yaw):
@@ -18,7 +16,6 @@ def rollout(kind, n, steps, inp, yaw):
     return st, ro.trace
 
 
-@needs_ref
 def test_yaw_register_stream_three_ways():
     n, steps = 48, 700
     inp = wl.plant_inputs(n, steps, seed=3)
@@ -29,13 +26,14 @@ def test_yaw_register_stream_three_ways():
     regs[0, 12] = 32767
     regs[1:, 11] = reg
     regs[1:, 12] = 32767
-    out = ol.imu_ref(np.zeros(layout.IS_WORDS * n, dtype=np.uint32), n, regs, None, want_out=True, do_init=True)
+    out = ol.reference_result("yaw_reg_imu", lambda kind: (ol.imu_port if kind == "port" else ol.imu_ref)(
+        np.zeros(layout.IS_WORDS * n, dtype=np.uint32), n, regs, None, want_out=True, do_init=True), "libref_imu.so")
     yaw_deg = out.view(np.float32)[1:, 2, :, 3]  # Data word 11 = angle[2] = getYawDate()
     rad = (yaw_deg * streams.DEG2RAD).astype(np.float32)  # the ISR's mymath::deg2rad
     np.testing.assert_array_equal(rad.view(np.uint32), streams.yaw_reg_to_rad(reg).view(np.uint32))
-    base = rollout("ref", n, steps, inp, np.ascontiguousarray(rad))
-    for kind in ("port", "ref"):
-        got = rollout(kind, n, steps, inp, reg)
+    base = ol.reference_result("yaw_reg_float", lambda kind: rollout(kind, n, steps, inp, np.ascontiguousarray(rad)), "libref_vdt.so")
+    for got in (rollout("port", n, steps, inp, reg),
+                ol.reference_result("yaw_reg_register", lambda kind: rollout(kind, n, steps, inp, reg), "libref_vdt.so")):
         np.testing.assert_array_equal(got[1], base[1])
         np.testing.assert_array_equal(got[0], base[0])
 
