@@ -619,6 +619,62 @@ int rk_stream_imu_samples(const rk_stream_desc_t *d_desc, int64_t n, int32_t n_u
 int rk_stream_arm_sequences(const rk_stream_desc_t *d_desc, int64_t n, void *d_seq, void *stream);
 
 /* =====================================================================================
+ * Vehicle sampling planner: one planning step for R robots with S candidates each is three calls on one stream,
+ *   rk_plan_sample_commands  nominal [n_seg][R]           -> candidates [n_seg][R*S]
+ *   rk_plan_rollout          R source states + candidates -> cost [R*S]       (source states untouched)
+ *   rk_plan_select           cost + candidates            -> new nominal [n_seg][R], best index / cost [R]
+ * after which the caller runs the first segment of the new nominal on its robots with rk_vdt_rollout.  Candidate j
+ * of robot r is instance r*S + j everywhere.  Every float result is defined as single IEEE float32 operations (round
+ * to nearest, no contraction) in the order written here; streams.plan_commands_v2 restates the sampler in numpy.
+ * Arguments are checked (RK_ERR_ARG): R >= 0, S >= 1, n_seg * S < 2^32, seg_len >= 1, 0 <= shift < n_seg, lambda >= 0
+ * and finite, state blocks and command tables 16-byte aligned.  R == 0 is a no-op.
+ * ===================================================================================== */
+typedef struct rk_plan_sample {
+  int64_t  first;     /* global index of robot 0 (sharded planners draw the same noise as one GPU would) */
+  uint32_t seed;
+  uint32_t rsv;
+  float    sigma[3];  /* noise scale of vx, vy (mm/s) and vth (rad/s) */
+  float    rsv2;
+} rk_plan_sample_t; /* 32 bytes */
+
+typedef struct rk_plan_cost {
+  const float *d_ref; /* float2 [n_seg][R]: where robot r should be (m) when segment s ends; s = n_seg-1 is the goal */
+  float w_pos;        /* weight of |pos - ref_s|^2 at the end of segments 0 .. n_seg-2 */
+  float w_goal;       /* weight of |pos - ref_{n_seg-1}|^2 after the last tick */
+  float w_cur;        /* weight of sum_w cur_tgt_w^2 at the end of every segment */
+  float rsv;
+} rk_plan_cost_t; /* 24 bytes */
+
+/* Candidate j of robot r (global index g = first + r), segment s: j == 0 is the nominal itself; otherwise, with
+ * h = streams.h32(seed, 40, g, s*S + j) and u_k = u01_32(lite32(h, 4a + k)), axis a gets
+ * xi_a = ((((u_0 + u_1) + u_2) + u_3) - 2) * 1.7320508f (Irwin-Hall, unit variance) and v_a = nom_a + sigma_a * xi_a.
+ * Then speed_limit_xy: ln = sqrtf(vx*vx + vy*vy); ln > p->limit_speed_mmps (L) -> vx = (vx*L)/ln, vy = (vy*L)/ln; vth is
+ * clamped to +-p->limit_rot_radps; kind = RK_CMD_MOVE (the nominal's kind is ignored).  d_cmd must not overlap d_nominal. */
+int rk_plan_sample_commands(const rk_vdt_params_t *p, const rk_plan_sample_t *s, const rk_vdt_cmd_t *d_nominal,
+                            int64_t R, int32_t S, int32_t n_seg, rk_vdt_cmd_t *d_cmd, void *stream);
+/* n_seg * seg_len closed-loop ticks (RK_SENSOR_PLANT) of candidate r*S + j from robot r's block of d_src_state (pitch R),
+ * command cell [s][r*S + j] applied before tick s*seg_len as rk_vdt_rollout applies d_cmd; no yaw stream and no task
+ * loop (the source heading is held).  At the end of segment s, with (x, y) the position words and c_k = (float) the
+ * sign-extended s16_rawCurr_tgt of wheel k:
+ *   dx = x - ref[s].x;  dy = y - ref[s].y;  e = dx*dx + dy*dy;  q = ((c0*c0 + c1*c1) + c2*c2) + c3*c3
+ *   J  = (J + (s < n_seg-1 ? w_pos : w_goal) * e) + w_cur * q          (J starts at 0)
+ * d_cost[r*S + j] = J.  No state is written.  The kernel is chosen as for rk_vdt_rollout (RK_OPT_* included); the costs
+ * do not depend on it. */
+int rk_plan_rollout(const rk_vdt_params_t *p, const void *d_src_state, int64_t R, int32_t S,
+                    const rk_vdt_cmd_t *d_cmd, int32_t n_seg, int32_t seg_len,
+                    const rk_plan_cost_t *cost, float *d_cost, void *stream);
+/* best[r] = argmin_j cost[r*S + j] (NaN counts as +inf, ties to the lowest j; all NaN: 0), best_cost[r] = that cost.
+ * nominal_out[s][r] takes segment s + shift of the candidates (the last segment repeated past the end):
+ *   lambda == 0: candidate best copied bit for bit;
+ *   lambda > 0:  vx, vy, vth = sum_j w_j v_j / sum_j w_j with w_j = expf(-(c_j - c_min) / lambda) (NaN cost: w = 0),
+ *                kind = RK_CMD_MOVE, in a fixed reduction order (repeatable bit for bit); a robot without a finite
+ *                minimum cost gets candidate best as under lambda == 0.
+ * d_best / d_best_cost may be NULL.  d_nominal_out must not overlap d_cmd. */
+int rk_plan_select(const float *d_cost, const rk_vdt_cmd_t *d_cmd, int64_t R, int32_t S, int32_t n_seg,
+                   float lambda, int32_t shift, rk_vdt_cmd_t *d_nominal_out, int32_t *d_best, float *d_best_cost,
+                   void *stream);
+
+/* =====================================================================================
  * RobotManager guard (SURVEY 8f-2): the vehicle-management block of RMT's routine_ros()
  * (src/RobotManager/RM_task_main.cpp:484-767), one call = K manager cycles of n robots.  Per
  * cycle: at most one ROS message is delivered through the callback the firmware runs for it

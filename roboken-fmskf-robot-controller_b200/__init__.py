@@ -17,4 +17,8 @@ def __getattr__(name):
         from . import vehicle as _v
 
         return _v if name == "vehicle" else _v.VehicleBatch
+    if name in ("planner", "VehiclePlanner"):
+        from . import planner as _p
+
+        return _p if name == "planner" else _p.VehiclePlanner
     raise AttributeError(name)

@@ -164,6 +164,18 @@ class TickRollout(C.Structure):
     ]
 
 
+class PlanSample(C.Structure):
+    """rk_plan_sample_t"""
+
+    _fields_ = [("first", C.c_int64), ("seed", C.c_uint32), ("rsv", C.c_uint32), ("sigma", C.c_float * 3), ("rsv2", C.c_float)]
+
+
+class PlanCost(C.Structure):
+    """rk_plan_cost_t"""
+
+    _fields_ = [("d_ref", C.c_void_p), ("w_pos", C.c_float), ("w_goal", C.c_float), ("w_cur", C.c_float), ("rsv", C.c_float)]
+
+
 _lib = None
 
 
@@ -209,6 +221,10 @@ def _proto(lib):
     lib.rk_stream_imu_samples.argtypes = [vp, C.c_int64, C.c_int32, vp, vp, vp]
     lib.rk_stream_imu_samples_yaw.argtypes = [vp, C.c_int64, C.c_int32, vp, vp, vp, vp]
     lib.rk_stream_arm_sequences.argtypes = [vp, C.c_int64, vp, vp]
+    lib.rk_plan_sample_commands.argtypes = [C.POINTER(VdtParams), C.POINTER(PlanSample), vp, C.c_int64, C.c_int32, C.c_int32, vp, vp]
+    lib.rk_plan_rollout.argtypes = [C.POINTER(VdtParams), vp, C.c_int64, C.c_int32, vp, C.c_int32, C.c_int32, C.POINTER(PlanCost), vp,
+                                    vp]
+    lib.rk_plan_select.argtypes = [vp, vp, C.c_int64, C.c_int32, C.c_int32, C.c_float, C.c_int32, vp, vp, vp, vp]
     lib.rk_adt_bldc_rx.argtypes = [C.POINTER(AdtParams), vp, C.c_int64, C.c_int, vp, vp, vp, vp]
     lib.rk_adt_mg_rx.argtypes = [C.POINTER(AdtParams), vp, C.c_int64, vp, vp, vp]
     lib.rk_selftest_div_rcp64.argtypes = [C.c_uint64, C.c_uint64, C.POINTER(C.c_uint32)]

@@ -69,16 +69,44 @@ RK_DEV bool yaw_enabled(const rk_vdt_rollout_t &a) {
 // big-endian, wire order from the low byte of the word
 RK_DEV uint32_t c610_tx_word(int32_t cur_a, int32_t cur_b) { return __byte_perm((uint32_t)cur_a, (uint32_t)cur_b, 0x4501); }
 
-template <int MODE, bool TRACE>
+// rk_plan_rollout: the PLAN instantiations of the rollout kernels run candidate i = r * S + j of n = R * S from robot
+// r's block of the source (pitch R, read only), form the stage cost at every segment end and store nothing else.
+struct PlanArgs {
+  int64_t       R;
+  int32_t       S;
+  const float2 *ref; // [n_seg][R], metres
+  float         w_pos, w_goal, w_cur;
+  float        *cost; // [R * S]
+};
+// J after the end of segment s (rk_plan_cost_t): the state is that after tick (s + 1) * seg_len - 1
+RK_DEV float plan_stage_cost(float J, const Veh &v, const PlanArgs &pl, int s, int n_seg, int64_t r) {
+  const float2 g = __ldg(pl.ref + (int64_t)s * pl.R + r);
+  const float  dx = fsub(v.pos[0], g.x), dy = fsub(v.pos[1], g.y);
+  const float  e = fadd(fmul(dx, dx), fmul(dy, dy));
+  float        c[4];
+#pragma unroll
+  for(int k = 0; k < 4; k++) c[k] = (float)v.m[k].cur_tgt;
+  const float q = fadd(fadd(fadd(fmul(c[0], c[0]), fmul(c[1], c[1])), fmul(c[2], c[2])), fmul(c[3], c[3]));
+  return fadd(fadd(J, fmul(s < n_seg - 1 ? pl.w_pos : pl.w_goal, e)), fmul(pl.w_cur, q));
+}
+
+template <int MODE, bool TRACE, bool PLAN = false>
 __global__ void __launch_bounds__(kRolloutThreads)
-vdt_rollout_kernel(const rk_vdt_params_t p, uint4 *__restrict__ state, int64_t n, const rk_vdt_rollout_t a) {
+vdt_rollout_kernel(const rk_vdt_params_t p, uint4 *__restrict__ state, int64_t n, const rk_vdt_rollout_t a, const PlanArgs pl) {
   __shared__ float s_tab[513];
   stage_sin_table(s_tab);
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if(i >= n) return;
 
-  Veh v;
-  load_veh(state, n, i, v);
+  Veh     v;
+  int64_t r = 0;
+  float   J = 0.0f;
+  if constexpr(PLAN) {
+    r = i / pl.S;
+    load_veh(state, pl.R, r, v);
+  } else {
+    load_veh(state, n, i, v);
+  }
   const Derived d = derive(p);
   float         cth, sth;
   yaw_trig(s_tab, v.pos[2], cth, sth);
@@ -96,6 +124,8 @@ vdt_rollout_kernel(const rk_vdt_params_t p, uint4 *__restrict__ state, int64_t n
   }
 
   for(int t = 0; t < a.steps; t++) {
+    if constexpr(PLAN)
+      if(t == sc.next_cmd && sc.seg > 0) J = plan_stage_cost(J, v, pl, sc.seg - 1, a.n_seg, r);
     sched_events(v, p, a, n, i, t, sc);
     if(t == next_yaw) { // can_tx_routine_intr -> set_now_yaw_world()   VD_task_main.cpp:368
       if(yaw_of_pf(a, load_yaw_pf(a, n, i, yk), yk, i, v.pos[2])) yaw_trig(s_tab, v.pos[2], cth, sth);
@@ -128,6 +158,10 @@ vdt_rollout_kernel(const rk_vdt_params_t p, uint4 *__restrict__ state, int64_t n
       tr[(int64_t)13 * n] = (a.task_period > 0) ? v.move_cnt : 0u;
       tr[(int64_t)14 * n] = c610_tx_word(v.m[0].cur_tgt, v.m[1].cur_tgt), tr[(int64_t)15 * n] = c610_tx_word(v.m[2].cur_tgt, v.m[3].cur_tgt);
     }
+  }
+  if constexpr(PLAN) {
+    pl.cost[i] = plan_stage_cost(J, v, pl, a.n_seg - 1, a.n_seg, r);
+    return;
   }
   store_veh(state, n, i, v);
   if(a.d_cost != nullptr && a.d_goal != nullptr) {
@@ -208,7 +242,9 @@ RK_DEV void yaw_feed_take(YawFeed &y, const rk_vdt_rollout_t &a, int64_t n, int6
 }
 
 // FLAGS: bit 0 FFSAT (ff_limit == 1: FMUL.SAT form of the feed-forward clamp), bit 1 KD0 (kd == 0, packed tick only)
-template <bool TRACE, int OCC, int FLAGS, bool PACKED, bool RESET = false>
+// PLAN: rk_plan_rollout (PlanArgs); segment ends are command ticks, so they are chunk boundaries and the stage cost is
+// formed outside the chunk loop.
+template <bool TRACE, int OCC, int FLAGS, bool PACKED, bool RESET = false, bool PLAN = false>
 #if defined(RK_FAST_MAXNREG) // tuning builds: the register budget given directly (finer occupancy steps with small CTAs)
 __global__ void __maxnreg__(RK_FAST_MAXNREG)
 #elif defined(RK_FAST_MINBLOCKS)
@@ -216,7 +252,8 @@ __global__ void __launch_bounds__(kFastThreads, RK_FAST_MINBLOCKS)
 #else
 __global__ void __launch_bounds__(kFastThreads, OCC * 128 / kFastThreads)
 #endif
-vdt_rollout_fast_kernel(const rk_vdt_params_t p, uint4 *__restrict__ state, int64_t n, const rk_vdt_rollout_t a, const CmdRcp rcp) {
+vdt_rollout_fast_kernel(const rk_vdt_params_t p, uint4 *__restrict__ state, int64_t n, const rk_vdt_rollout_t a, const CmdRcp rcp,
+                        const PlanArgs pl) {
   constexpr int  D0 = 1, D1 = 1, D2 = -1, D3 = -1; // VD_task_main.cpp:75-78 (host checks params match)
   constexpr bool FFSAT = (FLAGS & 1) != 0, KD0 = (FLAGS & 2) != 0;
   __shared__ float s_tab[513];
@@ -224,9 +261,17 @@ vdt_rollout_fast_kernel(const rk_vdt_params_t p, uint4 *__restrict__ state, int6
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if(i >= n) return;
 
-  Veh v;
-  if(RESET) v = Veh{}; // reset_state: the power-on block is all zeros -- nothing to load (and no memset in front of the kernel)
-  else load_veh(state, n, i, v);
+  Veh     v;
+  int64_t r = 0;
+  float   J = 0.0f;
+  if constexpr(PLAN) { // the S candidates of robot r read the same cells (one broadcast per warp)
+    r = i / pl.S;
+    load_veh(state, pl.R, r, v);
+  } else if(RESET) {
+    v = Veh{}; // reset_state: the power-on block is all zeros -- nothing to load (and no memset in front of the kernel)
+  } else {
+    load_veh(state, n, i, v);
+  }
   const Derived d = derive(p);
   FastConsts    fc;
   fast_consts(fc, p, d);
@@ -241,6 +286,8 @@ vdt_rollout_fast_kernel(const rk_vdt_params_t p, uint4 *__restrict__ state, int6
 
   int t = 0;
   while(t < K) {
+    if constexpr(PLAN)
+      if(t == sch.next_cmd && sch.seg > 0) J = plan_stage_cost(J, v, pl, sch.seg - 1, a.n_seg, r);
     sched_events(v, p, a, n, i, t, sch, RK_FAST_CMDRCP ? &rcp : nullptr); // commands, VDT::main messages and the move-time countdown due at this tick
     // run to the next event: a command, the countdown's automatic stop, or the last tick of the launch
     // (always a transcription tick).  Lanes of a warp whose countdowns fire at different ticks leave
@@ -296,6 +343,10 @@ vdt_rollout_fast_kernel(const rk_vdt_params_t p, uint4 *__restrict__ state, int6
                        v.m[2].cur_tgt, v.m[3].cur_tgt, (a.task_period > 0) ? v.move_cnt : 0u);
       t++;
     }
+  }
+  if constexpr(PLAN) { // the end state is discarded: 448 B per candidate not written
+    pl.cost[i] = plan_stage_cost(J, v, pl, a.n_seg - 1, a.n_seg, r);
+    return;
   }
   store_veh(state, n, i, v);
   if(a.d_cost != nullptr && a.d_goal != nullptr) {
@@ -527,9 +578,9 @@ static cudaError_t launch_rollout(const rk_vdt_params_t &p, void *d_state, int64
                                   cudaStream_t st) {
   const unsigned grid = (unsigned)((n + kRolloutThreads - 1) / kRolloutThreads);
   if(a.d_trace)
-    vdt_rollout_kernel<MODE, true><<<grid, kRolloutThreads, 0, st>>>(p, (uint4 *)d_state, n, a);
+    vdt_rollout_kernel<MODE, true><<<grid, kRolloutThreads, 0, st>>>(p, (uint4 *)d_state, n, a, PlanArgs{});
   else
-    vdt_rollout_kernel<MODE, false><<<grid, kRolloutThreads, 0, st>>>(p, (uint4 *)d_state, n, a);
+    vdt_rollout_kernel<MODE, false><<<grid, kRolloutThreads, 0, st>>>(p, (uint4 *)d_state, n, a, PlanArgs{});
   return cudaGetLastError();
 }
 
@@ -683,7 +734,7 @@ int rk_vdt_rollout(const rk_vdt_params_t *p, void *d_state, int64_t n, const rk_
       const unsigned grid  = (unsigned)((n + kFastThreads - 1) / kFastThreads);
       const int      flags = ((p->ff_limit == 1.0f && g_fast_ffsat) ? 1 : 0) | ((p->kd == 0.0f && g_fast_packed) ? 2 : 0);
       const CmdRcp rcp = make_cmd_rcp(*p);
-#define RK_LAUNCH_FAST3(TR, OCC, FL, PK) vdt_rollout_fast_kernel<TR, OCC, FL, PK><<<grid, kFastThreads, 0, st>>>(*p, (uint4 *)d_state, n, *args, rcp)
+#define RK_LAUNCH_FAST3(TR, OCC, FL, PK) vdt_rollout_fast_kernel<TR, OCC, FL, PK><<<grid, kFastThreads, 0, st>>>(*p, (uint4 *)d_state, n, *args, rcp, PlanArgs{})
 #define RK_LAUNCH_FAST(TR, OCC)                                    \
   do {                                                             \
     if(!g_fast_packed) {                                           \
@@ -699,7 +750,7 @@ int rk_vdt_rollout(const rk_vdt_params_t *p, void *d_state, int64_t n, const rk_
     }                                                              \
   } while(0)
       if(reset_in_kernel) {
-        vdt_rollout_fast_kernel<false, 4, 2, true, true><<<grid, kFastThreads, 0, st>>>(*p, (uint4 *)d_state, n, *args, rcp);
+        vdt_rollout_fast_kernel<false, 4, 2, true, true><<<grid, kFastThreads, 0, st>>>(*p, (uint4 *)d_state, n, *args, rcp, PlanArgs{});
       } else if(args->d_trace) {
         RK_LAUNCH_FAST(true, 4);
       } else {
@@ -740,6 +791,79 @@ int rk_vdt_rollout(const rk_vdt_params_t *p, void *d_state, int64_t n, const rk_
   default: set_error("rk_vdt_rollout: bad sensor_mode %d", args->sensor_mode); return RK_ERR_ARG;
   }
   if(e != cudaSuccess) return cuda_fail(e, "vdt_rollout_kernel launch");
+  return RK_OK;
+}
+
+} // extern "C"
+namespace rk {
+// rk_plan_rollout's kernel choice: the RK_SENSOR_PLANT dispatch of rk_vdt_rollout without trace and reset
+template <int OCC>
+static void launch_plan_fast(const rk_vdt_params_t &p, const void *d_src, int64_t n, const rk_vdt_rollout_t &a, const CmdRcp &rcp,
+                             const PlanArgs &pl, cudaStream_t st) {
+  const unsigned grid  = (unsigned)((n + kFastThreads - 1) / kFastThreads);
+  const int      flags = ((p.ff_limit == 1.0f && g_fast_ffsat) ? 1 : 0) | ((p.kd == 0.0f && g_fast_packed) ? 2 : 0);
+  uint4         *src   = (uint4 *)d_src; // read only under PLAN
+#define RK_LAUNCH_PLAN(FL, PK) vdt_rollout_fast_kernel<false, OCC, FL, PK, false, true><<<grid, kFastThreads, 0, st>>>(p, src, n, a, rcp, pl)
+  if(!g_fast_packed) {
+    if(flags & 1) RK_LAUNCH_PLAN(1, false);
+    else RK_LAUNCH_PLAN(0, false);
+  } else {
+    switch(flags) {
+    case 3: RK_LAUNCH_PLAN(3, true); break;
+    case 2: RK_LAUNCH_PLAN(2, true); break;
+    case 1: RK_LAUNCH_PLAN(1, true); break;
+    default: RK_LAUNCH_PLAN(0, true); break;
+    }
+  }
+#undef RK_LAUNCH_PLAN
+}
+} // namespace rk
+extern "C" {
+
+int rk_plan_rollout(const rk_vdt_params_t *p, const void *d_src_state, int64_t R, int32_t S, const rk_vdt_cmd_t *d_cmd, int32_t n_seg,
+                    int32_t seg_len, const rk_plan_cost_t *cost, float *d_cost, void *stream) {
+  if(!p || !cost) {
+    set_error("rk_plan_rollout: NULL params/cost");
+    return RK_ERR_ARG;
+  }
+  if(R < 0 || S < 1) {
+    set_error("rk_plan_rollout: need R >= 0 and S >= 1 (R = %lld, S = %d)", (long long)R, S);
+    return RK_ERR_ARG;
+  }
+  if(n_seg < 1 || seg_len < 1 || (int64_t)n_seg * seg_len > INT_MAX) {
+    set_error("rk_plan_rollout: need n_seg >= 1, seg_len >= 1 and n_seg * seg_len < 2^31 (n_seg = %d, seg_len = %d)", n_seg, seg_len);
+    return RK_ERR_ARG;
+  }
+  if((uint64_t)n_seg * (uint64_t)S >= (1ull << 32)) {
+    set_error("rk_plan_rollout: n_seg * S must be < 2^32");
+    return RK_ERR_ARG;
+  }
+  if(R == 0) return RK_OK;
+  if(int rc = check_block(d_src_state, "d_src_state")) return rc;
+  if(int rc = check_block(d_cmd, "d_cmd")) return rc;
+  if(!cost->d_ref || ((uintptr_t)cost->d_ref & 7u) || !d_cost || ((uintptr_t)d_cost & 3u)) {
+    set_error("rk_plan_rollout: cost->d_ref (8-byte aligned float2) and d_cost (float) must be non-NULL device pointers");
+    return RK_ERR_ARG;
+  }
+  if(int rc = require_device()) return rc;
+  rk_vdt_rollout_t a;
+  memset(&a, 0, sizeof(a));
+  a.steps = n_seg * seg_len, a.sensor_mode = RK_SENSOR_PLANT;
+  a.d_cmd = d_cmd, a.n_seg = n_seg, a.seg_len = seg_len;
+  PlanArgs pl;
+  pl.R = R, pl.S = S, pl.ref = reinterpret_cast<const float2 *>(cost->d_ref);
+  pl.w_pos = cost->w_pos, pl.w_goal = cost->w_goal, pl.w_cur = cost->w_cur, pl.cost = d_cost;
+  const int64_t n  = R * (int64_t)S;
+  cudaStream_t  st = (cudaStream_t)stream;
+  if(fast_path_usable(*p)) {
+    const CmdRcp rcp = make_cmd_rcp(*p);
+    if(g_fast_occupancy == 3) launch_plan_fast<3>(*p, d_src_state, n, a, rcp, pl, st);
+    else launch_plan_fast<4>(*p, d_src_state, n, a, rcp, pl, st);
+  } else {
+    const unsigned grid = (unsigned)((n + kRolloutThreads - 1) / kRolloutThreads);
+    vdt_rollout_kernel<RK_SENSOR_PLANT, false, true><<<grid, kRolloutThreads, 0, st>>>(*p, (uint4 *)d_src_state, n, a, pl);
+  }
+  RK_CUDA(cudaGetLastError());
   return RK_OK;
 }
 

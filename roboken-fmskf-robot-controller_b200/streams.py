@@ -515,3 +515,50 @@ def arm_sequences_v2(n, seed=0x5EED, first=0, max_len=32, min_len=2, seq_id=1, d
         wp[:, :, 1 + j] = (q.astype(np.float32) * np.float32(1.0 / 64.0)).view(np.uint32)
     wp[np.arange(32)[None, :] >= ln[:, None]] = 0
     return img
+
+
+def plan_xi_v2(h):
+    """The candidate noise of plan_commands_v2 under hash(es) h: float32 [..., 3] Irwin-Hall draws (four uniforms of lite32
+    draws 4a .. 4a+3 for axis a, summed left to right, centred and scaled to unit variance)."""
+    f32 = np.float32
+    xi = []
+    for a in range(3):
+        u = [_u01_32(lite32(h, 4 * a + k)) for k in range(4)]
+        xi.append((((u[0] + u[1]) + u[2]) + u[3] - f32(2.0)) * f32(1.7320508))
+    return np.stack(xi, axis=-1).astype(np.float32)
+
+
+def plan_commands_v2(nominal, S, seed=0x5EED, first=0, sigma=(100.0, 100.0, 1.0), params=None):
+    """Sampling-planner candidates around a nominal plan (rk_plan_sample_commands): nominal [n_seg, R] rk_vdt_cmd_t records
+    -> [n_seg, R*S], candidate j of robot r at column r*S + j.  Candidate 0 is the nominal; candidate j > 0 of segment s adds
+    sigma_a * xi_a with xi = plan_xi_v2(h32(seed, 40, first + r, s*S + j)).  Then the vehicle's limiters (params: the
+    rk_vdt_params_t, default firmware constants): |(vx, vy)| above limit_speed_mmps is scaled back onto it as
+    (v * L) / |v|, vth is clamped to +-limit_rot_radps; kind = RK_CMD_MOVE.  float32, one rounding per operation."""
+    p = params or _cabi.default_params()
+    f32 = np.float32
+    nominal = np.asarray(nominal)
+    if nominal.dtype.names is None:  # int32 / float32 [n_seg, R, 4] cells
+        cells = np.ascontiguousarray(nominal).view(np.uint32)
+        nominal = cells.view(np.dtype([("vx", "<f4"), ("vy", "<f4"), ("vth", "<f4"), ("kind", "<i4")])).reshape(cells.shape[:2])
+    n_seg, R = nominal.shape
+    inst = (np.arange(R, dtype=np.uint64) + np.uint64(first))[None, :, None]
+    idx = np.arange(n_seg, dtype=np.uint64)[:, None, None] * np.uint64(S) + np.arange(S, dtype=np.uint64)[None, None, :]
+    xi = plan_xi_v2(h32(seed, 40, inst, idx))  # [n_seg, R, S, 3]
+    v = []
+    for a, name in enumerate(("vx", "vy", "vth")):
+        nom = np.broadcast_to(nominal[name].astype(np.float32)[:, :, None], (n_seg, R, S))
+        noisy = (nom + f32(sigma[a]) * xi[..., a]).astype(np.float32)
+        noisy[:, :, 0] = nom[:, :, 0]  # j == 0: the nominal itself
+        v.append(noisy)
+    vx, vy, vth = v
+    L, rl = f32(p.limit_speed_mmps), f32(p.limit_rot_radps)
+    ln = np.sqrt(vx * vx + vy * vy, dtype=np.float32)
+    over = ln > L
+    safe = np.where(over, ln, f32(1.0))
+    vx = np.where(over, (vx * L) / safe, vx).astype(np.float32)
+    vy = np.where(over, (vy * L) / safe, vy).astype(np.float32)
+    vth = np.where(vth > rl, rl, np.where(vth < -rl, -rl, vth)).astype(np.float32)
+    cmd = np.zeros((n_seg, R * S), dtype=np.dtype([("vx", "<f4"), ("vy", "<f4"), ("vth", "<f4"), ("kind", "<i4")]))
+    cmd["vx"], cmd["vy"], cmd["vth"] = vx.reshape(n_seg, -1), vy.reshape(n_seg, -1), vth.reshape(n_seg, -1)
+    cmd["kind"] = _cabi.RK_CMD_MOVE
+    return cmd
