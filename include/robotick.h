@@ -663,6 +663,29 @@ int rk_plan_sample_commands(const rk_vdt_params_t *p, const rk_plan_sample_t *s,
 int rk_plan_rollout(const rk_vdt_params_t *p, const void *d_src_state, int64_t R, int32_t S,
                     const rk_vdt_cmd_t *d_cmd, int32_t n_seg, int32_t seg_len,
                     const rk_plan_cost_t *cost, float *d_cost, void *stream);
+
+typedef struct rk_plan_obstacles {
+  const float *d_obs;   /* float4 [m][R]: disc k of robot r at cell k*R + r = {cx, cy, radius, unused}, metres; 16-byte aligned */
+  int32_t m;            /* discs per robot, >= 0 */
+  int32_t check_period; /* P >= 1 ticks; seg_len % P == 0 */
+  float   w_obst;       /* >= 0, may be +INFINITY (a hard constraint); NaN rejected */
+  float   rsv;
+} rk_plan_obstacles_t;  /* 24 bytes */
+
+/* rk_plan_rollout with keep-out discs.  Checkpoints are the states after ticks c*P - 1, c = 1 .. K/P (K = n_seg *
+ * seg_len): every segment end is one, and so is the last tick.  O starts at 0; at each checkpoint, for k = 0 .. m-1 in
+ * order, with (x, y) the position words and {cx, cy, radius} disc k of robot r:
+ *   dx = x - cx;  dy = y - cy;  d2 = dx*dx + dy*dy;  pen = radius*radius - d2;  if (pen > 0) O = O + w_obst * pen
+ * (a NaN radius or centre contributes nothing; with w_obst = +inf one penetration makes O = +inf).
+ * d_cost[r*S + j] = J + O, J exactly the rk_plan_rollout cost, accumulated separately.  obst == NULL or m == 0 is
+ * rk_plan_rollout (the same kernel, the same bits); for J >= 0 so is w_obst == 0.  Everything else is as rk_plan_rollout:
+ * RK_SENSOR_PLANT, source states untouched, no state written, the kernel chosen by the same RK_OPT_* switches, and the
+ * cost does not depend on it.  RK_ERR_ARG besides rk_plan_rollout's checks: m < 0; m > 0 with d_obs NULL or not 16-byte
+ * aligned; P < 1 or seg_len % P != 0; w_obst < 0 or NaN.  R == 0 is a no-op. */
+int rk_plan_rollout_obstacles(const rk_vdt_params_t *p, const void *d_src_state, int64_t R, int32_t S,
+                              const rk_vdt_cmd_t *d_cmd, int32_t n_seg, int32_t seg_len,
+                              const rk_plan_cost_t *cost, const rk_plan_obstacles_t *obst,
+                              float *d_cost, void *stream);
 /* best[r] = argmin_j cost[r*S + j] (NaN counts as +inf, ties to the lowest j; all NaN: 0), best_cost[r] = that cost.
  * nominal_out[s][r] takes segment s + shift of the candidates (the last segment repeated past the end):
  *   lambda == 0: candidate best copied bit for bit;

@@ -176,6 +176,12 @@ class PlanCost(C.Structure):
     _fields_ = [("d_ref", C.c_void_p), ("w_pos", C.c_float), ("w_goal", C.c_float), ("w_cur", C.c_float), ("rsv", C.c_float)]
 
 
+class PlanObstacles(C.Structure):
+    """rk_plan_obstacles_t"""
+
+    _fields_ = [("d_obs", C.c_void_p), ("m", C.c_int32), ("check_period", C.c_int32), ("w_obst", C.c_float), ("rsv", C.c_float)]
+
+
 _lib = None
 
 
@@ -224,6 +230,8 @@ def _proto(lib):
     lib.rk_plan_sample_commands.argtypes = [C.POINTER(VdtParams), C.POINTER(PlanSample), vp, C.c_int64, C.c_int32, C.c_int32, vp, vp]
     lib.rk_plan_rollout.argtypes = [C.POINTER(VdtParams), vp, C.c_int64, C.c_int32, vp, C.c_int32, C.c_int32, C.POINTER(PlanCost), vp,
                                     vp]
+    lib.rk_plan_rollout_obstacles.argtypes = [C.POINTER(VdtParams), vp, C.c_int64, C.c_int32, vp, C.c_int32, C.c_int32, C.POINTER(PlanCost),
+                                              C.POINTER(PlanObstacles), vp, vp]
     lib.rk_plan_select.argtypes = [vp, vp, C.c_int64, C.c_int32, C.c_int32, C.c_float, C.c_int32, vp, vp, vp, vp]
     lib.rk_adt_bldc_rx.argtypes = [C.POINTER(AdtParams), vp, C.c_int64, C.c_int, vp, vp, vp, vp]
     lib.rk_adt_mg_rx.argtypes = [C.POINTER(AdtParams), vp, C.c_int64, vp, vp, vp]

@@ -5,6 +5,8 @@
 #include <stdio.h>
 #include <string.h>
 
+#include <type_traits>
+
 #include "rk_vehicle_fast2.cuh"
 
 namespace rk {
@@ -89,10 +91,34 @@ RK_DEV float plan_stage_cost(float J, const Veh &v, const PlanArgs &pl, int s, i
   const float q = fadd(fadd(fadd(fmul(c[0], c[0]), fmul(c[1], c[1])), fmul(c[2], c[2])), fmul(c[3], c[3]));
   return fadd(fadd(J, fmul(s < n_seg - 1 ? pl.w_pos : pl.w_goal, e)), fmul(pl.w_cur, q));
 }
+// rk_plan_rollout_obstacles: the keep-out discs on top of PlanArgs (the OBST instantiations; the others keep PlanArgs
+// itself, so their parameter block is unchanged)
+struct PlanObstArgs : PlanArgs {
+  const float4 *obs; // [m][R]: {cx, cy, radius, -}, metres
+  int32_t       m, P;
+  float         w_obst;
+};
+template <bool OBST>
+using PlanArgsOf = std::conditional_t<OBST, PlanObstArgs, PlanArgs>;
+// O after the checkpoint at position (x, y) (rk_plan_obstacles_t).  The S candidates of robot r read the same m cells
+// (one broadcast per warp); the discs are not staged in registers, the packed kernel has none to spare.  r fits 32 bits
+// (2^32 robots would take 1.9 TB of state), which keeps one register fewer live across the hot loop.
+RK_DEV float plan_obst_cost(float O, float x, float y, const PlanObstArgs &pl, uint32_t r) {
+  const float4 *q = pl.obs + r;
+#pragma unroll 1
+  for(int k = 0; k < pl.m; k++, q += pl.R) {
+    const float4 c   = __ldg(q);
+    const float  dx  = fsub(x, c.x), dy = fsub(y, c.y);
+    const float  pen = fsub(fmul(c.z, c.z), fadd(fmul(dx, dx), fmul(dy, dy)));
+    if(pen > 0.0f) O = fadd(O, fmul(pl.w_obst, pen));
+  }
+  return O;
+}
 
-template <int MODE, bool TRACE, bool PLAN = false>
+template <int MODE, bool TRACE, bool PLAN = false, bool OBST = false>
 __global__ void __launch_bounds__(kRolloutThreads)
-vdt_rollout_kernel(const rk_vdt_params_t p, uint4 *__restrict__ state, int64_t n, const rk_vdt_rollout_t a, const PlanArgs pl) {
+vdt_rollout_kernel(const rk_vdt_params_t p, uint4 *__restrict__ state, int64_t n, const rk_vdt_rollout_t a, const PlanArgsOf<OBST> pl) {
+  static_assert(PLAN || !OBST, "obstacles are a plan-rollout term");
   __shared__ float s_tab[513];
   stage_sin_table(s_tab);
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -123,9 +149,17 @@ vdt_rollout_kernel(const rk_vdt_params_t p, uint4 *__restrict__ state, int64_t n
     for(int k = 0; k < 4; k++) fpf[k] = __ldcs(fsrc + (int64_t)k * n);
   }
 
+  float O = 0.0f;
+  int   next_chk = 0;
+  if constexpr(OBST) next_chk = pl.P;
   for(int t = 0; t < a.steps; t++) {
     if constexpr(PLAN)
       if(t == sc.next_cmd && sc.seg > 0) J = plan_stage_cost(J, v, pl, sc.seg - 1, a.n_seg, r);
+    if constexpr(OBST)
+      if(t == next_chk) { // the state after tick t - 1
+        O = plan_obst_cost(O, v.pos[0], v.pos[1], pl, r);
+        next_chk += pl.P;
+      }
     sched_events(v, p, a, n, i, t, sc);
     if(t == next_yaw) { // can_tx_routine_intr -> set_now_yaw_world()   VD_task_main.cpp:368
       if(yaw_of_pf(a, load_yaw_pf(a, n, i, yk), yk, i, v.pos[2])) yaw_trig(s_tab, v.pos[2], cth, sth);
@@ -159,7 +193,10 @@ vdt_rollout_kernel(const rk_vdt_params_t p, uint4 *__restrict__ state, int64_t n
       tr[(int64_t)14 * n] = c610_tx_word(v.m[0].cur_tgt, v.m[1].cur_tgt), tr[(int64_t)15 * n] = c610_tx_word(v.m[2].cur_tgt, v.m[3].cur_tgt);
     }
   }
-  if constexpr(PLAN) {
+  if constexpr(OBST) { // the last checkpoint: t = K (seg_len % P == 0)
+    pl.cost[i] = fadd(plan_stage_cost(J, v, pl, a.n_seg - 1, a.n_seg, r), plan_obst_cost(O, v.pos[0], v.pos[1], pl, r));
+    return;
+  } else if constexpr(PLAN) {
     pl.cost[i] = plan_stage_cost(J, v, pl, a.n_seg - 1, a.n_seg, r);
     return;
   }
@@ -244,7 +281,10 @@ RK_DEV void yaw_feed_take(YawFeed &y, const rk_vdt_rollout_t &a, int64_t n, int6
 // FLAGS: bit 0 FFSAT (ff_limit == 1: FMUL.SAT form of the feed-forward clamp), bit 1 KD0 (kd == 0, packed tick only)
 // PLAN: rk_plan_rollout (PlanArgs); segment ends are command ticks, so they are chunk boundaries and the stage cost is
 // formed outside the chunk loop.
-template <bool TRACE, int OCC, int FLAGS, bool PACKED, bool RESET = false, bool PLAN = false>
+// OBST (with PLAN): rk_plan_rollout_obstacles (PlanObstArgs).  Plan rollouts have no yaw stream, so the yaw boundary's
+// cold branch inside the chunk loop takes the obstacle checkpoint instead (every P ticks, the same tick in every lane):
+// no new chunk boundary and no new loop-carried register besides O.
+template <bool TRACE, int OCC, int FLAGS, bool PACKED, bool RESET = false, bool PLAN = false, bool OBST = false>
 #if defined(RK_FAST_MAXNREG) // tuning builds: the register budget given directly (finer occupancy steps with small CTAs)
 __global__ void __maxnreg__(RK_FAST_MAXNREG)
 #elif defined(RK_FAST_MINBLOCKS)
@@ -253,7 +293,8 @@ __global__ void __launch_bounds__(kFastThreads, RK_FAST_MINBLOCKS)
 __global__ void __launch_bounds__(kFastThreads, OCC * 128 / kFastThreads)
 #endif
 vdt_rollout_fast_kernel(const rk_vdt_params_t p, uint4 *__restrict__ state, int64_t n, const rk_vdt_rollout_t a, const CmdRcp rcp,
-                        const PlanArgs pl) {
+                        const PlanArgsOf<OBST> pl) {
+  static_assert(PLAN || !OBST, "obstacles are a plan-rollout term");
   constexpr int  D0 = 1, D1 = 1, D2 = -1, D3 = -1; // VD_task_main.cpp:75-78 (host checks params match)
   constexpr bool FFSAT = (FLAGS & 1) != 0, KD0 = (FLAGS & 2) != 0;
   __shared__ float s_tab[513];
@@ -282,7 +323,9 @@ vdt_rollout_fast_kernel(const rk_vdt_params_t p, uint4 *__restrict__ state, int6
   Sched     sch;
   sched_init(sch, a);
   YawFeed yf;
-  yaw_feed_init(yf, a, n, i);
+  float   O = 0.0f;
+  if constexpr(OBST) yf.next = pl.P; // the next checkpoint: the state after tick yf.next - 1
+  else yaw_feed_init(yf, a, n, i);
 
   int t = 0;
   while(t < K) {
@@ -307,8 +350,13 @@ vdt_rollout_fast_kernel(const rk_vdt_params_t p, uint4 *__restrict__ state, int6
 #pragma unroll kFastUnroll
         for(; t < t_end; t++) {
           if(t == yf.next) {
-            yaw_feed_take(yf, a, n, i, s_tab, pth, cth, sth);
-            cs = make_float2(cth, sth), sc = make_float2(sth, cth);
+            if constexpr(OBST) {
+              O = plan_obst_cost(O, f.p.x, f.p.y, pl, r);
+              yf.next += pl.P;
+            } else {
+              yaw_feed_take(yf, a, n, i, s_tab, pth, cth, sth);
+              cs = make_float2(cth, sth), sc = make_float2(sth, cth);
+            }
           }
           float vel[3], tgt[3];
           fast_tick2<FFSAT, TRACE, KD0>(f, p, fc, cs, sc, nz, vel, tgt);
@@ -323,7 +371,14 @@ vdt_rollout_fast_kernel(const rk_vdt_params_t p, uint4 *__restrict__ state, int6
         to_fast<D0, D1, D2, D3>(v, f, p.ts, fc.B0);
 #pragma unroll kFastUnroll
         for(; t < t_end; t++) {
-          if(t == yf.next) yaw_feed_take(yf, a, n, i, s_tab, pth, cth, sth);
+          if(t == yf.next) {
+            if constexpr(OBST) {
+              O = plan_obst_cost(O, f.px, f.py, pl, r);
+              yf.next += pl.P;
+            } else {
+              yaw_feed_take(yf, a, n, i, s_tab, pth, cth, sth);
+            }
+          }
           float vel[3], tgt[3];
           fast_tick<D0, D1, D2, D3, FFSAT>(f, p, fc, cth, sth, vel, tgt);
           trace_row<TRACE>(a.d_trace, n, i, t, f.px, f.py, pth, vel, tgt, f.w[0].cur, f.w[1].cur, f.w[2].cur, f.w[3].cur,
@@ -334,7 +389,14 @@ vdt_rollout_fast_kernel(const rk_vdt_params_t p, uint4 *__restrict__ state, int6
         sched_skip_to(v, a, sch, t);
       }
     } else {
-      if(t == yf.next) yaw_feed_take(yf, a, n, i, s_tab, v.pos[2], cth, sth);
+      if(t == yf.next) {
+        if constexpr(OBST) {
+          O = plan_obst_cost(O, v.pos[0], v.pos[1], pl, r);
+          yf.next += pl.P;
+        } else {
+          yaw_feed_take(yf, a, n, i, s_tab, v.pos[2], cth, sth);
+        }
+      }
       const int32_t us = ((t + 1) * 1000) & 0x7FFF;
 #pragma unroll
       for(int k = 0; k < 4; k++) motor_rx(v.m[k], p.motor_dir[k], plant_frame(v.m[k]), us);
@@ -344,7 +406,10 @@ vdt_rollout_fast_kernel(const rk_vdt_params_t p, uint4 *__restrict__ state, int6
       t++;
     }
   }
-  if constexpr(PLAN) { // the end state is discarded: 448 B per candidate not written
+  if constexpr(OBST) { // the last checkpoint: t = K == yf.next (seg_len % P == 0)
+    pl.cost[i] = fadd(plan_stage_cost(J, v, pl, a.n_seg - 1, a.n_seg, r), plan_obst_cost(O, v.pos[0], v.pos[1], pl, r));
+    return;
+  } else if constexpr(PLAN) { // the end state is discarded: 448 B per candidate not written
     pl.cost[i] = plan_stage_cost(J, v, pl, a.n_seg - 1, a.n_seg, r);
     return;
   }
@@ -797,13 +862,14 @@ int rk_vdt_rollout(const rk_vdt_params_t *p, void *d_state, int64_t n, const rk_
 } // extern "C"
 namespace rk {
 // rk_plan_rollout's kernel choice: the RK_SENSOR_PLANT dispatch of rk_vdt_rollout without trace and reset
-template <int OCC>
+template <bool OBST, int OCC>
 static void launch_plan_fast(const rk_vdt_params_t &p, const void *d_src, int64_t n, const rk_vdt_rollout_t &a, const CmdRcp &rcp,
-                             const PlanArgs &pl, cudaStream_t st) {
+                             const PlanArgsOf<OBST> &pl, cudaStream_t st) {
   const unsigned grid  = (unsigned)((n + kFastThreads - 1) / kFastThreads);
   const int      flags = ((p.ff_limit == 1.0f && g_fast_ffsat) ? 1 : 0) | ((p.kd == 0.0f && g_fast_packed) ? 2 : 0);
   uint4         *src   = (uint4 *)d_src; // read only under PLAN
-#define RK_LAUNCH_PLAN(FL, PK) vdt_rollout_fast_kernel<false, OCC, FL, PK, false, true><<<grid, kFastThreads, 0, st>>>(p, src, n, a, rcp, pl)
+#define RK_LAUNCH_PLAN(FL, PK) \
+  vdt_rollout_fast_kernel<false, OCC, FL, PK, false, true, OBST><<<grid, kFastThreads, 0, st>>>(p, src, n, a, rcp, pl)
   if(!g_fast_packed) {
     if(flags & 1) RK_LAUNCH_PLAN(1, false);
     else RK_LAUNCH_PLAN(0, false);
@@ -817,32 +883,62 @@ static void launch_plan_fast(const rk_vdt_params_t &p, const void *d_src, int64_
   }
 #undef RK_LAUNCH_PLAN
 }
-} // namespace rk
-extern "C" {
-
-int rk_plan_rollout(const rk_vdt_params_t *p, const void *d_src_state, int64_t R, int32_t S, const rk_vdt_cmd_t *d_cmd, int32_t n_seg,
-                    int32_t seg_len, const rk_plan_cost_t *cost, float *d_cost, void *stream) {
+template <bool OBST>
+static void launch_plan(const rk_vdt_params_t &p, const void *d_src, int64_t n, const rk_vdt_rollout_t &a, const PlanArgsOf<OBST> &pl,
+                        cudaStream_t st) {
+  if(fast_path_usable(p)) {
+    const CmdRcp rcp = make_cmd_rcp(p);
+    if(g_fast_occupancy == 3) launch_plan_fast<OBST, 3>(p, d_src, n, a, rcp, pl, st);
+    else launch_plan_fast<OBST, 4>(p, d_src, n, a, rcp, pl, st);
+  } else {
+    const unsigned grid = (unsigned)((n + kRolloutThreads - 1) / kRolloutThreads);
+    vdt_rollout_kernel<RK_SENSOR_PLANT, false, true, OBST><<<grid, kRolloutThreads, 0, st>>>(p, (uint4 *)d_src, n, a, pl);
+  }
+}
+// rk_plan_rollout (ob == NULL) and rk_plan_rollout_obstacles: the same checks, and without discs the same kernels
+static int plan_rollout(const char *who, const rk_vdt_params_t *p, const void *d_src_state, int64_t R, int32_t S, const rk_vdt_cmd_t *d_cmd,
+                        int32_t n_seg, int32_t seg_len, const rk_plan_cost_t *cost, const rk_plan_obstacles_t *ob, float *d_cost,
+                        void *stream) {
   if(!p || !cost) {
-    set_error("rk_plan_rollout: NULL params/cost");
+    set_error("%s: NULL params/cost", who);
     return RK_ERR_ARG;
   }
   if(R < 0 || S < 1) {
-    set_error("rk_plan_rollout: need R >= 0 and S >= 1 (R = %lld, S = %d)", (long long)R, S);
+    set_error("%s: need R >= 0 and S >= 1 (R = %lld, S = %d)", who, (long long)R, S);
     return RK_ERR_ARG;
   }
   if(n_seg < 1 || seg_len < 1 || (int64_t)n_seg * seg_len > INT_MAX) {
-    set_error("rk_plan_rollout: need n_seg >= 1, seg_len >= 1 and n_seg * seg_len < 2^31 (n_seg = %d, seg_len = %d)", n_seg, seg_len);
+    set_error("%s: need n_seg >= 1, seg_len >= 1 and n_seg * seg_len < 2^31 (n_seg = %d, seg_len = %d)", who, n_seg, seg_len);
     return RK_ERR_ARG;
   }
   if((uint64_t)n_seg * (uint64_t)S >= (1ull << 32)) {
-    set_error("rk_plan_rollout: n_seg * S must be < 2^32");
+    set_error("%s: n_seg * S must be < 2^32", who);
     return RK_ERR_ARG;
+  }
+  if(ob) {
+    if(ob->m < 0) {
+      set_error("%s: need m >= 0 discs per robot (m = %d)", who, ob->m);
+      return RK_ERR_ARG;
+    }
+    if(ob->check_period < 1 || seg_len % ob->check_period != 0) {
+      set_error("%s: need check_period >= 1 dividing seg_len (check_period = %d, seg_len = %d)", who, ob->check_period, seg_len);
+      return RK_ERR_ARG;
+    }
+    if(!(ob->w_obst >= 0.0f)) {
+      set_error("%s: w_obst must be >= 0 (+inf allowed, NaN not)", who);
+      return RK_ERR_ARG;
+    }
   }
   if(R == 0) return RK_OK;
   if(int rc = check_block(d_src_state, "d_src_state")) return rc;
   if(int rc = check_block(d_cmd, "d_cmd")) return rc;
   if(!cost->d_ref || ((uintptr_t)cost->d_ref & 7u) || !d_cost || ((uintptr_t)d_cost & 3u)) {
-    set_error("rk_plan_rollout: cost->d_ref (8-byte aligned float2) and d_cost (float) must be non-NULL device pointers");
+    set_error("%s: cost->d_ref (8-byte aligned float2) and d_cost (float) must be non-NULL device pointers", who);
+    return RK_ERR_ARG;
+  }
+  const bool obst = ob && ob->m > 0;
+  if(obst && (!ob->d_obs || ((uintptr_t)ob->d_obs & 15u))) {
+    set_error("%s: obst->d_obs must be a non-NULL 16-byte aligned device pointer when m > 0", who);
     return RK_ERR_ARG;
   }
   if(int rc = require_device()) return rc;
@@ -850,21 +946,32 @@ int rk_plan_rollout(const rk_vdt_params_t *p, const void *d_src_state, int64_t R
   memset(&a, 0, sizeof(a));
   a.steps = n_seg * seg_len, a.sensor_mode = RK_SENSOR_PLANT;
   a.d_cmd = d_cmd, a.n_seg = n_seg, a.seg_len = seg_len;
-  PlanArgs pl;
+  PlanObstArgs pl;
   pl.R = R, pl.S = S, pl.ref = reinterpret_cast<const float2 *>(cost->d_ref);
   pl.w_pos = cost->w_pos, pl.w_goal = cost->w_goal, pl.w_cur = cost->w_cur, pl.cost = d_cost;
   const int64_t n  = R * (int64_t)S;
   cudaStream_t  st = (cudaStream_t)stream;
-  if(fast_path_usable(*p)) {
-    const CmdRcp rcp = make_cmd_rcp(*p);
-    if(g_fast_occupancy == 3) launch_plan_fast<3>(*p, d_src_state, n, a, rcp, pl, st);
-    else launch_plan_fast<4>(*p, d_src_state, n, a, rcp, pl, st);
+  if(obst) {
+    pl.obs = reinterpret_cast<const float4 *>(ob->d_obs), pl.m = ob->m, pl.P = ob->check_period, pl.w_obst = ob->w_obst;
+    launch_plan<true>(*p, d_src_state, n, a, pl, st);
   } else {
-    const unsigned grid = (unsigned)((n + kRolloutThreads - 1) / kRolloutThreads);
-    vdt_rollout_kernel<RK_SENSOR_PLANT, false, true><<<grid, kRolloutThreads, 0, st>>>(*p, (uint4 *)d_src_state, n, a, pl);
+    launch_plan<false>(*p, d_src_state, n, a, static_cast<const PlanArgs &>(pl), st);
   }
   RK_CUDA(cudaGetLastError());
   return RK_OK;
+}
+} // namespace rk
+extern "C" {
+
+int rk_plan_rollout(const rk_vdt_params_t *p, const void *d_src_state, int64_t R, int32_t S, const rk_vdt_cmd_t *d_cmd, int32_t n_seg,
+                    int32_t seg_len, const rk_plan_cost_t *cost, float *d_cost, void *stream) {
+  return plan_rollout("rk_plan_rollout", p, d_src_state, R, S, d_cmd, n_seg, seg_len, cost, nullptr, d_cost, stream);
+}
+
+int rk_plan_rollout_obstacles(const rk_vdt_params_t *p, const void *d_src_state, int64_t R, int32_t S, const rk_vdt_cmd_t *d_cmd,
+                              int32_t n_seg, int32_t seg_len, const rk_plan_cost_t *cost, const rk_plan_obstacles_t *obst, float *d_cost,
+                              void *stream) {
+  return plan_rollout("rk_plan_rollout_obstacles", p, d_src_state, R, S, d_cmd, n_seg, seg_len, cost, obst, d_cost, stream);
 }
 
 int rk_vdt_set_power(void *d_state, int64_t n, const uint8_t *d_on, void *stream) {

@@ -54,16 +54,31 @@ class VehiclePlanner:
                                                      self.R, self.S, self.n_seg, self.candidates.data_ptr(), self._stream()))
         return self.candidates
 
-    def rollout(self, src, ref, w_pos, w_goal, w_cur):
+    def rollout(self, src, ref, w_pos, w_goal, w_cur, obstacles=None, w_obst=0.0, check_period=None):
         """rk_plan_rollout: every candidate from its robot's state in `src` (a VehicleBatch of R robots, left untouched),
-        ranked against ref (float32 [n_seg, R, 2], metres: where each robot should be when each segment ends)."""
+        ranked against ref (float32 [n_seg, R, 2], metres: where each robot should be when each segment ends).
+
+        obstacles: keep-out discs, float32 [m, R, 4] = {cx, cy, radius, unused} in metres per robot (one world shared by
+        all robots: t.expand(m, R, 4).contiguous()).  Then rk_plan_rollout_obstacles adds w_obst * (radius^2 - d^2) for
+        every disc a candidate is inside of, every check_period ticks (default seg_len; it must divide seg_len);
+        w_obst = inf makes any penetrating candidate cost +inf."""
         assert src.n == self.R, "the source batch must hold the planner's R robots"
         assert ref.is_cuda and ref.is_contiguous() and ref.dtype == torch.float32 and tuple(ref.shape) == (self.n_seg, self.R, 2)
         c = _cabi.PlanCost()
         c.d_ref, c.w_pos, c.w_goal, c.w_cur = ref.data_ptr(), float(w_pos), float(w_goal), float(w_cur)
-        self._keep = ref
-        _cabi.check(self.lib.rk_plan_rollout(C.byref(self.params), src.state.data_ptr(), self.R, self.S, self.candidates.data_ptr(),
-                                             self.n_seg, self.seg_len, C.byref(c), self.cost.data_ptr(), self._stream()))
+        args = (C.byref(self.params), src.state.data_ptr(), self.R, self.S, self.candidates.data_ptr(), self.n_seg, self.seg_len, C.byref(c))
+        if obstacles is None:
+            self._keep = ref
+            _cabi.check(self.lib.rk_plan_rollout(*args, self.cost.data_ptr(), self._stream()))
+            return self.cost
+        assert (obstacles.is_cuda and obstacles.is_contiguous() and obstacles.dtype == torch.float32 and obstacles.dim() == 3
+                and tuple(obstacles.shape[1:]) == (self.R, 4)), "obstacles: float32 [m, R, 4] contiguous device tensor"
+        o = _cabi.PlanObstacles()
+        o.d_obs, o.m = obstacles.data_ptr(), obstacles.shape[0]
+        o.check_period = self.seg_len if check_period is None else int(check_period)
+        o.w_obst = float(w_obst)
+        self._keep = (ref, obstacles)
+        _cabi.check(self.lib.rk_plan_rollout_obstacles(*args, C.byref(o), self.cost.data_ptr(), self._stream()))
         return self.cost
 
     def select(self, lam, shift=1):
@@ -74,10 +89,10 @@ class VehiclePlanner:
                                             self._stream()))
         return self.nominal
 
-    def plan(self, src, ref, w_pos, w_goal, w_cur, lam=0.0, shift=1, seed=None):
+    def plan(self, src, ref, w_pos, w_goal, w_cur, lam=0.0, shift=1, seed=None, obstacles=None, w_obst=0.0, check_period=None):
         """One planning step (sample, rollout, select) on the current torch stream; returns the new nominal."""
         self.sample(seed=seed)
-        self.rollout(src, ref, w_pos, w_goal, w_cur)
+        self.rollout(src, ref, w_pos, w_goal, w_cur, obstacles=obstacles, w_obst=w_obst, check_period=check_period)
         return self.select(lam, shift)
 
     def first_command(self):
