@@ -57,7 +57,7 @@ __global__ void proof_small_kernel(ProofOut *out) {
   if(i < 65536) {
     const int r = i - 32768;
     if(plant_dang(r) != r * 8192 / 60000) atomicAdd(&out->dang_fail, 1u);
-    // the same step formed in float by the packed tick (RK_FAST_FDANG, rk_vehicle_fast2.cuh): trunc(RN(r * C))
+    // the same step formed in float by the packed tick (the float encoder step in fast_tick2, rk_vehicle_fast2.cuh): trunc(RN(r * C))
     if(truncf(fmul((float)r, kDangC)) != (float)(r * 8192 / 60000)) atomicAdd(&out->dang_fail, 1u);
   }
 }

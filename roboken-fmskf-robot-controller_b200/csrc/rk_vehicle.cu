@@ -115,6 +115,50 @@ RK_DEV float plan_obst_cost(float O, float x, float y, const PlanObstArgs &pl, u
   return O;
 }
 
+// The start state of thread i: under PLAN, candidate i = r * S + j starts from robot r's block (the S candidates of robot
+// r read the same cells: one broadcast per warp).  Returns r (0 without PLAN).
+template <bool PLAN>
+RK_DEV int64_t rollout_load(const uint4 *state, int64_t n, int64_t i, const PlanArgs &pl, Veh &v) {
+  if constexpr(PLAN) {
+    const int64_t r = i / pl.S;
+    load_veh(state, pl.R, r, v);
+    return r;
+  }
+  load_veh(state, n, i, v);
+  return 0;
+}
+// The end of a launch.  PLAN: the candidate's cost J (+ O after the last obstacle checkpoint, t = K: seg_len % P == 0);
+// the end state is discarded, 448 B per candidate not written.  Otherwise the end state, and its squared distance to the
+// goal if asked.
+template <bool PLAN, bool OBST>
+RK_DEV void rollout_store(uint4 *state, int64_t n, int64_t i, const rk_vdt_rollout_t &a, const PlanArgsOf<OBST> &pl, const Veh &v,
+                          float J, float O, int64_t r) {
+  if constexpr(OBST) {
+    pl.cost[i] = fadd(plan_stage_cost(J, v, pl, a.n_seg - 1, a.n_seg, r), plan_obst_cost(O, v.pos[0], v.pos[1], pl, r));
+  } else if constexpr(PLAN) {
+    pl.cost[i] = plan_stage_cost(J, v, pl, a.n_seg - 1, a.n_seg, r);
+  } else {
+    store_veh(state, n, i, v);
+    if(a.d_cost != nullptr && a.d_goal != nullptr) {
+      const float2 g  = reinterpret_cast<const float2 *>(a.d_goal)[i];
+      const float  dx = fsub(v.pos[0], g.x), dy = fsub(v.pos[1], g.y);
+      a.d_cost[i]     = fadd(fmul(dx, dx), fmul(dy, dy));
+    }
+  }
+}
+
+template <bool TRACE>
+RK_DEV void trace_row(uint32_t *d_trace, int64_t n, int64_t i, int t, float px, float py, float pth, const float vel[3],
+                      const float tgt[3], int c0, int c1, int c2, int c3, uint32_t cnt) {
+  if(!TRACE) return;
+  uint32_t *tr = d_trace + (int64_t)t * RK_VDT_TRACE_WORDS * n + i;
+  tr[0] = f2u(px), tr[n] = f2u(py), tr[2 * n] = f2u(pth);
+#pragma unroll
+  for(int j = 0; j < 3; j++) tr[(int64_t)(3 + j) * n] = f2u(vel[j]), tr[(int64_t)(6 + j) * n] = f2u(tgt[j]);
+  tr[9 * n] = (uint32_t)c0, tr[10 * n] = (uint32_t)c1, tr[11 * n] = (uint32_t)c2, tr[12 * n] = (uint32_t)c3;
+  tr[13 * n] = cnt, tr[14 * n] = c610_tx_word(c0, c1), tr[15 * n] = c610_tx_word(c2, c3);
+}
+
 template <int MODE, bool TRACE, bool PLAN = false, bool OBST = false>
 __global__ void __launch_bounds__(kRolloutThreads)
 vdt_rollout_kernel(const rk_vdt_params_t p, uint4 *__restrict__ state, int64_t n, const rk_vdt_rollout_t a, const PlanArgsOf<OBST> pl) {
@@ -124,15 +168,9 @@ vdt_rollout_kernel(const rk_vdt_params_t p, uint4 *__restrict__ state, int64_t n
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if(i >= n) return;
 
-  Veh     v;
-  int64_t r = 0;
-  float   J = 0.0f;
-  if constexpr(PLAN) {
-    r = i / pl.S;
-    load_veh(state, pl.R, r, v);
-  } else {
-    load_veh(state, n, i, v);
-  }
+  Veh           v;
+  const int64_t r = rollout_load<PLAN>(state, n, i, pl, v);
+  float         J = 0.0f;
   const Derived d = derive(p);
   float         cth, sth;
   yaw_trig(s_tab, v.pos[2], cth, sth);
@@ -179,33 +217,10 @@ vdt_rollout_kernel(const rk_vdt_params_t p, uint4 *__restrict__ state, int64_t n
       for(int k = 0; k < 4; k++) motor_rx(v.m[k], p.motor_dir[k], fr[k], us);
     }
     veh_update(v, p, d, cth, sth);
-    if(TRACE) {
-      uint32_t *tr = a.d_trace + (int64_t)t * RK_VDT_TRACE_WORDS * n + i;
-#pragma unroll
-      for(int j = 0; j < 3; j++) {
-        tr[(int64_t)j * n]       = f2u(v.pos[j]);
-        tr[(int64_t)(3 + j) * n] = f2u(v.vel[j]);
-        tr[(int64_t)(6 + j) * n] = f2u(v.tgt[j]);
-      }
-#pragma unroll
-      for(int k = 0; k < 4; k++) tr[(int64_t)(9 + k) * n] = (uint32_t)v.m[k].cur_tgt;
-      tr[(int64_t)13 * n] = (a.task_period > 0) ? v.move_cnt : 0u;
-      tr[(int64_t)14 * n] = c610_tx_word(v.m[0].cur_tgt, v.m[1].cur_tgt), tr[(int64_t)15 * n] = c610_tx_word(v.m[2].cur_tgt, v.m[3].cur_tgt);
-    }
+    trace_row<TRACE>(a.d_trace, n, i, t, v.pos[0], v.pos[1], v.pos[2], v.vel, v.tgt, v.m[0].cur_tgt, v.m[1].cur_tgt,
+                     v.m[2].cur_tgt, v.m[3].cur_tgt, (a.task_period > 0) ? v.move_cnt : 0u);
   }
-  if constexpr(OBST) { // the last checkpoint: t = K (seg_len % P == 0)
-    pl.cost[i] = fadd(plan_stage_cost(J, v, pl, a.n_seg - 1, a.n_seg, r), plan_obst_cost(O, v.pos[0], v.pos[1], pl, r));
-    return;
-  } else if constexpr(PLAN) {
-    pl.cost[i] = plan_stage_cost(J, v, pl, a.n_seg - 1, a.n_seg, r);
-    return;
-  }
-  store_veh(state, n, i, v);
-  if(a.d_cost != nullptr && a.d_goal != nullptr) {
-    const float2 g  = reinterpret_cast<const float2 *>(a.d_goal)[i];
-    const float  dx = fsub(v.pos[0], g.x), dy = fsub(v.pos[1], g.y);
-    a.d_cost[i]     = fadd(fmul(dx, dx), fmul(dy, dy));
-  }
+  rollout_store<PLAN, OBST>(state, n, i, a, pl, v, J, O, r);
 }
 
 // -----------------------------------------------------------------------------------------
@@ -215,33 +230,9 @@ vdt_rollout_kernel(const rk_vdt_params_t p, uint4 *__restrict__ state, int64_t n
 // the launch and any thread outside the fast path's domain run the transcription (veh_update), so the
 // stored state is complete and identical.
 // -----------------------------------------------------------------------------------------
-#ifndef RK_FAST_CMDRCP
-#define RK_FAST_CMDRCP 1
-#endif
-#ifndef RK_FAST_RESET_KERNEL
-#define RK_FAST_RESET_KERNEL 1
-#endif
-#ifndef RK_FAST_THREADS
-#define RK_FAST_THREADS 128
-#endif
-#ifndef RK_FAST_UNROLL
-#define RK_FAST_UNROLL 2
-#endif
-constexpr int kFastThreads = RK_FAST_THREADS;
-constexpr int kFastUnroll  = RK_FAST_UNROLL;
+constexpr int kFastThreads = 128;
+constexpr int kFastUnroll  = 2;
 constexpr int kMaxChunk    = 2048; // ticks per chunk: keeps the per-chunk angle sum exact (int32, or integers in float: |step| <= 4474)
-
-template <bool TRACE>
-RK_DEV void trace_row(uint32_t *d_trace, int64_t n, int64_t i, int t, float px, float py, float pth, const float vel[3],
-                      const float tgt[3], int c0, int c1, int c2, int c3, uint32_t cnt) {
-  if(!TRACE) return;
-  uint32_t *tr = d_trace + (int64_t)t * RK_VDT_TRACE_WORDS * n + i;
-  tr[0] = f2u(px), tr[n] = f2u(py), tr[2 * n] = f2u(pth);
-#pragma unroll
-  for(int j = 0; j < 3; j++) tr[(int64_t)(3 + j) * n] = f2u(vel[j]), tr[(int64_t)(6 + j) * n] = f2u(tgt[j]);
-  tr[9 * n] = (uint32_t)c0, tr[10 * n] = (uint32_t)c1, tr[11 * n] = (uint32_t)c2, tr[12 * n] = (uint32_t)c3;
-  tr[13 * n] = cnt, tr[14 * n] = c610_tx_word(c0, c1), tr[15 * n] = c610_tx_word(c2, c3);
-}
 
 RK_DEV void fast_consts(FastConsts &fc, const rk_vdt_params_t &p, const Derived &d) {
   fc.rcp_r = fdiv(1.0f, p.wheel_radius_mm), fc.rcp_s2 = fdiv(1.0f, p.sqrtf2), fc.rcp_l = fdiv(1.0f, p.wheel_l_mm);
@@ -278,6 +269,20 @@ RK_DEV void yaw_feed_take(YawFeed &y, const rk_vdt_rollout_t &a, int64_t n, int6
   }
 }
 
+// The cold branch of vdt_rollout_fast_kernel at t == yf.next.  OBST: the obstacle checkpoint at (x, y), the state after
+// tick t - 1; returns O with it added.  Otherwise the yaw boundary into (pth, cth, sth); returns O as it was.  (O by
+// value: taken by reference, it changes ptxas' register assignment in the OBST kernels.)
+template <bool OBST>
+RK_DEV float yaw_boundary(YawFeed &yf, float O, float x, float y, const PlanArgsOf<OBST> &pl, int64_t r, const rk_vdt_rollout_t &a,
+                          int64_t n, int64_t i, const float *s_tab, float &pth, float &cth, float &sth) {
+  if constexpr(OBST) {
+    O = plan_obst_cost(O, x, y, pl, r);
+    yf.next += pl.P;
+  } else {
+    yaw_feed_take(yf, a, n, i, s_tab, pth, cth, sth);
+  }
+  return O;
+}
 // FLAGS: bit 0 FFSAT (ff_limit == 1: FMUL.SAT form of the feed-forward clamp), bit 1 KD0 (kd == 0, packed tick only)
 // PLAN: rk_plan_rollout (PlanArgs); segment ends are command ticks, so they are chunk boundaries and the stage cost is
 // formed outside the chunk loop.
@@ -285,13 +290,7 @@ RK_DEV void yaw_feed_take(YawFeed &y, const rk_vdt_rollout_t &a, int64_t n, int6
 // cold branch inside the chunk loop takes the obstacle checkpoint instead (every P ticks, the same tick in every lane):
 // no new chunk boundary and no new loop-carried register besides O.
 template <bool TRACE, int OCC, int FLAGS, bool PACKED, bool RESET = false, bool PLAN = false, bool OBST = false>
-#if defined(RK_FAST_MAXNREG) // tuning builds: the register budget given directly (finer occupancy steps with small CTAs)
-__global__ void __maxnreg__(RK_FAST_MAXNREG)
-#elif defined(RK_FAST_MINBLOCKS)
-__global__ void __launch_bounds__(kFastThreads, RK_FAST_MINBLOCKS)
-#else
 __global__ void __launch_bounds__(kFastThreads, OCC * 128 / kFastThreads)
-#endif
 vdt_rollout_fast_kernel(const rk_vdt_params_t p, uint4 *__restrict__ state, int64_t n, const rk_vdt_rollout_t a, const CmdRcp rcp,
                         const PlanArgsOf<OBST> pl) {
   static_assert(PLAN || !OBST, "obstacles are a plan-rollout term");
@@ -305,14 +304,8 @@ vdt_rollout_fast_kernel(const rk_vdt_params_t p, uint4 *__restrict__ state, int6
   Veh     v;
   int64_t r = 0;
   float   J = 0.0f;
-  if constexpr(PLAN) { // the S candidates of robot r read the same cells (one broadcast per warp)
-    r = i / pl.S;
-    load_veh(state, pl.R, r, v);
-  } else if(RESET) {
-    v = Veh{}; // reset_state: the power-on block is all zeros -- nothing to load (and no memset in front of the kernel)
-  } else {
-    load_veh(state, n, i, v);
-  }
+  if(RESET) v = Veh{}; // reset_state: the power-on block is all zeros -- nothing to load (and no memset in front of the kernel)
+  else r = rollout_load<PLAN>(state, n, i, pl, v);
   const Derived d = derive(p);
   FastConsts    fc;
   fast_consts(fc, p, d);
@@ -331,13 +324,13 @@ vdt_rollout_fast_kernel(const rk_vdt_params_t p, uint4 *__restrict__ state, int6
   while(t < K) {
     if constexpr(PLAN)
       if(t == sch.next_cmd && sch.seg > 0) J = plan_stage_cost(J, v, pl, sch.seg - 1, a.n_seg, r);
-    sched_events(v, p, a, n, i, t, sch, RK_FAST_CMDRCP ? &rcp : nullptr); // commands, VDT::main messages and the move-time countdown due at this tick
+    sched_events(v, p, a, n, i, t, sch, &rcp); // commands, VDT::main messages and the move-time countdown due at this tick
     // run to the next event: a command, the countdown's automatic stop, or the last tick of the launch
     // (always a transcription tick).  Lanes of a warp whose countdowns fire at different ticks leave
     // the fast loop at different times; results do not depend on it.
     const int t_end = min(min(min(sch.next_cmd, sched_fire_tick(v, a, sch)), K - 1), t + kMaxChunk);
     if(t < t_end && fast_ok<D0, D1, D2, D3>(v, p) && fast_u_bounded<false>(v, p, fc) &&
-       !(PACKED && RK_FAST_FDANG && (f2u(v.pos[0]) == 0x80000000u || f2u(v.pos[1]) == 0x80000000u))) {
+       !(PACKED && (f2u(v.pos[0]) == 0x80000000u || f2u(v.pos[1]) == 0x80000000u))) {
       const int t0  = t;
       float     pth = v.pos[2];
       if(PACKED) { // FADD2 / FFMA2 form of the same tick (rk_vehicle_fast2.cuh)
@@ -350,13 +343,8 @@ vdt_rollout_fast_kernel(const rk_vdt_params_t p, uint4 *__restrict__ state, int6
 #pragma unroll kFastUnroll
         for(; t < t_end; t++) {
           if(t == yf.next) {
-            if constexpr(OBST) {
-              O = plan_obst_cost(O, f.p.x, f.p.y, pl, r);
-              yf.next += pl.P;
-            } else {
-              yaw_feed_take(yf, a, n, i, s_tab, pth, cth, sth);
-              cs = make_float2(cth, sth), sc = make_float2(sth, cth);
-            }
+            O = yaw_boundary<OBST>(yf, O, f.p.x, f.p.y, pl, r, a, n, i, s_tab, pth, cth, sth);
+            if constexpr(!OBST) cs = make_float2(cth, sth), sc = make_float2(sth, cth);
           }
           float vel[3], tgt[3];
           fast_tick2<FFSAT, TRACE, KD0>(f, p, fc, cs, sc, nz, vel, tgt);
@@ -371,14 +359,7 @@ vdt_rollout_fast_kernel(const rk_vdt_params_t p, uint4 *__restrict__ state, int6
         to_fast<D0, D1, D2, D3>(v, f, p.ts, fc.B0);
 #pragma unroll kFastUnroll
         for(; t < t_end; t++) {
-          if(t == yf.next) {
-            if constexpr(OBST) {
-              O = plan_obst_cost(O, f.px, f.py, pl, r);
-              yf.next += pl.P;
-            } else {
-              yaw_feed_take(yf, a, n, i, s_tab, pth, cth, sth);
-            }
-          }
+          if(t == yf.next) O = yaw_boundary<OBST>(yf, O, f.px, f.py, pl, r, a, n, i, s_tab, pth, cth, sth);
           float vel[3], tgt[3];
           fast_tick<D0, D1, D2, D3, FFSAT>(f, p, fc, cth, sth, vel, tgt);
           trace_row<TRACE>(a.d_trace, n, i, t, f.px, f.py, pth, vel, tgt, f.w[0].cur, f.w[1].cur, f.w[2].cur, f.w[3].cur,
@@ -389,14 +370,7 @@ vdt_rollout_fast_kernel(const rk_vdt_params_t p, uint4 *__restrict__ state, int6
         sched_skip_to(v, a, sch, t);
       }
     } else {
-      if(t == yf.next) {
-        if constexpr(OBST) {
-          O = plan_obst_cost(O, v.pos[0], v.pos[1], pl, r);
-          yf.next += pl.P;
-        } else {
-          yaw_feed_take(yf, a, n, i, s_tab, v.pos[2], cth, sth);
-        }
-      }
+      if(t == yf.next) O = yaw_boundary<OBST>(yf, O, v.pos[0], v.pos[1], pl, r, a, n, i, s_tab, v.pos[2], cth, sth);
       const int32_t us = ((t + 1) * 1000) & 0x7FFF;
 #pragma unroll
       for(int k = 0; k < 4; k++) motor_rx(v.m[k], p.motor_dir[k], plant_frame(v.m[k]), us);
@@ -406,19 +380,7 @@ vdt_rollout_fast_kernel(const rk_vdt_params_t p, uint4 *__restrict__ state, int6
       t++;
     }
   }
-  if constexpr(OBST) { // the last checkpoint: t = K == yf.next (seg_len % P == 0)
-    pl.cost[i] = fadd(plan_stage_cost(J, v, pl, a.n_seg - 1, a.n_seg, r), plan_obst_cost(O, v.pos[0], v.pos[1], pl, r));
-    return;
-  } else if constexpr(PLAN) { // the end state is discarded: 448 B per candidate not written
-    pl.cost[i] = plan_stage_cost(J, v, pl, a.n_seg - 1, a.n_seg, r);
-    return;
-  }
-  store_veh(state, n, i, v);
-  if(a.d_cost != nullptr && a.d_goal != nullptr) {
-    const float2 g  = reinterpret_cast<const float2 *>(a.d_goal)[i];
-    const float  dx = fsub(v.pos[0], g.x), dy = fsub(v.pos[1], g.y);
-    a.d_cost[i]     = fadd(fmul(dx, dx), fmul(dy, dy));
-  }
+  rollout_store<PLAN, OBST>(state, n, i, a, pl, v, J, O, r);
 }
 
 // -----------------------------------------------------------------------------------------
@@ -427,17 +389,11 @@ vdt_rollout_fast_kernel(const rk_vdt_params_t p, uint4 *__restrict__ state, int6
 // while tick t is computed.  Command ticks, the last tick and threads outside the fast domain run the
 // transcription on the same frames.
 // -----------------------------------------------------------------------------------------
-#ifndef RK_STREAM_OCC
-#define RK_STREAM_OCC 4
-#endif
-#ifndef RK_STREAM_RING
-#define RK_STREAM_RING 4
-#endif
 // The recorded frames reach each thread through its own ring in shared memory, filled kStreamRing ticks ahead by
 // cp.async (LDGSTS): the HBM latency of a tick's four frames hides behind kStreamRing ticks of arithmetic and costs no
 // registers.  Every thread copies and reads only its own slots ([stage][wheel][thread], conflict-free LDS.64), so
 // threads of a warp that sit in different chunk paths need no barrier between them.
-constexpr int kStreamRing = RK_STREAM_RING;
+constexpr int kStreamRing = 4;
 struct FrameRing {
   uint32_t                  base; // shared-memory address of this thread's slot (stage 0, wheel 0)
   const unsigned long long *src;  // the thread's column of d_frames
@@ -465,7 +421,7 @@ RK_DEV void frame_ring_take(const FrameRing &r, int t, uint64_t fr[4]) { // grou
   }
 }
 template <bool TRACE, int FLAGS>
-__global__ void __launch_bounds__(kFastThreads, RK_STREAM_OCC)
+__global__ void __launch_bounds__(kFastThreads, 4)
 vdt_rollout_stream_fast_kernel(const rk_vdt_params_t p, uint4 *__restrict__ state, int64_t n, const rk_vdt_rollout_t a, const CmdRcp rcp) {
   constexpr int  D0 = 1, D1 = 1, D2 = -1, D3 = -1;
   constexpr bool FFSAT = (FLAGS & 1) != 0, KD0 = (FLAGS & 2) != 0;
@@ -496,7 +452,7 @@ vdt_rollout_stream_fast_kernel(const rk_vdt_params_t p, uint4 *__restrict__ stat
 
   int t = 0;
   while(t < K) {
-    sched_events(v, p, a, n, i, t, sch, RK_FAST_CMDRCP ? &rcp : nullptr);
+    sched_events(v, p, a, n, i, t, sch, &rcp);
     // chunks are capped so the 32-bit per-chunk angle sum cannot overflow (|step| <= 40960)
     const int t_end = min(min(min(sch.next_cmd, sched_fire_tick(v, a, sch)), K - 1), t + 32768);
     if(t < t_end && fast_ok<D0, D1, D2, D3, true>(v, p) && fast_u_bounded<true>(v, p, fc)) {
@@ -541,12 +497,7 @@ vdt_rollout_stream_fast_kernel(const rk_vdt_params_t p, uint4 *__restrict__ stat
       t++;
     }
   }
-  store_veh(state, n, i, v);
-  if(a.d_cost != nullptr && a.d_goal != nullptr) {
-    const float2 g  = reinterpret_cast<const float2 *>(a.d_goal)[i];
-    const float  dx = fsub(v.pos[0], g.x), dy = fsub(v.pos[1], g.y);
-    a.d_cost[i]     = fadd(fmul(dx, dx), fmul(dy, dy));
-  }
+  rollout_store<false, false>(state, n, i, a, PlanArgs{}, v, 0.0f, 0.0f, 0);
 }
 
 // ---- small batched setters ------------------------------------------------------------
@@ -638,17 +589,6 @@ static int check_block(const void *p, const char *name) {
   return RK_OK;
 }
 
-template <int MODE>
-static cudaError_t launch_rollout(const rk_vdt_params_t &p, void *d_state, int64_t n, const rk_vdt_rollout_t &a,
-                                  cudaStream_t st) {
-  const unsigned grid = (unsigned)((n + kRolloutThreads - 1) / kRolloutThreads);
-  if(a.d_trace)
-    vdt_rollout_kernel<MODE, true><<<grid, kRolloutThreads, 0, st>>>(p, (uint4 *)d_state, n, a, PlanArgs{});
-  else
-    vdt_rollout_kernel<MODE, false><<<grid, kRolloutThreads, 0, st>>>(p, (uint4 *)d_state, n, a, PlanArgs{});
-  return cudaGetLastError();
-}
-
 bool fast_path_proven(const rk_vdt_params_t &p); // rk_exact.cu
 static CmdRcp make_cmd_rcp(const rk_vdt_params_t &p) { // the host's IEEE divisions (interp_set_rcp)
   CmdRcp r;
@@ -659,7 +599,7 @@ static CmdRcp make_cmd_rcp(const rk_vdt_params_t &p) { // the host's IEEE divisi
 int  tick_set_side_ctas(int v);                     // rk_tick.cu
 int  stream_set_ctas(int v);                        // rk_stream.cu
 
-static int g_fast_occupancy = 4;       // rk_set_option(RK_OPT_FAST_OCCUPANCY, 3|4|5): tuning
+static int g_fast_occupancy = 4;       // rk_set_option(RK_OPT_FAST_OCCUPANCY, 3|4): tuning
 static int g_fast_packed = 1;          // rk_set_option(RK_OPT_FAST_PACKED, 0|1): packed FP32 tick (default) or scalar
 static int g_fast_ffsat = 0;           // rk_set_option(RK_OPT_FAST_FFSAT, 0|1): FMUL.SAT form of the feed-forward clamp.  Off since
                                        // round 2: the packed tick is bound by FP32 lanes, the FMNMX form runs on the ALU pipe (8.83 vs 8.94 ms)
@@ -679,6 +619,47 @@ static bool fast_path_usable(const rk_vdt_params_t &p) {
   for(int k = 0; k < 3; k++)
     if(!(pos(p.accel_move[k]) && pos(p.jerk_move[k]) && pos(p.accel_stop[k]) && pos(p.jerk_stop[k]))) return false;
   return fast_path_proven(p);
+}
+
+// The compile-time configuration of one fast-kernel launch, from the params and the RK_OPT_FAST_* options
+struct FastCfg {
+  bool trace;  // TRACE (compiled at occupancy 4 only)
+  int  occ;    // OCC: resident CTAs per SM the kernel is compiled for (register budget), 3 or 4
+  int  flags;  // FLAGS: bit 0 FFSAT, bit 1 KD0
+  bool packed; // PACKED
+};
+static FastCfg fast_cfg(const rk_vdt_params_t &p, bool trace, bool stream) {
+  FastCfg c;
+  c.trace = trace;
+  c.occ   = (trace || g_fast_occupancy != 3) ? 4 : 3;
+  // KD0 specialises the packed tick only.  The stream kernel has no scalar form, so it is packed (and takes KD0)
+  // whatever RK_OPT_FAST_PACKED says.
+  c.packed = stream || g_fast_packed;
+  c.flags  = ((p.ff_limit == 1.0f && g_fast_ffsat) ? 1 : 0) | ((p.kd == 0.0f && c.packed) ? 2 : 0);
+  return c;
+}
+// Calls f(TRACE, OCC, FLAGS, PACKED) with c's values as std::integral_constants.  Only these combinations are compiled:
+// TRACE at occupancy 4, and the scalar tick without KD0.
+template <int V>
+using Int = std::integral_constant<int, V>;
+template <class F>
+static void with_fast_cfg(const FastCfg &c, F &&f) {
+  const auto flags = [&](auto tr, auto occ) {
+    if(!c.packed) {
+      if(c.flags & 1) f(tr, occ, Int<1>{}, std::false_type{});
+      else f(tr, occ, Int<0>{}, std::false_type{});
+      return;
+    }
+    switch(c.flags) {
+    case 3: f(tr, occ, Int<3>{}, std::true_type{}); break;
+    case 2: f(tr, occ, Int<2>{}, std::true_type{}); break;
+    case 1: f(tr, occ, Int<1>{}, std::true_type{}); break;
+    default: f(tr, occ, Int<0>{}, std::true_type{}); break;
+    }
+  };
+  if(c.trace) flags(std::true_type{}, Int<4>{});
+  else if(c.occ == 3) flags(std::false_type{}, Int<3>{});
+  else flags(std::false_type{}, Int<4>{});
 }
 
 } // namespace rk
@@ -782,117 +763,62 @@ int rk_vdt_rollout(const rk_vdt_params_t *p, void *d_state, int64_t n, const rk_
     return RK_ERR_ARG;
   }
   if(int rc = require_device()) return rc;
-  cudaStream_t st = (cudaStream_t)stream;
-  cudaError_t  e;
+  cudaStream_t  st    = (cudaStream_t)stream;
+  uint4        *state = (uint4 *)d_state;
+  const int     mode  = args->sensor_mode;
+  const bool    fast  = (mode == RK_SENSOR_PLANT || mode == RK_SENSOR_STREAM) && fast_path_usable(*p);
+  const FastCfg c     = fast_cfg(*p, args->d_trace != nullptr, mode == RK_SENSOR_STREAM);
   // reset_state: the power-on block is all zeros (static initialisation).  Done as a memset in front of the kernel: a
   // second load path inside the rollout kernels cost the hot loop 2 % through ptxas' register allocation (8.83 -> 8.99 ms).
   // ... except in the default configuration of the packed fast kernel, which has an instantiation that starts from
-  // zeros in registers (RK_FAST_RESET_KERNEL): no memset, no state load.
-  const bool reset_in_kernel = RK_FAST_RESET_KERNEL && args->reset_state && args->sensor_mode == RK_SENSOR_PLANT && !args->d_trace &&
-                               fast_path_usable(*p) && g_fast_packed && g_fast_occupancy != 3 && p->kd == 0.0f &&
-                               !(p->ff_limit == 1.0f && g_fast_ffsat);
+  // zeros in registers: no memset, no state load.
+  const bool reset_in_kernel = args->reset_state && mode == RK_SENSOR_PLANT && fast && !c.trace && c.occ == 4 && c.flags == 2 && c.packed;
   if(args->reset_state && !reset_in_kernel) RK_CUDA(cudaMemsetAsync(d_state, 0, (size_t)n * RK_VS_WORDS * 4u, st));
-  switch(args->sensor_mode) {
-  case RK_SENSOR_HOLD: e = launch_rollout<RK_SENSOR_HOLD>(*p, d_state, n, *args, st); break;
+  const unsigned grid  = (unsigned)((n + kFastThreads - 1) / kFastThreads);
+  const unsigned tgrid = (unsigned)((n + kRolloutThreads - 1) / kRolloutThreads);
+  const auto     transcription = [&](auto m) {
+    if(c.trace) vdt_rollout_kernel<m, true><<<tgrid, kRolloutThreads, 0, st>>>(*p, state, n, *args, PlanArgs{});
+    else vdt_rollout_kernel<m, false><<<tgrid, kRolloutThreads, 0, st>>>(*p, state, n, *args, PlanArgs{});
+  };
+  switch(mode) {
+  case RK_SENSOR_HOLD: transcription(Int<RK_SENSOR_HOLD>{}); break;
   case RK_SENSOR_PLANT:
-    if(fast_path_usable(*p)) {
-      const unsigned grid  = (unsigned)((n + kFastThreads - 1) / kFastThreads);
-      const int      flags = ((p->ff_limit == 1.0f && g_fast_ffsat) ? 1 : 0) | ((p->kd == 0.0f && g_fast_packed) ? 2 : 0);
-      const CmdRcp rcp = make_cmd_rcp(*p);
-#define RK_LAUNCH_FAST3(TR, OCC, FL, PK) vdt_rollout_fast_kernel<TR, OCC, FL, PK><<<grid, kFastThreads, 0, st>>>(*p, (uint4 *)d_state, n, *args, rcp, PlanArgs{})
-#define RK_LAUNCH_FAST(TR, OCC)                                    \
-  do {                                                             \
-    if(!g_fast_packed) {                                           \
-      if(flags & 1) RK_LAUNCH_FAST3(TR, OCC, 1, false);            \
-      else RK_LAUNCH_FAST3(TR, OCC, 0, false);                     \
-    } else {                                                       \
-      switch(flags) {                                              \
-      case 3: RK_LAUNCH_FAST3(TR, OCC, 3, true); break;            \
-      case 2: RK_LAUNCH_FAST3(TR, OCC, 2, true); break;            \
-      case 1: RK_LAUNCH_FAST3(TR, OCC, 1, true); break;            \
-      default: RK_LAUNCH_FAST3(TR, OCC, 0, true); break;           \
-      }                                                            \
-    }                                                              \
-  } while(0)
-      if(reset_in_kernel) {
-        vdt_rollout_fast_kernel<false, 4, 2, true, true><<<grid, kFastThreads, 0, st>>>(*p, (uint4 *)d_state, n, *args, rcp, PlanArgs{});
-      } else if(args->d_trace) {
-        RK_LAUNCH_FAST(true, 4);
-      } else {
-        switch(g_fast_occupancy) { // resident CTAs per SM the kernel is compiled for (register budget)
-        case 3: RK_LAUNCH_FAST(false, 3); break;
-        default: RK_LAUNCH_FAST(false, 4); break;
-        }
-      }
-#undef RK_LAUNCH_FAST
-#undef RK_LAUNCH_FAST3
-      e = cudaGetLastError();
-    } else {
-      e = launch_rollout<RK_SENSOR_PLANT>(*p, d_state, n, *args, st);
-    }
+    if(!fast) transcription(Int<RK_SENSOR_PLANT>{});
+    else if(reset_in_kernel)
+      vdt_rollout_fast_kernel<false, 4, 2, true, true><<<grid, kFastThreads, 0, st>>>(*p, state, n, *args, make_cmd_rcp(*p), PlanArgs{});
+    else
+      with_fast_cfg(c, [&](auto tr, auto occ, auto fl, auto pk) {
+        vdt_rollout_fast_kernel<tr, occ, fl, pk><<<grid, kFastThreads, 0, st>>>(*p, state, n, *args, make_cmd_rcp(*p), PlanArgs{});
+      });
     break;
   case RK_SENSOR_STREAM:
-    if(fast_path_usable(*p)) {
-      const unsigned grid  = (unsigned)((n + kFastThreads - 1) / kFastThreads);
-      const int      flags = ((p->ff_limit == 1.0f && g_fast_ffsat) ? 1 : 0) | ((p->kd == 0.0f) ? 2 : 0);
-      const CmdRcp   rcp   = make_cmd_rcp(*p);
-#define RK_LAUNCH_STREAM(TR)                                                                                                  \
-  do {                                                                                                                        \
-    switch(flags) {                                                                                                           \
-    case 3: vdt_rollout_stream_fast_kernel<TR, 3><<<grid, kFastThreads, 0, st>>>(*p, (uint4 *)d_state, n, *args, rcp); break;      \
-    case 2: vdt_rollout_stream_fast_kernel<TR, 2><<<grid, kFastThreads, 0, st>>>(*p, (uint4 *)d_state, n, *args, rcp); break;      \
-    case 1: vdt_rollout_stream_fast_kernel<TR, 1><<<grid, kFastThreads, 0, st>>>(*p, (uint4 *)d_state, n, *args, rcp); break;      \
-    default: vdt_rollout_stream_fast_kernel<TR, 0><<<grid, kFastThreads, 0, st>>>(*p, (uint4 *)d_state, n, *args, rcp); break;     \
-    }                                                                                                                         \
-  } while(0)
-      if(args->d_trace) RK_LAUNCH_STREAM(true);
-      else RK_LAUNCH_STREAM(false);
-#undef RK_LAUNCH_STREAM
-      e = cudaGetLastError();
-    } else {
-      e = launch_rollout<RK_SENSOR_STREAM>(*p, d_state, n, *args, st);
-    }
+    if(!fast) transcription(Int<RK_SENSOR_STREAM>{});
+    else
+      with_fast_cfg(c, [&](auto tr, auto, auto fl, auto) {
+        vdt_rollout_stream_fast_kernel<tr, fl><<<grid, kFastThreads, 0, st>>>(*p, state, n, *args, make_cmd_rcp(*p));
+      });
     break;
-  default: set_error("rk_vdt_rollout: bad sensor_mode %d", args->sensor_mode); return RK_ERR_ARG;
+  default: set_error("rk_vdt_rollout: bad sensor_mode %d", mode); return RK_ERR_ARG;
   }
-  if(e != cudaSuccess) return cuda_fail(e, "vdt_rollout_kernel launch");
+  if(cudaError_t e = cudaGetLastError(); e != cudaSuccess) return cuda_fail(e, "vdt_rollout_kernel launch");
   return RK_OK;
 }
 
 } // extern "C"
 namespace rk {
 // rk_plan_rollout's kernel choice: the RK_SENSOR_PLANT dispatch of rk_vdt_rollout without trace and reset
-template <bool OBST, int OCC>
-static void launch_plan_fast(const rk_vdt_params_t &p, const void *d_src, int64_t n, const rk_vdt_rollout_t &a, const CmdRcp &rcp,
-                             const PlanArgsOf<OBST> &pl, cudaStream_t st) {
-  const unsigned grid  = (unsigned)((n + kFastThreads - 1) / kFastThreads);
-  const int      flags = ((p.ff_limit == 1.0f && g_fast_ffsat) ? 1 : 0) | ((p.kd == 0.0f && g_fast_packed) ? 2 : 0);
-  uint4         *src   = (uint4 *)d_src; // read only under PLAN
-#define RK_LAUNCH_PLAN(FL, PK) \
-  vdt_rollout_fast_kernel<false, OCC, FL, PK, false, true, OBST><<<grid, kFastThreads, 0, st>>>(p, src, n, a, rcp, pl)
-  if(!g_fast_packed) {
-    if(flags & 1) RK_LAUNCH_PLAN(1, false);
-    else RK_LAUNCH_PLAN(0, false);
-  } else {
-    switch(flags) {
-    case 3: RK_LAUNCH_PLAN(3, true); break;
-    case 2: RK_LAUNCH_PLAN(2, true); break;
-    case 1: RK_LAUNCH_PLAN(1, true); break;
-    default: RK_LAUNCH_PLAN(0, true); break;
-    }
-  }
-#undef RK_LAUNCH_PLAN
-}
 template <bool OBST>
 static void launch_plan(const rk_vdt_params_t &p, const void *d_src, int64_t n, const rk_vdt_rollout_t &a, const PlanArgsOf<OBST> &pl,
                         cudaStream_t st) {
+  uint4 *src = (uint4 *)d_src; // read only under PLAN
   if(fast_path_usable(p)) {
-    const CmdRcp rcp = make_cmd_rcp(p);
-    if(g_fast_occupancy == 3) launch_plan_fast<OBST, 3>(p, d_src, n, a, rcp, pl, st);
-    else launch_plan_fast<OBST, 4>(p, d_src, n, a, rcp, pl, st);
+    const unsigned grid = (unsigned)((n + kFastThreads - 1) / kFastThreads);
+    with_fast_cfg(fast_cfg(p, false, false), [&](auto, auto occ, auto fl, auto pk) {
+      vdt_rollout_fast_kernel<false, occ, fl, pk, false, true, OBST><<<grid, kFastThreads, 0, st>>>(p, src, n, a, make_cmd_rcp(p), pl);
+    });
   } else {
     const unsigned grid = (unsigned)((n + kRolloutThreads - 1) / kRolloutThreads);
-    vdt_rollout_kernel<RK_SENSOR_PLANT, false, true, OBST><<<grid, kRolloutThreads, 0, st>>>(p, (uint4 *)d_src, n, a, pl);
+    vdt_rollout_kernel<RK_SENSOR_PLANT, false, true, OBST><<<grid, kRolloutThreads, 0, st>>>(p, src, n, a, pl);
   }
 }
 // rk_plan_rollout (ob == NULL) and rk_plan_rollout_obstacles: the same checks, and without discs the same kernels

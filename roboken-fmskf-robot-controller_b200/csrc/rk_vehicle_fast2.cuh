@@ -66,7 +66,7 @@ struct FastInterp1 { // the theta interpolator, same scheme
 };
 struct FastWheel2 { // two wheels of equal direction, lane-paired
   int32_t rpm[2], cur[2], dsum[2];
-  float2  dsf; // RK_FAST_FDANG: the chunk's angle sums kept as exact integers in float (|sum| < 2^24, see kMaxChunk);
+  float2  dsf; // fast_tick2: the chunk's angle sums kept as exact integers in float (|sum| < 2^24, see kMaxChunk);
                // w01.dsf = {wheel 0, wheel 2}, w23.dsf = {wheel 1, wheel 3} -- the pairing the odometry consumes the steps in
   float2  prev_val, integ, lpf_y, b0x;
   float2  x_l; // the IIR input of the last executed tick (prev_X_)
@@ -173,7 +173,7 @@ RK_DEV void from_fast2_common(Veh &v, const FastVeh2 &f, FastWheel w[4]) {
   fast_interp2_store(f.xy, v.it[0], v.it[1]);
   fast_interp1_store(f.th, v.it[2]);
   w[0] = lane_wheel(f.w01, 0), w[1] = lane_wheel(f.w01, 1), w[2] = lane_wheel(f.w23, 0), w[3] = lane_wheel(f.w23, 1);
-  // the float angle sums (RK_FAST_FDANG; zero otherwise) in their odometry pairing
+  // the float angle sums of fast_tick2 (zero on the stream tick, which sums in dsum) in their odometry pairing
   w[0].dsum += (int32_t)f.w01.dsf.x, w[2].dsum += (int32_t)f.w01.dsf.y, w[1].dsum += (int32_t)f.w23.dsf.x, w[3].dsum += (int32_t)f.w23.dsf.y;
 #pragma unroll
   for(int k = 0; k < 4; k++) v.c[k].prev_val = w[k].prev_val, v.c[k].integ = w[k].integ, v.c[k].lpf_y = w[k].lpf_y, v.c[k].lpf_x = w[k].lpf_x;
@@ -195,16 +195,6 @@ struct Sense {
   float  d0, d2;     // (float)(s64_rawAngleSum - s64_rawAngleSumPrev) of wheels 0, 2   VD_vehicle_controller.cpp:37-41
   float2 d13;        // ... and of wheels 1, 3, paired as the odometry consumes them
 };
-
-// plant step + collapsed rx_callback for one wheel (see fast_wheel_sense)
-template <int DIR>
-RK_DEV void fast_wheel_sense2(int32_t &rpm, int32_t cur, int32_t &dsum, float &rwf, float &df) {
-  rpm += ((cur * 4 - rpm) >> 4);
-  const int32_t rw   = (DIR == 1) ? rpm : -rpm;
-  const int32_t dang = plant_dang(rw);
-  dsum += dang;
-  rwf = (float)rw, df = (float)dang;
-}
 
 // ---- RK_SENSOR_STREAM on the fast tick: the wheel feedback comes from recorded C610 frames, so rx_callback
 // (VD_motor_if_m2006.cpp:32-72) runs in full -- big-endian fields, direction, the +-4096 unwrap -- instead of the
@@ -337,16 +327,13 @@ RK_DEV void fast_tick2_core(FastVeh2 &f, const rk_vdt_params_t &p, const FastCon
   fast_wheel_ctrl2<-1, FFSAT, KD0>(f.w23, p, fc, t23, now23, nz);
 }
 
-// RK_FAST_FDANG: the plant's encoder step rpm * 8192 / 60000 (truncating) formed in FLOAT from the float wheel speed the
+// The plant's encoder step rpm * 8192 / 60000 (truncating) formed in FLOAT from the float wheel speed the
 // tick needs anyway: trunc(RN(rw * C)) with C = RN(8192 / 60000) equals the integer division for every int16 rw (all
 // 65536 checked by tests/test_cabi_cpu.py::test_float_encoder_step_is_exact and on the device by rk_exact.cu's
 // proof_small_kernel); FRND runs on the otherwise idle conversion unit, the products and the angle sums pair up as
 // packed ops, and six half-rate ALU cycles per wheel (sign fix, I2FP, integer accumulate) disappear.  A negative speed
 // below one count gives -0.0 where the integer path gives +0.0; the step only enters the position sums, where the sign of
-// a zero term is immaterial unless the position word itself is -0.0 -- fast_ok2() keeps such a (never produced) state out.
-#ifndef RK_FAST_FDANG
-#define RK_FAST_FDANG 1
-#endif
+// a zero term is immaterial unless the position word itself is -0.0 -- the fast kernel's chunk test keeps such a (never produced) state out.
 constexpr float kDangC = 0.13653333485126495f; // RN(8192 / 60000)
 template <int DIR>
 RK_DEV void fast_wheel_rpm2(int32_t &rpm, int32_t cur, float &rwf) {
@@ -357,22 +344,13 @@ template <bool FFSAT, bool TRACE, bool KD0>
 RK_DEV void fast_tick2(FastVeh2 &f, const rk_vdt_params_t &p, const FastConsts &fc, float2 cs, float2 sc, float nz,
                        float vel[3], float tgt[3]) {
   Sense s;
-  if(RK_FAST_FDANG) {
-    fast_wheel_rpm2<1>(f.w01.rpm[0], f.w01.cur[0], s.rw01.x);
-    fast_wheel_rpm2<1>(f.w01.rpm[1], f.w01.cur[1], s.rw01.y);
-    fast_wheel_rpm2<-1>(f.w23.rpm[0], f.w23.cur[0], s.rw23.x);
-    fast_wheel_rpm2<-1>(f.w23.rpm[1], f.w23.cur[1], s.rw23.y);
-    const float2 q01 = mul2(s.rw01, bc2(kDangC), nz), q23 = mul2(s.rw23, bc2(kDangC), nz);
-    s.d0 = truncf(q01.x), s.d2 = truncf(q23.x), s.d13 = make_float2(truncf(q01.y), truncf(q23.y));
-    f.w01.dsf = add2(f.w01.dsf, make_float2(s.d0, s.d2)), f.w23.dsf = add2(f.w23.dsf, s.d13);
-  } else {
-    float d1, d3;
-    fast_wheel_sense2<1>(f.w01.rpm[0], f.w01.cur[0], f.w01.dsum[0], s.rw01.x, s.d0);
-    fast_wheel_sense2<1>(f.w01.rpm[1], f.w01.cur[1], f.w01.dsum[1], s.rw01.y, d1);
-    fast_wheel_sense2<-1>(f.w23.rpm[0], f.w23.cur[0], f.w23.dsum[0], s.rw23.x, s.d2);
-    fast_wheel_sense2<-1>(f.w23.rpm[1], f.w23.cur[1], f.w23.dsum[1], s.rw23.y, d3);
-    s.d13 = make_float2(d1, d3);
-  }
+  fast_wheel_rpm2<1>(f.w01.rpm[0], f.w01.cur[0], s.rw01.x);
+  fast_wheel_rpm2<1>(f.w01.rpm[1], f.w01.cur[1], s.rw01.y);
+  fast_wheel_rpm2<-1>(f.w23.rpm[0], f.w23.cur[0], s.rw23.x);
+  fast_wheel_rpm2<-1>(f.w23.rpm[1], f.w23.cur[1], s.rw23.y);
+  const float2 q01 = mul2(s.rw01, bc2(kDangC), nz), q23 = mul2(s.rw23, bc2(kDangC), nz);
+  s.d0 = truncf(q01.x), s.d2 = truncf(q23.x), s.d13 = make_float2(truncf(q01.y), truncf(q23.y));
+  f.w01.dsf = add2(f.w01.dsf, make_float2(s.d0, s.d2)), f.w23.dsf = add2(f.w23.dsf, s.d13);
   fast_tick2_core<FFSAT, TRACE, KD0>(f, p, fc, cs, sc, nz, vel, tgt, s);
 }
 // the same tick fed by four recorded frames (RK_SENSOR_STREAM)

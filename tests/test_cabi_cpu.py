@@ -169,8 +169,8 @@ def test_ctypes_structs_match_the_header(tmp_path):
 
 def test_float_encoder_step_is_exact():
     """The packed vehicle tick forms the plant's encoder step rpm * 8192 / 60000 (C truncating division) in float as
-    trunc(RN(rpm * C)), C = RN(8192 / 60000) (rk_vehicle_fast2.cuh, RK_FAST_FDANG): equal for every int16 rpm.  The same
-    check runs on the device before the fast path is enabled (rk_exact.cu)."""
+    trunc(RN(rpm * C)), C = RN(8192 / 60000) (the float encoder step in fast_tick2, rk_vehicle_fast2.cuh): equal for every
+    int16 rpm.  The same check runs on the device before the fast path is enabled (rk_exact.cu)."""
     rw = np.arange(-32768, 32768, dtype=np.int64)
     want = np.sign(rw) * ((np.abs(rw) * 8192) // 60000)
     c = np.float32(0.13653333485126495)
