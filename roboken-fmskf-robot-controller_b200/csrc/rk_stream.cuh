@@ -29,6 +29,10 @@ RK_DEV uint32_t lite32(uint32_t h, uint32_t k) {
 RK_DEV float    u01_32(uint32_t h) { return fmul((float)(h >> 8), 1.0f / 16777216.0f); }
 
 
+// Whether sample `upd` of streams.imu_samples_v2 carries a quaternion frame.  px = h32_prefix(seed, 20, robot).
+RK_DEV bool stream_imu_have(uint32_t px, uint32_t upd, uint32_t drop_every) {
+  return drop_every == 0u || (lite32(h32_idx(px, upd), 8u) % drop_every) != 0u;
+}
 // One WT901 register snapshot of streams.imu_samples_v2: the two 128-bit cells rk_imt_update consumes and the
 // quaternion-frame flag.  px = h32_prefix(seed, 20, robot), upd = the sample's update index.
 RK_DEV void stream_imu_sample(uint32_t px, uint32_t upd, uint32_t drop_every, uint4 &c0, uint4 &c1, bool &have) {
@@ -48,13 +52,12 @@ RK_DEV void stream_imu_sample(uint32_t px, uint32_t upd, uint32_t drop_every, ui
   for(int k = 0; k < 4; k++) q[k] = (uint32_t)__float2int_rn(fmul(g[k], sc)) & 0xFFFFu;
   w[6] = q[0] | (q[1] << 16), w[7] = q[2] | (q[3] << 16);
   c0 = make_uint4(w[0], w[1], w[2], w[3]), c1 = make_uint4(w[4], w[5], w[6], w[7]);
-  have = drop_every == 0u || (lite32(b, 8u) % drop_every) != 0u;
+  have = stream_imu_have(px, upd, drop_every);
 }
 // only what the vehicle needs of a sample: the Yaw register and the flag
 RK_DEV void stream_imu_yaw(uint32_t px, uint32_t upd, uint32_t drop_every, int16_t &yaw, bool &have) {
-  const uint32_t b = h32_idx(px, upd);
-  yaw  = (int16_t)(lite32(b, 5u) >> 16);
-  have = drop_every == 0u || (lite32(b, 8u) % drop_every) != 0u;
+  yaw  = (int16_t)(lite32(h32_idx(px, upd), 5u) >> 16);
+  have = stream_imu_have(px, upd, drop_every);
 }
 
 } // namespace rk

@@ -10,11 +10,12 @@
 //     rk_vdt_rollout_t::d_imu_regs), so the IMU kernel is no longer its predecessor.  The one word it
 //     needs from the IMU block -- Data.angle[2] at launch, held if update 0 carries no quaternion frame --
 //     is snapshot into the caller's scratch before anything else runs;
-//   * the IMU update (HBM-bound) and the arm tick (latency-bound) run on a high-priority side stream on
-//     a CAPPED grid of one CTA per SM that strides over the batch.  The vehicle kernel fills the register
-//     file with four 128-thread CTAs per SM and gains only 4 % from the fourth; whenever one of its CTAs
-//     retires, the pending high-priority CTA takes the slot, so the two small kernels execute inside the
-//     vehicle rollout's shadow instead of after it.
+//   * the IMU update (one frame per robot: nothing reads the IMU block inside the launch, so only the last
+//     sample with a quaternion frame is read -- rk_imu.cu, imt_last_frame) and the arm tick (latency-bound)
+//     run on a high-priority side stream on a CAPPED grid of one CTA per SM that strides over the batch.  The
+//     vehicle kernel fills the register file with four 128-thread CTAs per SM and gains only 4 % from the
+//     fourth; whenever one of its CTAs retires, the pending high-priority CTA takes the slot, so the two small
+//     kernels execute inside the vehicle rollout's shadow instead of after it.
 #include <mutex>
 
 #include "rk_common.cuh"
