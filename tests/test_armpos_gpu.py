@@ -12,7 +12,8 @@ pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
 
 
-def gpu_pos_script(n, script, astate):
+def gpu_pos_script(n, script, astate, trace=True):
+    """The script's outputs; without `trace` each update's trace output is None (the kernel runs untraced)."""
     ab = ArmBatch(n, DEV)
     ab.load_state_soa(astate)
     pb = ArmPositioningBatch(ab)
@@ -23,9 +24,9 @@ def gpu_pos_script(n, script, astate):
         elif step[0] == "push":
             pb.push_cmd(torch.from_numpy(step[1].view(np.int32)).to(DEV), None if step[2] is None else torch.from_numpy(step[2]).to(DEV))
         elif step[0] == "update":
-            tr = torch.zeros((step[1], layout.ADT_TRACE_WORDS, n), dtype=torch.int32, device=DEV)
+            tr = torch.zeros((step[1], layout.ADT_TRACE_WORDS, n), dtype=torch.int32, device=DEV) if trace else None
             pb.update(step[1], tr)
-            outs.append(tr.cpu().numpy().view(np.uint32))
+            outs.append(tr.cpu().numpy().view(np.uint32) if trace else None)
         elif step[0] == "status":
             outs.append(pb.cmd_status(torch.from_numpy(np.asarray(step[1], dtype=np.uint32).view(np.int32)).to(DEV)).cpu().numpy())
         torch.cuda.synchronize()
@@ -33,14 +34,20 @@ def gpu_pos_script(n, script, astate):
     return outs
 
 
-@pytest.mark.parametrize("n,seed", [(1, 1), (300, 2), (4100, 3)])
-def test_positioning_mode_vs_port(n, seed):
+_POS_CASES = [(1, 1), (300, 2), (4100, 3)]
+
+
+# Untraced runs launch the kernel instantiations without a trace; they are held to the state blocks after every step.
+@pytest.mark.parametrize("n,seed,trace", [(n, s, True) for n, s in _POS_CASES] + [(n, s, False) for n, s in _POS_CASES],
+                         ids=[f"{n}-{s}" for n, s in _POS_CASES] + [f"{n}-{s}-untraced" for n, s in _POS_CASES])
+def test_positioning_mode_vs_port(n, seed, trace):
     st0 = bringup_state(n, seed)
     sc = pos_script(n, seed)
-    got, exp = gpu_pos_script(n, sc, st0), run_pos_script("port", n, sc, st0)[2]
+    got, exp = gpu_pos_script(n, sc, st0, trace), run_pos_script("port", n, sc, st0)[2]
     assert len(got) == len(exp)
     for k, (x, y) in enumerate(zip(got, exp)):
-        np.testing.assert_array_equal(x, y, err_msg=f"output {k}")
+        if x is not None:
+            np.testing.assert_array_equal(x, y, err_msg=f"output {k}")
 
 
 def test_positioning_mode_vs_compiled_reference():
