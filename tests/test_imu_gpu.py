@@ -1,4 +1,4 @@
-"""GPU parity: rk_imt_update (C-ABI) vs the oracle / golden fixture, bit-exact."""
+"""GPU parity: rk_imt_update / rk_imt_update_yaw (C-ABI) vs the oracle / golden fixture, bit-exact."""
 import os
 
 import numpy as np
@@ -6,7 +6,7 @@ import pytest
 import torch
 
 import oracle_lib as ol
-from roboken_fmskf_robot_controller_b200 import layout, streams
+from roboken_fmskf_robot_controller_b200 import _cabi, layout, streams
 from roboken_fmskf_robot_controller_b200.imu import Imu, ImuBatch
 
 pytestmark = pytest.mark.gpu
@@ -46,6 +46,36 @@ def test_imu_vs_port(n, K, seed):
     st2, out2 = gpu_imu(n, regs2, have2, state=st)
     np.testing.assert_array_equal(out2, oa)
     np.testing.assert_array_equal(st2, a)
+
+
+@pytest.mark.parametrize("do_init", [True, False])
+@pytest.mark.parametrize("with_have", [True, False])
+@pytest.mark.parametrize("with_out", [True, False])
+def test_imu_yaw_entry_vs_port(with_out, with_have, do_init):
+    """rk_imt_update_yaw, with the output page and with the yaw alone: every update's yaw is the port's Data.angle[2]
+    times DEG2RAD in float32, and the page and the state block are the port's, bit for bit."""
+    n, K = 1000, 9
+    seed = 20 + 4 * with_out + 2 * with_have + do_init
+    regs, have = streams.imu_samples(n, K, seed=seed, drop_every=3)
+    have = have if with_have else None
+    st0 = np.zeros(layout.IS_WORDS * n, dtype=np.uint32)
+    ol.imu_port(st0, n, streams.imu_samples(n, 1, seed=seed + 100)[0], None, do_init=True)  # a booted block
+    exp = st0.copy()
+    oe = ol.imu_port(exp, n, regs, have, want_out=True, do_init=do_init)
+    yaw_exp = (np.ascontiguousarray(oe[:, 2, :, 3]).view(np.float32) * streams.DEG2RAD).astype(np.float32)  # Data.angle[2]
+    ib = ImuBatch(n, DEV)
+    ib.load_state_soa(st0)
+    regs_d = torch.from_numpy(streams.imu_cells(regs)).to(DEV)
+    have_d = None if have is None else torch.from_numpy(have).to(DEV)
+    out = torch.zeros((K, 4, n, 4), dtype=torch.float32, device=DEV) if with_out else None
+    yaw = torch.zeros((K, n), dtype=torch.float32, device=DEV)
+    _cabi.check(ib.lib.rk_imt_update_yaw(ib.state.data_ptr(), n, K, regs_d.data_ptr(), None if have_d is None else have_d.data_ptr(),
+                                         None if out is None else out.data_ptr(), yaw.data_ptr(), int(do_init), None))
+    torch.cuda.synchronize()
+    np.testing.assert_array_equal(yaw.cpu().numpy().view(np.uint32), yaw_exp.view(np.uint32))
+    if with_out:
+        np.testing.assert_array_equal(out.cpu().numpy().view(np.uint32), oe)
+    np.testing.assert_array_equal(ib.state.cpu().numpy().view(np.uint32), exp)
 
 
 def test_imu_extreme_registers():
