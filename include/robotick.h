@@ -63,7 +63,7 @@ enum {
   RK_OPT_STREAM_CTAS = 6,    /* rk_stream_*: at most this many CTAs per SM (0, the default: full grids).  A planner that expands
                               * the next batch's streams beside a running rollout keeps them out of its way.  Scheduling only. */
   RK_OPT_TICK_SIDE_CTAS = 4  /* rk_tick_rollout: CTAs per SM its IMU / arm kernels may occupy beside the vehicle
-                              * rollout (default 1; 0 = full grids).  Scheduling only, results do not depend on it. */
+                              * rollout (0, the default: full grids).  Scheduling only, results do not depend on it. */
 };
 int rk_set_option(int option, int value);
 /* 1 if the exhaustive on-device proofs that gate the issue-optimised kernel hold for these

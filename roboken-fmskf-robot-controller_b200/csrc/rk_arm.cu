@@ -505,7 +505,72 @@ RK_DEV void arm_trace_row(uint32_t *tr, int64_t n, const ArmLoop &a, uint32_t w1
   tr[14 * n] = 0u, tr[15 * n] = 0u;
 }
 
-template <bool TRACE, int DIVC, int UNROLL>
+// Jumping over ticks (the untraced launch with the MG joint in position control).  Inside a segment a LAZY tick only
+// advances cyc, forms tgt[0] and runs the ICS update on it (the MG targets it shifts are constant there, and the last two
+// ticks of the launch, which stay real, rewrite them), so the non-final ticks of a segment can be replaced by their end
+// state.  The ICS update of one tick is exact to reproduce over a window: its deg100 is a chain of RN operations with
+// one fixed operand and a truncation toward zero on the remaining count, so it is monotone over the window, and tp is
+// monotone in deg100.  So "active" (|deg100| <= 18000) and "send" (active, torque on, 3500 <= tp <= 11500) each hold on
+// one contiguous run of ticks; the window leaves what the last sending tick and then the last active tick leave.
+
+// the ICS joint's raw target, and the argument of its deg100 conversion, on the segment tick with remaining count r
+RK_DEV float seg_tgt0(const ArmLoop &a, int32_t r) { return fadd(fsub(a.now_tgt[0], fmul(a.move[0], (float)r)), a.ofs[0]); }
+RK_DEV float ics_arg(const ArmLoop &a, const ArmConsts &c, int32_t r) { return fmul(fmul(seg_tgt0(a, r), c.dir_y0), 100.0f); }
+// where the tick with remaining count r lies against the interval of `active` (send = false) or of `send` (send = true):
+// -1 below, 0 inside, +1 above; monotone in deg100
+RK_DEV int ics_side(const ArmLoop &a, const ArmConsts &c, int32_t r, bool send) {
+  const int deg100 = f2i_x86(ics_arg(a, c, r));
+  if(deg100 < -18000 || deg100 > 18000) return deg100 < 0 ? -1 : 1;
+  const int tp = (deg100 * 2963) / 10000 + 7500;
+  return !send ? 0 : (tp < 3500 ? -1 : (tp > 11500 ? 1 : 0));
+}
+// the last of the window's j ticks (tick k has remaining count left - k) inside the interval, or -1: the last tick if it
+// is inside; else the ticks past the same bound form a suffix, and the one before it is checked against the other bound
+RK_DEV int32_t ics_last(const ArmLoop &a, const ArmConsts &c, int32_t left, int32_t j, bool send) {
+  const int s = ics_side(a, c, left - (j - 1), send);
+  if(s == 0) return j - 1;
+  int32_t lo = 0, hi = j - 1;
+#pragma unroll 1
+  while(lo < hi) {
+    const int32_t m = lo + (hi - lo) / 2;
+    if(ics_side(a, c, left - m, send) == s) hi = m;
+    else lo = m + 1;
+  }
+  return (lo > 0 && ics_side(a, c, left - (lo - 1), send) == 0) ? lo - 1 : -1;
+}
+RK_DEV void ics_window_tick(ArmLoop &a, const ArmConsts &c, int32_t r) {
+  RK_ICS_UPDATE(seg_tgt0(a, r), c.dir_y0, c.y0_conn, c.y0_on, a.ics_pos, a.ics_servo)
+  a.y0_pos  = active ? now_pos : a.y0_pos;
+  a.y0_seen = a.y0_seen || active;
+}
+RK_DEV bool arm_idle(const ArmLoop &a) { return a.state == RK_ASTATE_STANDBY && a.exec == a.head; }
+
+// The index of the next tick to run for real, after ticks [0, t) have run (`idle`: the last of them started in STANDBY
+// with nothing queued).  Ticks K-2 and K-1 always run: loop_finish_mg needs their MG targets, the stored block their
+// targets and frames.  An idle tick is a fixed point -- IS_COMP is set, and the ICS update of an unchanged target rewrites
+// what it wrote -- so the ticks after it are skipped.  Inside a segment, the next min(cnt - cyc, K-2 - t) ticks are its
+// non-final ticks, jumped over in one step unless the ICS conversion of a target at either end of the window is out of
+// f2i_x86's range or NaN (huge or infinite waypoints), which breaks the monotonicity: those windows run tick by tick.
+RK_DEV int loop_jump(ArmLoop &a, const ArmConsts &c, int t, int K, bool idle) {
+  if(t >= K - 2) return t;
+  if(idle) return K - 2;
+  const int32_t left = (int32_t)((uint32_t)a.cnt - (uint32_t)a.cyc); // remaining count of the next tick
+  if(a.state != RK_ASTATE_MOVING || a.cnt <= a.cyc || left <= 0) return t;
+  const int32_t j = min(left, K - 2 - t), last = left - (j - 1);
+  if(!(fabsf(ics_arg(a, c, left)) < 2147483648.0f && fabsf(ics_arg(a, c, last)) < 2147483648.0f)) return t;
+  if(c.y0_conn) {
+    const int32_t ls = c.y0_on ? ics_last(a, c, left, j, true) : -1, la = ics_last(a, c, left, j, false);
+    if(ls >= 0) ics_window_tick(a, c, left - ls);
+    if(la >= 0) ics_window_tick(a, c, left - la);
+  }
+  a.tgt[0] = seg_tgt0(a, last);
+  a.mg_pp  = j > 1 ? a.tgt[1] : a.mg_pre;
+  a.mg_pre = a.tgt[1];
+  a.cyc += j;
+  return t + j;
+}
+
+template <bool TRACE, int DIVC>
 RK_DEV void adt_update_body(int64_t i, const rk_adt_params_t &p, uint4 *__restrict__ state, const uint4 *__restrict__ tab, int64_t n, int K,
                             uint32_t *__restrict__ trace, float mg_rcp) {
   ArmLoop  a;
@@ -524,17 +589,28 @@ RK_DEV void adt_update_body(int64_t i, const rk_adt_params_t &p, uint4 *__restri
     ring_fetch(a, tab, n, i, fs, fi, a.sel);
     a.pf_key = ring_key(fs, fi);
   }
-  if(c.mg_pos) {
-    if(K > 0) { // the first tick sees the stored is_torque_on_prev flags, the others run on launch constants (STEADY)
-      loop_tick<DIVC, false, false, !TRACE>(a, p, c, state, tab, n, i, K <= 2);
-      if(TRACE) arm_trace_row(trace + i, n, a, a.state, a.cmd_idx);
+  // the first tick sees the stored is_torque_on_prev flags, the others run on launch constants (STEADY)
+  if(c.mg_pos && !TRACE) { // one real tick per iteration, then as far as loop_jump allows
+    if(K > 0) {
+      bool idle = arm_idle(a);
+      loop_tick<DIVC, false, false, true>(a, p, c, state, tab, n, i, K <= 2);
+#pragma unroll 1
+      for(int t = loop_jump(a, c, 1, K, idle); t < K; t = loop_jump(a, c, t + 1, K, idle)) {
+        idle = arm_idle(a);
+        loop_tick<DIVC, false, true, true>(a, p, c, state, tab, n, i, t >= K - 2);
+      }
+      loop_finish_mg<DIVC>(a, c);
     }
-#pragma unroll UNROLL
+  } else if(c.mg_pos) { // every tick writes a trace row
+    if(K > 0) {
+      loop_tick<DIVC, false, false, false>(a, p, c, state, tab, n, i, K <= 2);
+      arm_trace_row(trace + i, n, a, a.state, a.cmd_idx);
+    }
+#pragma unroll 1
     for(int t = 1; t < K; t++) {
-      loop_tick<DIVC, false, true, !TRACE>(a, p, c, state, tab, n, i, t >= K - 2);
-      if(TRACE) arm_trace_row(trace + (int64_t)t * RK_ADT_TRACE_WORDS * n + i, n, a, a.state, a.cmd_idx);
+      loop_tick<DIVC, false, true, false>(a, p, c, state, tab, n, i, t >= K - 2);
+      arm_trace_row(trace + (int64_t)t * RK_ADT_TRACE_WORDS * n + i, n, a, a.state, a.cmd_idx);
     }
-    if(!TRACE && K > 0) loop_finish_mg<DIVC>(a, c);
   } else {
 #pragma unroll 1
     for(int t = 0; t < K; t++) {
@@ -546,12 +622,12 @@ RK_DEV void adt_update_body(int64_t i, const rk_adt_params_t &p, uint4 *__restri
   loop_store(state, n, i, a, jflags, K > 0);
 }
 // One thread per arm; CTAs stride over the batch when the grid is capped (see imt_update_kernel).
-template <bool TRACE, int DIVC, int UNROLL = 1>
+template <bool TRACE, int DIVC>
 __global__ void __launch_bounds__(128, 5)
 adt_update_kernel(const rk_adt_params_t p, uint4 *__restrict__ state, const uint4 *__restrict__ tab, int64_t n, int K,
                   uint32_t *__restrict__ trace, float mg_rcp) {
   for(int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
-    adt_update_body<TRACE, DIVC, UNROLL>(i, p, state, tab, n, K, trace, mg_rcp);
+    adt_update_body<TRACE, DIVC>(i, p, state, tab, n, K, trace, mg_rcp);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -1174,12 +1250,8 @@ int rk::adt_update_launch(const rk_adt_params_t *p, void *d_state, const void *d
   with_divc(p->ctrl_time_s[RK_AJ_P1], [&](auto dv, float rcp) {
     uint4       *s = (uint4 *)d_state;
     const uint4 *t = (const uint4 *)d_cmdtab;
-    // Alone, the tick loop unrolled 4x is fastest (5.40 -> 5.09 ms per 2^20 x 1000).  Beside the vehicle rollout of
-    // rk_tick_rollout the larger loop loses far more in the shared instruction caches than it gains (full tick 162.6 ->
-    // 188.5 ms per pass), so a capped launch (max_ctas > 0: the side stream) runs the rolled loop.
     if(d_trace) adt_update_kernel<true, dv><<<grid, 128, 0, st>>>(*p, s, t, n, K, d_trace, rcp);
-    else if(max_ctas > 0) adt_update_kernel<false, dv><<<grid, 128, 0, st>>>(*p, s, t, n, K, d_trace, rcp);
-    else adt_update_kernel<false, dv, 4><<<grid, 128, 0, st>>>(*p, s, t, n, K, d_trace, rcp);
+    else adt_update_kernel<false, dv><<<grid, 128, 0, st>>>(*p, s, t, n, K, d_trace, rcp);
   });
   RK_CUDA(cudaGetLastError());
   return RK_OK;

@@ -11,11 +11,13 @@
 //     needs from the IMU block -- Data.angle[2] at launch, held if update 0 carries no quaternion frame --
 //     is snapshot into the caller's scratch before anything else runs;
 //   * the IMU update (one frame per robot: nothing reads the IMU block inside the launch, so only the last
-//     sample with a quaternion frame is read -- rk_imu.cu, imt_last_frame) and the arm tick (latency-bound)
-//     run on a high-priority side stream on a CAPPED grid of one CTA per SM that strides over the batch.  The
-//     vehicle kernel fills the register file with four 128-thread CTAs per SM and gains only 4 % from the
-//     fourth; whenever one of its CTAs retires, the pending high-priority CTA takes the slot, so the two small
-//     kernels execute inside the vehicle rollout's shadow instead of after it.
+//     sample with a quaternion frame is read -- rk_imu.cu, imt_last_frame) and the arm tick (a few real ticks
+//     per segment -- rk_arm.cu, loop_jump) run on a high-priority side stream.  The vehicle kernel fills the
+//     register file with four 128-thread CTAs per SM; whenever one of its CTAs retires, a pending
+//     high-priority CTA takes the slot, so the two small kernels execute inside the vehicle rollout's shadow
+//     instead of after it.  Their grids are uncapped by default: each side CTA then finishes its 128 or 256
+//     robots and gives the slot back, where a capped grid of one CTA per SM holds a vehicle slot for the
+//     whole latency-bound stride over the batch (RK_OPT_TICK_SIDE_CTAS caps them; DESIGN.md 3.5).
 #include <mutex>
 
 #include "rk_common.cuh"
@@ -31,7 +33,7 @@ struct TickStreams {
 static bool g_tick_timeline = false;
 static std::mutex  g_tick_mu; // held across the whole fork / launch / join sequence: the event pair is per device
 static TickStreams g_tick[64];
-static int         g_tick_side_ctas_per_sm = 1; // rk_set_option(RK_OPT_TICK_SIDE_CTAS, 0..8): 0 = uncapped grids
+static int         g_tick_side_ctas_per_sm = 0; // rk_set_option(RK_OPT_TICK_SIDE_CTAS, 0..8): 0 = uncapped grids
 
 int tick_set_side_ctas(int v) {
   if(v < 0 || v > 8) return RK_ERR_ARG;

@@ -2,7 +2,7 @@
 """Where the kernels of rk_tick_rollout run relative to each other: a few chunks back to back on one or two lanes with
 the library's diagnostic timestamps (rk_tick_debug_timeline), plus CUDA events around the caller-side setup kernels.
 
-    python tools/tick_timeline.py [--n 1048576] [--chunks 4] [--lanes 2] [--side-ctas 1]"""
+    python tools/tick_timeline.py [--n 1048576] [--chunks 4] [--lanes 2] [--side-ctas 0]"""
 import argparse
 import ctypes as C
 import os
@@ -20,7 +20,7 @@ ap = argparse.ArgumentParser()
 ap.add_argument("--n", type=int, default=1 << 20)
 ap.add_argument("--chunks", type=int, default=4)
 ap.add_argument("--lanes", type=int, default=2)
-ap.add_argument("--side-ctas", type=int, default=1)
+ap.add_argument("--side-ctas", type=int, default=0)
 ap.add_argument("--ticks", type=int, default=1000)
 a = ap.parse_args()
 dev = torch.device("cuda", 0)
