@@ -697,6 +697,53 @@ int rk_plan_select(const float *d_cost, const rk_vdt_cmd_t *d_cmd, int64_t R, in
                    float lambda, int32_t shift, rk_vdt_cmd_t *d_nominal_out, int32_t *d_best, float *d_best_cost,
                    void *stream);
 
+/* Cross-entropy planning (CEM): several sample -> rollout -> refit rounds per planning step from the same source states,
+ * each drawing the candidates from a per-robot, per-segment distribution (nominal, sigma table) and refitting it to the
+ * round's k best candidates:
+ *   rk_plan_sample_commands_sigma  nominal + sigma [n_seg][R]  -> candidates [n_seg][R*S]
+ *   rk_plan_rollout(_obstacles)    as above                    -> cost [R*S]
+ *   rk_plan_refit                  cost + candidates + sigma   -> new nominal + sigma [n_seg][R], best index / cost [R] */
+
+/* rk_plan_sample_commands with the noise scale taken per robot and segment: axis a of candidate j > 0 of robot r,
+ * segment s is nom_a + d_sigma[s*R + r][a] * xi_a.  xi, the hash, j == 0, the limiters and kind are exactly those of
+ * rk_plan_sample_commands, and s->sigma is ignored.  So a table holding s->sigma in every cell gives the same bits as
+ * rk_plan_sample_commands.  d_sigma: float4 [n_seg][R] {sx, sy, sth, unused}, 16-byte aligned, and it must not overlap
+ * d_cmd.  Argument checks as rk_plan_sample_commands, plus d_sigma NULL, misaligned or overlapping d_cmd (RK_ERR_ARG). */
+int rk_plan_sample_commands_sigma(const rk_vdt_params_t *p, const rk_plan_sample_t *s, const rk_vdt_cmd_t *d_nominal,
+                                  const float *d_sigma, int64_t R, int32_t S, int32_t n_seg, rk_vdt_cmd_t *d_cmd, void *stream);
+
+typedef struct rk_plan_refit {
+  int32_t elite;        /* k, 1 <= k <= S */
+  float   alpha;        /* smoothing toward the previous distribution, 0 <= alpha <= 1 (0: none) */
+  float   sigma_min[3]; /* floor of the refitted sigma, finite and >= 0 */
+  float   rsv;
+} rk_plan_refit_t;      /* 24 bytes */
+
+/* Refit of robot r's distribution to its elite candidates.  Every float operation is one IEEE float32 operation (round to
+ * nearest, no contraction) in the order written.
+ *   Order:  candidates are ordered by (cost, j), costs compared as floats (-0 equals +0), ties to the lower j.
+ *   Elites: E_r = the first k_eff = min(k, number of finite costs of r) candidates in that order; a NaN or +-inf cost is
+ *           never an elite (a candidate priced +inf by w_obst = INFINITY never weighs in the mean).
+ *   Best:   d_best / d_best_cost exactly as rk_plan_select writes them (argmin, NaN as +inf, all NaN: 0); either may be NULL.
+ *   Output segment s reads source segment ss = min(s + shift, n_seg - 1), as rk_plan_select does.  Per axis a, with v the
+ *   axis-a word of the candidate's cell [ss][r*S + j] and the elites taken in ascending j:
+ *     m   = (((v_e0 + v_e1) + ...) + v_e(k_eff-1)) / (float)k_eff     (the sum starts from the first elite)
+ *     q   = ((0 + (v_e0 - m)*(v_e0 - m)) + ...) + (v_e(k_eff-1) - m)*(v_e(k_eff-1) - m)
+ *     sd  = sqrtf(q / (float)k_eff)
+ *     alpha > 0:  mean = alpha*c0 + (1 - alpha)*m,  sig = alpha*sigma_in[ss][a] + (1 - alpha)*sd
+ *                 (c0: candidate 0 of robot r in segment ss, the centre that segment was drawn around)
+ *     alpha == 0: mean = m,  sig = sd
+ *   sigma_out[s][r] = {fmaxf(sig_x, sigma_min[0]), fmaxf(sig_y, sigma_min[1]), fmaxf(sig_th, sigma_min[2]), 0} and
+ *   nominal_out[s][r] = {mean_x, mean_y, mean_th, RK_CMD_MOVE}.  k_eff == 0 (no finite cost): nominal_out[s][r] is candidate
+ *   best of segment ss and sigma_out[s][r] is sigma_in[ss][r], both copied bit for bit.
+ * d_sigma_in / d_sigma_out: float4 [n_seg][R], 16-byte aligned.  RK_ERR_ARG: rk_plan_select's checks; rf NULL; elite
+ * outside [1, S]; alpha NaN or outside [0, 1]; a sigma_min NaN, negative or inf; a NULL or misaligned sigma table;
+ * d_nominal_out overlapping d_cmd; d_sigma_out overlapping d_sigma_in, except the same table with shift == 0 (each robot
+ * and segment reads only its own cell then).  R == 0 is a no-op.  No limit on S or k beyond n_seg * S < 2^32. */
+int rk_plan_refit(const float *d_cost, const rk_vdt_cmd_t *d_cmd, const float *d_sigma_in, int64_t R, int32_t S,
+                  int32_t n_seg, const rk_plan_refit_t *rf, int32_t shift, rk_vdt_cmd_t *d_nominal_out,
+                  float *d_sigma_out, int32_t *d_best, float *d_best_cost, void *stream);
+
 /* =====================================================================================
  * RobotManager guard (SURVEY 8f-2): the vehicle-management block of RMT's routine_ros()
  * (src/RobotManager/RM_task_main.cpp:484-767), one call = K manager cycles of n robots.  Per

@@ -182,6 +182,12 @@ class PlanObstacles(C.Structure):
     _fields_ = [("d_obs", C.c_void_p), ("m", C.c_int32), ("check_period", C.c_int32), ("w_obst", C.c_float), ("rsv", C.c_float)]
 
 
+class PlanRefit(C.Structure):
+    """rk_plan_refit_t"""
+
+    _fields_ = [("elite", C.c_int32), ("alpha", C.c_float), ("sigma_min", C.c_float * 3), ("rsv", C.c_float)]
+
+
 _lib = None
 
 
@@ -233,6 +239,9 @@ def _proto(lib):
     lib.rk_plan_rollout_obstacles.argtypes = [C.POINTER(VdtParams), vp, C.c_int64, C.c_int32, vp, C.c_int32, C.c_int32, C.POINTER(PlanCost),
                                               C.POINTER(PlanObstacles), vp, vp]
     lib.rk_plan_select.argtypes = [vp, vp, C.c_int64, C.c_int32, C.c_int32, C.c_float, C.c_int32, vp, vp, vp, vp]
+    lib.rk_plan_sample_commands_sigma.argtypes = [C.POINTER(VdtParams), C.POINTER(PlanSample), vp, vp, C.c_int64, C.c_int32, C.c_int32, vp,
+                                                  vp]
+    lib.rk_plan_refit.argtypes = [vp, vp, vp, C.c_int64, C.c_int32, C.c_int32, C.POINTER(PlanRefit), C.c_int32, vp, vp, vp, vp, vp]
     lib.rk_adt_bldc_rx.argtypes = [C.POINTER(AdtParams), vp, C.c_int64, C.c_int, vp, vp, vp, vp]
     lib.rk_adt_mg_rx.argtypes = [C.POINTER(AdtParams), vp, C.c_int64, vp, vp, vp]
     lib.rk_selftest_div_rcp64.argtypes = [C.c_uint64, C.c_uint64, C.POINTER(C.c_uint32)]

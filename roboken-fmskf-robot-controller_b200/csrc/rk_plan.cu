@@ -28,9 +28,12 @@ struct PlanSampleArgs {
   float    sigma[3], limit_speed, limit_rot;
 };
 
-// one thread per (segment, candidate): blockIdx.y strides the segments, x runs over the R*S candidates of one segment
+// one thread per (segment, candidate): blockIdx.y strides the segments, x runs over the R*S candidates of one segment.
+// kSigmaTable: the noise scale of segment s, robot r is cell s*R + r of `sigma` (rk_plan_sample_commands_sigma) instead
+// of a.sigma; the table comes last among the parameters so that the other instantiation's parameter offsets stay put.
+template <bool kSigmaTable>
 __global__ void __launch_bounds__(RK_PLAN_BLOCK)
-plan_sample_kernel(const PlanSampleArgs a, const uint4 *__restrict__ nominal, uint4 *__restrict__ cmd) {
+plan_sample_kernel(const PlanSampleArgs a, const uint4 *__restrict__ nominal, uint4 *__restrict__ cmd, const float4 *__restrict__ sigma) {
   const int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   const int64_t n = a.R * (int64_t)a.S;
   if(c >= n) return;
@@ -42,8 +45,13 @@ plan_sample_kernel(const PlanSampleArgs a, const uint4 *__restrict__ nominal, ui
     float       v[3] = {u2f(nq.x), u2f(nq.y), u2f(nq.z)};
     if(j != 0u) {
       const uint32_t h = h32_idx(px, (uint32_t)s * (uint32_t)a.S + j);
+      float          sg[3] = {a.sigma[0], a.sigma[1], a.sigma[2]};
+      if constexpr(kSigmaTable) {
+        const float4 t = __ldg(sigma + (int64_t)s * a.R + r); // like the nominal, one cell per robot and segment
+        sg[0] = t.x, sg[1] = t.y, sg[2] = t.z;
+      }
 #pragma unroll
-      for(int ax = 0; ax < 3; ax++) v[ax] = fadd(v[ax], fmul(a.sigma[ax], plan_xi(h, (uint32_t)ax)));
+      for(int ax = 0; ax < 3; ax++) v[ax] = fadd(v[ax], fmul(sg[ax], plan_xi(h, (uint32_t)ax)));
     }
     // speed_limit_xy / speed_limit_rot (VD_task_main.cpp:127-142): a vector inside the limits passes unchanged
     const float ln = fsqrt(fadd(fmul(v[0], v[0]), fmul(v[1], v[1])));
@@ -67,18 +75,12 @@ RK_DEV float plan_weight(float c, float cmin, float lambda) {
   return isnan(w) ? 0.0f : w;
 }
 
-// one warp per robot, lanes striding over the S contiguous candidates
-__global__ void __launch_bounds__(RK_PLAN_BLOCK)
-plan_select_kernel(const float *__restrict__ cost, const uint4 *__restrict__ cmd, int64_t R, int S, int n_seg, float lambda, int shift,
-                   uint4 *__restrict__ nom, int32_t *__restrict__ best_out, float *__restrict__ best_cost_out) {
-  const int64_t r    = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-  const int     lane = threadIdx.x & 31;
-  if(r >= R) return; // whole warps leave together
-  const int64_t n  = R * (int64_t)S;
-  const float  *cr = cost + r * S;
-
-  float bk = __int_as_float(0x7F800000);
-  int   bj = INT_MAX;
+// The robot's best candidate (key, j) over its S costs cr, the same in every lane; lane 0 writes best / best_cost where
+// asked.  Returns j and leaves the key in bk.
+RK_DEV int plan_argmin(const float *__restrict__ cr, int S, int64_t r, int lane, int32_t *__restrict__ best_out,
+                       float *__restrict__ best_cost_out, float &bk) {
+  bk     = __int_as_float(0x7F800000);
+  int bj = INT_MAX;
   for(int j = lane; j < S; j += 32) {
     const float k = plan_key(__ldg(cr + j));
     if(plan_better(k, j, bk, bj)) bk = k, bj = j;
@@ -94,6 +96,21 @@ plan_select_kernel(const float *__restrict__ cost, const uint4 *__restrict__ cmd
     if(best_out) best_out[r] = best;
     if(best_cost_out) best_cost_out[r] = __ldg(cr + best);
   }
+  return best;
+}
+
+// one warp per robot, lanes striding over the S contiguous candidates
+__global__ void __launch_bounds__(RK_PLAN_BLOCK)
+plan_select_kernel(const float *__restrict__ cost, const uint4 *__restrict__ cmd, int64_t R, int S, int n_seg, float lambda, int shift,
+                   uint4 *__restrict__ nom, int32_t *__restrict__ best_out, float *__restrict__ best_cost_out) {
+  const int64_t r    = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int     lane = threadIdx.x & 31;
+  if(r >= R) return; // whole warps leave together
+  const int64_t n  = R * (int64_t)S;
+  const float  *cr = cost + r * S;
+
+  float     bk;
+  const int best = plan_argmin(cr, S, r, lane, best_out, best_cost_out, bk);
 
   float wsum = 0.0f;
   if(lambda > 0.0f) {
@@ -124,6 +141,103 @@ plan_select_kernel(const float *__restrict__ cost, const uint4 *__restrict__ cmd
   }
 }
 
+struct PlanRefitArgs {
+  int64_t R;
+  int32_t S, n_seg, k, shift;
+  float   alpha, sigma_min[3];
+};
+
+// order-preserving u32 image of a finite cost; -0 is made +0 first, so that the two are one key as they are one float
+RK_DEV uint32_t plan_order(float c) {
+  const uint32_t u = f2u(c == 0.0f ? 0.0f : c);
+  return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+}
+// Elite bits of candidates j0 .. j0+31 (bit i: candidate j0 + i), the same in every lane: finite keys below the
+// threshold key, and those at it while fewer than `take` came before (at_thr counts the ones before j0: ascending j).
+RK_DEV uint32_t plan_elite_bits(const float *__restrict__ cr, int S, int j0, int lane, uint32_t thr, int take, int &at_thr) {
+  const int      j     = j0 + lane;
+  const float    c     = j < S ? __ldg(cr + j) : __int_as_float(0x7FC00000);
+  const bool     fin   = isfinite(c);
+  const uint32_t key   = plan_order(c);
+  const uint32_t below = __ballot_sync(0xFFFFFFFFu, fin && key < thr);
+  const uint32_t at    = __ballot_sync(0xFFFFFFFFu, fin && key == thr);
+  const int      rank  = at_thr + __popc(at & ((1u << lane) - 1u));
+  at_thr += __popc(at);
+  return below | __ballot_sync(0xFFFFFFFFu, ((at >> lane) & 1u) && rank < take);
+}
+
+// one warp per robot, shaped like plan_select_kernel: the argmin; the key of the k_eff-th elite, fixed bit by bit from
+// the top with warp-wide counts; then lanes own (segment, axis) pairs and walk the candidates 32 at a time in ascending
+// j, the elites of each 32 as one ballot, reading the elite cells only.  sigma_in and sigma_out may be one table (shift == 0: each lane reads its own word first).
+__global__ void __launch_bounds__(RK_PLAN_BLOCK)
+plan_refit_kernel(const PlanRefitArgs a, const float *__restrict__ cost, const uint4 *__restrict__ cmd, const float4 *sigma_in,
+                  uint4 *__restrict__ nom, float4 *sigma_out, int32_t *__restrict__ best_out, float *__restrict__ best_cost_out) {
+  const int64_t r    = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int     lane = threadIdx.x & 31;
+  if(r >= a.R) return; // whole warps leave together
+  const int     S = a.S, n_seg = a.n_seg;
+  const int64_t n  = a.R * (int64_t)S;
+  const float  *cr = cost + r * S;
+
+  float     bk;
+  const int best = plan_argmin(cr, S, r, lane, best_out, best_cost_out, bk);
+  int       fin  = 0;
+  for(int j = lane; j < S; j += 32) fin += isfinite(__ldg(cr + j)) ? 1 : 0;
+  const int k_eff = min(a.k, (int)__reduce_add_sync(0xFFFFFFFFu, (unsigned)fin));
+  if(k_eff == 0) { // no finite cost: candidate `best` and the incoming sigma, bit for bit, one lane per segment
+    for(int s = lane; s < n_seg; s += 32) {
+      const int ss                    = min(s + a.shift, n_seg - 1);
+      nom[(int64_t)s * a.R + r]       = __ldg(cmd + (int64_t)ss * n + r * S + best);
+      sigma_out[(int64_t)s * a.R + r] = sigma_in[(int64_t)ss * a.R + r];
+    }
+    return;
+  }
+
+  uint32_t thr  = 0u;    // order key of the k_eff-th elite
+  int      take = k_eff; // ends as that elite's rank among the candidates whose key is thr
+  for(int b = 31; b >= 0; b--) {
+    const uint32_t hi  = 0xFFFFFFFFu << b;
+    int            cnt = 0; // finite keys equal to thr above bit b, with bit b clear
+    for(int j = lane; j < S; j += 32) {
+      const float c = __ldg(cr + j);
+      cnt += (isfinite(c) && ((plan_order(c) ^ thr) & hi) == 0u) ? 1 : 0;
+    }
+    cnt = (int)__reduce_add_sync(0xFFFFFFFFu, (unsigned)cnt);
+    if(take > cnt) take -= cnt, thr |= 1u << b;
+  }
+
+  const float kf = (float)k_eff, beta = fsub(1.0f, a.alpha);
+  for(int p0 = 0; p0 < 3 * n_seg; p0 += 32) { // every lane takes part in the ballots; lanes past the end do not store
+    const int    p = min(p0 + lane, 3 * n_seg - 1), s = p / 3, ax = p - 3 * s;
+    const int    ss = min(s + a.shift, n_seg - 1);
+    const float *cv = (const float *)(cmd + (int64_t)ss * n + r * S) + ax; // axis ax of candidate j is cv[4*j]
+    float        sum = -0.0f; // -0 + v == v for every v: the sum starts from the first elite
+    for(int j0 = 0, at = 0; j0 < S; j0 += 32)
+      for(uint32_t m = plan_elite_bits(cr, S, j0, lane, thr, take, at); m != 0u; m &= m - 1u) // ascending j
+        sum = fadd(sum, __ldg(cv + 4 * (int64_t)(j0 + __ffs(m) - 1)));
+    const float m = fdiv(sum, kf);
+    float       q = 0.0f;
+    for(int j0 = 0, at = 0; j0 < S; j0 += 32)
+      for(uint32_t e = plan_elite_bits(cr, S, j0, lane, thr, take, at); e != 0u; e &= e - 1u) {
+        const float d = fsub(__ldg(cv + 4 * (int64_t)(j0 + __ffs(e) - 1)), m);
+        q             = fadd(q, fmul(d, d));
+      }
+    const float sd   = fsqrt(fdiv(q, kf));
+    float       mean = m, sig = sd;
+    if(a.alpha > 0.0f) {
+      const float sin = ((const float *)(sigma_in + (int64_t)ss * a.R + r))[ax];
+      mean            = fadd(fmul(a.alpha, __ldg(cv)), fmul(beta, m));
+      sig             = fadd(fmul(a.alpha, sin), fmul(beta, sd));
+    }
+    if(p0 + lane >= 3 * n_seg) continue;
+    const float lo = ax == 0 ? a.sigma_min[0] : (ax == 1 ? a.sigma_min[1] : a.sigma_min[2]);
+    float      *no = (float *)(nom + (int64_t)s * a.R + r);
+    float      *so = (float *)(sigma_out + (int64_t)s * a.R + r);
+    no[ax] = mean, so[ax] = fmaxf(sig, lo);
+    if(ax == 0) ((uint32_t *)no)[3] = (uint32_t)RK_CMD_MOVE, so[3] = 0.0f;
+  }
+}
+
 static bool overlap(const void *a, size_t na, const void *b, size_t nb) {
   const uintptr_t x = (uintptr_t)a, y = (uintptr_t)b;
   return x < y + nb && y < x + na;
@@ -148,15 +262,9 @@ static int plan_check_table(const char *who, const void *ptr, const char *name) 
   return RK_OK;
 }
 
-} // namespace rk
-
-using namespace rk;
-
-extern "C" {
-
-int rk_plan_sample_commands(const rk_vdt_params_t *p, const rk_plan_sample_t *s, const rk_vdt_cmd_t *d_nominal, int64_t R, int32_t S,
-                            int32_t n_seg, rk_vdt_cmd_t *d_cmd, void *stream) {
-  static const char *who = "rk_plan_sample_commands";
+// rk_plan_sample_commands, and with `table` rk_plan_sample_commands_sigma (d_sigma: float4 [n_seg][R])
+static int plan_sample(const char *who, const rk_vdt_params_t *p, const rk_plan_sample_t *s, const rk_vdt_cmd_t *d_nominal, bool table,
+                       const float *d_sigma, int64_t R, int32_t S, int32_t n_seg, rk_vdt_cmd_t *d_cmd, void *stream) {
   if(!p || !s) {
     set_error("%s: NULL params/sample", who);
     return RK_ERR_ARG;
@@ -170,30 +278,38 @@ int rk_plan_sample_commands(const rk_vdt_params_t *p, const rk_plan_sample_t *s,
     set_error("%s: d_cmd must not overlap d_nominal", who);
     return RK_ERR_ARG;
   }
+  if(table) {
+    if(int rc = plan_check_table(who, d_sigma, "d_sigma")) return rc;
+    if(overlap(d_sigma, (size_t)n_seg * R * 16u, d_cmd, (size_t)n_seg * n * 16u)) {
+      set_error("%s: d_cmd must not overlap d_sigma", who);
+      return RK_ERR_ARG;
+    }
+  }
   if(int rc = require_device()) return rc;
   PlanSampleArgs a;
   a.first = s->first, a.R = R, a.S = S, a.n_seg = n_seg, a.seed = s->seed;
   for(int k = 0; k < 3; k++) a.sigma[k] = s->sigma[k];
   a.limit_speed = p->limit_speed_mmps, a.limit_rot = p->limit_rot_radps;
   const dim3 grid((unsigned)((n + RK_PLAN_BLOCK - 1) / RK_PLAN_BLOCK), (unsigned)min(n_seg, 65535));
-  plan_sample_kernel<<<grid, RK_PLAN_BLOCK, 0, (cudaStream_t)stream>>>(a, (const uint4 *)d_nominal, (uint4 *)d_cmd);
+  if(table)
+    plan_sample_kernel<true><<<grid, RK_PLAN_BLOCK, 0, (cudaStream_t)stream>>>(a, (const uint4 *)d_nominal, (uint4 *)d_cmd, (const float4 *)d_sigma);
+  else
+    plan_sample_kernel<false><<<grid, RK_PLAN_BLOCK, 0, (cudaStream_t)stream>>>(a, (const uint4 *)d_nominal, (uint4 *)d_cmd, nullptr);
   RK_CUDA(cudaGetLastError());
   return RK_OK;
 }
 
-int rk_plan_select(const float *d_cost, const rk_vdt_cmd_t *d_cmd, int64_t R, int32_t S, int32_t n_seg, float lambda, int32_t shift,
-                   rk_vdt_cmd_t *d_nominal_out, int32_t *d_best, float *d_best_cost, void *stream) {
-  static const char *who = "rk_plan_select";
+// the arguments rk_plan_select and rk_plan_refit share: sizes and shift first, then (R > 0) the tables
+static int plan_check_choice(const char *who, int64_t R, int32_t S, int32_t n_seg, int32_t shift) {
   if(int rc = plan_check_rs(who, R, S, n_seg)) return rc;
   if(shift < 0 || shift >= n_seg) {
     set_error("%s: need 0 <= shift < n_seg (shift = %d, n_seg = %d)", who, shift, n_seg);
     return RK_ERR_ARG;
   }
-  if(!(lambda >= 0.0f) || isinf(lambda)) {
-    set_error("%s: lambda must be finite and >= 0", who);
-    return RK_ERR_ARG;
-  }
-  if(R == 0) return RK_OK;
+  return RK_OK;
+}
+static int plan_check_choice_tables(const char *who, const float *d_cost, const rk_vdt_cmd_t *d_cmd, int64_t R, int32_t S, int32_t n_seg,
+                                    const rk_vdt_cmd_t *d_nominal_out) {
   if(!d_cost || ((uintptr_t)d_cost & 3u)) {
     set_error("%s: d_cost must be a non-NULL float device pointer", who);
     return RK_ERR_ARG;
@@ -204,11 +320,83 @@ int rk_plan_select(const float *d_cost, const rk_vdt_cmd_t *d_cmd, int64_t R, in
     set_error("%s: d_nominal_out must not overlap d_cmd", who);
     return RK_ERR_ARG;
   }
+  return RK_OK;
+}
+
+} // namespace rk
+
+using namespace rk;
+
+extern "C" {
+
+int rk_plan_sample_commands(const rk_vdt_params_t *p, const rk_plan_sample_t *s, const rk_vdt_cmd_t *d_nominal, int64_t R, int32_t S,
+                            int32_t n_seg, rk_vdt_cmd_t *d_cmd, void *stream) {
+  return plan_sample("rk_plan_sample_commands", p, s, d_nominal, false, nullptr, R, S, n_seg, d_cmd, stream);
+}
+
+int rk_plan_sample_commands_sigma(const rk_vdt_params_t *p, const rk_plan_sample_t *s, const rk_vdt_cmd_t *d_nominal, const float *d_sigma,
+                                  int64_t R, int32_t S, int32_t n_seg, rk_vdt_cmd_t *d_cmd, void *stream) {
+  return plan_sample("rk_plan_sample_commands_sigma", p, s, d_nominal, true, d_sigma, R, S, n_seg, d_cmd, stream);
+}
+
+int rk_plan_select(const float *d_cost, const rk_vdt_cmd_t *d_cmd, int64_t R, int32_t S, int32_t n_seg, float lambda, int32_t shift,
+                   rk_vdt_cmd_t *d_nominal_out, int32_t *d_best, float *d_best_cost, void *stream) {
+  static const char *who = "rk_plan_select";
+  if(int rc = plan_check_choice(who, R, S, n_seg, shift)) return rc;
+  if(!(lambda >= 0.0f) || isinf(lambda)) {
+    set_error("%s: lambda must be finite and >= 0", who);
+    return RK_ERR_ARG;
+  }
+  if(R == 0) return RK_OK;
+  if(int rc = plan_check_choice_tables(who, d_cost, d_cmd, R, S, n_seg, d_nominal_out)) return rc;
   if(int rc = require_device()) return rc;
   const unsigned warps_per_block = RK_PLAN_BLOCK / 32;
   const unsigned grid            = (unsigned)((R + warps_per_block - 1) / warps_per_block);
   plan_select_kernel<<<grid, RK_PLAN_BLOCK, 0, (cudaStream_t)stream>>>(d_cost, (const uint4 *)d_cmd, R, S, n_seg, lambda, shift,
                                                                         (uint4 *)d_nominal_out, d_best, d_best_cost);
+  RK_CUDA(cudaGetLastError());
+  return RK_OK;
+}
+
+int rk_plan_refit(const float *d_cost, const rk_vdt_cmd_t *d_cmd, const float *d_sigma_in, int64_t R, int32_t S, int32_t n_seg,
+                  const rk_plan_refit_t *rf, int32_t shift, rk_vdt_cmd_t *d_nominal_out, float *d_sigma_out, int32_t *d_best,
+                  float *d_best_cost, void *stream) {
+  static const char *who = "rk_plan_refit";
+  if(int rc = plan_check_choice(who, R, S, n_seg, shift)) return rc;
+  if(!rf) {
+    set_error("%s: NULL refit", who);
+    return RK_ERR_ARG;
+  }
+  if(rf->elite < 1 || rf->elite > S) {
+    set_error("%s: need 1 <= elite <= S (elite = %d, S = %d)", who, rf->elite, S);
+    return RK_ERR_ARG;
+  }
+  if(!(rf->alpha >= 0.0f && rf->alpha <= 1.0f)) {
+    set_error("%s: alpha must be in [0, 1]", who);
+    return RK_ERR_ARG;
+  }
+  for(int k = 0; k < 3; k++)
+    if(!(rf->sigma_min[k] >= 0.0f) || isinf(rf->sigma_min[k])) {
+      set_error("%s: sigma_min[%d] must be finite and >= 0", who, k);
+      return RK_ERR_ARG;
+    }
+  if(R == 0) return RK_OK;
+  if(int rc = plan_check_choice_tables(who, d_cost, d_cmd, R, S, n_seg, d_nominal_out)) return rc;
+  if(int rc = plan_check_table(who, d_sigma_in, "d_sigma_in")) return rc;
+  if(int rc = plan_check_table(who, d_sigma_out, "d_sigma_out")) return rc;
+  const size_t nsig = (size_t)n_seg * R * 16u;
+  if(overlap(d_sigma_out, nsig, d_sigma_in, nsig) && !(shift == 0 && d_sigma_out == d_sigma_in)) {
+    set_error("%s: d_sigma_out must not overlap d_sigma_in, unless shift == 0 and they are the same table", who);
+    return RK_ERR_ARG;
+  }
+  if(int rc = require_device()) return rc;
+  PlanRefitArgs a;
+  a.R = R, a.S = S, a.n_seg = n_seg, a.k = rf->elite, a.shift = shift, a.alpha = rf->alpha;
+  for(int k = 0; k < 3; k++) a.sigma_min[k] = rf->sigma_min[k];
+  const unsigned warps_per_block = RK_PLAN_BLOCK / 32;
+  const unsigned grid            = (unsigned)((R + warps_per_block - 1) / warps_per_block);
+  plan_refit_kernel<<<grid, RK_PLAN_BLOCK, 0, (cudaStream_t)stream>>>(a, d_cost, (const uint4 *)d_cmd, (const float4 *)d_sigma_in,
+                                                                       (uint4 *)d_nominal_out, (float4 *)d_sigma_out, d_best, d_best_cost);
   RK_CUDA(cudaGetLastError());
   return RK_OK;
 }

@@ -528,12 +528,15 @@ def plan_xi_v2(h):
     return np.stack(xi, axis=-1).astype(np.float32)
 
 
-def plan_commands_v2(nominal, S, seed=0x5EED, first=0, sigma=(100.0, 100.0, 1.0), params=None):
+def plan_commands_v2(nominal, S, seed=0x5EED, first=0, sigma=(100.0, 100.0, 1.0), params=None, sigma_table=None):
     """Sampling-planner candidates around a nominal plan (rk_plan_sample_commands): nominal [n_seg, R] rk_vdt_cmd_t records
     -> [n_seg, R*S], candidate j of robot r at column r*S + j.  Candidate 0 is the nominal; candidate j > 0 of segment s adds
     sigma_a * xi_a with xi = plan_xi_v2(h32(seed, 40, first + r, s*S + j)).  Then the vehicle's limiters (params: the
     rk_vdt_params_t, default firmware constants): |(vx, vy)| above limit_speed_mmps is scaled back onto it as
-    (v * L) / |v|, vth is clamped to +-limit_rot_radps; kind = RK_CMD_MOVE.  float32, one rounding per operation."""
+    (v * L) / |v|, vth is clamped to +-limit_rot_radps; kind = RK_CMD_MOVE.  float32, one rounding per operation.
+
+    sigma_table: float32 [n_seg, R, 4] {sx, sy, sth, unused} (rk_plan_sample_commands_sigma): segment s of robot r draws
+    with the scale of cell [s, r] instead of `sigma`."""
     p = params or _cabi.default_params()
     f32 = np.float32
     nominal = np.asarray(nominal)
@@ -544,10 +547,16 @@ def plan_commands_v2(nominal, S, seed=0x5EED, first=0, sigma=(100.0, 100.0, 1.0)
     inst = (np.arange(R, dtype=np.uint64) + np.uint64(first))[None, :, None]
     idx = np.arange(n_seg, dtype=np.uint64)[:, None, None] * np.uint64(S) + np.arange(S, dtype=np.uint64)[None, None, :]
     xi = plan_xi_v2(h32(seed, 40, inst, idx))  # [n_seg, R, S, 3]
+    if sigma_table is None:
+        scale = [f32(x) for x in sigma]
+    else:
+        tab = np.asarray(sigma_table, dtype=np.float32)
+        assert tab.shape == (n_seg, R, 4), "sigma_table: float32 [n_seg, R, 4]"
+        scale = [tab[:, :, a, None] for a in range(3)]
     v = []
     for a, name in enumerate(("vx", "vy", "vth")):
         nom = np.broadcast_to(nominal[name].astype(np.float32)[:, :, None], (n_seg, R, S))
-        noisy = (nom + f32(sigma[a]) * xi[..., a]).astype(np.float32)
+        noisy = (nom + scale[a] * xi[..., a]).astype(np.float32)
         noisy[:, :, 0] = nom[:, :, 0]  # j == 0: the nominal itself
         v.append(noisy)
     vx, vy, vth = v

@@ -10,8 +10,14 @@ for every M and every --check-period P (default seg_len), each alternated with r
 and reports obst_over_plan.  The discs are seeded around the robots' positions, within the candidates' reach, so that
 part of the candidates enter them.
 
+With --cem ITERS:ELITE the run also times the two ends of a cross-entropy round, rk_plan_sample_commands_sigma and
+rk_plan_refit (ELITE elites), each alternated with its counterpart rk_plan_sample_commands / rk_plan_select, and reports
+them against the plan rollout.  Then, from the same robots, it plans --cem-steps closed-loop steps three ways at the same
+rollout budget -- CEM with ITERS rounds of S / ITERS candidates, argmin and MPPI (--lam) over S candidates -- executing
+the first segment of each new plan, and reports the last step's best cost and the final distance to the goal.
+
     python tools/bench_plan.py [--R 4096] [--S 256] [--n-seg 8] [--seg-len 125] [--reps 10] [--out FILE]
-                               [--obstacles 1,8 --check-period 125,25,10]
+                               [--obstacles 1,8 --check-period 125,25,10] [--cem 4:8 --cem-steps 8 --lam 1e-3]
 """
 import argparse
 import json
@@ -53,6 +59,33 @@ def int_list(args):
     return [int(x) for a in args for x in str(a).split(",") if x != ""]
 
 
+def compare_planners(a, src, goal, ref, iters, elite):
+    """--cem-steps closed-loop steps from the robots in src (left untouched) for CEM (iters x S/iters, elite), argmin and
+    MPPI (S candidates): the last step's best cost and the final distance to the goal, median and mean over the robots."""
+    R, S, n_seg, seg_len, dev = a.R, a.S, a.n_seg, a.seg_len, src.state.device
+    out = {}
+    for name, s_step in (("cem", S // iters), ("argmin", S), ("mppi", S)):
+        pl = VehiclePlanner(R, s_step, n_seg, seg_len, dev)
+        vb = VehicleBatch(R, dev)
+        vb.state.copy_(src.state)
+        for step in range(a.cem_steps):
+            if name == "cem":
+                pl.plan_cem(vb, ref, 1.0, 10.0, 1e-9, iters, elite, seed=step)
+            else:
+                pl.plan(vb, ref, 1.0, 10.0, 1e-9, lam=a.lam if name == "mppi" else 0.0, seed=step)
+            vb.rollout(seg_len, sensor_mode=_cabi.RK_SENSOR_PLANT, cmd=pl.first_command(), seg_len=seg_len)
+        torch.cuda.synchronize()
+        aos = layout.soa_to_aos(vb.state.cpu().numpy().view(np.uint32), R, layout.VS_WORDS)
+        pos = aos[:, [layout.VS_POS_X, layout.VS_POS_Y]].view(np.float32).astype(np.float64)
+        d = np.hypot(*(pos - goal.cpu().numpy()).T)
+        bc = pl.best_cost.cpu().numpy().astype(np.float64)
+        out[name] = {"rollouts_per_step": S if name != "cem" else iters * s_step,
+                     "best_cost_median": float(np.median(bc)), "best_cost_mean": float(np.mean(bc)),
+                     "goal_dist_m_median": float(np.median(d)), "goal_dist_m_mean": float(np.mean(d))}
+    out["steps"], out["lam"] = a.cem_steps, a.lam
+    return out
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--R", type=int, default=4096)
@@ -63,7 +96,11 @@ def main():
     ap.add_argument("--out", default=None)
     ap.add_argument("--obstacles", action="append", default=[], help="discs per robot (comma list or repeated; 0: none)")
     ap.add_argument("--check-period", action="append", default=[], help="obstacle check period in ticks (comma list or repeated)")
+    ap.add_argument("--cem", default=None, help="ITERS:ELITE: time the cross-entropy round's sampler and refit, and compare planners")
+    ap.add_argument("--cem-steps", type=int, default=8, help="closed-loop planning steps of the planner comparison")
+    ap.add_argument("--lam", type=float, default=1e-3, help="MPPI temperature of the planner comparison")
     a = ap.parse_args()
+    cem_iters, cem_elite = (int(x) for x in a.cem.split(":")) if a.cem else (0, 0)
     obst_m = [m for m in int_list(a.obstacles) if m > 0]
     obst_p = int_list(a.check_period) or [a.seg_len]
     if not torch.cuda.is_available():
@@ -113,19 +150,33 @@ def main():
     def obst_rollout(m, P):
         pl.rollout(src, ref, 1.0, 10.0, 1e-9, obstacles=discs[m], w_obst=1e3, check_period=P)
 
+    def sample_sigma():
+        pl.sample(nominal=nominal, seed=5, sigma_table=pl.sigma_table)
+
+    def refit():
+        pl.refit(cem_elite, shift=1)
+
     # warm-up: every shape once (the first rollout also runs the fast path's on-device proofs)
     sample(), plan_rollout(), select(), fork(), plain_rollout()
+    if a.cem:
+        sample_sigma(), refit()
     for m in obst_m:
         for P in obst_p:
             obst_rollout(m, P)
     torch.cuda.synchronize()
     src_before = src.state.clone()
     t = {"sample": [], "plan_rollout": [], "select": [], "plain_rollout": []}
+    if a.cem:
+        t.update(sample_sigma=[], refit=[])
     t_obst = {}
     for _ in range(a.reps):
         t["sample"].append(timed(sample))
+        if a.cem:
+            t["sample_sigma"].append(timed(sample_sigma))
         t["plan_rollout"].append(timed(plan_rollout))
         t["select"].append(timed(select))
+        if a.cem:
+            t["refit"].append(timed(refit))
         fork()
         torch.cuda.synchronize()
         t["plain_rollout"].append(timed(plain_rollout))
@@ -162,6 +213,12 @@ def main():
                          "ms_min_obst": round(float(np.min(to)), 4), "ms_max_obst": round(float(np.max(to)), 4),
                          "obst_over_plan": mo / mp, "penetrating_fraction": hit})
         res["obstacles"] = rows
+    if a.cem:
+        res["cem"] = {"iters": cem_iters, "elite": cem_elite,
+                      "sample_sigma_over_sample": med["sample_sigma"] / med["sample"],
+                      "refit_over_select": med["refit"] / med["select"],
+                      "sample_sigma_plus_refit_over_rollout": (med["sample_sigma"] + med["refit"]) / med["plan_rollout"],
+                      "compare": compare_planners(a, src, goal, ref, cem_iters, cem_elite)}
     line = json.dumps(res)
     print(line)
     if a.out:
