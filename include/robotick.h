@@ -744,6 +744,37 @@ int rk_plan_refit(const float *d_cost, const rk_vdt_cmd_t *d_cmd, const float *d
                   int32_t n_seg, const rk_plan_refit_t *rf, int32_t shift, rk_vdt_cmd_t *d_nominal_out,
                   float *d_sigma_out, int32_t *d_best, float *d_best_cost, void *stream);
 
+/* Moving keep-out discs and predicted paths (fleet planning): every robot of a planner keeps clear of the positions its
+ * peers' nominal plans predict, checkpoint by checkpoint.  One fleet step on one stream:
+ *   rk_plan_rollout_moving (S = 1, d_cmd = nominal, m = 0, d_path)  R states + nominal   -> path [n_ck][R]
+ *   rk_plan_peer_discs                                               path + peer indices -> discs [n_ck][M][R]
+ *   rk_plan_sample_commands, rk_plan_rollout_moving (the discs), rk_plan_select as above
+ * Positions are checked at checkpoints only, and the peers replan every step, so this is avoidance by cost, not a
+ * guarantee (INTEGRATION.md §2). */
+
+/* rk_plan_rollout_obstacles with a disc table per checkpoint, and optionally the candidates' paths.  obst is required;
+ * n_ck = n_seg * seg_len / P.  obst->d_obs is float4 [n_ck][m][R]: cell (c*m + k)*R + r is disc k of robot r at
+ * checkpoint c + 1, the state after tick (c + 1)*P - 1.  The checkpoints, the per-disc formula, its float32 order, NaN
+ * discs and w_obst = +inf are those of rk_plan_rollout_obstacles; checkpoint c reads its own table.  So a table repeating
+ * one [m][R] table at every checkpoint gives rk_plan_rollout_obstacles' bits, and m == 0 gives rk_plan_rollout's.
+ * d_path (NULL: not written): float2 [n_ck][R*S], 8-byte aligned; cell c*R*S + i = the position words (x, y) of
+ * candidate i at checkpoint c + 1, bit for bit the words the cost read.  Writing it never changes d_cost.
+ * RK_ERR_ARG: rk_plan_rollout_obstacles' checks, obst NULL, and d_path not 8-byte aligned. */
+int rk_plan_rollout_moving(const rk_vdt_params_t *p, const void *d_src_state, int64_t R, int32_t S,
+                           const rk_vdt_cmd_t *d_cmd, int32_t n_seg, int32_t seg_len,
+                           const rk_plan_cost_t *cost, const rk_plan_obstacles_t *obst,
+                           float *d_path, float *d_cost, void *stream);
+
+/* Peer discs from predicted paths: d_path float2 [n_ck][R] (8-byte aligned), d_peer int32 [m][R], d_obs float4
+ * [n_ck][M][R] (16-byte aligned).  For c < n_ck, k < m, r < R with q = d_peer[k*R + r], cell (c*M + k0 + k)*R + r becomes
+ *   {path[c][q].x, path[c][q].y, radius, 0}   if 0 <= q < R and q != r,
+ *   {0, 0, NaN, 0}                             otherwise (a disc that contributes nothing; nothing out of range is read).
+ * Cells of slots outside [k0, k0 + m) are not touched, so static discs or several peer sets can share one table.
+ * RK_ERR_ARG: R < 0, n_ck < 0, m < 0, k0 < 0, k0 + m > M, radius NaN, inf or < 0, a NULL or misaligned table (when
+ * R, n_ck and m are > 0), d_obs overlapping d_path.  R, n_ck or m == 0 is a no-op. */
+int rk_plan_peer_discs(const float *d_path, int64_t R, int32_t n_ck, const int32_t *d_peer, int32_t m, float radius,
+                       float *d_obs, int32_t M, int32_t k0, void *stream);
+
 /* =====================================================================================
  * RobotManager guard (SURVEY 8f-2): the vehicle-management block of RMT's routine_ros()
  * (src/RobotManager/RM_task_main.cpp:484-767), one call = K manager cycles of n robots.  Per

@@ -238,6 +238,9 @@ def _proto(lib):
                                     vp]
     lib.rk_plan_rollout_obstacles.argtypes = [C.POINTER(VdtParams), vp, C.c_int64, C.c_int32, vp, C.c_int32, C.c_int32, C.POINTER(PlanCost),
                                               C.POINTER(PlanObstacles), vp, vp]
+    lib.rk_plan_rollout_moving.argtypes = [C.POINTER(VdtParams), vp, C.c_int64, C.c_int32, vp, C.c_int32, C.c_int32, C.POINTER(PlanCost),
+                                           C.POINTER(PlanObstacles), vp, vp, vp]
+    lib.rk_plan_peer_discs.argtypes = [vp, C.c_int64, C.c_int32, vp, C.c_int32, C.c_float, vp, C.c_int32, C.c_int32, vp]
     lib.rk_plan_select.argtypes = [vp, vp, C.c_int64, C.c_int32, C.c_int32, C.c_float, C.c_int32, vp, vp, vp, vp]
     lib.rk_plan_sample_commands_sigma.argtypes = [C.POINTER(VdtParams), C.POINTER(PlanSample), vp, vp, C.c_int64, C.c_int32, C.c_int32, vp,
                                                   vp]

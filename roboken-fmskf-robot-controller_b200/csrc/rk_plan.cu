@@ -238,6 +238,28 @@ plan_refit_kernel(const PlanRefitArgs a, const float *__restrict__ cost, const u
   }
 }
 
+// rk_plan_peer_discs: one thread per (checkpoint, robot), x over the robots (coalesced stores), y striding the
+// checkpoints.  The peer index is checked before the path is read, so nothing out of range is read.
+__global__ void __launch_bounds__(RK_PLAN_BLOCK)
+plan_peer_discs_kernel(const float2 *__restrict__ path, int64_t R, int n_ck, const int32_t *__restrict__ peer, int m, float radius,
+                       float4 *__restrict__ obs, int M, int k0) {
+  const int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if(r >= R) return;
+  for(int c = blockIdx.y; c < n_ck; c += gridDim.y) {
+    const float2 *pc = path + (int64_t)c * R;
+    float4       *oc = obs + ((int64_t)c * M + k0) * R + r;
+    for(int k = 0; k < m; k++) {
+      const int32_t q = __ldg(peer + (int64_t)k * R + r);
+      float4        d = make_float4(0.0f, 0.0f, __int_as_float(0x7FC00000), 0.0f); // contributes nothing
+      if(q >= 0 && q < R && q != r) {
+        const float2 x = __ldg(pc + q);
+        d              = make_float4(x.x, x.y, radius, 0.0f);
+      }
+      oc[(int64_t)k * R] = d;
+    }
+  }
+}
+
 static bool overlap(const void *a, size_t na, const void *b, size_t nb) {
   const uintptr_t x = (uintptr_t)a, y = (uintptr_t)b;
   return x < y + nb && y < x + na;
@@ -397,6 +419,39 @@ int rk_plan_refit(const float *d_cost, const rk_vdt_cmd_t *d_cmd, const float *d
   const unsigned grid            = (unsigned)((R + warps_per_block - 1) / warps_per_block);
   plan_refit_kernel<<<grid, RK_PLAN_BLOCK, 0, (cudaStream_t)stream>>>(a, d_cost, (const uint4 *)d_cmd, (const float4 *)d_sigma_in,
                                                                        (uint4 *)d_nominal_out, (float4 *)d_sigma_out, d_best, d_best_cost);
+  RK_CUDA(cudaGetLastError());
+  return RK_OK;
+}
+
+int rk_plan_peer_discs(const float *d_path, int64_t R, int32_t n_ck, const int32_t *d_peer, int32_t m, float radius, float *d_obs, int32_t M,
+                       int32_t k0, void *stream) {
+  static const char *who = "rk_plan_peer_discs";
+  if(R < 0 || n_ck < 0 || m < 0) {
+    set_error("%s: need R, n_ck and m >= 0 (R = %lld, n_ck = %d, m = %d)", who, (long long)R, n_ck, m);
+    return RK_ERR_ARG;
+  }
+  if(k0 < 0 || (int64_t)k0 + m > M) {
+    set_error("%s: need 0 <= k0 and k0 + m <= M (k0 = %d, m = %d, M = %d)", who, k0, m, M);
+    return RK_ERR_ARG;
+  }
+  if(!(radius >= 0.0f) || isinf(radius)) {
+    set_error("%s: radius must be finite and >= 0", who);
+    return RK_ERR_ARG;
+  }
+  if(R == 0 || n_ck == 0 || m == 0) return RK_OK;
+  if(!d_path || ((uintptr_t)d_path & 7u) || !d_peer || ((uintptr_t)d_peer & 3u)) {
+    set_error("%s: d_path (8-byte aligned float2) and d_peer (int32) must be non-NULL device pointers", who);
+    return RK_ERR_ARG;
+  }
+  if(int rc = plan_check_table(who, d_obs, "d_obs")) return rc;
+  if(overlap(d_obs, (size_t)n_ck * M * R * 16u, d_path, (size_t)n_ck * R * 8u)) {
+    set_error("%s: d_obs must not overlap d_path", who);
+    return RK_ERR_ARG;
+  }
+  if(int rc = require_device()) return rc;
+  const dim3 grid((unsigned)((R + RK_PLAN_BLOCK - 1) / RK_PLAN_BLOCK), (unsigned)min(n_ck, 65535));
+  plan_peer_discs_kernel<<<grid, RK_PLAN_BLOCK, 0, (cudaStream_t)stream>>>((const float2 *)d_path, R, n_ck, d_peer, m, radius,
+                                                                            (float4 *)d_obs, M, k0);
   RK_CUDA(cudaGetLastError());
   return RK_OK;
 }

@@ -98,8 +98,15 @@ struct PlanObstArgs : PlanArgs {
   int32_t       m, P;
   float         w_obst;
 };
-template <bool OBST>
-using PlanArgsOf = std::conditional_t<OBST, PlanObstArgs, PlanArgs>;
+// rk_plan_rollout_moving: a disc table per checkpoint, and the candidates' positions at the checkpoints if path != NULL
+struct PlanMovingArgs : PlanObstArgs {
+  float2 *path; // [n_ck][R * S], metres
+};
+// OBST: 0 no discs (PlanArgs), kObstStatic rk_plan_rollout_obstacles (PlanObstArgs), kObstMoving rk_plan_rollout_moving
+// (PlanMovingArgs)
+constexpr int kObstStatic = 1, kObstMoving = 2;
+template <int OBST>
+using PlanArgsOf = std::conditional_t<OBST == kObstMoving, PlanMovingArgs, std::conditional_t<OBST == kObstStatic, PlanObstArgs, PlanArgs>>;
 // O after the checkpoint at position (x, y) (rk_plan_obstacles_t).  The S candidates of robot r read the same m cells
 // (one broadcast per warp); the discs are not staged in registers, the packed kernel has none to spare.  r fits 32 bits
 // (2^32 robots would take 1.9 TB of state), which keeps one register fewer live across the hot loop.
@@ -111,6 +118,23 @@ RK_DEV float plan_obst_cost(float O, float x, float y, const PlanObstArgs &pl, u
     const float  dx  = fsub(x, c.x), dy = fsub(y, c.y);
     const float  pen = fsub(fmul(c.z, c.z), fadd(fmul(dx, dx), fmul(dy, dy)));
     if(pen > 0.0f) O = fadd(O, fmul(pl.w_obst, pen));
+  }
+  return O;
+}
+// O after checkpoint c + 1 (0-based c) of rk_plan_rollout_moving at position (x, y): first the path cell of candidate i
+// (n = R * S) if asked, then plan_obst_cost on checkpoint c's table.  Only the table differs from rk_plan_obstacles_t.
+// Unlike the static table, each checkpoint's cells are new to L1, and the serial disc loop would wait on m misses in a
+// row; so every checkpoint but the last (at t = K, `last`) prefetches the next table's m cells into L1, P ticks ahead
+// and without holding a register.
+RK_DEV float plan_moving_cost(float O, float x, float y, const PlanMovingArgs &pl, uint32_t r, int64_t n, int64_t i, int c, bool last) {
+  if(pl.path != nullptr) __stcs(pl.path + (int64_t)c * n + i, make_float2(x, y));
+  PlanObstArgs q = pl;
+  q.obs += (int64_t)c * pl.m * pl.R;
+  O = plan_obst_cost(O, x, y, q, r);
+  if(!last) {
+    const float4 *nx = q.obs + (int64_t)pl.m * pl.R + r;
+#pragma unroll 1
+    for(int k = 0; k < pl.m; k++, nx += pl.R) asm volatile("prefetch.global.L1 [%0];" ::"l"(nx));
   }
   return O;
 }
@@ -130,10 +154,12 @@ RK_DEV int64_t rollout_load(const uint4 *state, int64_t n, int64_t i, const Plan
 // The end of a launch.  PLAN: the candidate's cost J (+ O after the last obstacle checkpoint, t = K: seg_len % P == 0);
 // the end state is discarded, 448 B per candidate not written.  Otherwise the end state, and its squared distance to the
 // goal if asked.
-template <bool PLAN, bool OBST>
+template <bool PLAN, int OBST>
 RK_DEV void rollout_store(uint4 *state, int64_t n, int64_t i, const rk_vdt_rollout_t &a, const PlanArgsOf<OBST> &pl, const Veh &v,
                           float J, float O, int64_t r) {
-  if constexpr(OBST) {
+  if constexpr(OBST == kObstMoving) {
+    pl.cost[i] = fadd(plan_stage_cost(J, v, pl, a.n_seg - 1, a.n_seg, r), plan_moving_cost(O, v.pos[0], v.pos[1], pl, r, n, i, a.steps / pl.P - 1, true));
+  } else if constexpr(OBST) {
     pl.cost[i] = fadd(plan_stage_cost(J, v, pl, a.n_seg - 1, a.n_seg, r), plan_obst_cost(O, v.pos[0], v.pos[1], pl, r));
   } else if constexpr(PLAN) {
     pl.cost[i] = plan_stage_cost(J, v, pl, a.n_seg - 1, a.n_seg, r);
@@ -159,7 +185,7 @@ RK_DEV void trace_row(uint32_t *d_trace, int64_t n, int64_t i, int t, float px, 
   tr[13 * n] = cnt, tr[14 * n] = c610_tx_word(c0, c1), tr[15 * n] = c610_tx_word(c2, c3);
 }
 
-template <int MODE, bool TRACE, bool PLAN = false, bool OBST = false>
+template <int MODE, bool TRACE, bool PLAN = false, int OBST = 0>
 __global__ void __launch_bounds__(kRolloutThreads)
 vdt_rollout_kernel(const rk_vdt_params_t p, uint4 *__restrict__ state, int64_t n, const rk_vdt_rollout_t a, const PlanArgsOf<OBST> pl) {
   static_assert(PLAN || !OBST, "obstacles are a plan-rollout term");
@@ -195,7 +221,8 @@ vdt_rollout_kernel(const rk_vdt_params_t p, uint4 *__restrict__ state, int64_t n
       if(t == sc.next_cmd && sc.seg > 0) J = plan_stage_cost(J, v, pl, sc.seg - 1, a.n_seg, r);
     if constexpr(OBST)
       if(t == next_chk) { // the state after tick t - 1
-        O = plan_obst_cost(O, v.pos[0], v.pos[1], pl, r);
+        if constexpr(OBST == kObstMoving) O = plan_moving_cost(O, v.pos[0], v.pos[1], pl, r, n, i, next_chk / pl.P - 1, false);
+        else O = plan_obst_cost(O, v.pos[0], v.pos[1], pl, r);
         next_chk += pl.P;
       }
     sched_events(v, p, a, n, i, t, sc);
@@ -272,10 +299,13 @@ RK_DEV void yaw_feed_take(YawFeed &y, const rk_vdt_rollout_t &a, int64_t n, int6
 // The cold branch of vdt_rollout_fast_kernel at t == yf.next.  OBST: the obstacle checkpoint at (x, y), the state after
 // tick t - 1; returns O with it added.  Otherwise the yaw boundary into (pth, cth, sth); returns O as it was.  (O by
 // value: taken by reference, it changes ptxas' register assignment in the OBST kernels.)
-template <bool OBST>
+template <int OBST>
 RK_DEV float yaw_boundary(YawFeed &yf, float O, float x, float y, const PlanArgsOf<OBST> &pl, int64_t r, const rk_vdt_rollout_t &a,
                           int64_t n, int64_t i, const float *s_tab, float &pth, float &cth, float &sth) {
-  if constexpr(OBST) {
+  if constexpr(OBST == kObstMoving) { // checkpoint yf.next / P, from the tick itself: no loop-carried checkpoint index
+    O = plan_moving_cost(O, x, y, pl, r, n, i, yf.next / pl.P - 1, false);
+    yf.next += pl.P;
+  } else if constexpr(OBST) {
     O = plan_obst_cost(O, x, y, pl, r);
     yf.next += pl.P;
   } else {
@@ -286,10 +316,10 @@ RK_DEV float yaw_boundary(YawFeed &yf, float O, float x, float y, const PlanArgs
 // FLAGS: bit 0 FFSAT (ff_limit == 1: FMUL.SAT form of the feed-forward clamp), bit 1 KD0 (kd == 0, packed tick only)
 // PLAN: rk_plan_rollout (PlanArgs); segment ends are command ticks, so they are chunk boundaries and the stage cost is
 // formed outside the chunk loop.
-// OBST (with PLAN): rk_plan_rollout_obstacles (PlanObstArgs).  Plan rollouts have no yaw stream, so the yaw boundary's
-// cold branch inside the chunk loop takes the obstacle checkpoint instead (every P ticks, the same tick in every lane):
-// no new chunk boundary and no new loop-carried register besides O.
-template <bool TRACE, int OCC, int FLAGS, bool PACKED, bool RESET = false, bool PLAN = false, bool OBST = false>
+// OBST (with PLAN): rk_plan_rollout_obstacles (kObstStatic) or rk_plan_rollout_moving (kObstMoving).  Plan rollouts have
+// no yaw stream, so the yaw boundary's cold branch inside the chunk loop takes the obstacle checkpoint instead (every P
+// ticks, the same tick in every lane): no new chunk boundary and no new loop-carried register besides O.
+template <bool TRACE, int OCC, int FLAGS, bool PACKED, bool RESET = false, bool PLAN = false, int OBST = 0>
 __global__ void __launch_bounds__(kFastThreads, OCC * 128 / kFastThreads)
 vdt_rollout_fast_kernel(const rk_vdt_params_t p, uint4 *__restrict__ state, int64_t n, const rk_vdt_rollout_t a, const CmdRcp rcp,
                         const PlanArgsOf<OBST> pl) {
@@ -497,7 +527,7 @@ vdt_rollout_stream_fast_kernel(const rk_vdt_params_t p, uint4 *__restrict__ stat
       t++;
     }
   }
-  rollout_store<false, false>(state, n, i, a, PlanArgs{}, v, 0.0f, 0.0f, 0);
+  rollout_store<false, 0>(state, n, i, a, PlanArgs{}, v, 0.0f, 0.0f, 0);
 }
 
 // ---- small batched setters ------------------------------------------------------------
@@ -807,7 +837,7 @@ int rk_vdt_rollout(const rk_vdt_params_t *p, void *d_state, int64_t n, const rk_
 } // extern "C"
 namespace rk {
 // rk_plan_rollout's kernel choice: the RK_SENSOR_PLANT dispatch of rk_vdt_rollout without trace and reset
-template <bool OBST>
+template <int OBST>
 static void launch_plan(const rk_vdt_params_t &p, const void *d_src, int64_t n, const rk_vdt_rollout_t &a, const PlanArgsOf<OBST> &pl,
                         cudaStream_t st) {
   uint4 *src = (uint4 *)d_src; // read only under PLAN
@@ -821,12 +851,21 @@ static void launch_plan(const rk_vdt_params_t &p, const void *d_src, int64_t n, 
     vdt_rollout_kernel<RK_SENSOR_PLANT, false, true, OBST><<<grid, kRolloutThreads, 0, st>>>(p, src, n, a, pl);
   }
 }
-// rk_plan_rollout (ob == NULL) and rk_plan_rollout_obstacles: the same checks, and without discs the same kernels
+// rk_plan_rollout (ob == NULL), rk_plan_rollout_obstacles and rk_plan_rollout_moving (moving): the same checks, and
+// without discs or path the same kernels
 static int plan_rollout(const char *who, const rk_vdt_params_t *p, const void *d_src_state, int64_t R, int32_t S, const rk_vdt_cmd_t *d_cmd,
-                        int32_t n_seg, int32_t seg_len, const rk_plan_cost_t *cost, const rk_plan_obstacles_t *ob, float *d_cost,
-                        void *stream) {
+                        int32_t n_seg, int32_t seg_len, const rk_plan_cost_t *cost, const rk_plan_obstacles_t *ob, bool moving,
+                        float *d_path, float *d_cost, void *stream) {
   if(!p || !cost) {
     set_error("%s: NULL params/cost", who);
+    return RK_ERR_ARG;
+  }
+  if(moving && !ob) {
+    set_error("%s: obst is required", who);
+    return RK_ERR_ARG;
+  }
+  if((uintptr_t)d_path & 7u) {
+    set_error("%s: d_path must be 8-byte aligned", who);
     return RK_ERR_ARG;
   }
   if(R < 0 || S < 1) {
@@ -872,16 +911,18 @@ static int plan_rollout(const char *who, const rk_vdt_params_t *p, const void *d
   memset(&a, 0, sizeof(a));
   a.steps = n_seg * seg_len, a.sensor_mode = RK_SENSOR_PLANT;
   a.d_cmd = d_cmd, a.n_seg = n_seg, a.seg_len = seg_len;
-  PlanObstArgs pl;
+  PlanMovingArgs pl;
   pl.R = R, pl.S = S, pl.ref = reinterpret_cast<const float2 *>(cost->d_ref);
   pl.w_pos = cost->w_pos, pl.w_goal = cost->w_goal, pl.w_cur = cost->w_cur, pl.cost = d_cost;
   const int64_t n  = R * (int64_t)S;
   cudaStream_t  st = (cudaStream_t)stream;
-  if(obst) {
+  if(obst || d_path) {
     pl.obs = reinterpret_cast<const float4 *>(ob->d_obs), pl.m = ob->m, pl.P = ob->check_period, pl.w_obst = ob->w_obst;
-    launch_plan<true>(*p, d_src_state, n, a, pl, st);
+    pl.path = reinterpret_cast<float2 *>(d_path);
+    if(moving) launch_plan<kObstMoving>(*p, d_src_state, n, a, pl, st);
+    else launch_plan<kObstStatic>(*p, d_src_state, n, a, static_cast<const PlanObstArgs &>(pl), st);
   } else {
-    launch_plan<false>(*p, d_src_state, n, a, static_cast<const PlanArgs &>(pl), st);
+    launch_plan<0>(*p, d_src_state, n, a, static_cast<const PlanArgs &>(pl), st);
   }
   RK_CUDA(cudaGetLastError());
   return RK_OK;
@@ -891,13 +932,19 @@ extern "C" {
 
 int rk_plan_rollout(const rk_vdt_params_t *p, const void *d_src_state, int64_t R, int32_t S, const rk_vdt_cmd_t *d_cmd, int32_t n_seg,
                     int32_t seg_len, const rk_plan_cost_t *cost, float *d_cost, void *stream) {
-  return plan_rollout("rk_plan_rollout", p, d_src_state, R, S, d_cmd, n_seg, seg_len, cost, nullptr, d_cost, stream);
+  return plan_rollout("rk_plan_rollout", p, d_src_state, R, S, d_cmd, n_seg, seg_len, cost, nullptr, false, nullptr, d_cost, stream);
 }
 
 int rk_plan_rollout_obstacles(const rk_vdt_params_t *p, const void *d_src_state, int64_t R, int32_t S, const rk_vdt_cmd_t *d_cmd,
                               int32_t n_seg, int32_t seg_len, const rk_plan_cost_t *cost, const rk_plan_obstacles_t *obst, float *d_cost,
                               void *stream) {
-  return plan_rollout("rk_plan_rollout_obstacles", p, d_src_state, R, S, d_cmd, n_seg, seg_len, cost, obst, d_cost, stream);
+  return plan_rollout("rk_plan_rollout_obstacles", p, d_src_state, R, S, d_cmd, n_seg, seg_len, cost, obst, false, nullptr, d_cost, stream);
+}
+
+int rk_plan_rollout_moving(const rk_vdt_params_t *p, const void *d_src_state, int64_t R, int32_t S, const rk_vdt_cmd_t *d_cmd, int32_t n_seg,
+                           int32_t seg_len, const rk_plan_cost_t *cost, const rk_plan_obstacles_t *obst, float *d_path, float *d_cost,
+                           void *stream) {
+  return plan_rollout("rk_plan_rollout_moving", p, d_src_state, R, S, d_cmd, n_seg, seg_len, cost, obst, true, d_path, d_cost, stream);
 }
 
 int rk_vdt_set_power(void *d_state, int64_t n, const uint8_t *d_on, void *stream) {

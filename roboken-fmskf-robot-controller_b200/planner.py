@@ -4,7 +4,8 @@ One planning step for R robots with S candidates each: sample candidate command 
 every candidate out from its robot's current state and rank it by a stage cost, then pick (argmin) or blend (MPPI) the
 candidates into the next nominal plan.  Candidate j of robot r is column r*S + j of every table.  The cross-entropy
 method (plan_cem) runs several sample -> rollout -> refit rounds per step, refitting a per-robot, per-segment mean and
-sigma to each round's elite candidates.
+sigma to each round's elite candidates.  For fleets, predict() gives where each robot's nominal plan takes it and
+peer_discs() turns those paths into moving keep-out discs for the robot's peers (fleet_peers builds the usual grouping).
 """
 import ctypes as C
 
@@ -40,6 +41,8 @@ class VehiclePlanner:
             self._sigma_cell = torch.tensor(self.sigma + (0.0,), dtype=torch.float32, **kw)
             self.sigma_table = self._sigma_cell.expand(self.n_seg, self.R, 4).contiguous()
             self._sigma_next = torch.empty_like(self.sigma_table)  # the refit's output when it shifts the plan
+            self._pred_cost = torch.zeros(self.R, dtype=torch.float32, **kw)  # predict(): the S = 1 rollout's unused cost
+            self._pred_ref = torch.zeros((self.n_seg, self.R, 2), dtype=torch.float32, **kw)
         self._keep = None
 
     def _stream(self):
@@ -67,32 +70,91 @@ class VehiclePlanner:
             _cabi.check(self.lib.rk_plan_sample_commands_sigma(C.byref(self.params), C.byref(s), nom, sig, *tail))
         return self.candidates
 
-    def rollout(self, src, ref, w_pos, w_goal, w_cur, obstacles=None, w_obst=0.0, check_period=None):
+    def n_ck(self, check_period):
+        """Checkpoints of a plan rollout every check_period ticks: n_seg * seg_len / check_period."""
+        P = int(check_period)
+        assert P >= 1 and self.seg_len % P == 0, "check_period must divide seg_len"
+        return self.n_seg * self.seg_len // P
+
+    def rollout(self, src, ref, w_pos, w_goal, w_cur, obstacles=None, w_obst=0.0, check_period=None, path=None):
         """rk_plan_rollout: every candidate from its robot's state in `src` (a VehicleBatch of R robots, left untouched),
         ranked against ref (float32 [n_seg, R, 2], metres: where each robot should be when each segment ends).
 
         obstacles: keep-out discs, float32 [m, R, 4] = {cx, cy, radius, unused} in metres per robot (one world shared by
         all robots: t.expand(m, R, 4).contiguous()).  Then rk_plan_rollout_obstacles adds w_obst * (radius^2 - d^2) for
         every disc a candidate is inside of, every check_period ticks (default seg_len; it must divide seg_len);
-        w_obst = inf makes any penetrating candidate cost +inf."""
+        w_obst = inf makes any penetrating candidate cost +inf.  A 4-D table float32 [n_ck, m, R, 4] (n_ck =
+        self.n_ck(check_period)) gives each checkpoint its own discs (rk_plan_rollout_moving): moving obstacles, or the
+        peers' predicted paths (peer_discs).
+
+        path: float32 [n_ck, R*S, 2], receives every candidate's position at every checkpoint (rk_plan_rollout_moving; with
+        a 4-D table or no obstacles).  It never changes the cost."""
         assert src.n == self.R, "the source batch must hold the planner's R robots"
         assert ref.is_cuda and ref.is_contiguous() and ref.dtype == torch.float32 and tuple(ref.shape) == (self.n_seg, self.R, 2)
         c = _cabi.PlanCost()
         c.d_ref, c.w_pos, c.w_goal, c.w_cur = ref.data_ptr(), float(w_pos), float(w_goal), float(w_cur)
         args = (C.byref(self.params), src.state.data_ptr(), self.R, self.S, self.candidates.data_ptr(), self.n_seg, self.seg_len, C.byref(c))
-        if obstacles is None:
+        if obstacles is None and path is None:
             self._keep = ref
             _cabi.check(self.lib.rk_plan_rollout(*args, self.cost.data_ptr(), self._stream()))
             return self.cost
-        assert (obstacles.is_cuda and obstacles.is_contiguous() and obstacles.dtype == torch.float32 and obstacles.dim() == 3
-                and tuple(obstacles.shape[1:]) == (self.R, 4)), "obstacles: float32 [m, R, 4] contiguous device tensor"
+        P = self.seg_len if check_period is None else int(check_period)
         o = _cabi.PlanObstacles()
-        o.d_obs, o.m = obstacles.data_ptr(), obstacles.shape[0]
-        o.check_period = self.seg_len if check_period is None else int(check_period)
-        o.w_obst = float(w_obst)
-        self._keep = (ref, obstacles)
-        _cabi.check(self.lib.rk_plan_rollout_obstacles(*args, C.byref(o), self.cost.data_ptr(), self._stream()))
+        o.check_period, o.w_obst = P, float(w_obst)
+        if obstacles is not None:
+            assert (obstacles.is_cuda and obstacles.is_contiguous() and obstacles.dtype == torch.float32 and obstacles.dim() in (3, 4)
+                    and tuple(obstacles.shape[-2:]) == (self.R, 4)), "obstacles: float32 [m, R, 4] or [n_ck, m, R, 4] contiguous device tensor"
+            o.d_obs, o.m = obstacles.data_ptr(), obstacles.shape[-3]
+        self._keep = (ref, obstacles, path)
+        if obstacles is not None and obstacles.dim() == 3:
+            assert path is None, "path: with a 4-D obstacles table or none"
+            _cabi.check(self.lib.rk_plan_rollout_obstacles(*args, C.byref(o), self.cost.data_ptr(), self._stream()))
+            return self.cost
+        n_ck = self.n_ck(P)
+        assert obstacles is None or obstacles.shape[0] == n_ck, f"obstacles: {n_ck} checkpoint tables of [m, R, 4]"
+        if path is not None:
+            assert (path.is_cuda and path.is_contiguous() and path.dtype == torch.float32
+                    and tuple(path.shape) == (n_ck, self.R * self.S, 2)), f"path: float32 [{n_ck}, {self.R * self.S}, 2] device tensor"
+        _cabi.check(self.lib.rk_plan_rollout_moving(*args, C.byref(o), None if path is None else path.data_ptr(), self.cost.data_ptr(),
+                                                    self._stream()))
         return self.cost
+
+    def predict(self, src, check_period):
+        """Where each robot's nominal plan takes it from its state in `src`: float32 [n_ck, R, 2], metres, the position at
+        every checkpoint (ticks check_period - 1, 2*check_period - 1, ...).  rk_plan_rollout_moving with S = 1, the nominal
+        as the candidates, no discs and a path."""
+        assert src.n == self.R, "the source batch must hold the planner's R robots"
+        n_ck = self.n_ck(check_period)
+        path = torch.empty((n_ck, self.R, 2), dtype=torch.float32, device=self.device)
+        c = _cabi.PlanCost()
+        c.d_ref = self._pred_ref.data_ptr()
+        o = _cabi.PlanObstacles()
+        o.check_period = int(check_period)
+        _cabi.check(self.lib.rk_plan_rollout_moving(C.byref(self.params), src.state.data_ptr(), self.R, 1, self.nominal.data_ptr(), self.n_seg,
+                                                    self.seg_len, C.byref(c), C.byref(o), path.data_ptr(), self._pred_cost.data_ptr(),
+                                                    self._stream()))
+        return path
+
+    def peer_discs(self, path, peers, radius, out=None, k0=0):
+        """rk_plan_peer_discs: for every checkpoint, disc k0 + k of robot r is centred where robot peers[k, r] is predicted
+        to be, with `radius` (metres: the sum of the two bodies' radii and a margin); a peer index outside [0, R) or equal
+        to r gives a disc that contributes nothing.  path: float32 [n_ck, R, 2] (predict); peers: int32 [m, R].
+        out: float32 [n_ck, M, R, 4] whose slots k0 .. k0+m-1 are written and the others left as they are (default: a new
+        [n_ck, m, R, 4] table, k0 = 0).  Returns the table, ready for rollout / plan(obstacles=...)."""
+        n_ck = path.shape[0]
+        assert (path.is_cuda and path.is_contiguous() and path.dtype == torch.float32
+                and tuple(path.shape) == (n_ck, self.R, 2)), "path: float32 [n_ck, R, 2] device tensor"
+        assert (peers.is_cuda and peers.is_contiguous() and peers.dtype == torch.int32 and peers.dim() == 2
+                and peers.shape[1] == self.R), "peers: int32 [m, R] device tensor"
+        m = peers.shape[0]
+        if out is None:
+            assert k0 == 0, "k0 > 0 needs out"
+            out = torch.empty((n_ck, m, self.R, 4), dtype=torch.float32, device=self.device)
+        assert (out.is_cuda and out.is_contiguous() and out.dtype == torch.float32 and out.dim() == 4
+                and out.shape[0] == n_ck and tuple(out.shape[2:]) == (self.R, 4)), "out: float32 [n_ck, M, R, 4] device tensor"
+        _cabi.check(self.lib.rk_plan_peer_discs(path.data_ptr(), self.R, n_ck, peers.data_ptr(), m, float(radius), out.data_ptr(), out.shape[1],
+                                                int(k0), self._stream()))
+        return out
 
     def select(self, lam, shift=1):
         """rk_plan_select into the planner's nominal: lam == 0 takes the best candidate, lam > 0 the MPPI-weighted mean;
@@ -118,7 +180,8 @@ class VehiclePlanner:
         return self.nominal
 
     def plan(self, src, ref, w_pos, w_goal, w_cur, lam=0.0, shift=1, seed=None, obstacles=None, w_obst=0.0, check_period=None):
-        """One planning step (sample, rollout, select) on the current torch stream; returns the new nominal."""
+        """One planning step (sample, rollout, select) on the current torch stream; returns the new nominal.  obstacles
+        as in rollout (3-D static or 4-D per-checkpoint discs)."""
         self.sample(seed=seed)
         self.rollout(src, ref, w_pos, w_goal, w_cur, obstacles=obstacles, w_obst=w_obst, check_period=check_period)
         return self.select(lam, shift)
@@ -146,3 +209,15 @@ class VehiclePlanner:
         """The command the robots execute next: a [1, R, 4] view of the nominal, ready for
         VehicleBatch.rollout(seg_len, cmd=planner.first_command(), seg_len=seg_len)."""
         return self.nominal[:1]
+
+
+def fleet_peers(R, G, device="cuda:0"):
+    """int32 [G-1, R] peer table of fleets of G robots: robot r belongs to group r // G, and its peers are the other G-1
+    robots of the group in ascending order (-1 where a short last group has fewer; such a disc contributes nothing)."""
+    R, G = int(R), int(G)
+    assert R >= 0 and G >= 1, "R >= 0 and G >= 1"
+    r = torch.arange(R, dtype=torch.int64)
+    j = torch.arange(G - 1, dtype=torch.int64)[:, None]  # peer slot k
+    rank = r % G
+    q = (r - rank)[None, :] + j + (j >= rank[None, :]).to(torch.int64)  # skip the robot itself
+    return torch.where(q < R, q, -1).to(torch.int32).contiguous().to(device)

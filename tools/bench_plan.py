@@ -16,8 +16,20 @@ them against the plan rollout.  Then, from the same robots, it plans --cem-steps
 rollout budget -- CEM with ITERS rounds of S / ITERS candidates, argmin and MPPI (--lam) over S candidates -- executing
 the first segment of each new plan, and reports the last step's best cost and the final distance to the goal.
 
+With --moving M:P (a comma list or repeated) the run also times, for every pair, rk_plan_rollout_moving with a table of
+M discs per robot that differs at every checkpoint, alternated with rk_plan_rollout_obstacles at the same M and P and with
+rk_plan_rollout_moving writing every candidate's path; then VehiclePlanner.predict (S = 1 over the R robots) and
+rk_plan_peer_discs of fleets of --fleet G robots (default 8).  It reports moving_over_static and path_over_moving.
+
+With --fleet G the run also plays the circle swap at size: R / G groups of G robots on a --fleet-circle (m) circle, each
+heading for the antipodal point, with and without peer discs (radius 2 * --fleet-body + --fleet-margin, weight
+--fleet-w, checked every --fleet-period ticks), under argmin (S candidates) and CEM (--cem ITERS:ELITE, default 4:8, at
+the same rollout budget), for --fleet-steps steps.  It reports the share of groups in which two robots came closer than
+2 * body radius, the median / minimum over groups of the least pairwise distance, and the median distance to the goal.
+
     python tools/bench_plan.py [--R 4096] [--S 256] [--n-seg 8] [--seg-len 125] [--reps 10] [--out FILE]
                                [--obstacles 1,8 --check-period 125,25,10] [--cem 4:8 --cem-steps 8 --lam 1e-3]
+                               [--moving 1:125,8:25] [--fleet 8 --fleet-steps 60]
 """
 import argparse
 import json
@@ -33,13 +45,13 @@ import torch  # noqa: E402
 
 import roboken_fmskf_robot_controller_b200 as rk  # noqa: E402
 from roboken_fmskf_robot_controller_b200 import _cabi, layout, streams  # noqa: E402
-from roboken_fmskf_robot_controller_b200.planner import VehiclePlanner  # noqa: E402
+from roboken_fmskf_robot_controller_b200.planner import VehiclePlanner, fleet_peers  # noqa: E402
 from roboken_fmskf_robot_controller_b200.vehicle import VehicleBatch  # noqa: E402
 
 
-def power_limit():
+def power_limit(query="power.limit"):
     try:
-        out = subprocess.run(["nvidia-smi", "--query-gpu=power.limit", "--format=csv,noheader", "-i", str(torch.cuda.current_device())],
+        out = subprocess.run(["nvidia-smi", f"--query-gpu={query}", "--format=csv,noheader", "-i", str(torch.cuda.current_device())],
                              capture_output=True, text=True, timeout=30).stdout.strip()
         return out or "unknown"
     except Exception:
@@ -86,6 +98,62 @@ def compare_planners(a, src, goal, ref, iters, elite):
     return out
 
 
+def circle_swap(R, G, circle, dev):
+    """Start states and goals float32 [R, 2] of the circle swap: group g = r // G on a circle of radius `circle` around its
+    own centre (a grid 3 circles apart), robot r at angle 2 pi (r % G) / G + 0.3 g, the goal at the antipodal point."""
+    g = np.arange(R) // G
+    side = int(np.ceil(np.sqrt(R // G + 1)))
+    centre = 3.0 * circle * np.stack([g % side, g // side], axis=1).astype(np.float64)
+    ang = 2.0 * np.pi * (np.arange(R) % G) / G + 0.3 * g
+    u = np.stack([np.cos(ang), np.sin(ang)], axis=1)
+    start, goal = (centre + circle * u).astype(np.float32), (centre - circle * u).astype(np.float32)
+    aos = np.zeros((R, layout.VS_WORDS), dtype=np.uint32)
+    aos[:, layout.VS_POS_X], aos[:, layout.VS_POS_Y] = start[:, 0].view(np.uint32), start[:, 1].view(np.uint32)
+    vb = VehicleBatch(R, dev)
+    vb.load_state_aos(aos)
+    return vb, torch.from_numpy(goal).to(dev)
+
+
+def fleet_report(a, G, dev):
+    """The circle swap with and without peer discs, under argmin and CEM at the same rollout budget (see the docstring)."""
+    R, S, n_seg, seg_len, P = a.R, a.S, a.n_seg, a.seg_len, a.fleet_period
+    iters, elite = (int(x) for x in (a.cem or "4:8").split(":"))
+    body, radius = a.fleet_body, 2 * a.fleet_body + a.fleet_margin
+    peers = fleet_peers(R, G, dev)
+    out = {"G": G, "groups": R // G, "circle_m": a.fleet_circle, "body_radius_m": body, "disc_radius_m": radius, "w_obst": a.fleet_w,
+           "check_period": P, "steps": a.fleet_steps, "cem": {"iters": iters, "elite": elite}}
+    for mode in ("argmin", "cem"):
+        for avoid in (False, True):
+            vb, goal = circle_swap(R, G, a.fleet_circle, dev)
+            ref = goal.unsqueeze(0).expand(n_seg, R, 2).contiguous()
+            pl = VehiclePlanner(R, S // iters if mode == "cem" else S, n_seg, seg_len, dev)
+            tr = torch.zeros((seg_len, _cabi.RK_VDT_TRACE_WORDS, R), dtype=torch.int32, device=dev)
+            least = torch.full((R // G,), float("inf"), dtype=torch.float64, device=dev)
+            eye = torch.eye(G, dtype=torch.bool, device=dev)
+            for step in range(a.fleet_steps):
+                discs = None
+                if avoid:
+                    discs = pl.peer_discs(pl.predict(vb, check_period=P), peers, radius=radius)
+                kw = dict(shift=0, seed=step, obstacles=discs, w_obst=a.fleet_w, check_period=P)
+                if mode == "cem":
+                    pl.plan_cem(vb, ref, 1.0, 10.0, 1e-9, iters, elite, **kw)
+                else:
+                    pl.plan(vb, ref, 1.0, 10.0, 1e-9, lam=0.0, **kw)
+                vb.rollout(seg_len, sensor_mode=_cabi.RK_SENSOR_PLANT, cmd=pl.first_command(), seg_len=seg_len, trace=tr)
+                pos = tr[:, :2].view(torch.float32).double().reshape(seg_len, 2, R // G, G)
+                d = torch.hypot(pos[:, 0, :, :, None] - pos[:, 0, :, None, :], pos[:, 1, :, :, None] - pos[:, 1, :, None, :])
+                least = torch.minimum(least, d.masked_fill(eye, float("inf")).amin(dim=(0, 2, 3)))
+            aos = layout.soa_to_aos(vb.state.cpu().numpy().view(np.uint32), R, layout.VS_WORDS)
+            pos = aos[:, [layout.VS_POS_X, layout.VS_POS_Y]].view(np.float32).astype(np.float64)
+            dg = np.hypot(*(pos - goal.cpu().numpy()).T)
+            lc = least.cpu().numpy()
+            out[f"{mode}_{'peer_discs' if avoid else 'none'}"] = {
+                "rollouts_per_step": S if mode == "argmin" else iters * (S // iters),
+                "groups_with_collision": float(np.mean(lc < 2 * body)), "least_pair_m_median": float(np.median(lc)),
+                "least_pair_m_min": float(np.min(lc)), "goal_dist_m_median": float(np.median(dg))}
+    return out
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--R", type=int, default=4096)
@@ -99,7 +167,16 @@ def main():
     ap.add_argument("--cem", default=None, help="ITERS:ELITE: time the cross-entropy round's sampler and refit, and compare planners")
     ap.add_argument("--cem-steps", type=int, default=8, help="closed-loop planning steps of the planner comparison")
     ap.add_argument("--lam", type=float, default=1e-3, help="MPPI temperature of the planner comparison")
+    ap.add_argument("--moving", action="append", default=[], help="M:P pairs (comma list or repeated): time moving discs and paths")
+    ap.add_argument("--fleet", type=int, default=None, help="G: play the circle swap with fleets of G robots")
+    ap.add_argument("--fleet-steps", type=int, default=60)
+    ap.add_argument("--fleet-circle", type=float, default=1.0)
+    ap.add_argument("--fleet-body", type=float, default=0.15)
+    ap.add_argument("--fleet-margin", type=float, default=0.1)
+    ap.add_argument("--fleet-w", type=float, default=1e3)
+    ap.add_argument("--fleet-period", type=int, default=25)
     a = ap.parse_args()
+    moving = [tuple(int(v) for v in x.split(":")) for arg in a.moving for x in arg.split(",") if x]
     cem_iters, cem_elite = (int(x) for x in a.cem.split(":")) if a.cem else (0, 0)
     obst_m = [m for m in int_list(a.obstacles) if m > 0]
     obst_p = int_list(a.check_period) or [a.seg_len]
@@ -150,6 +227,35 @@ def main():
     def obst_rollout(m, P):
         pl.rollout(src, ref, 1.0, 10.0, 1e-9, obstacles=discs[m], w_obst=1e3, check_period=P)
 
+    # moving discs: a table per checkpoint, the discs of the static table moved by up to 20 mm per checkpoint
+    mov, static_m = {}, {}
+    if moving:
+        aos = layout.soa_to_aos(src.state.cpu().numpy().view(np.uint32), R, layout.VS_WORDS)
+        pos0 = aos[:, [layout.VS_POS_X, layout.VS_POS_Y]].view(np.float32)
+        rng_m = np.random.default_rng(12)
+    for m, P in moving:
+        n_ck = K // P
+        d = np.zeros((m, R, 4), dtype=np.float32)
+        d[:, :, :2] = pos0[None] + rng_m.uniform(-0.15, 0.15, (m, R, 2))
+        d[:, :, 2] = rng_m.uniform(0.02, 0.08, (m, R))
+        static_m[m] = torch.from_numpy(d).to(dev)
+        walk = np.cumsum(rng_m.uniform(-0.02, 0.02, (n_ck, m, R, 2)), axis=0).astype(np.float32)
+        t4 = np.repeat(d[None], n_ck, axis=0)
+        t4[..., :2] += walk
+        mov[(m, P)] = torch.from_numpy(t4).to(dev)
+    if moving:
+        n_ck_max = max(K // P for _, P in moving)
+        path_buf = torch.empty((n_ck_max, n, 2), dtype=torch.float32, device=dev)
+        G_m = a.fleet or 8
+        peers_m = fleet_peers(R, G_m, dev)
+
+    def static_rollout(m, P):
+        pl.rollout(src, ref, 1.0, 10.0, 1e-9, obstacles=static_m[m], w_obst=1e3, check_period=P)
+
+    def moving_rollout(m, P, path=False):
+        p = path_buf[: K // P] if path else None
+        pl.rollout(src, ref, 1.0, 10.0, 1e-9, obstacles=mov[(m, P)], w_obst=1e3, check_period=P, path=p)
+
     def sample_sigma():
         pl.sample(nominal=nominal, seed=5, sigma_table=pl.sigma_table)
 
@@ -163,12 +269,18 @@ def main():
     for m in obst_m:
         for P in obst_p:
             obst_rollout(m, P)
+    for m, P in moving:
+        static_rollout(m, P), moving_rollout(m, P), moving_rollout(m, P, True)
+    if moving:
+        pred = {P: pl.predict(src, P) for P in sorted({P for _, P in moving})}
+        for P in pred:
+            pl.peer_discs(pred[P], peers_m, 0.4)
     torch.cuda.synchronize()
     src_before = src.state.clone()
     t = {"sample": [], "plan_rollout": [], "select": [], "plain_rollout": []}
     if a.cem:
         t.update(sample_sigma=[], refit=[])
-    t_obst = {}
+    t_obst, t_mov = {}, {}
     for _ in range(a.reps):
         t["sample"].append(timed(sample))
         if a.cem:
@@ -185,6 +297,15 @@ def main():
                 tp, to = t_obst.setdefault((m, P), ([], []))
                 tp.append(timed(plan_rollout))
                 to.append(timed(lambda: obst_rollout(m, P)))
+        for m, P in moving:  # static, moving and moving with paths, alternated
+            ts, tm, tpth = t_mov.setdefault((m, P), ([], [], []))
+            ts.append(timed(lambda: static_rollout(m, P)))
+            tm.append(timed(lambda: moving_rollout(m, P)))
+            tpth.append(timed(lambda: moving_rollout(m, P, True)))
+        if moving:
+            for P in pred:
+                t_mov.setdefault(("predict", P), []).append(timed(lambda: pl.predict(src, P)))
+                t_mov.setdefault(("peer_discs", P), []).append(timed(lambda: pl.peer_discs(pred[P], peers_m, 0.4)))
     assert torch.equal(src.state, src_before), "the plan rollout modified its source states"
     med = {k: float(np.median(v)) for k, v in t.items()}
     res = {
@@ -213,6 +334,26 @@ def main():
                          "ms_min_obst": round(float(np.min(to)), 4), "ms_max_obst": round(float(np.max(to)), 4),
                          "obst_over_plan": mo / mp, "penetrating_fraction": hit})
         res["obstacles"] = rows
+    if moving:
+        rows = []
+        for m, P in moving:
+            ts, tm, tpth = (float(np.median(v)) for v in t_mov[(m, P)])
+            moving_rollout(m, P)
+            mc = pl.cost.clone()
+            moving_rollout(m, P, True)
+            same = bool(torch.equal(pl.cost.view(torch.int32), mc.view(torch.int32)))
+            rows.append({"m": m, "check_period": P, "ms_median_static": round(ts, 4), "ms_median_moving": round(tm, 4),
+                         "ms_median_moving_path": round(tpth, 4), "moving_over_static": tm / ts, "path_over_moving": tpth / tm,
+                         "path_bytes": (K // P) * n * 8, "path_store_ms": tpth - tm, "cost_same_with_path": same})
+        res["moving"] = rows
+        res["predict"] = [{"check_period": P, "robots": R, "ms_median": round(float(np.median(t_mov[("predict", P)])), 4),
+                           "ms_min": round(float(np.min(t_mov[("predict", P)])), 4)} for P in pred]
+        res["peer_discs"] = [{"check_period": P, "G": G_m, "cells": (K // P) * (G_m - 1) * R,
+                              "ms_median": round(float(np.median(t_mov[("peer_discs", P)])), 4)} for P in pred]
+    if moving or a.fleet:
+        res["max_sm_clock"] = power_limit("clocks.max.sm")
+    if a.fleet:
+        res["fleet"] = fleet_report(a, a.fleet, dev)
     if a.cem:
         res["cem"] = {"iters": cem_iters, "elite": cem_elite,
                       "sample_sigma_over_sample": med["sample_sigma"] / med["sample"],
