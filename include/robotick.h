@@ -775,6 +775,38 @@ int rk_plan_rollout_moving(const rk_vdt_params_t *p, const void *d_src_state, in
 int rk_plan_peer_discs(const float *d_path, int64_t R, int32_t n_ck, const int32_t *d_peer, int32_t m, float radius,
                        float *d_obs, int32_t M, int32_t k0, void *stream);
 
+/* Cost maps: a grid of cell costs, stored once per world (not per robot) and looked up at every checkpoint, one cell load
+ * whatever the world holds -- walls, corridors, shelving.  It shares the checkpoints and the accumulator O with the discs,
+ * so peer discs and a building map compose in one rollout.  The robot is a point read at checkpoints only: inflate walls by
+ * the body radius plus the distance covered in P ticks (at most 0.4 mm per tick at 400 mm/s), see INTEGRATION.md §2. */
+typedef struct rk_plan_map {
+  const float   *d_cells;  /* float [n_maps][height][width]: cell (ix, iy) of map k at (k*height + iy)*width + ix; 4-byte aligned */
+  const int32_t *d_map_of; /* int32 [R]: the map of robot r; NULL: map 0 for every robot */
+  int32_t n_maps, width, height;  /* >= 1 each; n_maps*height*width < 2^31; width, height <= 2^24 */
+  float   x0, y0;          /* metres: the outer corner of cell (0, 0); finite */
+  float   inv_res;         /* cells per metre; finite, > 0 */
+  float   outside;         /* the value of every point off the grid; may be +inf; NaN rejected */
+  float   w_map;           /* >= 0, may be +inf; NaN rejected */
+} rk_plan_map_t;           /* 48 bytes */
+
+/* rk_plan_rollout_moving plus a map term.  obst is required (it gives check_period; m may be 0), d_path as there.  At each
+ * checkpoint: the path cell is stored, discs k = 0 .. m-1 are added to O exactly as rk_plan_rollout_moving does, then the
+ * map term is added to the same O.  Each operation is one IEEE float32 operation in the written order, no contraction:
+ *   k = d_map_of ? d_map_of[r] : 0;        k < 0 or k >= n_maps: no map term for robot r
+ *   u = (x - x0) * inv_res;  v = (y - y0) * inv_res
+ *   c = (u >= 0 && u < (float)width && v >= 0 && v < (float)height) ? cells[(k*height + (int)v)*width + (int)u] : outside
+ *   if (c > 0) O = O + w_map * c
+ * So a NaN position reads `outside`; NaN, zero and negative cells contribute nothing; a +inf cell, or w_map = +inf with a
+ * cell above 0, makes O = +inf (a hard wall).  d_cost = J + O.  map == NULL or w_map == 0 is rk_plan_rollout_moving (the
+ * same kernel and bits, never 0 * inf).  Cells are read with ordinary loads: no texture filtering.
+ * RK_ERR_ARG: rk_plan_rollout_moving's checks; d_cells NULL or not 4-byte aligned; d_map_of not 4-byte aligned; n_maps,
+ * width or height < 1, width or height > 2^24, n_maps*height*width >= 2^31; x0, y0 or inv_res not finite, inv_res <= 0;
+ * outside NaN; w_map < 0 or NaN.  R == 0 is a no-op. */
+int rk_plan_rollout_map(const rk_vdt_params_t *p, const void *d_src_state, int64_t R, int32_t S,
+                        const rk_vdt_cmd_t *d_cmd, int32_t n_seg, int32_t seg_len, const rk_plan_cost_t *cost,
+                        const rk_plan_obstacles_t *obst, const rk_plan_map_t *map, float *d_path, float *d_cost,
+                        void *stream);
+
 /* =====================================================================================
  * RobotManager guard (SURVEY 8f-2): the vehicle-management block of RMT's routine_ros()
  * (src/RobotManager/RM_task_main.cpp:484-767), one call = K manager cycles of n robots.  Per

@@ -17,8 +17,8 @@ def __getattr__(name):
         from . import vehicle as _v
 
         return _v if name == "vehicle" else _v.VehicleBatch
-    if name in ("planner", "VehiclePlanner"):
+    if name in ("planner", "VehiclePlanner", "CostMap"):
         from . import planner as _p
 
-        return _p if name == "planner" else _p.VehiclePlanner
+        return _p if name == "planner" else getattr(_p, name)
     raise AttributeError(name)

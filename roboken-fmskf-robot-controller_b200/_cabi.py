@@ -182,6 +182,13 @@ class PlanObstacles(C.Structure):
     _fields_ = [("d_obs", C.c_void_p), ("m", C.c_int32), ("check_period", C.c_int32), ("w_obst", C.c_float), ("rsv", C.c_float)]
 
 
+class PlanMap(C.Structure):
+    """rk_plan_map_t"""
+
+    _fields_ = [("d_cells", C.c_void_p), ("d_map_of", C.c_void_p), ("n_maps", C.c_int32), ("width", C.c_int32), ("height", C.c_int32),
+                ("x0", C.c_float), ("y0", C.c_float), ("inv_res", C.c_float), ("outside", C.c_float), ("w_map", C.c_float)]
+
+
 class PlanRefit(C.Structure):
     """rk_plan_refit_t"""
 
@@ -240,6 +247,8 @@ def _proto(lib):
                                               C.POINTER(PlanObstacles), vp, vp]
     lib.rk_plan_rollout_moving.argtypes = [C.POINTER(VdtParams), vp, C.c_int64, C.c_int32, vp, C.c_int32, C.c_int32, C.POINTER(PlanCost),
                                            C.POINTER(PlanObstacles), vp, vp, vp]
+    lib.rk_plan_rollout_map.argtypes = [C.POINTER(VdtParams), vp, C.c_int64, C.c_int32, vp, C.c_int32, C.c_int32, C.POINTER(PlanCost),
+                                        C.POINTER(PlanObstacles), C.POINTER(PlanMap), vp, vp, vp]
     lib.rk_plan_peer_discs.argtypes = [vp, C.c_int64, C.c_int32, vp, C.c_int32, C.c_float, vp, C.c_int32, C.c_int32, vp]
     lib.rk_plan_select.argtypes = [vp, vp, C.c_int64, C.c_int32, C.c_int32, C.c_float, C.c_int32, vp, vp, vp, vp]
     lib.rk_plan_sample_commands_sigma.argtypes = [C.POINTER(VdtParams), C.POINTER(PlanSample), vp, vp, C.c_int64, C.c_int32, C.c_int32, vp,

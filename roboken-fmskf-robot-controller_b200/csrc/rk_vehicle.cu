@@ -98,9 +98,14 @@ struct PlanObstArgs : PlanArgs {
   int32_t       m, P;
   float         w_obst;
 };
-// rk_plan_rollout_moving: a disc table per checkpoint, and the candidates' positions at the checkpoints if path != NULL
+// rk_plan_rollout_moving: a disc table per checkpoint, and the candidates' positions at the checkpoints if path != NULL.
+// rk_plan_rollout_map: the cost grid (rk_plan_map_t) if cells != NULL; the host leaves it NULL for w_map == 0.
 struct PlanMovingArgs : PlanObstArgs {
-  float2 *path; // [n_ck][R * S], metres
+  float2        *path;   // [n_ck][R * S], metres
+  const float   *cells;  // [n_maps][height][width]
+  const int32_t *map_of; // [R]; NULL: map 0
+  int32_t        n_maps, width, height;
+  float          x0, y0, inv_res, outside, w_map;
 };
 // OBST: 0 no discs (PlanArgs), kObstStatic rk_plan_rollout_obstacles (PlanObstArgs), kObstMoving rk_plan_rollout_moving
 // (PlanMovingArgs)
@@ -121,11 +126,23 @@ RK_DEV float plan_obst_cost(float O, float x, float y, const PlanObstArgs &pl, u
   }
   return O;
 }
+// O after the map term of rk_plan_rollout_map at position (x, y).  The map index is read here, at the checkpoint (one
+// broadcast per warp), not held across the tick loop.  The cell index fits 32 bits (n_maps * height * width < 2^31), and
+// (int) truncates a u in [0, width) to its cell.  A NaN position fails every comparison and reads `outside`.
+RK_DEV float plan_map_cost(float O, float x, float y, const PlanMovingArgs &pl, uint32_t r) {
+  const int32_t k = pl.map_of != nullptr ? __ldg(pl.map_of + r) : 0;
+  if((uint32_t)k >= (uint32_t)pl.n_maps) return O; // no map term for this robot
+  const float u = fmul(fsub(x, pl.x0), pl.inv_res), v = fmul(fsub(y, pl.y0), pl.inv_res);
+  float       c = pl.outside;
+  if(u >= 0.0f && u < (float)pl.width && v >= 0.0f && v < (float)pl.height) c = __ldg(pl.cells + (k * pl.height + (int)v) * pl.width + (int)u);
+  if(c > 0.0f) O = fadd(O, fmul(pl.w_map, c));
+  return O;
+}
 // O after checkpoint c + 1 (0-based c) of rk_plan_rollout_moving at position (x, y): first the path cell of candidate i
-// (n = R * S) if asked, then plan_obst_cost on checkpoint c's table.  Only the table differs from rk_plan_obstacles_t.
-// Unlike the static table, each checkpoint's cells are new to L1, and the serial disc loop would wait on m misses in a
-// row; so every checkpoint but the last (at t = K, `last`) prefetches the next table's m cells into L1, P ticks ahead
-// and without holding a register.
+// (n = R * S) if asked, then plan_obst_cost on checkpoint c's table, then the map term into the same O if there is a map.
+// Only the table differs from rk_plan_obstacles_t.  Unlike the static table, each checkpoint's cells are new to L1, and
+// the serial disc loop would wait on m misses in a row; so every checkpoint but the last (at t = K, `last`) prefetches the
+// next table's m cells into L1, P ticks ahead and without holding a register.
 RK_DEV float plan_moving_cost(float O, float x, float y, const PlanMovingArgs &pl, uint32_t r, int64_t n, int64_t i, int c, bool last) {
   if(pl.path != nullptr) __stcs(pl.path + (int64_t)c * n + i, make_float2(x, y));
   PlanObstArgs q = pl;
@@ -136,6 +153,7 @@ RK_DEV float plan_moving_cost(float O, float x, float y, const PlanMovingArgs &p
 #pragma unroll 1
     for(int k = 0; k < pl.m; k++, nx += pl.R) asm volatile("prefetch.global.L1 [%0];" ::"l"(nx));
   }
+  if(pl.cells != nullptr) O = plan_map_cost(O, x, y, pl, r);
   return O;
 }
 
@@ -851,11 +869,11 @@ static void launch_plan(const rk_vdt_params_t &p, const void *d_src, int64_t n, 
     vdt_rollout_kernel<RK_SENSOR_PLANT, false, true, OBST><<<grid, kRolloutThreads, 0, st>>>(p, src, n, a, pl);
   }
 }
-// rk_plan_rollout (ob == NULL), rk_plan_rollout_obstacles and rk_plan_rollout_moving (moving): the same checks, and
-// without discs or path the same kernels
+// rk_plan_rollout (ob == NULL), rk_plan_rollout_obstacles, rk_plan_rollout_moving (moving) and rk_plan_rollout_map
+// (moving, map): the same checks, and without discs, path or map the same kernels
 static int plan_rollout(const char *who, const rk_vdt_params_t *p, const void *d_src_state, int64_t R, int32_t S, const rk_vdt_cmd_t *d_cmd,
                         int32_t n_seg, int32_t seg_len, const rk_plan_cost_t *cost, const rk_plan_obstacles_t *ob, bool moving,
-                        float *d_path, float *d_cost, void *stream) {
+                        const rk_plan_map_t *map, float *d_path, float *d_cost, void *stream) {
   if(!p || !cost) {
     set_error("%s: NULL params/cost", who);
     return RK_ERR_ARG;
@@ -894,6 +912,27 @@ static int plan_rollout(const char *who, const rk_vdt_params_t *p, const void *d
       return RK_ERR_ARG;
     }
   }
+  if(map) {
+    if(map->n_maps < 1 || map->width < 1 || map->height < 1 || map->width > (1 << 24) || map->height > (1 << 24) ||
+       (int64_t)map->n_maps * map->height * map->width > INT_MAX) {
+      set_error("%s: need n_maps, width, height >= 1, width, height <= 2^24 and n_maps * height * width < 2^31 (n_maps = %d, "
+                "width = %d, height = %d)",
+                who, map->n_maps, map->width, map->height);
+      return RK_ERR_ARG;
+    }
+    if(!isfinite(map->x0) || !isfinite(map->y0) || !isfinite(map->inv_res) || !(map->inv_res > 0.0f)) {
+      set_error("%s: map x0, y0 and inv_res must be finite, and inv_res > 0", who);
+      return RK_ERR_ARG;
+    }
+    if(isnan(map->outside)) {
+      set_error("%s: map outside must not be NaN (+-inf allowed)", who);
+      return RK_ERR_ARG;
+    }
+    if(!(map->w_map >= 0.0f)) {
+      set_error("%s: w_map must be >= 0 (+inf allowed, NaN not)", who);
+      return RK_ERR_ARG;
+    }
+  }
   if(R == 0) return RK_OK;
   if(int rc = check_block(d_src_state, "d_src_state")) return rc;
   if(int rc = check_block(d_cmd, "d_cmd")) return rc;
@@ -906,6 +945,11 @@ static int plan_rollout(const char *who, const rk_vdt_params_t *p, const void *d
     set_error("%s: obst->d_obs must be a non-NULL 16-byte aligned device pointer when m > 0", who);
     return RK_ERR_ARG;
   }
+  if(map && (!map->d_cells || ((uintptr_t)map->d_cells & 3u) || ((uintptr_t)map->d_map_of & 3u))) {
+    set_error("%s: map->d_cells (float) must be a non-NULL device pointer and map->d_map_of (int32, may be NULL) 4-byte aligned", who);
+    return RK_ERR_ARG;
+  }
+  const bool use_map = map && map->w_map > 0.0f; // w_map == 0 is the rollout without the map (and never 0 * inf)
   if(int rc = require_device()) return rc;
   rk_vdt_rollout_t a;
   memset(&a, 0, sizeof(a));
@@ -916,9 +960,14 @@ static int plan_rollout(const char *who, const rk_vdt_params_t *p, const void *d
   pl.w_pos = cost->w_pos, pl.w_goal = cost->w_goal, pl.w_cur = cost->w_cur, pl.cost = d_cost;
   const int64_t n  = R * (int64_t)S;
   cudaStream_t  st = (cudaStream_t)stream;
-  if(obst || d_path) {
+  if(obst || d_path || use_map) {
     pl.obs = reinterpret_cast<const float4 *>(ob->d_obs), pl.m = ob->m, pl.P = ob->check_period, pl.w_obst = ob->w_obst;
     pl.path = reinterpret_cast<float2 *>(d_path);
+    pl.cells = use_map ? map->d_cells : nullptr, pl.map_of = use_map ? map->d_map_of : nullptr;
+    if(use_map) {
+      pl.n_maps = map->n_maps, pl.width = map->width, pl.height = map->height;
+      pl.x0 = map->x0, pl.y0 = map->y0, pl.inv_res = map->inv_res, pl.outside = map->outside, pl.w_map = map->w_map;
+    }
     if(moving) launch_plan<kObstMoving>(*p, d_src_state, n, a, pl, st);
     else launch_plan<kObstStatic>(*p, d_src_state, n, a, static_cast<const PlanObstArgs &>(pl), st);
   } else {
@@ -932,19 +981,25 @@ extern "C" {
 
 int rk_plan_rollout(const rk_vdt_params_t *p, const void *d_src_state, int64_t R, int32_t S, const rk_vdt_cmd_t *d_cmd, int32_t n_seg,
                     int32_t seg_len, const rk_plan_cost_t *cost, float *d_cost, void *stream) {
-  return plan_rollout("rk_plan_rollout", p, d_src_state, R, S, d_cmd, n_seg, seg_len, cost, nullptr, false, nullptr, d_cost, stream);
+  return plan_rollout("rk_plan_rollout", p, d_src_state, R, S, d_cmd, n_seg, seg_len, cost, nullptr, false, nullptr, nullptr, d_cost, stream);
 }
 
 int rk_plan_rollout_obstacles(const rk_vdt_params_t *p, const void *d_src_state, int64_t R, int32_t S, const rk_vdt_cmd_t *d_cmd,
                               int32_t n_seg, int32_t seg_len, const rk_plan_cost_t *cost, const rk_plan_obstacles_t *obst, float *d_cost,
                               void *stream) {
-  return plan_rollout("rk_plan_rollout_obstacles", p, d_src_state, R, S, d_cmd, n_seg, seg_len, cost, obst, false, nullptr, d_cost, stream);
+  return plan_rollout("rk_plan_rollout_obstacles", p, d_src_state, R, S, d_cmd, n_seg, seg_len, cost, obst, false, nullptr, nullptr, d_cost, stream);
 }
 
 int rk_plan_rollout_moving(const rk_vdt_params_t *p, const void *d_src_state, int64_t R, int32_t S, const rk_vdt_cmd_t *d_cmd, int32_t n_seg,
                            int32_t seg_len, const rk_plan_cost_t *cost, const rk_plan_obstacles_t *obst, float *d_path, float *d_cost,
                            void *stream) {
-  return plan_rollout("rk_plan_rollout_moving", p, d_src_state, R, S, d_cmd, n_seg, seg_len, cost, obst, true, d_path, d_cost, stream);
+  return plan_rollout("rk_plan_rollout_moving", p, d_src_state, R, S, d_cmd, n_seg, seg_len, cost, obst, true, nullptr, d_path, d_cost, stream);
+}
+
+int rk_plan_rollout_map(const rk_vdt_params_t *p, const void *d_src_state, int64_t R, int32_t S, const rk_vdt_cmd_t *d_cmd, int32_t n_seg,
+                        int32_t seg_len, const rk_plan_cost_t *cost, const rk_plan_obstacles_t *obst, const rk_plan_map_t *map, float *d_path,
+                        float *d_cost, void *stream) {
+  return plan_rollout("rk_plan_rollout_map", p, d_src_state, R, S, d_cmd, n_seg, seg_len, cost, obst, true, map, d_path, d_cost, stream);
 }
 
 int rk_vdt_set_power(void *d_state, int64_t n, const uint8_t *d_on, void *stream) {

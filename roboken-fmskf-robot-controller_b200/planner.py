@@ -6,6 +6,8 @@ candidates into the next nominal plan.  Candidate j of robot r is column r*S + j
 method (plan_cem) runs several sample -> rollout -> refit rounds per step, refitting a per-robot, per-segment mean and
 sigma to each round's elite candidates.  For fleets, predict() gives where each robot's nominal plan takes it and
 peer_discs() turns those paths into moving keep-out discs for the robot's peers (fleet_peers builds the usual grouping).
+A CostMap, a grid of cell costs shared by the robots of a world, prices walls and shelving at every checkpoint, alone or
+together with discs.
 """
 import ctypes as C
 
@@ -13,6 +15,43 @@ import torch
 
 from . import _cabi
 from .vehicle import _dev_index
+
+
+class CostMap:
+    """A cost grid for rk_plan_rollout_map: cells float32 [H, W] (one world) or [n_maps, H, W], contiguous, on the
+    planner's device; cell (ix, iy) of map k covers x in [x0 + ix*resolution, x0 + (ix+1)*resolution) and likewise y, with
+    (x0, y0) = origin in metres.  A point off the grid reads `outside` (+inf: leaving the grid is a hard wall).  map_of:
+    int32 [R] device tensor, the map of each robot (an index outside [0, n_maps) gives that robot no map term); None: map 0
+    for every robot.  Cells above 0 add w_map * cell to a candidate's cost at every checkpoint; zero, negative and NaN cells
+    add nothing.  The robot is a point read at checkpoints: inflate walls by the body radius plus the distance covered in
+    check_period ticks.  Cells may be changed in place between planning steps.
+
+    inv_res = float32(1 / resolution) is computed once here and passed as is, so a restatement can use the same bits;
+    x0, y0 and outside are likewise the float32 values the device reads."""
+
+    def __init__(self, cells, origin, resolution, outside=float("inf"), map_of=None):
+        assert (cells.is_cuda and cells.is_contiguous() and cells.dtype == torch.float32 and cells.dim() in (2, 3)
+                and cells.numel() > 0), "cells: float32 [H, W] or [n_maps, H, W] contiguous device tensor"
+        self.cells = cells if cells.dim() == 3 else cells[None]
+        self.n_maps, self.height, self.width = (int(d) for d in self.cells.shape)
+        resolution = float(resolution)
+        assert resolution > 0 and resolution < float("inf"), "resolution: metres per cell, finite and > 0"
+        self.resolution = resolution
+        self.x0, self.y0 = (C.c_float(float(v)).value for v in origin)
+        self.inv_res = C.c_float(1.0 / resolution).value
+        self.outside = C.c_float(float(outside)).value
+        if map_of is not None:
+            assert (map_of.is_cuda and map_of.is_contiguous() and map_of.dtype == torch.int32 and map_of.dim() == 1
+                    and map_of.device == cells.device), "map_of: int32 [R] contiguous tensor on the cells' device"
+        self.map_of = map_of
+
+    def struct(self, w_map):
+        """The rk_plan_map_t of this map with weight w_map."""
+        m = _cabi.PlanMap()
+        m.d_cells, m.d_map_of = self.cells.data_ptr(), None if self.map_of is None else self.map_of.data_ptr()
+        m.n_maps, m.width, m.height = self.n_maps, self.width, self.height
+        m.x0, m.y0, m.inv_res, m.outside, m.w_map = self.x0, self.y0, self.inv_res, self.outside, float(w_map)
+        return m
 
 
 class VehiclePlanner:
@@ -76,7 +115,7 @@ class VehiclePlanner:
         assert P >= 1 and self.seg_len % P == 0, "check_period must divide seg_len"
         return self.n_seg * self.seg_len // P
 
-    def rollout(self, src, ref, w_pos, w_goal, w_cur, obstacles=None, w_obst=0.0, check_period=None, path=None):
+    def rollout(self, src, ref, w_pos, w_goal, w_cur, obstacles=None, w_obst=0.0, check_period=None, path=None, costmap=None, w_map=0.0):
         """rk_plan_rollout: every candidate from its robot's state in `src` (a VehicleBatch of R robots, left untouched),
         ranked against ref (float32 [n_seg, R, 2], metres: where each robot should be when each segment ends).
 
@@ -88,13 +127,24 @@ class VehiclePlanner:
         peers' predicted paths (peer_discs).
 
         path: float32 [n_ck, R*S, 2], receives every candidate's position at every checkpoint (rk_plan_rollout_moving; with
-        a 4-D table or no obstacles).  It never changes the cost."""
+        a 4-D table or no obstacles).  It never changes the cost.
+
+        costmap (a CostMap on the planner's device): rk_plan_rollout_map adds w_map * cell at every checkpoint (cells > 0
+        only; w_map = inf makes every such cell a hard wall), into the same sum as the discs.  Without obstacles the
+        checkpoints are every check_period ticks (default seg_len) with no discs.  A 3-D static disc table is then repeated
+        for every checkpoint (obstacles.expand(n_ck, m, R, 4).contiguous(), the same bits as the static table): a copy of
+        n_ck * m * R * 16 bytes written on every call, so pass a 4-D table to keep one."""
         assert src.n == self.R, "the source batch must hold the planner's R robots"
         assert ref.is_cuda and ref.is_contiguous() and ref.dtype == torch.float32 and tuple(ref.shape) == (self.n_seg, self.R, 2)
         c = _cabi.PlanCost()
         c.d_ref, c.w_pos, c.w_goal, c.w_cur = ref.data_ptr(), float(w_pos), float(w_goal), float(w_cur)
         args = (C.byref(self.params), src.state.data_ptr(), self.R, self.S, self.candidates.data_ptr(), self.n_seg, self.seg_len, C.byref(c))
-        if obstacles is None and path is None:
+        if costmap is not None:
+            assert costmap.cells.device.index == self.dev_index, "costmap: on the planner's device"
+            assert costmap.map_of is None or costmap.map_of.shape[0] == self.R, f"costmap.map_of: int32 [{self.R}]"
+            if obstacles is not None and obstacles.dim() == 3:
+                obstacles = obstacles.expand(self.n_ck(self.seg_len if check_period is None else check_period), *obstacles.shape).contiguous()
+        if obstacles is None and path is None and costmap is None:
             self._keep = ref
             _cabi.check(self.lib.rk_plan_rollout(*args, self.cost.data_ptr(), self._stream()))
             return self.cost
@@ -115,8 +165,13 @@ class VehiclePlanner:
         if path is not None:
             assert (path.is_cuda and path.is_contiguous() and path.dtype == torch.float32
                     and tuple(path.shape) == (n_ck, self.R * self.S, 2)), f"path: float32 [{n_ck}, {self.R * self.S}, 2] device tensor"
-        _cabi.check(self.lib.rk_plan_rollout_moving(*args, C.byref(o), None if path is None else path.data_ptr(), self.cost.data_ptr(),
-                                                    self._stream()))
+        pth = None if path is None else path.data_ptr()
+        if costmap is None:
+            _cabi.check(self.lib.rk_plan_rollout_moving(*args, C.byref(o), pth, self.cost.data_ptr(), self._stream()))
+        else:
+            self._keep = (ref, obstacles, path, costmap)
+            mp = costmap.struct(w_map)
+            _cabi.check(self.lib.rk_plan_rollout_map(*args, C.byref(o), C.byref(mp), pth, self.cost.data_ptr(), self._stream()))
         return self.cost
 
     def predict(self, src, check_period):
@@ -179,19 +234,21 @@ class VehiclePlanner:
             self.sigma_table, self._sigma_next = out, self.sigma_table
         return self.nominal
 
-    def plan(self, src, ref, w_pos, w_goal, w_cur, lam=0.0, shift=1, seed=None, obstacles=None, w_obst=0.0, check_period=None):
+    def plan(self, src, ref, w_pos, w_goal, w_cur, lam=0.0, shift=1, seed=None, obstacles=None, w_obst=0.0, check_period=None,
+             costmap=None, w_map=0.0):
         """One planning step (sample, rollout, select) on the current torch stream; returns the new nominal.  obstacles
-        as in rollout (3-D static or 4-D per-checkpoint discs)."""
+        (3-D static or 4-D per-checkpoint discs) and costmap as in rollout."""
         self.sample(seed=seed)
-        self.rollout(src, ref, w_pos, w_goal, w_cur, obstacles=obstacles, w_obst=w_obst, check_period=check_period)
+        self.rollout(src, ref, w_pos, w_goal, w_cur, obstacles=obstacles, w_obst=w_obst, check_period=check_period, costmap=costmap,
+                     w_map=w_map)
         return self.select(lam, shift)
 
     def plan_cem(self, src, ref, w_pos, w_goal, w_cur, iters, elite, alpha=0.0, sigma_min=(0.0, 0.0, 0.0), shift=1, seed=None,
-                 obstacles=None, w_obst=0.0, check_period=None):
+                 obstacles=None, w_obst=0.0, check_period=None, costmap=None, w_map=0.0):
         """One cross-entropy planning step on the current torch stream; returns the new nominal.
 
         sigma_table is reset to the planner's sigma, then `iters` rounds of sample (around the nominal, with the table) ->
-        rollout (obstacles as in rollout) -> refit to the `elite` best candidates.  Every round but the last refits with
+        rollout (obstacles and costmap as in rollout) -> refit to the `elite` best candidates.  Every round but the last refits with
         shift = 0, so that the next round samples around the same segments; the last one with `shift`.  Round i draws with
         seed (seed + i * 0x9E3779B9) mod 2^32 (seed: the planner's own when None).  iters = 1, elite = 1, alpha = 0 is
         plan(..., lam=0) bit for bit while no cost is -inf (never, with non-negative weights).  NaN and +-inf costs are never
@@ -201,7 +258,8 @@ class VehiclePlanner:
         self.sigma_table.copy_(self._sigma_cell.expand_as(self.sigma_table))
         for i in range(int(iters)):
             self.sample(seed=(base + i * 0x9E3779B9) & 0xFFFFFFFF, sigma_table=self.sigma_table)
-            self.rollout(src, ref, w_pos, w_goal, w_cur, obstacles=obstacles, w_obst=w_obst, check_period=check_period)
+            self.rollout(src, ref, w_pos, w_goal, w_cur, obstacles=obstacles, w_obst=w_obst, check_period=check_period, costmap=costmap,
+                         w_map=w_map)
             self.refit(elite, alpha, sigma_min, shift if i == int(iters) - 1 else 0)
         return self.nominal
 

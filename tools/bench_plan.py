@@ -27,10 +27,21 @@ heading for the antipodal point, with and without peer discs (radius 2 * --fleet
 the same rollout budget), for --fleet-steps steps.  It reports the share of groups in which two robots came closer than
 2 * body radius, the median / minimum over groups of the least pairwise distance, and the median distance to the goal.
 
+With --map CELLS:P (a comma list or repeated) the run also times rk_plan_rollout_map on a square world of CELLS x CELLS
+5 cm cells (800 cells: 40 m, 2.56 MB) holding random rectangular walls, with m = 0 and 8 moving discs per robot checked
+every P ticks, each alternated with rk_plan_rollout_moving on the same discs (m = 0: with a path, so that the moving
+kernel runs), and reports map_over_moving.  Then it plays the wall scenario at size (R robots, each in its own lane with
+a wall across it and a gap to the side, --map-steps steps under argmin and CEM --cem ITERS:ELITE, default 4:8) and
+reports the share of robots that ever enter a wall cell, with and without the map, and the distance to the goal.
+--parent-lib LIB also times LIB's rk_plan_rollout_moving (a build of another tree, loaded side by side) alternated with
+this tree's on the same inputs, and checks that both give the same bits.
+
     python tools/bench_plan.py [--R 4096] [--S 256] [--n-seg 8] [--seg-len 125] [--reps 10] [--out FILE]
                                [--obstacles 1,8 --check-period 125,25,10] [--cem 4:8 --cem-steps 8 --lam 1e-3]
-                               [--moving 1:125,8:25] [--fleet 8 --fleet-steps 60]
+                               [--moving 1:125,8:25] [--fleet 8 --fleet-steps 60] [--map 800:125,800:25,800:5]
+                               [--parent-lib path/to/librobotick_b200.so]
 """
+import ctypes as C
 import argparse
 import json
 import os
@@ -45,7 +56,7 @@ import torch  # noqa: E402
 
 import roboken_fmskf_robot_controller_b200 as rk  # noqa: E402
 from roboken_fmskf_robot_controller_b200 import _cabi, layout, streams  # noqa: E402
-from roboken_fmskf_robot_controller_b200.planner import VehiclePlanner, fleet_peers  # noqa: E402
+from roboken_fmskf_robot_controller_b200.planner import CostMap, VehiclePlanner, fleet_peers  # noqa: E402
 from roboken_fmskf_robot_controller_b200.vehicle import VehicleBatch  # noqa: E402
 
 
@@ -154,6 +165,67 @@ def fleet_report(a, G, dev):
     return out
 
 
+def wall_world(R, dev, cell=0.05):
+    """The wall scenario of tests/plan_map_ref.py at size: robot r in lane x in [r - 0.5, r + 0.5), a 0.1 m wall band across
+    y = 0 with a 0.3 m gap centred 0.25 m east (even r) or west (odd r) of the lane's line, start 0.35 m south of the band,
+    goal 0.35 m north.  Returns (wall bool [H, W] on the host, CostMap of the wall inflated by one cell, starts, goals)."""
+    W, H = 20 * R, 24
+    x0, y0 = -0.5, -0.6
+    xc = x0 + (np.arange(W) + 0.5) * cell
+    yc = y0 + (np.arange(H) + 0.5) * cell
+    lane = np.floor(xc - x0).astype(np.int64)
+    gap = np.abs(xc - (lane + 0.25 * np.where(lane % 2 == 0, 1.0, -1.0))) < 0.15
+    wall = (np.abs(yc) < 0.05)[:, None] & ~gap[None, :]
+    g = np.pad(wall, 1)
+    grown = np.zeros_like(wall)
+    for dy in range(3):
+        for dx in range(3):
+            grown |= g[dy:dy + H, dx:dx + W]
+    cm = CostMap(torch.from_numpy(grown.astype(np.float32)).to(dev), (x0, y0), cell)
+    starts = np.stack([np.arange(R, dtype=np.float64), np.full(R, -0.40)], axis=1).astype(np.float32)
+    goals = np.stack([np.arange(R, dtype=np.float64), np.full(R, 0.40)], axis=1).astype(np.float32)
+    return wall, cm, starts, goals
+
+
+def wall_report(a, dev, iters, elite):
+    """The wall scenario at size under argmin (S candidates) and CEM (iters rounds of S / iters), with and without the map:
+    the share of robots that ever enter a wall cell and the distance to the goal after --map-steps steps."""
+    R, n_seg, seg_len, P = a.R, a.n_seg, a.seg_len, 25
+    wall, cm, starts, goals = wall_world(R, dev)
+    ref = torch.from_numpy(np.ascontiguousarray(np.broadcast_to(goals, (n_seg, R, 2)))).to(dev)
+    aos = np.zeros((R, layout.VS_WORDS), dtype=np.uint32)
+    aos[:, layout.VS_POS_X], aos[:, layout.VS_POS_Y] = starts[:, 0].view(np.uint32), starts[:, 1].view(np.uint32)
+    out = {"robots": R, "steps": a.map_steps, "check_period": P, "w_map": 1e4, "cell_m": 0.05, "inflation_cells": 1}
+    for mode in ("argmin", "cem"):
+        for use_map in (False, True):
+            S = a.S if mode == "argmin" else a.S // iters
+            pl = VehiclePlanner(R, S, n_seg, seg_len, dev, sigma=(250.0, 250.0, 0.2), seed=0xA11)
+            vb = VehicleBatch(R, dev)
+            vb.load_state_soa(layout.aos_to_soa(aos))
+            tr = torch.empty((seg_len, _cabi.RK_VDT_TRACE_WORDS, R), dtype=torch.int32, device=dev)
+            hit = np.zeros(R, dtype=bool)
+            kw = dict(check_period=P, costmap=cm if use_map else None, w_map=1e4)
+            for it in range(a.map_steps):
+                if mode == "argmin":
+                    pl.plan(vb, ref, 1.0, 10.0, 1e-9, lam=0.0, shift=0, seed=0xA11 + it, **kw)
+                else:
+                    pl.plan_cem(vb, ref, 1.0, 10.0, 1e-9, iters, elite, 0.0, (40.0, 40.0, 0.05), shift=0, seed=0xA11 + it, **kw)
+                vb.rollout(seg_len, sensor_mode=_cabi.RK_SENSOR_PLANT, cmd=pl.first_command(), seg_len=seg_len, trace=tr)
+                t = tr.cpu().numpy().view(np.uint32)
+                u = ((t[:, 0].view(np.float32) - np.float32(-0.5)) * np.float32(20.0))
+                v = ((t[:, 1].view(np.float32) - np.float32(-0.6)) * np.float32(20.0))
+                ok = (u >= 0) & (u < wall.shape[1]) & (v >= 0) & (v < wall.shape[0])
+                hit |= (ok & wall[np.where(ok, v, 0).astype(np.int64), np.where(ok, u, 0).astype(np.int64)]).any(axis=0)
+            st = layout.soa_to_aos(vb.state.cpu().numpy().view(np.uint32), R, layout.VS_WORDS)
+            pos = st[:, [layout.VS_POS_X, layout.VS_POS_Y]].view(np.float32)
+            d = np.hypot(pos[:, 0] - goals[:, 0], pos[:, 1] - goals[:, 1])
+            out[f"{mode}_{'map' if use_map else 'no_map'}"] = {
+                "S": S, "entered_wall_share": float(hit.mean()), "goal_dist_median_m": float(np.median(d)),
+                "goal_dist_p90_m": float(np.quantile(d, 0.9)), "within_0.1m_share": float((d < 0.1).mean()),
+                "north_of_wall_share": float((pos[:, 1] > 0.05).mean())}
+    return out
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--R", type=int, default=4096)
@@ -175,8 +247,12 @@ def main():
     ap.add_argument("--fleet-margin", type=float, default=0.1)
     ap.add_argument("--fleet-w", type=float, default=1e3)
     ap.add_argument("--fleet-period", type=int, default=25)
+    ap.add_argument("--map", action="append", default=[], help="CELLS:P pairs (comma list or repeated): time cost maps")
+    ap.add_argument("--map-steps", type=int, default=40, help="planning steps of the wall scenario")
+    ap.add_argument("--parent-lib", default=None, help="another build's library: time its rk_plan_rollout_moving side by side")
     a = ap.parse_args()
     moving = [tuple(int(v) for v in x.split(":")) for arg in a.moving for x in arg.split(",") if x]
+    maps = [tuple(int(v) for v in x.split(":")) for arg in a.map for x in arg.split(",") if x]
     cem_iters, cem_elite = (int(x) for x in a.cem.split(":")) if a.cem else (0, 0)
     obst_m = [m for m in int_list(a.obstacles) if m > 0]
     obst_p = int_list(a.check_period) or [a.seg_len]
@@ -256,6 +332,64 @@ def main():
         p = path_buf[: K // P] if path else None
         pl.rollout(src, ref, 1.0, 10.0, 1e-9, obstacles=mov[(m, P)], w_obst=1e3, check_period=P, path=p)
 
+    # cost maps: CELLS x CELLS cells of 5 cm centred on the origin, walls of 1 - 4 cells by 4 - 40 cells at random, one per
+    # 160 cells of area, each cell of a wall costing 1.  The robots of these rollouts are the mid-move robots moved to
+    # random places over the world (1 m from its edge), so that their cells are spread over the whole map as in a
+    # building, not all in the few cells around the origin; discs around them as for --moving
+    worlds, map_tabs = {}, {}
+    if maps:
+        aos = layout.soa_to_aos(src.state.cpu().numpy().view(np.uint32), R, layout.VS_WORDS)
+        rng_w = np.random.default_rng(13)
+        half = max(c for c, _ in maps) * 0.05 / 2
+        pos1 = rng_w.uniform(-half + 1.0, half - 1.0, (R, 2)).astype(np.float32)
+        aos[:, layout.VS_POS_X], aos[:, layout.VS_POS_Y] = pos1[:, 0].view(np.uint32), pos1[:, 1].view(np.uint32)
+        src_map = VehicleBatch(R, dev)
+        src_map.load_state_soa(layout.aos_to_soa(aos))
+        map_path = torch.empty((K // min(P for _, P in maps), n, 2), dtype=torch.float32, device=dev)
+        ref_map = (torch.from_numpy(pos1).to(dev) + goal).unsqueeze(0).expand(n_seg, R, 2).contiguous()
+    for cells_n, P in maps:
+        if cells_n not in worlds:
+            g = np.zeros((cells_n, cells_n), dtype=np.float32)
+            for _ in range(cells_n * cells_n // 160):
+                h, w = (rng_w.integers(1, 5), rng_w.integers(4, 41))[:: 1 if rng_w.random() < 0.5 else -1]
+                y, x = rng_w.integers(0, cells_n - h), rng_w.integers(0, cells_n - w)
+                g[y:y + h, x:x + w] = 1.0
+            half = cells_n * 0.05 / 2
+            worlds[cells_n] = CostMap(torch.from_numpy(g).to(dev), (-half, -half), 0.05)
+        n_ck = K // P
+        for m in (0, 8):
+            d = np.zeros((m, R, 4), dtype=np.float32)
+            d[:, :, :2] = pos1[None] + rng_w.uniform(-0.15, 0.15, (m, R, 2))
+            d[:, :, 2] = rng_w.uniform(0.02, 0.08, (m, R))
+            t4 = np.repeat(d[None], n_ck, axis=0)
+            t4[..., :2] += np.cumsum(rng_w.uniform(-0.02, 0.02, (n_ck, m, R, 2)), axis=0).astype(np.float32)
+            map_tabs[(m, P)] = torch.from_numpy(t4).to(dev)
+
+    def map_moving(cells_n, P, m, use_map):
+        p = map_path[: K // P] if m == 0 else None  # m = 0 without a path would run rk_plan_rollout's kernel
+        pl.rollout(src_map, ref_map, 1.0, 10.0, 1e-9, obstacles=map_tabs[(m, P)], w_obst=1e3, check_period=P, path=p,
+                   costmap=worlds[cells_n] if use_map else None, w_map=1.0)
+
+    parent = None
+    if a.parent_lib:
+        assert maps, "--parent-lib times the discs of --map"
+        parent = C.CDLL(os.path.abspath(a.parent_lib), mode=C.RTLD_LOCAL)
+        parent.rk_plan_rollout_moving.argtypes = pl.lib.rk_plan_rollout_moving.argtypes
+        par_cost = torch.empty(n, dtype=torch.float32, device=dev)
+        par_P = sorted({P for _, P in maps} or {P for _, P in moving} or {seg_len})
+        par_tabs = map_tabs if maps else {}
+
+    def parent_moving(P, m, lib):
+        c = _cabi.PlanCost()
+        c.d_ref, c.w_pos, c.w_goal, c.w_cur = ref_map.data_ptr(), 1.0, 10.0, 1e-9
+        o = _cabi.PlanObstacles()
+        tab = par_tabs[(m, P)]
+        o.d_obs, o.m, o.check_period, o.w_obst = tab.data_ptr(), m, P, 1e3
+        out = pl.cost if lib is pl.lib else par_cost
+        pth = map_path[: K // P].data_ptr() if m == 0 else None
+        _cabi.check(lib.rk_plan_rollout_moving(C.byref(pl.params), src_map.state.data_ptr(), R, S, pl.candidates.data_ptr(), n_seg, seg_len,
+                                               C.byref(c), C.byref(o), pth, out.data_ptr(), C.c_void_p(torch.cuda.current_stream().cuda_stream)))
+
     def sample_sigma():
         pl.sample(nominal=nominal, seed=5, sigma_table=pl.sigma_table)
 
@@ -275,12 +409,19 @@ def main():
         pred = {P: pl.predict(src, P) for P in sorted({P for _, P in moving})}
         for P in pred:
             pl.peer_discs(pred[P], peers_m, 0.4)
+    for cells_n, P in maps:
+        for m in (0, 8):
+            map_moving(cells_n, P, m, False), map_moving(cells_n, P, m, True)
+    if parent is not None:
+        for P in par_P:
+            for m in (0, 8):
+                parent_moving(P, m, parent), parent_moving(P, m, pl.lib)
     torch.cuda.synchronize()
     src_before = src.state.clone()
     t = {"sample": [], "plan_rollout": [], "select": [], "plain_rollout": []}
     if a.cem:
         t.update(sample_sigma=[], refit=[])
-    t_obst, t_mov = {}, {}
+    t_obst, t_mov, t_map, t_par = {}, {}, {}, {}
     for _ in range(a.reps):
         t["sample"].append(timed(sample))
         if a.cem:
@@ -306,6 +447,17 @@ def main():
             for P in pred:
                 t_mov.setdefault(("predict", P), []).append(timed(lambda: pl.predict(src, P)))
                 t_mov.setdefault(("peer_discs", P), []).append(timed(lambda: pl.peer_discs(pred[P], peers_m, 0.4)))
+        for cells_n, P in maps:  # the moving rollout and the map rollout on the same discs, alternated
+            for m in (0, 8):
+                tm, tmap = t_map.setdefault((cells_n, P, m), ([], []))
+                tm.append(timed(lambda: map_moving(cells_n, P, m, False)))
+                tmap.append(timed(lambda: map_moving(cells_n, P, m, True)))
+        if parent is not None:  # the same rk_plan_rollout_moving call from the other build and from this one, alternated
+            for P in par_P:
+                for m in (0, 8):
+                    tpar, tthis = t_par.setdefault((P, m), ([], []))
+                    tpar.append(timed(lambda: parent_moving(P, m, parent)))
+                    tthis.append(timed(lambda: parent_moving(P, m, pl.lib)))
     assert torch.equal(src.state, src_before), "the plan rollout modified its source states"
     med = {k: float(np.median(v)) for k, v in t.items()}
     res = {
@@ -350,7 +502,32 @@ def main():
                            "ms_min": round(float(np.min(t_mov[("predict", P)])), 4)} for P in pred]
         res["peer_discs"] = [{"check_period": P, "G": G_m, "cells": (K // P) * (G_m - 1) * R,
                               "ms_median": round(float(np.median(t_mov[("peer_discs", P)])), 4)} for P in pred]
-    if moving or a.fleet:
+    if maps:
+        rows = []
+        for (cells_n, P, m), (tm, tmap) in t_map.items():
+            map_moving(cells_n, P, m, False)
+            base = pl.cost.clone()
+            map_moving(cells_n, P, m, True)
+            rows.append({"cells": cells_n, "map_bytes": cells_n * cells_n * 4, "check_period": P, "m": m,
+                         "ms_median_moving": round(float(np.median(tm)), 4), "ms_median_map": round(float(np.median(tmap)), 4),
+                         "ms_min_map": round(float(np.min(tmap)), 4), "ms_max_map": round(float(np.max(tmap)), 4),
+                         "map_over_moving": float(np.median(tmap) / np.median(tm)),
+                         "priced_fraction": (pl.cost != base).float().mean().item()})
+        res["map"] = rows
+        res["wall"] = wall_report(a, dev, *((cem_iters, cem_elite) if a.cem else (4, 8)))
+    if parent is not None:
+        rows = []
+        for (P, m), (tpar, tthis) in t_par.items():
+            parent_moving(P, m, parent)
+            parent_moving(P, m, pl.lib)
+            torch.cuda.synchronize()
+            rows.append({"check_period": P, "m": m, "path": m == 0, "ms_median_parent": round(float(np.median(tpar)), 4),
+                         "ms_median_this": round(float(np.median(tthis)), 4), "this_over_parent": float(np.median(tthis) / np.median(tpar)),
+                         "ms_min_max_parent": [round(float(np.min(tpar)), 4), round(float(np.max(tpar)), 4)],
+                         "ms_min_max_this": [round(float(np.min(tthis)), 4), round(float(np.max(tthis)), 4)],
+                         "same_bits": bool(torch.equal(par_cost.view(torch.int32), pl.cost.view(torch.int32)))})
+        res["parent_moving"] = rows
+    if moving or a.fleet or maps:
         res["max_sm_clock"] = power_limit("clocks.max.sm")
     if a.fleet:
         res["fleet"] = fleet_report(a, a.fleet, dev)
