@@ -807,6 +807,81 @@ int rk_plan_rollout_map(const rk_vdt_params_t *p, const void *d_src_state, int64
                         const rk_plan_obstacles_t *obst, const rk_plan_map_t *map, float *d_path, float *d_cost,
                         void *stream);
 
+/* Cost-to-go fields (navigation functions): the shortest-path distance from a goal through the free cells of a cost map,
+ * built on the device.  Used as a rollout's terminal cost it has no local minimum except at the goal, so robots route
+ * around walls and out of dead ends that the straight-line goal term w_goal * |pos - goal|^2 traps them in.
+ *   rk_plan_cost_to_go     map + goals [n_fields]                -> fields [n_fields][fh][fw] (synchronises the stream)
+ *   rk_plan_rollout_field  rk_plan_rollout_map + the field term  -> cost [R*S]
+ * Build fields when goals or the map change, not every planning step (INTEGRATION.md §2). */
+typedef struct rk_plan_ctg {
+  float step_axial, step_diag; /* metres per axial / diagonal step; finite, > 0 (e.g. float(res), float(res * sqrt(2))) */
+  float k_cost;                /* extra traversal cost per unit of cell cost; finite, >= 0 */
+  float lethal;                /* a cell with c >= lethal is not traversable; > 0, may be +inf (then only +inf cells block) */
+} rk_plan_ctg_t;               /* 16 bytes */
+
+/* Field f is a fw x fh window of map k = d_field_map[f] (NULL: 0) of `map`; window cell (ix, iy) is map cell
+ * (ox + ix, oy + iy), (ox, oy) = d_offset[f] (NULL: (0, 0)).  Cell (ix, iy) of field f is d_field[(f*fh + iy)*fw + ix].
+ * Every operation is one IEEE float32 operation in the written order, no contraction:
+ *   cost     c = map cell (ox + ix, oy + iy) of map k, or map->outside where that cell is off the map
+ *   blocked  c >= lethal  (NaN compares false: a NaN cell never blocks)
+ *   factor   t = c > 0 ? 1 + k_cost*c : 1
+ *   goal     gu = (gx - map->x0)*map->inv_res, gv likewise.  If gu >= (float)ox && gu < (float)(ox + fw) and the same for
+ *            gv, the goal cell is ((int)floorf(gu) - ox, (int)floorf(gv) - oy).  Otherwise the field has no goal and is
+ *            +inf everywhere: a NaN goal, a goal off the window, k outside [0, n_maps), or a window whose |ox|, |oy|,
+ *            |ox + fw| or |oy + fh| exceeds 2^24 (where (float) is no longer exact).
+ *   edges    the goal cell gets D = 0, even if blocked.  An edge p -> q runs to each of the 8 neighbours q of p that lies
+ *            in the window and is not blocked; a diagonal edge also needs both cells that share a side with p and with q
+ *            to be in the window and unblocked (no corner cutting).  Its weight is w = step * t_q (step_axial or
+ *            step_diag).
+ *   field    D(q) = the minimum over all paths from the goal of the left fold D = D + w; +inf where no path reaches q
+ *            (blocked cells other than the goal included).
+ * The bits do not depend on the order of relaxation: fl(a + w) is monotone in a and w >= 0, so every relaxation keeps D(q)
+ * an upper bound that some path attains, and any order that runs to a fixed point (Bellman-Ford in any order, chaotic
+ * in-place updates, or a float32 Dijkstra) stops at the same minimum.  The device relaxes 32 x 32 tiles in rounds, each
+ * tile in place in shared memory until it stops changing, and runs the next round over the tiles that changed and their
+ * neighbours; the host enqueues rounds in batches and reads the number of changed tiles after each batch, so the call
+ * synchronises `stream`.  It ends after the first round that changes nothing; no cap is needed, since values only
+ * decrease over finitely many floats.  *rounds_out (may be NULL) = the number of rounds that changed a cell.
+ * d_goal: float2 [n_fields] metres, 8-byte aligned; d_field_map: int32 [n_fields] (may be NULL); d_offset: int2
+ * [n_fields], 8-byte aligned (may be NULL); d_field: float [n_fields][fh][fw]; d_work: rk_plan_cost_to_go_work_bytes()
+ * bytes of device memory, 4-byte aligned, owned by the caller (nothing is allocated).
+ * RK_ERR_ARG, checked before any device call: map NULL or failing rk_plan_rollout_map's map checks (w_map is ignored);
+ * spec NULL; a step not finite or <= 0; k_cost negative, NaN or inf; lethal NaN or <= 0; n_fields, fw or fh < 1; fw or
+ * fh > 2^24; n_fields*fh*fw >= 2^31; d_goal, d_field or d_work NULL; a misaligned table. */
+int rk_plan_cost_to_go(const rk_plan_map_t *map, const rk_plan_ctg_t *spec, const float *d_goal, const int32_t *d_field_map,
+                       const int32_t *d_offset, int32_t n_fields, int32_t fw, int32_t fh, float *d_field, void *d_work,
+                       int32_t *rounds_out, void *stream);
+/* Bytes of d_work for rk_plan_cost_to_go; 0 for sizes it rejects. */
+size_t rk_plan_cost_to_go_work_bytes(int32_t n_fields, int32_t fw, int32_t fh);
+
+typedef struct rk_plan_field {
+  const float   *d_field;    /* float [n_fields][fh][fw] (rk_plan_cost_to_go's, or any caller's grid); 4-byte aligned */
+  const int32_t *d_field_of; /* int32 [R]: the field of robot r; NULL: field 0 for every robot */
+  const int32_t *d_offset;   /* int2 [n_fields]: the grid cell of window cell (0, 0); NULL: (0, 0); 8-byte aligned */
+  int32_t n_fields, fw, fh;  /* >= 1 each; n_fields*fh*fw < 2^31; fw, fh <= 2^24 */
+  float   x0, y0, inv_res;   /* the map's grid: the outer corner of grid cell (0, 0), cells per metre; finite, inv_res > 0 */
+  float   outside;           /* the value off the window; may be +inf; NaN rejected */
+  float   w_field;           /* finite, >= 0 */
+} rk_plan_field_t;           /* 56 bytes */
+
+/* rk_plan_rollout_map plus a terminal cost-to-go term, read at the state after the last tick (after the last checkpoint's
+ * map term), into the same O.  One IEEE float32 operation each, in the written order:
+ *   f = d_field_of ? d_field_of[r] : 0;     f < 0 or f >= n_fields: no term for robot r
+ *   u = (x - x0) * inv_res;  v = (y - y0) * inv_res;  (ox, oy) = d_offset ? d_offset[f] : (0, 0)
+ *   c = field cell ((int)floorf(u) - ox, (int)floorf(v) - oy) of field f if (u, v) lies in the window by the comparisons
+ *       of rk_plan_cost_to_go's goal cell (the same 2^24 rule), else outside
+ *   if (c > 0) O = O + w_field * c;         d_cost = J + O
+ * With ox, oy >= 0 this is the cell plan_map reads for the same map grid.  A blocked or unreachable cell (+inf) prices
+ * the candidate at +inf; a NaN cell adds nothing.  map may be NULL (no map term).  field == NULL or w_field == 0 is
+ * rk_plan_rollout_map (the same kernel and bits).
+ * RK_ERR_ARG: rk_plan_rollout_map's checks; n_fields, fw or fh < 1, fw or fh > 2^24, n_fields*fh*fw >= 2^31; x0, y0 or
+ * inv_res not finite, inv_res <= 0; outside NaN; w_field negative, NaN or inf; d_field NULL, or a misaligned table.
+ * R == 0 is a no-op. */
+int rk_plan_rollout_field(const rk_vdt_params_t *p, const void *d_src_state, int64_t R, int32_t S,
+                          const rk_vdt_cmd_t *d_cmd, int32_t n_seg, int32_t seg_len, const rk_plan_cost_t *cost,
+                          const rk_plan_obstacles_t *obst, const rk_plan_map_t *map, const rk_plan_field_t *field,
+                          float *d_path, float *d_cost, void *stream);
+
 /* =====================================================================================
  * RobotManager guard (SURVEY 8f-2): the vehicle-management block of RMT's routine_ros()
  * (src/RobotManager/RM_task_main.cpp:484-767), one call = K manager cycles of n robots.  Per

@@ -17,7 +17,7 @@ def __getattr__(name):
         from . import vehicle as _v
 
         return _v if name == "vehicle" else _v.VehicleBatch
-    if name in ("planner", "VehiclePlanner", "CostMap"):
+    if name in ("planner", "VehiclePlanner", "CostMap", "CostToGo"):
         from . import planner as _p
 
         return _p if name == "planner" else getattr(_p, name)

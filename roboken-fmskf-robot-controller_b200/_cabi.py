@@ -189,6 +189,19 @@ class PlanMap(C.Structure):
                 ("x0", C.c_float), ("y0", C.c_float), ("inv_res", C.c_float), ("outside", C.c_float), ("w_map", C.c_float)]
 
 
+class PlanCtg(C.Structure):
+    """rk_plan_ctg_t"""
+
+    _fields_ = [("step_axial", C.c_float), ("step_diag", C.c_float), ("k_cost", C.c_float), ("lethal", C.c_float)]
+
+
+class PlanField(C.Structure):
+    """rk_plan_field_t"""
+
+    _fields_ = [("d_field", C.c_void_p), ("d_field_of", C.c_void_p), ("d_offset", C.c_void_p), ("n_fields", C.c_int32), ("fw", C.c_int32),
+                ("fh", C.c_int32), ("x0", C.c_float), ("y0", C.c_float), ("inv_res", C.c_float), ("outside", C.c_float), ("w_field", C.c_float)]
+
+
 class PlanRefit(C.Structure):
     """rk_plan_refit_t"""
 
@@ -249,6 +262,12 @@ def _proto(lib):
                                            C.POINTER(PlanObstacles), vp, vp, vp]
     lib.rk_plan_rollout_map.argtypes = [C.POINTER(VdtParams), vp, C.c_int64, C.c_int32, vp, C.c_int32, C.c_int32, C.POINTER(PlanCost),
                                         C.POINTER(PlanObstacles), C.POINTER(PlanMap), vp, vp, vp]
+    lib.rk_plan_rollout_field.argtypes = [C.POINTER(VdtParams), vp, C.c_int64, C.c_int32, vp, C.c_int32, C.c_int32, C.POINTER(PlanCost),
+                                          C.POINTER(PlanObstacles), C.POINTER(PlanMap), C.POINTER(PlanField), vp, vp, vp]
+    lib.rk_plan_cost_to_go.argtypes = [C.POINTER(PlanMap), C.POINTER(PlanCtg), vp, vp, vp, C.c_int32, C.c_int32, C.c_int32, vp, vp,
+                                       C.POINTER(C.c_int32), vp]
+    lib.rk_plan_cost_to_go_work_bytes.argtypes = [C.c_int32, C.c_int32, C.c_int32]
+    lib.rk_plan_cost_to_go_work_bytes.restype = C.c_size_t
     lib.rk_plan_peer_discs.argtypes = [vp, C.c_int64, C.c_int32, vp, C.c_int32, C.c_float, vp, C.c_int32, C.c_int32, vp]
     lib.rk_plan_select.argtypes = [vp, vp, C.c_int64, C.c_int32, C.c_int32, C.c_float, C.c_int32, vp, vp, vp, vp]
     lib.rk_plan_sample_commands_sigma.argtypes = [C.POINTER(VdtParams), C.POINTER(PlanSample), vp, vp, C.c_int64, C.c_int32, C.c_int32, vp,

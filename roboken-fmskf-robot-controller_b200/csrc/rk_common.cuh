@@ -48,6 +48,16 @@ RK_DEV void st_plane(uint4 *blk, int64_t n, int pl, int64_t i, uint4 v) { __stcs
 RK_DEV float u2f(uint32_t u) { return __uint_as_float(u); }
 RK_DEV uint32_t f2u(float f) { return __float_as_uint(f); }
 
+// The cost-to-go window cell under grid coordinates (u, v) (rk_plan_cost_to_go's goal cell and rk_plan_rollout_field's
+// lookup): a window of w x h cells whose cell (0, 0) is grid cell o.  False when (u, v) is off the window, NaN, or the
+// window's edges |o| or |o + size| exceed 2^24, where (float) would no longer be exact.
+RK_DEV bool plan_window_cell(float u, float v, int2 o, int32_t w, int32_t h, int &ix, int &iy) {
+  if(!(o.x >= -(1 << 24) && o.x <= (1 << 24) - w && o.y >= -(1 << 24) && o.y <= (1 << 24) - h)) return false;
+  if(!(u >= (float)o.x && u < (float)(o.x + w) && v >= (float)o.y && v < (float)(o.y + h))) return false;
+  ix = (int)floorf(u) - o.x, iy = (int)floorf(v) - o.y;
+  return true;
+}
+
 } // namespace rk
 
 // ---- host-side error plumbing --------------------------------------------------------
@@ -60,6 +70,10 @@ int imt_update_launch(void *d_state, int64_t n, int32_t K, const int16_t *d_regs
                       float *d_yaw_rad, int do_init, int max_ctas, void *stream, const void *d_desc = nullptr);
 int adt_update_launch(const rk_adt_params_t *p, void *d_state, const void *d_cmdtab, int64_t n, int32_t K, uint32_t *d_trace,
                       int max_ctas, void *stream);
+// rk_plan_rollout_map's checks of an rk_plan_map_t, shared with rk_plan_cost_to_go: the grid (sizes, origin, resolution,
+// outside; not w_map) and the tables
+int plan_check_map_grid(const char *who, const rk_plan_map_t *map);
+int plan_check_map_tables(const char *who, const rk_plan_map_t *map);
 } // namespace rk
 
 #define RK_CUDA(call)                                        \

@@ -1,6 +1,7 @@
 // rk_plan.cu -- the two ends of a planning step around rk_plan_rollout (rk_vehicle.cu): candidate commands sampled
 // around a nominal plan, and the per-robot choice among the candidates' costs (include/robotick.h, "Vehicle sampling
-// planner").  Candidate j of robot r is instance r*S + j, so a robot's S candidates are contiguous in every table.
+// planner"); and the planner kernels outside the rollout: peer discs and cost-to-go fields.  Candidate j of robot r is
+// instance r*S + j, so a robot's S candidates are contiguous in every table.
 #include <limits.h>
 #include <math.h>
 
@@ -260,6 +261,138 @@ plan_peer_discs_kernel(const float2 *__restrict__ path, int64_t R, int n_ck, con
   }
 }
 
+// rk_plan_cost_to_go: one CTA per 32 x 32 tile of a field window, tiles numbered field-major then row-major.  Each
+// thread owns column tx of rows ty, ty + 8, ty + 16, ty + 24 of its tile.
+constexpr int kCtgTile = 32, kCtgHalo = kCtgTile + 2, kCtgThreads = 256, kCtgRows = kCtgThreads / kCtgTile;
+constexpr int kCtgMaxBatch = 64; // rounds per batch at most (the batch doubles from 4)
+
+struct CtgArgs {
+  const float   *cells; // the map, [n_maps][height][width]
+  int32_t        n_maps, width, height;
+  float          x0, y0, inv_res, outside;
+  float          step_a, step_d, k_cost, lethal;
+  const float2  *goal;      // [n_fields]
+  const int32_t *field_map; // [n_fields]; NULL: map 0
+  const int2    *offset;    // [n_fields]; NULL: (0, 0)
+  int32_t        fw, fh, tiles_x, tiles_y;
+  float         *field; // [n_fields][fh][fw]
+};
+
+struct CtgTile {
+  int  f, x0, y0; // the field, and the window cell of the tile's cell (0, 0)
+  int  k;         // the field's map
+  int2 o;         // the field's offset
+};
+RK_DEV CtgTile ctg_tile(const CtgArgs &a, int t) {
+  const int per = a.tiles_x * a.tiles_y, f = t / per, q = t - f * per, ty = q / a.tiles_x;
+  CtgTile c;
+  c.f = f, c.x0 = (q - ty * a.tiles_x) * kCtgTile, c.y0 = ty * kCtgTile;
+  c.k = a.field_map != nullptr ? __ldg(a.field_map + f) : 0;
+  c.o = a.offset != nullptr ? __ldg(a.offset + f) : make_int2(0, 0);
+  return c;
+}
+// The cost c of window cell (ix, iy) (in the window, of a field whose map index is in range and |offset| <= 2^24)
+RK_DEV float ctg_cost(const CtgArgs &a, const CtgTile &c, int ix, int iy) {
+  const int mx = c.o.x + ix, my = c.o.y + iy;
+  return (mx >= 0 && mx < a.width && my >= 0 && my < a.height) ? __ldg(a.cells + (c.k * a.height + my) * a.width + mx) : a.outside;
+}
+
+// D = +inf over the tile's cells, 0 at the goal cell; dirty[t] = the goal lies in tile t
+__global__ void __launch_bounds__(kCtgThreads) plan_ctg_init_kernel(const CtgArgs a, uint32_t *__restrict__ dirty) {
+  const CtgTile c = ctg_tile(a, blockIdx.x);
+  int           gx = -1, gy = -1;
+  if((uint32_t)c.k < (uint32_t)a.n_maps) {
+    const float2 g = __ldg(a.goal + c.f);
+    plan_window_cell(fmul(fsub(g.x, a.x0), a.inv_res), fmul(fsub(g.y, a.y0), a.inv_res), c.o, a.fw, a.fh, gx, gy);
+  }
+  float *D = a.field + (int64_t)c.f * a.fh * a.fw;
+  for(int q = threadIdx.x; q < kCtgTile * kCtgTile; q += kCtgThreads) {
+    const int ix = c.x0 + (q & (kCtgTile - 1)), iy = c.y0 + q / kCtgTile;
+    if(ix < a.fw && iy < a.fh) D[iy * a.fw + ix] = (ix == gx && iy == gy) ? 0.0f : __int_as_float(0x7F800000);
+  }
+  if(threadIdx.x == 0) dirty[blockIdx.x] = (gx >= c.x0 && gx < c.x0 + kCtgTile && gy >= c.y0 && gy < c.y0 + kCtgTile) ? 1u : 0u;
+}
+
+// One round: a tile runs if it or one of its 8 neighbours changed in the previous round (dirty_in).  It loads D with a
+// 1-cell halo into shared memory, relaxes its cells in place until a sweep changes nothing, writes back the cells that
+// decreased, and reports in dirty_out (every tile writes its flag, so the buffer needs no clearing) and *count.
+// Other tiles may write the halo's cells during the round: a read sees the old or the new value, both upper bounds that
+// some path attains, and a tile that changed runs its neighbours again in the next round.
+__global__ void __launch_bounds__(kCtgThreads)
+plan_ctg_relax_kernel(const CtgArgs a, const uint32_t *__restrict__ dirty_in, uint32_t *__restrict__ dirty_out, int32_t *__restrict__ count) {
+  __shared__ float   sD[kCtgHalo][kCtgHalo];
+  __shared__ uint8_t sOk[kCtgHalo][kCtgHalo]; // in the window and not blocked
+  const int          t  = blockIdx.x;
+  const int          per = a.tiles_x * a.tiles_y, tq = t % per, tyi = tq / a.tiles_x, txi = tq - tyi * a.tiles_x;
+  bool               go = false;
+  if(threadIdx.x < 9) {
+    const int ny = tyi + (int)threadIdx.x / 3 - 1, nx = txi + (int)threadIdx.x % 3 - 1;
+    go = ny >= 0 && ny < a.tiles_y && nx >= 0 && nx < a.tiles_x && dirty_in[t - tq + ny * a.tiles_x + nx] != 0u;
+  }
+  if(!__syncthreads_or(go)) {
+    if(threadIdx.x == 0) dirty_out[t] = 0u;
+    return;
+  }
+  const CtgTile c = ctg_tile(a, t);
+  float        *D = a.field + (int64_t)c.f * a.fh * a.fw;
+  for(int q = threadIdx.x; q < kCtgHalo * kCtgHalo; q += kCtgThreads) {
+    const int hy = q / kCtgHalo, hx = q - hy * kCtgHalo, ix = c.x0 + hx - 1, iy = c.y0 + hy - 1;
+    float     d  = __int_as_float(0x7F800000);
+    bool      ok = false;
+    if(ix >= 0 && ix < a.fw && iy >= 0 && iy < a.fh) d = D[iy * a.fw + ix], ok = !(ctg_cost(a, c, ix, iy) >= a.lethal);
+    sD[hy][hx] = d, sOk[hy][hx] = ok;
+  }
+  __syncthreads();
+  const int tx = threadIdx.x & (kCtgTile - 1), ty = threadIdx.x / kCtgTile, x = tx + 1;
+  float     wa[4], wd[4], d0[4];
+  uint32_t  diag = 0u; // bits 4j .. 4j+3: the diagonal edges into row j's cell that may be taken (-,-), (+,-), (-,+), (+,+)
+  bool      mine[4];
+#pragma unroll
+  for(int j = 0; j < 4; j++) {
+    const int y = ty + kCtgRows * j + 1;
+    mine[j]     = sOk[y][x] != 0;
+    d0[j]       = sD[y][x];
+    wa[j] = wd[j] = 0.0f;
+    if(mine[j]) {
+      const float cq = ctg_cost(a, c, c.x0 + tx, c.y0 + y - 1);
+      const float tq = cq > 0.0f ? fadd(1.0f, fmul(a.k_cost, cq)) : 1.0f;
+      wa[j] = fmul(a.step_a, tq), wd[j] = fmul(a.step_d, tq);
+      const bool l = sOk[y][x - 1], r = sOk[y][x + 1], dn = sOk[y - 1][x], up = sOk[y + 1][x];
+      diag |= ((l && dn ? 1u : 0u) | (r && dn ? 2u : 0u) | (l && up ? 4u : 0u) | (r && up ? 8u : 0u)) << (4 * j);
+    }
+  }
+  const float inf = __int_as_float(0x7F800000);
+  volatile float(*s)[kCtgHalo] = sD;
+  for(;;) {
+    bool ch = false;
+#pragma unroll
+    for(int j = 0; j < 4; j++) {
+      if(!mine[j]) continue;
+      const int      y = ty + kCtgRows * j + 1;
+      const uint32_t b = diag >> (4 * j);
+      // fl(a + w) is monotone in a: the least of the candidates D(p) + w is the least D(p) plus w
+      const float ma = fminf(fminf(s[y][x - 1], s[y][x + 1]), fminf(s[y - 1][x], s[y + 1][x]));
+      const float md = fminf(fminf((b & 1u) ? s[y - 1][x - 1] : inf, (b & 2u) ? s[y - 1][x + 1] : inf),
+                             fminf((b & 4u) ? s[y + 1][x - 1] : inf, (b & 8u) ? s[y + 1][x + 1] : inf));
+      const float nd = fminf(fadd(ma, wa[j]), fadd(md, wd[j]));
+      if(nd < s[y][x]) s[y][x] = nd, ch = true;
+    }
+    if(!__syncthreads_or(ch)) break;
+  }
+  bool changed = false;
+#pragma unroll
+  for(int j = 0; j < 4; j++) {
+    const int   y = ty + kCtgRows * j + 1;
+    const float d = sD[y][x];
+    if(mine[j] && d < d0[j]) D[(c.y0 + y - 1) * a.fw + c.x0 + tx] = d, changed = true;
+  }
+  changed = __syncthreads_or(changed);
+  if(threadIdx.x == 0) {
+    dirty_out[t] = changed ? 1u : 0u;
+    if(changed) atomicAdd(count, 1);
+  }
+}
+
 static bool overlap(const void *a, size_t na, const void *b, size_t nb) {
   const uintptr_t x = (uintptr_t)a, y = (uintptr_t)b;
   return x < y + nb && y < x + na;
@@ -343,6 +476,12 @@ static int plan_check_choice_tables(const char *who, const float *d_cost, const 
     return RK_ERR_ARG;
   }
   return RK_OK;
+}
+
+// Tiles of a cost-to-go build; 0 for sizes rk_plan_cost_to_go rejects
+static int64_t ctg_tiles(int32_t n_fields, int32_t fw, int32_t fh) {
+  if(n_fields < 1 || fw < 1 || fh < 1 || fw > (1 << 24) || fh > (1 << 24) || (int64_t)n_fields * fh * fw > INT_MAX) return 0;
+  return (int64_t)n_fields * ((fw + kCtgTile - 1) / kCtgTile) * ((fh + kCtgTile - 1) / kCtgTile);
 }
 
 } // namespace rk
@@ -453,6 +592,75 @@ int rk_plan_peer_discs(const float *d_path, int64_t R, int32_t n_ck, const int32
   plan_peer_discs_kernel<<<grid, RK_PLAN_BLOCK, 0, (cudaStream_t)stream>>>((const float2 *)d_path, R, n_ck, d_peer, m, radius,
                                                                             (float4 *)d_obs, M, k0);
   RK_CUDA(cudaGetLastError());
+  return RK_OK;
+}
+
+size_t rk_plan_cost_to_go_work_bytes(int32_t n_fields, int32_t fw, int32_t fh) {
+  const int64_t T = ctg_tiles(n_fields, fw, fh);
+  return T == 0 ? 0 : (size_t)(kCtgMaxBatch + 2 * T) * sizeof(uint32_t);
+}
+
+int rk_plan_cost_to_go(const rk_plan_map_t *map, const rk_plan_ctg_t *spec, const float *d_goal, const int32_t *d_field_map,
+                       const int32_t *d_offset, int32_t n_fields, int32_t fw, int32_t fh, float *d_field, void *d_work, int32_t *rounds_out,
+                       void *stream) {
+  static const char *who = "rk_plan_cost_to_go";
+  if(!map || !spec) {
+    set_error("%s: NULL map/spec", who);
+    return RK_ERR_ARG;
+  }
+  if(int rc = plan_check_map_grid(who, map)) return rc;
+  if(int rc = plan_check_map_tables(who, map)) return rc;
+  if(!isfinite(spec->step_axial) || !(spec->step_axial > 0.0f) || !isfinite(spec->step_diag) || !(spec->step_diag > 0.0f)) {
+    set_error("%s: step_axial and step_diag must be finite and > 0", who);
+    return RK_ERR_ARG;
+  }
+  if(!(spec->k_cost >= 0.0f) || isinf(spec->k_cost)) {
+    set_error("%s: k_cost must be finite and >= 0", who);
+    return RK_ERR_ARG;
+  }
+  if(!(spec->lethal > 0.0f)) {
+    set_error("%s: lethal must be > 0 (+inf allowed, NaN not)", who);
+    return RK_ERR_ARG;
+  }
+  const int64_t T = ctg_tiles(n_fields, fw, fh);
+  if(T == 0) {
+    set_error("%s: need n_fields, fw, fh >= 1, fw, fh <= 2^24 and n_fields * fh * fw < 2^31 (n_fields = %d, fw = %d, fh = %d)", who,
+              n_fields, fw, fh);
+    return RK_ERR_ARG;
+  }
+  if(!d_goal || ((uintptr_t)d_goal & 7u) || ((uintptr_t)d_field_map & 3u) || ((uintptr_t)d_offset & 7u) || !d_field ||
+     ((uintptr_t)d_field & 3u) || !d_work || ((uintptr_t)d_work & 3u)) {
+    set_error("%s: d_goal (float2) and d_offset (int2, may be NULL) must be 8-byte aligned, d_field_map (int32, may be NULL), "
+              "d_field (float) and d_work 4-byte aligned, and d_goal, d_field and d_work non-NULL",
+              who);
+    return RK_ERR_ARG;
+  }
+  if(int rc = require_device()) return rc;
+  CtgArgs a;
+  a.cells = map->d_cells, a.n_maps = map->n_maps, a.width = map->width, a.height = map->height;
+  a.x0 = map->x0, a.y0 = map->y0, a.inv_res = map->inv_res, a.outside = map->outside;
+  a.step_a = spec->step_axial, a.step_d = spec->step_diag, a.k_cost = spec->k_cost, a.lethal = spec->lethal;
+  a.goal = (const float2 *)d_goal, a.field_map = d_field_map, a.offset = (const int2 *)d_offset;
+  a.fw = fw, a.fh = fh, a.tiles_x = (fw + kCtgTile - 1) / kCtgTile, a.tiles_y = (fh + kCtgTile - 1) / kCtgTile;
+  a.field = d_field;
+  int32_t     *count = (int32_t *)d_work;
+  uint32_t    *dirty[2] = {(uint32_t *)d_work + kCtgMaxBatch, (uint32_t *)d_work + kCtgMaxBatch + T};
+  cudaStream_t st = (cudaStream_t)stream;
+  plan_ctg_init_kernel<<<(unsigned)T, kCtgThreads, 0, st>>>(a, dirty[0]);
+  RK_CUDA(cudaGetLastError());
+  int32_t rounds = 0, host[kCtgMaxBatch];
+  for(int batch = 4, cur = 0;; batch = min(2 * batch, kCtgMaxBatch)) {
+    RK_CUDA(cudaMemsetAsync(count, 0, batch * sizeof(int32_t), st));
+    for(int b = 0; b < batch; b++, cur ^= 1) plan_ctg_relax_kernel<<<(unsigned)T, kCtgThreads, 0, st>>>(a, dirty[cur], dirty[cur ^ 1], count + b);
+    RK_CUDA(cudaGetLastError());
+    RK_CUDA(cudaMemcpyAsync(host, count, batch * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    RK_CUDA(cudaStreamSynchronize(st));
+    int b = 0;
+    while(b < batch && host[b] != 0) b++;
+    rounds += b;
+    if(b < batch) break; // a round changed nothing: every later one is empty
+  }
+  if(rounds_out) *rounds_out = rounds;
   return RK_OK;
 }
 

@@ -100,12 +100,18 @@ struct PlanObstArgs : PlanArgs {
 };
 // rk_plan_rollout_moving: a disc table per checkpoint, and the candidates' positions at the checkpoints if path != NULL.
 // rk_plan_rollout_map: the cost grid (rk_plan_map_t) if cells != NULL; the host leaves it NULL for w_map == 0.
+// rk_plan_rollout_field: the cost-to-go term (rk_plan_field_t) if field != NULL; likewise NULL for w_field == 0.
 struct PlanMovingArgs : PlanObstArgs {
   float2        *path;   // [n_ck][R * S], metres
   const float   *cells;  // [n_maps][height][width]
   const int32_t *map_of; // [R]; NULL: map 0
   int32_t        n_maps, width, height;
   float          x0, y0, inv_res, outside, w_map;
+  const float   *field;    // [n_fields][fh][fw]
+  const int32_t *field_of; // [R]; NULL: field 0
+  const int2    *f_offset; // [n_fields]; NULL: (0, 0)
+  int32_t        n_fields, fw, fh;
+  float          fx0, fy0, finv_res, foutside, w_field;
 };
 // OBST: 0 no discs (PlanArgs), kObstStatic rk_plan_rollout_obstacles (PlanObstArgs), kObstMoving rk_plan_rollout_moving
 // (PlanMovingArgs)
@@ -156,6 +162,19 @@ RK_DEV float plan_moving_cost(float O, float x, float y, const PlanMovingArgs &p
   if(pl.cells != nullptr) O = plan_map_cost(O, x, y, pl, r);
   return O;
 }
+// O after the cost-to-go term of rk_plan_rollout_field at the end position (x, y): one field index, one offset and one
+// cell load per candidate, in the epilogue only, so that the checkpoint branch inside the tick loop does not grow.
+RK_DEV float plan_field_cost(float O, float x, float y, const PlanMovingArgs &pl, uint32_t r) {
+  const int32_t f = pl.field_of != nullptr ? __ldg(pl.field_of + r) : 0;
+  if((uint32_t)f >= (uint32_t)pl.n_fields) return O; // no term for this robot
+  const int2  o = pl.f_offset != nullptr ? __ldg(pl.f_offset + f) : make_int2(0, 0);
+  const float u = fmul(fsub(x, pl.fx0), pl.finv_res), v = fmul(fsub(y, pl.fy0), pl.finv_res);
+  float       c = pl.foutside;
+  int         ix, iy;
+  if(plan_window_cell(u, v, o, pl.fw, pl.fh, ix, iy)) c = __ldg(pl.field + (f * pl.fh + iy) * pl.fw + ix);
+  if(c > 0.0f) O = fadd(O, fmul(pl.w_field, c));
+  return O;
+}
 
 // The start state of thread i: under PLAN, candidate i = r * S + j starts from robot r's block (the S candidates of robot
 // r read the same cells: one broadcast per warp).  Returns r (0 without PLAN).
@@ -176,7 +195,9 @@ template <bool PLAN, int OBST>
 RK_DEV void rollout_store(uint4 *state, int64_t n, int64_t i, const rk_vdt_rollout_t &a, const PlanArgsOf<OBST> &pl, const Veh &v,
                           float J, float O, int64_t r) {
   if constexpr(OBST == kObstMoving) {
-    pl.cost[i] = fadd(plan_stage_cost(J, v, pl, a.n_seg - 1, a.n_seg, r), plan_moving_cost(O, v.pos[0], v.pos[1], pl, r, n, i, a.steps / pl.P - 1, true));
+    O = plan_moving_cost(O, v.pos[0], v.pos[1], pl, r, n, i, a.steps / pl.P - 1, true);
+    if(pl.field != nullptr) O = plan_field_cost(O, v.pos[0], v.pos[1], pl, r);
+    pl.cost[i] = fadd(plan_stage_cost(J, v, pl, a.n_seg - 1, a.n_seg, r), O);
   } else if constexpr(OBST) {
     pl.cost[i] = fadd(plan_stage_cost(J, v, pl, a.n_seg - 1, a.n_seg, r), plan_obst_cost(O, v.pos[0], v.pos[1], pl, r));
   } else if constexpr(PLAN) {
@@ -869,11 +890,37 @@ static void launch_plan(const rk_vdt_params_t &p, const void *d_src, int64_t n, 
     vdt_rollout_kernel<RK_SENSOR_PLANT, false, true, OBST><<<grid, kRolloutThreads, 0, st>>>(p, src, n, a, pl);
   }
 }
-// rk_plan_rollout (ob == NULL), rk_plan_rollout_obstacles, rk_plan_rollout_moving (moving) and rk_plan_rollout_map
-// (moving, map): the same checks, and without discs, path or map the same kernels
+int plan_check_map_grid(const char *who, const rk_plan_map_t *map) {
+  if(map->n_maps < 1 || map->width < 1 || map->height < 1 || map->width > (1 << 24) || map->height > (1 << 24) ||
+     (int64_t)map->n_maps * map->height * map->width > INT_MAX) {
+    set_error("%s: need n_maps, width, height >= 1, width, height <= 2^24 and n_maps * height * width < 2^31 (n_maps = %d, "
+              "width = %d, height = %d)",
+              who, map->n_maps, map->width, map->height);
+    return RK_ERR_ARG;
+  }
+  if(!isfinite(map->x0) || !isfinite(map->y0) || !isfinite(map->inv_res) || !(map->inv_res > 0.0f)) {
+    set_error("%s: map x0, y0 and inv_res must be finite, and inv_res > 0", who);
+    return RK_ERR_ARG;
+  }
+  if(isnan(map->outside)) {
+    set_error("%s: map outside must not be NaN (+-inf allowed)", who);
+    return RK_ERR_ARG;
+  }
+  return RK_OK;
+}
+int plan_check_map_tables(const char *who, const rk_plan_map_t *map) {
+  if(!map->d_cells || ((uintptr_t)map->d_cells & 3u) || ((uintptr_t)map->d_map_of & 3u)) {
+    set_error("%s: map->d_cells (float) must be a non-NULL device pointer and map->d_map_of (int32, may be NULL) 4-byte aligned", who);
+    return RK_ERR_ARG;
+  }
+  return RK_OK;
+}
+// rk_plan_rollout (ob == NULL), rk_plan_rollout_obstacles, rk_plan_rollout_moving (moving), rk_plan_rollout_map (moving,
+// map) and rk_plan_rollout_field (moving, map, field): the same checks, and without discs, path, map or field the same
+// kernels
 static int plan_rollout(const char *who, const rk_vdt_params_t *p, const void *d_src_state, int64_t R, int32_t S, const rk_vdt_cmd_t *d_cmd,
                         int32_t n_seg, int32_t seg_len, const rk_plan_cost_t *cost, const rk_plan_obstacles_t *ob, bool moving,
-                        const rk_plan_map_t *map, float *d_path, float *d_cost, void *stream) {
+                        const rk_plan_map_t *map, const rk_plan_field_t *field, float *d_path, float *d_cost, void *stream) {
   if(!p || !cost) {
     set_error("%s: NULL params/cost", who);
     return RK_ERR_ARG;
@@ -913,23 +960,29 @@ static int plan_rollout(const char *who, const rk_vdt_params_t *p, const void *d
     }
   }
   if(map) {
-    if(map->n_maps < 1 || map->width < 1 || map->height < 1 || map->width > (1 << 24) || map->height > (1 << 24) ||
-       (int64_t)map->n_maps * map->height * map->width > INT_MAX) {
-      set_error("%s: need n_maps, width, height >= 1, width, height <= 2^24 and n_maps * height * width < 2^31 (n_maps = %d, "
-                "width = %d, height = %d)",
-                who, map->n_maps, map->width, map->height);
-      return RK_ERR_ARG;
-    }
-    if(!isfinite(map->x0) || !isfinite(map->y0) || !isfinite(map->inv_res) || !(map->inv_res > 0.0f)) {
-      set_error("%s: map x0, y0 and inv_res must be finite, and inv_res > 0", who);
-      return RK_ERR_ARG;
-    }
-    if(isnan(map->outside)) {
-      set_error("%s: map outside must not be NaN (+-inf allowed)", who);
-      return RK_ERR_ARG;
-    }
+    if(int rc = plan_check_map_grid(who, map)) return rc;
     if(!(map->w_map >= 0.0f)) {
       set_error("%s: w_map must be >= 0 (+inf allowed, NaN not)", who);
+      return RK_ERR_ARG;
+    }
+  }
+  if(field) {
+    if(field->n_fields < 1 || field->fw < 1 || field->fh < 1 || field->fw > (1 << 24) || field->fh > (1 << 24) ||
+       (int64_t)field->n_fields * field->fh * field->fw > INT_MAX) {
+      set_error("%s: need n_fields, fw, fh >= 1, fw, fh <= 2^24 and n_fields * fh * fw < 2^31 (n_fields = %d, fw = %d, fh = %d)", who,
+                field->n_fields, field->fw, field->fh);
+      return RK_ERR_ARG;
+    }
+    if(!isfinite(field->x0) || !isfinite(field->y0) || !isfinite(field->inv_res) || !(field->inv_res > 0.0f)) {
+      set_error("%s: field x0, y0 and inv_res must be finite, and inv_res > 0", who);
+      return RK_ERR_ARG;
+    }
+    if(isnan(field->outside)) {
+      set_error("%s: field outside must not be NaN (+-inf allowed)", who);
+      return RK_ERR_ARG;
+    }
+    if(!(field->w_field >= 0.0f) || isinf(field->w_field)) {
+      set_error("%s: w_field must be finite and >= 0", who);
       return RK_ERR_ARG;
     }
   }
@@ -945,11 +998,16 @@ static int plan_rollout(const char *who, const rk_vdt_params_t *p, const void *d
     set_error("%s: obst->d_obs must be a non-NULL 16-byte aligned device pointer when m > 0", who);
     return RK_ERR_ARG;
   }
-  if(map && (!map->d_cells || ((uintptr_t)map->d_cells & 3u) || ((uintptr_t)map->d_map_of & 3u))) {
-    set_error("%s: map->d_cells (float) must be a non-NULL device pointer and map->d_map_of (int32, may be NULL) 4-byte aligned", who);
+  if(map)
+    if(int rc = plan_check_map_tables(who, map)) return rc;
+  if(field && (!field->d_field || ((uintptr_t)field->d_field & 3u) || ((uintptr_t)field->d_field_of & 3u) || ((uintptr_t)field->d_offset & 7u))) {
+    set_error("%s: field->d_field (float) must be a non-NULL device pointer, field->d_field_of (int32) 4-byte and field->d_offset "
+              "(int2) 8-byte aligned (both may be NULL)",
+              who);
     return RK_ERR_ARG;
   }
-  const bool use_map = map && map->w_map > 0.0f; // w_map == 0 is the rollout without the map (and never 0 * inf)
+  const bool use_map   = map && map->w_map > 0.0f;         // w_map == 0 is the rollout without the map (and never 0 * inf)
+  const bool use_field = field && field->w_field > 0.0f; // likewise
   if(int rc = require_device()) return rc;
   rk_vdt_rollout_t a;
   memset(&a, 0, sizeof(a));
@@ -960,13 +1018,19 @@ static int plan_rollout(const char *who, const rk_vdt_params_t *p, const void *d
   pl.w_pos = cost->w_pos, pl.w_goal = cost->w_goal, pl.w_cur = cost->w_cur, pl.cost = d_cost;
   const int64_t n  = R * (int64_t)S;
   cudaStream_t  st = (cudaStream_t)stream;
-  if(obst || d_path || use_map) {
+  if(obst || d_path || use_map || use_field) {
     pl.obs = reinterpret_cast<const float4 *>(ob->d_obs), pl.m = ob->m, pl.P = ob->check_period, pl.w_obst = ob->w_obst;
     pl.path = reinterpret_cast<float2 *>(d_path);
     pl.cells = use_map ? map->d_cells : nullptr, pl.map_of = use_map ? map->d_map_of : nullptr;
     if(use_map) {
       pl.n_maps = map->n_maps, pl.width = map->width, pl.height = map->height;
       pl.x0 = map->x0, pl.y0 = map->y0, pl.inv_res = map->inv_res, pl.outside = map->outside, pl.w_map = map->w_map;
+    }
+    pl.field = use_field ? field->d_field : nullptr;
+    if(use_field) {
+      pl.field_of = field->d_field_of, pl.f_offset = reinterpret_cast<const int2 *>(field->d_offset);
+      pl.n_fields = field->n_fields, pl.fw = field->fw, pl.fh = field->fh;
+      pl.fx0 = field->x0, pl.fy0 = field->y0, pl.finv_res = field->inv_res, pl.foutside = field->outside, pl.w_field = field->w_field;
     }
     if(moving) launch_plan<kObstMoving>(*p, d_src_state, n, a, pl, st);
     else launch_plan<kObstStatic>(*p, d_src_state, n, a, static_cast<const PlanObstArgs &>(pl), st);
@@ -981,25 +1045,31 @@ extern "C" {
 
 int rk_plan_rollout(const rk_vdt_params_t *p, const void *d_src_state, int64_t R, int32_t S, const rk_vdt_cmd_t *d_cmd, int32_t n_seg,
                     int32_t seg_len, const rk_plan_cost_t *cost, float *d_cost, void *stream) {
-  return plan_rollout("rk_plan_rollout", p, d_src_state, R, S, d_cmd, n_seg, seg_len, cost, nullptr, false, nullptr, nullptr, d_cost, stream);
+  return plan_rollout("rk_plan_rollout", p, d_src_state, R, S, d_cmd, n_seg, seg_len, cost, nullptr, false, nullptr, nullptr, nullptr, d_cost, stream);
 }
 
 int rk_plan_rollout_obstacles(const rk_vdt_params_t *p, const void *d_src_state, int64_t R, int32_t S, const rk_vdt_cmd_t *d_cmd,
                               int32_t n_seg, int32_t seg_len, const rk_plan_cost_t *cost, const rk_plan_obstacles_t *obst, float *d_cost,
                               void *stream) {
-  return plan_rollout("rk_plan_rollout_obstacles", p, d_src_state, R, S, d_cmd, n_seg, seg_len, cost, obst, false, nullptr, nullptr, d_cost, stream);
+  return plan_rollout("rk_plan_rollout_obstacles", p, d_src_state, R, S, d_cmd, n_seg, seg_len, cost, obst, false, nullptr, nullptr, nullptr, d_cost, stream);
 }
 
 int rk_plan_rollout_moving(const rk_vdt_params_t *p, const void *d_src_state, int64_t R, int32_t S, const rk_vdt_cmd_t *d_cmd, int32_t n_seg,
                            int32_t seg_len, const rk_plan_cost_t *cost, const rk_plan_obstacles_t *obst, float *d_path, float *d_cost,
                            void *stream) {
-  return plan_rollout("rk_plan_rollout_moving", p, d_src_state, R, S, d_cmd, n_seg, seg_len, cost, obst, true, nullptr, d_path, d_cost, stream);
+  return plan_rollout("rk_plan_rollout_moving", p, d_src_state, R, S, d_cmd, n_seg, seg_len, cost, obst, true, nullptr, nullptr, d_path, d_cost, stream);
 }
 
 int rk_plan_rollout_map(const rk_vdt_params_t *p, const void *d_src_state, int64_t R, int32_t S, const rk_vdt_cmd_t *d_cmd, int32_t n_seg,
                         int32_t seg_len, const rk_plan_cost_t *cost, const rk_plan_obstacles_t *obst, const rk_plan_map_t *map, float *d_path,
                         float *d_cost, void *stream) {
-  return plan_rollout("rk_plan_rollout_map", p, d_src_state, R, S, d_cmd, n_seg, seg_len, cost, obst, true, map, d_path, d_cost, stream);
+  return plan_rollout("rk_plan_rollout_map", p, d_src_state, R, S, d_cmd, n_seg, seg_len, cost, obst, true, map, nullptr, d_path, d_cost, stream);
+}
+
+int rk_plan_rollout_field(const rk_vdt_params_t *p, const void *d_src_state, int64_t R, int32_t S, const rk_vdt_cmd_t *d_cmd, int32_t n_seg,
+                          int32_t seg_len, const rk_plan_cost_t *cost, const rk_plan_obstacles_t *obst, const rk_plan_map_t *map,
+                          const rk_plan_field_t *field, float *d_path, float *d_cost, void *stream) {
+  return plan_rollout("rk_plan_rollout_field", p, d_src_state, R, S, d_cmd, n_seg, seg_len, cost, obst, true, map, field, d_path, d_cost, stream);
 }
 
 int rk_vdt_set_power(void *d_state, int64_t n, const uint8_t *d_on, void *stream) {

@@ -7,7 +7,8 @@ method (plan_cem) runs several sample -> rollout -> refit rounds per step, refit
 sigma to each round's elite candidates.  For fleets, predict() gives where each robot's nominal plan takes it and
 peer_discs() turns those paths into moving keep-out discs for the robot's peers (fleet_peers builds the usual grouping).
 A CostMap, a grid of cell costs shared by the robots of a world, prices walls and shelving at every checkpoint, alone or
-together with discs.
+together with discs; its cost_to_go() builds CostToGo fields, shortest-path distances to goals around the walls, that
+price each candidate's end position instead of the straight line to the goal.
 """
 import ctypes as C
 
@@ -52,6 +53,78 @@ class CostMap:
         m.n_maps, m.width, m.height = self.n_maps, self.width, self.height
         m.x0, m.y0, m.inv_res, m.outside, m.w_map = self.x0, self.y0, self.inv_res, self.outside, float(w_map)
         return m
+
+    def cost_to_go(self, goals, size=None, offsets=None, k_cost=0.0, lethal=float("inf"), field_map=None, field_of=None,
+                   outside=float("inf")):
+        """rk_plan_cost_to_go on the current torch stream of the map's device (the call synchronises it): one field per goal,
+        the shortest-path distance in metres from goals[f] (float32 [n_fields, 2], metres) through the cells below `lethal`,
+        each step weighted by 1 + k_cost * cell for cells above 0, with no corner cutting.  size = (fh, fw): the window of
+        every field (default: the whole map); offsets: int32 [n_fields, 2], the map cell (ox, oy) of window cell (0, 0)
+        (default 0, 0); field_map: int32 [n_fields], the map of each field (default map 0).  field_of and outside go to
+        the returned CostToGo.  Build fields when goals or the map change, not every planning step."""
+        dev = self.cells.device
+        goals = torch.as_tensor(goals, dtype=torch.float32, device=dev).contiguous()
+        assert goals.dim() == 2 and goals.shape[1] == 2 and goals.shape[0] >= 1, "goals: float32 [n_fields, 2]"
+        n = goals.shape[0]
+        fh, fw = (self.height, self.width) if size is None else (int(size[0]), int(size[1]))
+        if offsets is not None:
+            offsets = torch.as_tensor(offsets, dtype=torch.int32, device=dev).contiguous()
+            assert tuple(offsets.shape) == (n, 2), f"offsets: int32 [{n}, 2]"
+        if field_map is not None:
+            field_map = torch.as_tensor(field_map, dtype=torch.int32, device=dev).contiguous()
+            assert tuple(field_map.shape) == (n,), f"field_map: int32 [{n}]"
+        lib = _cabi.load()
+        work_bytes = lib.rk_plan_cost_to_go_work_bytes(n, fw, fh)
+        assert work_bytes > 0, "n_fields, fw, fh >= 1, fw, fh <= 2^24 and n_fields * fh * fw < 2^31"
+        field = torch.empty((n, fh, fw), dtype=torch.float32, device=dev)
+        work = torch.empty((work_bytes + 3) // 4, dtype=torch.int32, device=dev)
+        spec = _cabi.PlanCtg()
+        spec.step_axial = C.c_float(self.resolution).value
+        spec.step_diag = C.c_float(self.resolution * 2.0 ** 0.5).value
+        spec.k_cost, spec.lethal = float(k_cost), float(lethal)
+        rounds = C.c_int32(0)
+        di = _dev_index(dev)
+        _cabi.check(lib.rk_set_device(di))
+        mp = self.struct(0.0)
+        _cabi.check(lib.rk_plan_cost_to_go(C.byref(mp), C.byref(spec), goals.data_ptr(), None if field_map is None else field_map.data_ptr(),
+                                           None if offsets is None else offsets.data_ptr(), n, fw, fh, field.data_ptr(), work.data_ptr(),
+                                           C.byref(rounds), C.c_void_p(torch.cuda.current_stream(di).cuda_stream)))
+        ctg = CostToGo(field, self, offsets=offsets, field_of=field_of, outside=outside)
+        ctg.rounds = rounds.value
+        return ctg
+
+
+class CostToGo:
+    """A cost-to-go field for rk_plan_rollout_field: field float32 [n_fields, fh, fw] (CostMap.cost_to_go's, or any caller's
+    grid) on the grid of `costmap` (its origin and resolution); offsets int32 [n_fields, 2], the grid cell of each
+    window's cell (0, 0) (None: 0, 0); field_of int32 [R], the field of each robot (None: field 0; an index outside
+    [0, n_fields) adds no term); outside: the value off a window.  The term w_field * cell is added once, at the end of
+    each candidate's rollout; a +inf cell (blocked or unreachable) prices the candidate at +inf.  rounds: the relaxation
+    rounds of the build (None for a caller's grid)."""
+
+    def __init__(self, field, costmap, offsets=None, field_of=None, outside=float("inf")):
+        assert (field.is_cuda and field.is_contiguous() and field.dtype == torch.float32 and field.dim() == 3
+                and field.numel() > 0), "field: float32 [n_fields, fh, fw] contiguous device tensor"
+        self.field, self.costmap = field, costmap
+        self.n_fields, self.fh, self.fw = (int(d) for d in field.shape)
+        for t, shape, what in ((offsets, (self.n_fields, 2), "offsets"), (field_of, None, "field_of")):
+            if t is not None:
+                assert (t.is_cuda and t.is_contiguous() and t.dtype == torch.int32 and t.device == field.device
+                        and (shape is None and t.dim() == 1 or tuple(t.shape) == shape)), f"{what}: int32 contiguous tensor on the field's device"
+        self.offsets, self.field_of = offsets, field_of
+        self.outside = C.c_float(float(outside)).value
+        self.rounds = None
+
+    def struct(self, w_field):
+        """The rk_plan_field_t of this field with weight w_field."""
+        f = _cabi.PlanField()
+        f.d_field = self.field.data_ptr()
+        f.d_field_of = None if self.field_of is None else self.field_of.data_ptr()
+        f.d_offset = None if self.offsets is None else self.offsets.data_ptr()
+        f.n_fields, f.fw, f.fh = self.n_fields, self.fw, self.fh
+        cm = self.costmap
+        f.x0, f.y0, f.inv_res, f.outside, f.w_field = cm.x0, cm.y0, cm.inv_res, self.outside, float(w_field)
+        return f
 
 
 class VehiclePlanner:
@@ -115,7 +188,8 @@ class VehiclePlanner:
         assert P >= 1 and self.seg_len % P == 0, "check_period must divide seg_len"
         return self.n_seg * self.seg_len // P
 
-    def rollout(self, src, ref, w_pos, w_goal, w_cur, obstacles=None, w_obst=0.0, check_period=None, path=None, costmap=None, w_map=0.0):
+    def rollout(self, src, ref, w_pos, w_goal, w_cur, obstacles=None, w_obst=0.0, check_period=None, path=None, costmap=None, w_map=0.0,
+                field=None, w_field=0.0):
         """rk_plan_rollout: every candidate from its robot's state in `src` (a VehicleBatch of R robots, left untouched),
         ranked against ref (float32 [n_seg, R, 2], metres: where each robot should be when each segment ends).
 
@@ -133,7 +207,11 @@ class VehiclePlanner:
         only; w_map = inf makes every such cell a hard wall), into the same sum as the discs.  Without obstacles the
         checkpoints are every check_period ticks (default seg_len) with no discs.  A 3-D static disc table is then repeated
         for every checkpoint (obstacles.expand(n_ck, m, R, 4).contiguous(), the same bits as the static table): a copy of
-        n_ck * m * R * 16 bytes written on every call, so pass a 4-D table to keep one."""
+        n_ck * m * R * 16 bytes written on every call, so pass a 4-D table to keep one.
+
+        field (a CostToGo on the planner's device): rk_plan_rollout_field adds w_field * cell (cells > 0 only; finite
+        w_field) of the robot's field under each candidate's end position, once, after the last checkpoint; costmap may
+        then be None.  With a field, drop w_pos and keep w_goal small (INTEGRATION.md §2)."""
         assert src.n == self.R, "the source batch must hold the planner's R robots"
         assert ref.is_cuda and ref.is_contiguous() and ref.dtype == torch.float32 and tuple(ref.shape) == (self.n_seg, self.R, 2)
         c = _cabi.PlanCost()
@@ -142,9 +220,12 @@ class VehiclePlanner:
         if costmap is not None:
             assert costmap.cells.device.index == self.dev_index, "costmap: on the planner's device"
             assert costmap.map_of is None or costmap.map_of.shape[0] == self.R, f"costmap.map_of: int32 [{self.R}]"
-            if obstacles is not None and obstacles.dim() == 3:
-                obstacles = obstacles.expand(self.n_ck(self.seg_len if check_period is None else check_period), *obstacles.shape).contiguous()
-        if obstacles is None and path is None and costmap is None:
+        if field is not None:
+            assert field.field.device.index == self.dev_index, "field: on the planner's device"
+            assert field.field_of is None or field.field_of.shape[0] == self.R, f"field.field_of: int32 [{self.R}]"
+        if (costmap is not None or field is not None) and obstacles is not None and obstacles.dim() == 3:
+            obstacles = obstacles.expand(self.n_ck(self.seg_len if check_period is None else check_period), *obstacles.shape).contiguous()
+        if obstacles is None and path is None and costmap is None and field is None:
             self._keep = ref
             _cabi.check(self.lib.rk_plan_rollout(*args, self.cost.data_ptr(), self._stream()))
             return self.cost
@@ -166,12 +247,17 @@ class VehiclePlanner:
             assert (path.is_cuda and path.is_contiguous() and path.dtype == torch.float32
                     and tuple(path.shape) == (n_ck, self.R * self.S, 2)), f"path: float32 [{n_ck}, {self.R * self.S}, 2] device tensor"
         pth = None if path is None else path.data_ptr()
-        if costmap is None:
+        if costmap is None and field is None:
             _cabi.check(self.lib.rk_plan_rollout_moving(*args, C.byref(o), pth, self.cost.data_ptr(), self._stream()))
-        else:
+        elif field is None:
             self._keep = (ref, obstacles, path, costmap)
             mp = costmap.struct(w_map)
             _cabi.check(self.lib.rk_plan_rollout_map(*args, C.byref(o), C.byref(mp), pth, self.cost.data_ptr(), self._stream()))
+        else:
+            self._keep = (ref, obstacles, path, costmap, field)
+            mp = None if costmap is None else C.byref(costmap.struct(w_map))
+            fd = field.struct(w_field)
+            _cabi.check(self.lib.rk_plan_rollout_field(*args, C.byref(o), mp, C.byref(fd), pth, self.cost.data_ptr(), self._stream()))
         return self.cost
 
     def predict(self, src, check_period):
@@ -235,20 +321,20 @@ class VehiclePlanner:
         return self.nominal
 
     def plan(self, src, ref, w_pos, w_goal, w_cur, lam=0.0, shift=1, seed=None, obstacles=None, w_obst=0.0, check_period=None,
-             costmap=None, w_map=0.0):
+             costmap=None, w_map=0.0, field=None, w_field=0.0):
         """One planning step (sample, rollout, select) on the current torch stream; returns the new nominal.  obstacles
-        (3-D static or 4-D per-checkpoint discs) and costmap as in rollout."""
+        (3-D static or 4-D per-checkpoint discs), costmap and field as in rollout."""
         self.sample(seed=seed)
         self.rollout(src, ref, w_pos, w_goal, w_cur, obstacles=obstacles, w_obst=w_obst, check_period=check_period, costmap=costmap,
-                     w_map=w_map)
+                     w_map=w_map, field=field, w_field=w_field)
         return self.select(lam, shift)
 
     def plan_cem(self, src, ref, w_pos, w_goal, w_cur, iters, elite, alpha=0.0, sigma_min=(0.0, 0.0, 0.0), shift=1, seed=None,
-                 obstacles=None, w_obst=0.0, check_period=None, costmap=None, w_map=0.0):
+                 obstacles=None, w_obst=0.0, check_period=None, costmap=None, w_map=0.0, field=None, w_field=0.0):
         """One cross-entropy planning step on the current torch stream; returns the new nominal.
 
         sigma_table is reset to the planner's sigma, then `iters` rounds of sample (around the nominal, with the table) ->
-        rollout (obstacles and costmap as in rollout) -> refit to the `elite` best candidates.  Every round but the last refits with
+        rollout (obstacles, costmap and field as in rollout) -> refit to the `elite` best candidates.  Every round but the last refits with
         shift = 0, so that the next round samples around the same segments; the last one with `shift`.  Round i draws with
         seed (seed + i * 0x9E3779B9) mod 2^32 (seed: the planner's own when None).  iters = 1, elite = 1, alpha = 0 is
         plan(..., lam=0) bit for bit while no cost is -inf (never, with non-negative weights).  NaN and +-inf costs are never
@@ -259,7 +345,7 @@ class VehiclePlanner:
         for i in range(int(iters)):
             self.sample(seed=(base + i * 0x9E3779B9) & 0xFFFFFFFF, sigma_table=self.sigma_table)
             self.rollout(src, ref, w_pos, w_goal, w_cur, obstacles=obstacles, w_obst=w_obst, check_period=check_period, costmap=costmap,
-                         w_map=w_map)
+                         w_map=w_map, field=field, w_field=w_field)
             self.refit(elite, alpha, sigma_min, shift if i == int(iters) - 1 else 0)
         return self.nominal
 

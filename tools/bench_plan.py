@@ -36,10 +36,19 @@ reports the share of robots that ever enter a wall cell, with and without the ma
 --parent-lib LIB also times LIB's rk_plan_rollout_moving (a build of another tree, loaded side by side) alternated with
 this tree's on the same inputs, and checks that both give the same bits.
 
+With --field CELLS:G the run also times rk_plan_cost_to_go on the random-wall world of --map (CELLS x CELLS cells, walls
+lethal) with G whole-map fields, and on a serpentine maze of the same size as the worst case (one path that crosses
+every tile row back and forth), reporting ms and relaxation rounds; then rk_plan_rollout_field (field of robot r: r % G)
+alternated with rk_plan_rollout_map on the same inputs at P = 125, 25 and 5, with a path and no discs, and with
+--parent-lib LIB's rk_plan_rollout_map alternated with this tree's.  Then it plays the wall scenario and a dead end (a U
+of shelving that opens toward the robot, its goal straight behind the U's bottom) at size, under argmin and CEM, with
+the map and with or without each robot's cost-to-go field over its 20-cell lane, and reports the share of robots within
+0.1 m of their goals.
+
     python tools/bench_plan.py [--R 4096] [--S 256] [--n-seg 8] [--seg-len 125] [--reps 10] [--out FILE]
                                [--obstacles 1,8 --check-period 125,25,10] [--cem 4:8 --cem-steps 8 --lam 1e-3]
                                [--moving 1:125,8:25] [--fleet 8 --fleet-steps 60] [--map 800:125,800:25,800:5]
-                               [--parent-lib path/to/librobotick_b200.so]
+                               [--field 800:16] [--parent-lib path/to/librobotick_b200.so]
 """
 import ctypes as C
 import argparse
@@ -47,6 +56,7 @@ import json
 import os
 import subprocess
 import sys
+import time
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
@@ -56,7 +66,7 @@ import torch  # noqa: E402
 
 import roboken_fmskf_robot_controller_b200 as rk  # noqa: E402
 from roboken_fmskf_robot_controller_b200 import _cabi, layout, streams  # noqa: E402
-from roboken_fmskf_robot_controller_b200.planner import CostMap, VehiclePlanner, fleet_peers  # noqa: E402
+from roboken_fmskf_robot_controller_b200.planner import CostMap, CostToGo, VehiclePlanner, fleet_peers  # noqa: E402
 from roboken_fmskf_robot_controller_b200.vehicle import VehicleBatch  # noqa: E402
 
 
@@ -187,6 +197,171 @@ def wall_world(R, dev, cell=0.05):
     return wall, cm, starts, goals
 
 
+def random_walls(cells_n, rng):
+    """The --map world: CELLS x CELLS cells, walls of 1 - 4 by 4 - 40 cells at random (one per 160 cells of area) costing 1."""
+    g = np.zeros((cells_n, cells_n), dtype=np.float32)
+    for _ in range(cells_n * cells_n // 160):
+        h, w = (rng.integers(1, 5), rng.integers(4, 41))[:: 1 if rng.random() < 0.5 else -1]
+        y, x = rng.integers(0, cells_n - h), rng.integers(0, cells_n - w)
+        g[y:y + h, x:x + w] = 1.0
+    return g
+
+
+def serpentine(cells_n, corridor=3):
+    """A maze of cells_n x cells_n: a +inf wall row after every `corridor` free rows, open at alternating ends."""
+    g = np.zeros((cells_n, cells_n), np.float32)
+    for k, y in enumerate(range(corridor, cells_n, corridor + 1)):
+        g[y, :] = np.inf
+        g[y, -1 if k % 2 == 0 else 0] = 0.0
+    return g
+
+
+def inflate(wall, n=1):
+    H, W = wall.shape
+    grown = wall.copy()
+    for _ in range(n):
+        g = np.pad(grown, 1)
+        grown = np.zeros_like(wall)
+        for dy in range(3):
+            for dx in range(3):
+                grown |= g[dy:dy + H, dx:dx + W]
+    return grown
+
+
+def dead_end_world(R, dev, cell=0.05):
+    """The dead end of tests/plan_field_ref.py at size: lane r (x in [r - 0.5, r + 0.5), y in [-0.8, 0.8)) holds a U of
+    shelving, a bar across y in [0.10, 0.15) for |x - r| < 0.2 and arms down to y = -0.30 at 0.15 <= |x - r| < 0.2; start
+    (r, -0.45), goal (r, 0.50).  Returns (wall, CostMap of the wall inflated by one cell, starts, goals)."""
+    W, H = 20 * R, 32
+    x0, y0 = -0.5, -0.8
+    xc = x0 + (np.arange(W) + 0.5) * cell
+    yc = y0 + (np.arange(H) + 0.5) * cell
+    dx = xc - np.floor(xc - x0) - x0 - 0.5
+    bar = (np.abs(dx) < 0.2)[None, :] & ((yc >= 0.10) & (yc < 0.15))[:, None]
+    arms = ((np.abs(dx) >= 0.15) & (np.abs(dx) < 0.2))[None, :] & ((yc >= -0.30) & (yc < 0.15))[:, None]
+    wall = bar | arms
+    cm = CostMap(torch.from_numpy(inflate(wall).astype(np.float32)).to(dev), (x0, y0), cell)
+    starts = np.stack([np.arange(R, dtype=np.float64), np.full(R, -0.45)], axis=1).astype(np.float32)
+    goals = np.stack([np.arange(R, dtype=np.float64), np.full(R, 0.50)], axis=1).astype(np.float32)
+    return wall, cm, starts, goals
+
+
+def field_play(a, dev, world, steps, iters, elite):
+    """A scenario at size under argmin and CEM, with the map, with and without each robot's lane field (w_pos 0, w_goal 1,
+    w_field 10 with it; w_pos 1, w_goal 10 without): the share of robots within 0.1 m of the goal after `steps` steps."""
+    R, n_seg, seg_len, P = a.R, a.n_seg, a.seg_len, 25
+    wall, cm, starts, goals = world(R, dev)
+    ref = torch.from_numpy(np.ascontiguousarray(np.broadcast_to(goals, (n_seg, R, 2)))).to(dev)
+    aos = np.zeros((R, layout.VS_WORDS), dtype=np.uint32)
+    aos[:, layout.VS_POS_X], aos[:, layout.VS_POS_Y] = starts[:, 0].view(np.uint32), starts[:, 1].view(np.uint32)
+    offs = np.stack([np.arange(R) * 20, np.zeros(R, np.int64)], axis=1).astype(np.int32)
+    ctg = cm.cost_to_go(goals, size=(cm.height, 20), offsets=offs, lethal=1.0, field_of=torch.arange(R, dtype=torch.int32, device=dev))
+    out = {"robots": R, "steps": steps, "check_period": P, "w_map": 1e4, "field_bytes": ctg.field.numel() * 4, "build_rounds": ctg.rounds}
+    for mode in ("argmin", "cem"):
+        for use_field in (False, True):
+            S = a.S if mode == "argmin" else a.S // iters
+            pl = VehiclePlanner(R, S, n_seg, seg_len, dev, sigma=(250.0, 250.0, 0.2), seed=0xA11)
+            vb = VehicleBatch(R, dev)
+            vb.load_state_soa(layout.aos_to_soa(aos))
+            w = (0.0, 1.0, 1e-9) if use_field else (1.0, 10.0, 1e-9)
+            kw = dict(check_period=P, costmap=cm, w_map=1e4, field=ctg if use_field else None, w_field=10.0)
+            for it in range(steps):
+                if mode == "argmin":
+                    pl.plan(vb, ref, *w, lam=0.0, shift=0, seed=0xA11 + it, **kw)
+                else:
+                    pl.plan_cem(vb, ref, *w, iters, elite, 0.0, (40.0, 40.0, 0.05), shift=0, seed=0xA11 + it, **kw)
+                vb.rollout(seg_len, sensor_mode=_cabi.RK_SENSOR_PLANT, cmd=pl.first_command(), seg_len=seg_len)
+            st = layout.soa_to_aos(vb.state.cpu().numpy().view(np.uint32), R, layout.VS_WORDS)
+            pos = st[:, [layout.VS_POS_X, layout.VS_POS_Y]].view(np.float32)
+            d = np.hypot(pos[:, 0] - goals[:, 0], pos[:, 1] - goals[:, 1])
+            out[f"{mode}_{'field' if use_field else 'no_field'}"] = {
+                "S": S, "goal_dist_median_m": float(np.median(d)), "goal_dist_p90_m": float(np.quantile(d, 0.9)),
+                "within_0.1m_share": float((d < 0.1).mean())}
+    return out
+
+
+def field_bench(a, dev, pl, src, goal, cells_n, G, parent, iters, elite):
+    """--field: the builder's time and rounds, rk_plan_rollout_field against rk_plan_rollout_map (and the parent's map
+    rollout), and the two scenarios at size."""
+    R, S, n_seg, seg_len = a.R, a.S, a.n_seg, a.seg_len
+    n, K = R * S, n_seg * seg_len
+    rng = np.random.default_rng(21)
+    half = cells_n * 0.05 / 2
+    g = random_walls(cells_n, rng)
+    cm = CostMap(torch.from_numpy(g).to(dev), (-half, -half), 0.05)
+    free = np.argwhere(g == 0)
+    pick = free[rng.choice(len(free), G, replace=False)]
+    goals = np.stack([-half + (pick[:, 1] + 0.5) * 0.05, -half + (pick[:, 0] + 0.5) * 0.05], axis=1).astype(np.float32)
+    maze = CostMap(torch.from_numpy(serpentine(cells_n)).to(dev), (-half, -half), 0.05)
+    corner = np.array([[-half + 0.025, -half + 0.025]], np.float32)
+    out = {"cells": cells_n, "G": G, "builder": {}}
+    for name, m, gl in (("random_walls", cm, goals), ("maze", maze, corner)):
+        ms, rounds = [], None
+        for _ in range(3 if name == "maze" else a.reps):
+            torch.cuda.synchronize()
+            t0 = time.perf_counter()
+            ctg = m.cost_to_go(gl, lethal=1.0)  # synchronises the stream
+            ms.append((time.perf_counter() - t0) * 1e3)
+            rounds = ctg.rounds
+        out["builder"][name] = {"fields": len(gl), "ms_median": round(float(np.median(ms)), 3), "ms_min": round(float(np.min(ms)), 3),
+                                "rounds": rounds, "reachable_fraction": float(torch.isfinite(ctg.field).float().mean())}
+    field = cm.cost_to_go(goals, lethal=1.0, field_of=(torch.arange(R, dtype=torch.int32, device=dev) % G).contiguous())
+    # the robots spread over the world as for --map, each heading for its field's goal
+    aos = layout.soa_to_aos(src.state.cpu().numpy().view(np.uint32), R, layout.VS_WORDS)
+    pos1 = rng.uniform(-half + 1.0, half - 1.0, (R, 2)).astype(np.float32)
+    aos[:, layout.VS_POS_X], aos[:, layout.VS_POS_Y] = pos1[:, 0].view(np.uint32), pos1[:, 1].view(np.uint32)
+    src_f = VehicleBatch(R, dev)
+    src_f.load_state_soa(layout.aos_to_soa(aos))
+    ref_f = (torch.from_numpy(pos1).to(dev) + goal).unsqueeze(0).expand(n_seg, R, 2).contiguous()
+    path = torch.empty((K // 5, n, 2), dtype=torch.float32, device=dev)
+    par_cost = torch.empty(n, dtype=torch.float32, device=dev)
+
+    def roll(P, use_field):
+        pl.rollout(src_f, ref_f, 1.0, 10.0, 1e-9, check_period=P, path=path[: K // P], costmap=cm, w_map=1.0,
+                   field=field if use_field else None, w_field=10.0)
+
+    def parent_map(P, lib):
+        c = _cabi.PlanCost()
+        c.d_ref, c.w_pos, c.w_goal, c.w_cur = ref_f.data_ptr(), 1.0, 10.0, 1e-9
+        o = _cabi.PlanObstacles()
+        o.check_period = P
+        mp = cm.struct(1.0)
+        out_c = pl.cost if lib is pl.lib else par_cost
+        _cabi.check(lib.rk_plan_rollout_map(C.byref(pl.params), src_f.state.data_ptr(), R, S, pl.candidates.data_ptr(), n_seg, seg_len,
+                                            C.byref(c), C.byref(o), C.byref(mp), path[: K // P].data_ptr(), out_c.data_ptr(),
+                                            C.c_void_p(torch.cuda.current_stream().cuda_stream)))
+
+    rows, prow = [], []
+    for P in (125, 25, 5):
+        roll(P, False), roll(P, True)
+        tm, tf = [], []
+        for _ in range(a.reps):
+            tm.append(timed(lambda: roll(P, False)))
+            tf.append(timed(lambda: roll(P, True)))
+        roll(P, False)
+        base = pl.cost.clone()
+        roll(P, True)
+        rows.append({"check_period": P, "ms_median_map": round(float(np.median(tm)), 4), "ms_median_field": round(float(np.median(tf)), 4),
+                     "ms_min_max_field": [round(float(np.min(tf)), 4), round(float(np.max(tf)), 4)],
+                     "field_over_map": float(np.median(tf) / np.median(tm)), "priced_fraction": (pl.cost != base).float().mean().item()})
+        if parent is not None:
+            parent_map(P, parent), parent_map(P, pl.lib)
+            tp, tt = [], []
+            for _ in range(a.reps):
+                tp.append(timed(lambda: parent_map(P, parent)))
+                tt.append(timed(lambda: parent_map(P, pl.lib)))
+            torch.cuda.synchronize()
+            prow.append({"check_period": P, "ms_median_parent": round(float(np.median(tp)), 4), "ms_median_this": round(float(np.median(tt)), 4),
+                         "this_over_parent": float(np.median(tt) / np.median(tp)),
+                         "same_bits": bool(torch.equal(par_cost.view(torch.int32), pl.cost.view(torch.int32)))})
+    out["rollout"] = rows
+    if parent is not None:
+        out["parent_map"] = prow
+    out["wall"] = field_play(a, dev, wall_world, a.map_steps, iters, elite)
+    out["dead_end"] = field_play(a, dev, dead_end_world, a.field_steps, iters, elite)
+    return out
+
+
 def wall_report(a, dev, iters, elite):
     """The wall scenario at size under argmin (S candidates) and CEM (iters rounds of S / iters), with and without the map:
     the share of robots that ever enter a wall cell and the distance to the goal after --map-steps steps."""
@@ -250,6 +425,8 @@ def main():
     ap.add_argument("--map", action="append", default=[], help="CELLS:P pairs (comma list or repeated): time cost maps")
     ap.add_argument("--map-steps", type=int, default=40, help="planning steps of the wall scenario")
     ap.add_argument("--parent-lib", default=None, help="another build's library: time its rk_plan_rollout_moving side by side")
+    ap.add_argument("--field", default=None, help="CELLS:G: time cost-to-go fields and play the wall and dead-end scenarios")
+    ap.add_argument("--field-steps", type=int, default=60, help="planning steps of the dead-end scenario")
     a = ap.parse_args()
     moving = [tuple(int(v) for v in x.split(":")) for arg in a.moving for x in arg.split(",") if x]
     maps = [tuple(int(v) for v in x.split(":")) for arg in a.map for x in arg.split(",") if x]
@@ -349,13 +526,8 @@ def main():
         ref_map = (torch.from_numpy(pos1).to(dev) + goal).unsqueeze(0).expand(n_seg, R, 2).contiguous()
     for cells_n, P in maps:
         if cells_n not in worlds:
-            g = np.zeros((cells_n, cells_n), dtype=np.float32)
-            for _ in range(cells_n * cells_n // 160):
-                h, w = (rng_w.integers(1, 5), rng_w.integers(4, 41))[:: 1 if rng_w.random() < 0.5 else -1]
-                y, x = rng_w.integers(0, cells_n - h), rng_w.integers(0, cells_n - w)
-                g[y:y + h, x:x + w] = 1.0
             half = cells_n * 0.05 / 2
-            worlds[cells_n] = CostMap(torch.from_numpy(g).to(dev), (-half, -half), 0.05)
+            worlds[cells_n] = CostMap(torch.from_numpy(random_walls(cells_n, rng_w)).to(dev), (-half, -half), 0.05)
         n_ck = K // P
         for m in (0, 8):
             d = np.zeros((m, R, 4), dtype=np.float32)
@@ -372,9 +544,10 @@ def main():
 
     parent = None
     if a.parent_lib:
-        assert maps, "--parent-lib times the discs of --map"
+        assert maps or a.field, "--parent-lib times the discs of --map or the map rollout of --field"
         parent = C.CDLL(os.path.abspath(a.parent_lib), mode=C.RTLD_LOCAL)
         parent.rk_plan_rollout_moving.argtypes = pl.lib.rk_plan_rollout_moving.argtypes
+        parent.rk_plan_rollout_map.argtypes = pl.lib.rk_plan_rollout_map.argtypes
         par_cost = torch.empty(n, dtype=torch.float32, device=dev)
         par_P = sorted({P for _, P in maps} or {P for _, P in moving} or {seg_len})
         par_tabs = map_tabs if maps else {}
@@ -412,7 +585,7 @@ def main():
     for cells_n, P in maps:
         for m in (0, 8):
             map_moving(cells_n, P, m, False), map_moving(cells_n, P, m, True)
-    if parent is not None:
+    if parent is not None and maps:
         for P in par_P:
             for m in (0, 8):
                 parent_moving(P, m, parent), parent_moving(P, m, pl.lib)
@@ -452,7 +625,7 @@ def main():
                 tm, tmap = t_map.setdefault((cells_n, P, m), ([], []))
                 tm.append(timed(lambda: map_moving(cells_n, P, m, False)))
                 tmap.append(timed(lambda: map_moving(cells_n, P, m, True)))
-        if parent is not None:  # the same rk_plan_rollout_moving call from the other build and from this one, alternated
+        if parent is not None and maps:  # the same rk_plan_rollout_moving call from the other build and from this one, alternated
             for P in par_P:
                 for m in (0, 8):
                     tpar, tthis = t_par.setdefault((P, m), ([], []))
@@ -515,7 +688,7 @@ def main():
                          "priced_fraction": (pl.cost != base).float().mean().item()})
         res["map"] = rows
         res["wall"] = wall_report(a, dev, *((cem_iters, cem_elite) if a.cem else (4, 8)))
-    if parent is not None:
+    if parent is not None and maps:
         rows = []
         for (P, m), (tpar, tthis) in t_par.items():
             parent_moving(P, m, parent)
@@ -527,7 +700,10 @@ def main():
                          "ms_min_max_this": [round(float(np.min(tthis)), 4), round(float(np.max(tthis)), 4)],
                          "same_bits": bool(torch.equal(par_cost.view(torch.int32), pl.cost.view(torch.int32)))})
         res["parent_moving"] = rows
-    if moving or a.fleet or maps:
+    if a.field:
+        cells_n, G = (int(v) for v in a.field.split(":"))
+        res["field"] = field_bench(a, dev, pl, src, goal, cells_n, G, parent, *((cem_iters, cem_elite) if a.cem else (4, 8)))
+    if moving or a.fleet or maps or a.field:
         res["max_sm_clock"] = power_limit("clocks.max.sm")
     if a.fleet:
         res["fleet"] = fleet_report(a, a.fleet, dev)
