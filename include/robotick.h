@@ -778,7 +778,8 @@ int rk_plan_peer_discs(const float *d_path, int64_t R, int32_t n_ck, const int32
 /* Cost maps: a grid of cell costs, stored once per world (not per robot) and looked up at every checkpoint, one cell load
  * whatever the world holds -- walls, corridors, shelving.  It shares the checkpoints and the accumulator O with the discs,
  * so peer discs and a building map compose in one rollout.  The robot is a point read at checkpoints only: inflate walls by
- * the body radius plus the distance covered in P ticks (at most 0.4 mm per tick at 400 mm/s), see INTEGRATION.md §2. */
+ * the body radius plus the distance covered in P ticks (at most 0.4 mm per tick at 400 mm/s) with rk_plan_inflate, see
+ * INTEGRATION.md §2. */
 typedef struct rk_plan_map {
   const float   *d_cells;  /* float [n_maps][height][width]: cell (ix, iy) of map k at (k*height + iy)*width + ix; 4-byte aligned */
   const int32_t *d_map_of; /* int32 [R]: the map of robot r; NULL: map 0 for every robot */
@@ -881,6 +882,35 @@ int rk_plan_rollout_field(const rk_vdt_params_t *p, const void *d_src_state, int
                           const rk_vdt_cmd_t *d_cmd, int32_t n_seg, int32_t seg_len, const rk_plan_cost_t *cost,
                           const rk_plan_obstacles_t *obst, const rk_plan_map_t *map, const rk_plan_field_t *field,
                           float *d_path, float *d_cost, void *stream);
+
+/* Cost-map inflation: every cell priced by its Euclidean distance to the nearest obstacle of its map, through a table the
+ * caller fills (a ROS-style inflation profile, planner.inflation_table), so that robots keep their body clear of walls.
+ * The maps and fields above treat the robot as a point; an inflated map is what they should read.  Meant to run when the
+ * map changes, not every step. */
+typedef struct rk_plan_inflate {
+  const float *d_table;  /* float [n_table]: the cost at squared cell distance d2 = 0 .. n_table-1; 4-byte aligned */
+  int32_t      n_table;  /* 1 .. 65536 (so only obstacles within 255 cells matter) */
+  float        lethal;   /* a cell c >= lethal is an obstacle; > 0, may be +inf; NaN rejected */
+} rk_plan_inflate_t;     /* 16 bytes */
+
+/* d_dst: float [n_maps][height][width], the inflated cells of `map` (d_cells; map_of, x0, y0, inv_res and w_map are not
+ * used, but x0, y0, inv_res and outside pass rk_plan_rollout_map's map checks).  Every step is integer, or a comparison of
+ * float32 values, so the output has one right answer:
+ *   obstacle  a cell of map k with c >= lethal (NaN never); the cells off the grid are obstacles exactly when
+ *             map->outside >= lethal (the rule rk_plan_cost_to_go uses off the map)
+ *   distance  d2(q) = the least (qx - ox)^2 + (qy - oy)^2 over the obstacles o of the same map, exact in integers (maps do
+ *             not see each other's obstacles), "none" without an obstacle.  The nearest off-grid obstacle is always the
+ *             axial one: min((x+1)^2, (W-x)^2, (y+1)^2, (H-y)^2).
+ *   output    with c the source cell: if d2 < n_table, v = d_table[d2] and out = (v > c || c != c) ? v : c; otherwise
+ *             out = c.  So the larger value wins, a NaN source cell takes the table's value, and signed zeros keep the
+ *             source's bits.
+ * The call is asynchronous on `stream` (no host read, no synchronise).  d_work: rk_plan_inflate_work_bytes() bytes of device
+ * memory, 4-byte aligned, owned by the caller.  d_dst and d_work must not overlap each other, the cells or the table.
+ * RK_ERR_ARG, checked before any device call: map or spec NULL; the map checks of rk_plan_cost_to_go; n_table outside
+ * [1, 65536]; lethal NaN or <= 0; d_table, d_dst or d_work NULL or not 4-byte aligned; an overlap. */
+int rk_plan_inflate(const rk_plan_map_t *map, const rk_plan_inflate_t *spec, float *d_dst, void *d_work, void *stream);
+/* Bytes of d_work for rk_plan_inflate; 0 for sizes it rejects. */
+size_t rk_plan_inflate_work_bytes(int32_t n_maps, int32_t width, int32_t height);
 
 /* =====================================================================================
  * RobotManager guard (SURVEY 8f-2): the vehicle-management block of RMT's routine_ros()

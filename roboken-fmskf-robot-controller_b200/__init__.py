@@ -12,13 +12,14 @@ __all__ = ["_cabi", "layout", "streams", "RobotickError", "default_params", "loa
 
 
 def __getattr__(name):
-    # torch-dependent modules are imported lazily so that layout/streams stay light
+    # torch-dependent modules are imported lazily so that layout/streams stay light.  import_module, not `from . import`:
+    # the latter first probes this module for the attribute, which would call __getattr__ again.
+    import importlib
+
     if name in ("vehicle", "VehicleBatch"):
-        from . import vehicle as _v
-
+        _v = importlib.import_module(".vehicle", __name__)
         return _v if name == "vehicle" else _v.VehicleBatch
-    if name in ("planner", "VehiclePlanner", "CostMap", "CostToGo"):
-        from . import planner as _p
-
+    if name in ("planner", "VehiclePlanner", "CostMap", "CostToGo", "inflation_table"):
+        _p = importlib.import_module(".planner", __name__)
         return _p if name == "planner" else getattr(_p, name)
     raise AttributeError(name)

@@ -202,6 +202,12 @@ class PlanField(C.Structure):
                 ("fh", C.c_int32), ("x0", C.c_float), ("y0", C.c_float), ("inv_res", C.c_float), ("outside", C.c_float), ("w_field", C.c_float)]
 
 
+class PlanInflate(C.Structure):
+    """rk_plan_inflate_t"""
+
+    _fields_ = [("d_table", C.c_void_p), ("n_table", C.c_int32), ("lethal", C.c_float)]
+
+
 class PlanRefit(C.Structure):
     """rk_plan_refit_t"""
 
@@ -268,6 +274,9 @@ def _proto(lib):
                                        C.POINTER(C.c_int32), vp]
     lib.rk_plan_cost_to_go_work_bytes.argtypes = [C.c_int32, C.c_int32, C.c_int32]
     lib.rk_plan_cost_to_go_work_bytes.restype = C.c_size_t
+    lib.rk_plan_inflate.argtypes = [C.POINTER(PlanMap), C.POINTER(PlanInflate), vp, vp, vp]
+    lib.rk_plan_inflate_work_bytes.argtypes = [C.c_int32, C.c_int32, C.c_int32]
+    lib.rk_plan_inflate_work_bytes.restype = C.c_size_t
     lib.rk_plan_peer_discs.argtypes = [vp, C.c_int64, C.c_int32, vp, C.c_int32, C.c_float, vp, C.c_int32, C.c_int32, vp]
     lib.rk_plan_select.argtypes = [vp, vp, C.c_int64, C.c_int32, C.c_int32, C.c_float, C.c_int32, vp, vp, vp, vp]
     lib.rk_plan_sample_commands_sigma.argtypes = [C.POINTER(VdtParams), C.POINTER(PlanSample), vp, vp, C.c_int64, C.c_int32, C.c_int32, vp,

@@ -1,6 +1,6 @@
 // rk_plan.cu -- the two ends of a planning step around rk_plan_rollout (rk_vehicle.cu): candidate commands sampled
 // around a nominal plan, and the per-robot choice among the candidates' costs (include/robotick.h, "Vehicle sampling
-// planner"); and the planner kernels outside the rollout: peer discs and cost-to-go fields.  Candidate j of robot r is
+// planner"); and the planner kernels outside the rollout: peer discs, cost-to-go fields and map inflation.  Candidate j of robot r is
 // instance r*S + j, so a robot's S candidates are contiguous in every table.
 #include <limits.h>
 #include <math.h>
@@ -393,6 +393,104 @@ plan_ctg_relax_kernel(const CtgArgs a, const uint32_t *__restrict__ dirty_in, ui
   }
 }
 
+// rk_plan_inflate: an exact squared Euclidean distance transform truncated at rmax = floor(sqrt(n_table - 1)) cells, which
+// keeps every d2 < n_table exact, in two passes.  The column pass writes g = min(vertical distance to the nearest
+// obstacle of the column, rmax + 1) to the work space; the row pass takes min over |dx| <= rmax of dx^2 + g(x + dx)^2 and
+// applies the table.  A capped g gives d2 >= (rmax + 1)^2 >= n_table, which the table treats as no obstacle.
+constexpr int kInflThreads = 128, kInflChunk = 64, kInflMaxR = 255; // kInflChunk: the bits of one mask word
+
+struct InflateArgs {
+  const float *cells; // [n_maps][height][width]
+  const float *table; // [n_table]
+  float       *dst;   // [n_maps][height][width]
+  int32_t      n_maps, width, height, rmax, n_table;
+  float        lethal;
+  bool         edge; // the cells off the grid are obstacles
+};
+
+// One thread per (map, chunk of 64 rows, column), x fastest.  Bit i of the mask is row y0 + i; the rows above and below
+// the chunk are searched only as far as rmax from its ends, and the off-grid rows -1 and H count when edge is set.
+__global__ void __launch_bounds__(kInflThreads) plan_inflate_cols_kernel(const InflateArgs a, int chunks, uint16_t *__restrict__ g) {
+  const int64_t t = (int64_t)blockIdx.x * kInflThreads + threadIdx.x;
+  const int     W = a.width, H = a.height, R = a.rmax, lim = R + 1;
+  if(t >= (int64_t)a.n_maps * chunks * W) return;
+  const int64_t q = t / W;
+  const int     x = (int)(t - q * W), ch = (int)(q % chunks), k = (int)(q / chunks);
+  const int     y0 = ch * kInflChunk, n = min(kInflChunk, H - y0);
+  const float  *col = a.cells + (int64_t)k * H * W + x;
+  uint64_t      m = 0;
+#pragma unroll 8
+  for(int i = 0; i < n; i++) m |= (__ldg(col + (int64_t)(y0 + i) * W) >= a.lethal ? 1ull : 0ull) << i;
+  int above = y0 - lim; // the nearest obstacle row before the chunk, or a row far enough to cap
+  for(int y = y0 - 1; y >= y0 - R; y--) {
+    if(y < 0) {
+      if(a.edge) above = -1;
+      break;
+    }
+    if(__ldg(col + (int64_t)y * W) >= a.lethal) {
+      above = y;
+      break;
+    }
+  }
+  const int y1 = y0 + n;
+  int       below = y1 - 1 + lim; // the nearest obstacle row after the chunk, or a row far enough to cap
+  for(int y = y1; y <= y1 - 1 + R; y++) {
+    if(y >= H) {
+      if(a.edge) below = H;
+      break;
+    }
+    if(__ldg(col + (int64_t)y * W) >= a.lethal) {
+      below = y;
+      break;
+    }
+  }
+  uint16_t *gc = g + (int64_t)k * H * W + x;
+  for(int i = 0; i < n; i++) {
+    const int      y = y0 + i;
+    const uint64_t lo = m & (~0ull >> (63 - i)), hi = m >> i;
+    const int      up = lo ? __clzll((long long)lo) - (63 - i) : y - above;
+    const int      dn = hi ? __ffsll((long long)hi) - 1 : below - y;
+    gc[(int64_t)y * W] = (uint16_t)min(min(up, dn), lim);
+  }
+}
+
+// One CTA per (map, row, segment of 128 columns): g^2 of the segment and rmax columns on each side in shared memory
+// ((rmax + 1)^2 off the grid: the off-grid columns are the axial terms below).  Each thread walks dx outward and stops
+// once dx^2 alone reaches its best.
+__global__ void __launch_bounds__(kInflThreads) plan_inflate_rows_kernel(const InflateArgs a, int segs, const uint16_t *__restrict__ g) {
+  __shared__ int sg[kInflThreads + 2 * kInflMaxR];
+  const int64_t  row = blockIdx.x / segs; // k*H + y
+  const int      W = a.width, R = a.rmax, x0 = (int)(blockIdx.x - row * segs) * kInflThreads, lim2 = (R + 1) * (R + 1);
+  const uint16_t *gr = g + row * W;
+  for(int i = threadIdx.x; i < kInflThreads + 2 * R; i += kInflThreads) {
+    const int x = x0 - R + i;
+    int       v = lim2;
+    if(x >= 0 && x < W) {
+      const int d = gr[x];
+      v           = d * d;
+    }
+    sg[i] = v;
+  }
+  __syncthreads();
+  const int x = x0 + (int)threadIdx.x;
+  if(x >= W) return;
+  const int *s    = sg + R + threadIdx.x; // s[dx]: g^2 at column x + dx
+  int        best = s[0];
+  for(int dx = 1; dx <= R && dx * dx < best; dx++) best = min(best, dx * dx + min(s[-dx], s[dx]));
+  if(a.edge) {
+    if(x + 1 <= R) best = min(best, (x + 1) * (x + 1));
+    if(W - x <= R) best = min(best, (W - x) * (W - x));
+  }
+  const int64_t i = row * W + x;
+  const float   c = __ldg(a.cells + i);
+  float         o = c;
+  if(best < a.n_table) {
+    const float v = __ldg(a.table + best);
+    o             = (v > c || isnan(c)) ? v : c;
+  }
+  a.dst[i] = o;
+}
+
 static bool overlap(const void *a, size_t na, const void *b, size_t nb) {
   const uintptr_t x = (uintptr_t)a, y = (uintptr_t)b;
   return x < y + nb && y < x + na;
@@ -482,6 +580,12 @@ static int plan_check_choice_tables(const char *who, const float *d_cost, const 
 static int64_t ctg_tiles(int32_t n_fields, int32_t fw, int32_t fh) {
   if(n_fields < 1 || fw < 1 || fh < 1 || fw > (1 << 24) || fh > (1 << 24) || (int64_t)n_fields * fh * fw > INT_MAX) return 0;
   return (int64_t)n_fields * ((fw + kCtgTile - 1) / kCtgTile) * ((fh + kCtgTile - 1) / kCtgTile);
+}
+
+// Cells of an inflation (the map-grid size rule); 0 for sizes rk_plan_inflate rejects
+static int64_t infl_cells(int32_t n_maps, int32_t width, int32_t height) {
+  if(n_maps < 1 || width < 1 || height < 1 || width > (1 << 24) || height > (1 << 24) || (int64_t)n_maps * height * width > INT_MAX) return 0;
+  return (int64_t)n_maps * height * width;
 }
 
 } // namespace rk
@@ -661,6 +765,57 @@ int rk_plan_cost_to_go(const rk_plan_map_t *map, const rk_plan_ctg_t *spec, cons
     if(b < batch) break; // a round changed nothing: every later one is empty
   }
   if(rounds_out) *rounds_out = rounds;
+  return RK_OK;
+}
+
+size_t rk_plan_inflate_work_bytes(int32_t n_maps, int32_t width, int32_t height) {
+  const int64_t n = infl_cells(n_maps, width, height);
+  return n == 0 ? 0 : ((size_t)n * sizeof(uint16_t) + 3u) & ~(size_t)3u;
+}
+
+int rk_plan_inflate(const rk_plan_map_t *map, const rk_plan_inflate_t *spec, float *d_dst, void *d_work, void *stream) {
+  static const char *who = "rk_plan_inflate";
+  if(!map || !spec) {
+    set_error("%s: NULL map/spec", who);
+    return RK_ERR_ARG;
+  }
+  if(int rc = plan_check_map_grid(who, map)) return rc;
+  if(int rc = plan_check_map_tables(who, map)) return rc;
+  if(spec->n_table < 1 || spec->n_table > 65536) {
+    set_error("%s: need 1 <= n_table <= 65536 (n_table = %d)", who, spec->n_table);
+    return RK_ERR_ARG;
+  }
+  if(!(spec->lethal > 0.0f)) {
+    set_error("%s: lethal must be > 0 (+inf allowed, NaN not)", who);
+    return RK_ERR_ARG;
+  }
+  if(!spec->d_table || ((uintptr_t)spec->d_table & 3u) || !d_dst || ((uintptr_t)d_dst & 3u) || !d_work || ((uintptr_t)d_work & 3u)) {
+    set_error("%s: d_table, d_dst and d_work must be non-NULL 4-byte aligned device pointers", who);
+    return RK_ERR_ARG;
+  }
+  const int64_t n       = infl_cells(map->n_maps, map->width, map->height);
+  const size_t  n_cells = (size_t)n * 4u, n_work = rk_plan_inflate_work_bytes(map->n_maps, map->width, map->height);
+  const size_t  n_tab   = (size_t)spec->n_table * 4u;
+  if(overlap(d_dst, n_cells, map->d_cells, n_cells) || overlap(d_dst, n_cells, d_work, n_work) || overlap(d_dst, n_cells, spec->d_table, n_tab) ||
+     overlap(d_work, n_work, map->d_cells, n_cells) || overlap(d_work, n_work, spec->d_table, n_tab)) {
+    set_error("%s: d_dst and d_work must not overlap each other, the cells or the table", who);
+    return RK_ERR_ARG;
+  }
+  if(int rc = require_device()) return rc;
+  int r = (int)sqrt((double)(spec->n_table - 1)); // rmax = floor(sqrt(n_table - 1)), made exact in integers
+  while(r * r > spec->n_table - 1) r--;
+  while((r + 1) * (r + 1) <= spec->n_table - 1) r++;
+  InflateArgs a;
+  a.cells = map->d_cells, a.table = spec->d_table, a.dst = d_dst;
+  a.n_maps = map->n_maps, a.width = map->width, a.height = map->height, a.rmax = r, a.n_table = spec->n_table;
+  a.lethal = spec->lethal, a.edge = map->outside >= spec->lethal;
+  const int          chunks = (map->height + kInflChunk - 1) / kInflChunk, segs = (map->width + kInflThreads - 1) / kInflThreads;
+  const int64_t      col_threads = (int64_t)map->n_maps * chunks * map->width;
+  const cudaStream_t st = (cudaStream_t)stream;
+  uint16_t          *g = (uint16_t *)d_work;
+  plan_inflate_cols_kernel<<<(unsigned)((col_threads + kInflThreads - 1) / kInflThreads), kInflThreads, 0, st>>>(a, chunks, g);
+  plan_inflate_rows_kernel<<<(unsigned)((int64_t)map->n_maps * map->height * segs), kInflThreads, 0, st>>>(a, segs, g);
+  RK_CUDA(cudaGetLastError());
   return RK_OK;
 }
 

@@ -8,7 +8,8 @@ sigma to each round's elite candidates.  For fleets, predict() gives where each 
 peer_discs() turns those paths into moving keep-out discs for the robot's peers (fleet_peers builds the usual grouping).
 A CostMap, a grid of cell costs shared by the robots of a world, prices walls and shelving at every checkpoint, alone or
 together with discs; its cost_to_go() builds CostToGo fields, shortest-path distances to goals around the walls, that
-price each candidate's end position instead of the straight line to the goal.
+price each candidate's end position instead of the straight line to the goal.  CostMap.inflate prices every cell by its
+distance to the nearest wall through an inflation_table, so that plans and paths keep the robot's body clear of walls.
 """
 import ctypes as C
 
@@ -25,7 +26,7 @@ class CostMap:
     int32 [R] device tensor, the map of each robot (an index outside [0, n_maps) gives that robot no map term); None: map 0
     for every robot.  Cells above 0 add w_map * cell to a candidate's cost at every checkpoint; zero, negative and NaN cells
     add nothing.  The robot is a point read at checkpoints: inflate walls by the body radius plus the distance covered in
-    check_period ticks.  Cells may be changed in place between planning steps.
+    check_period ticks (inflate, inflation_table).  Cells may be changed in place between planning steps.
 
     inv_res = float32(1 / resolution) is computed once here and passed as is, so a restatement can use the same bits;
     x0, y0 and outside are likewise the float32 values the device reads."""
@@ -92,6 +93,46 @@ class CostMap:
         ctg = CostToGo(field, self, offsets=offsets, field_of=field_of, outside=outside)
         ctg.rounds = rounds.value
         return ctg
+
+    def inflate(self, table, lethal=float("inf")):
+        """rk_plan_inflate on the current torch stream of the map's device (asynchronous): a new CostMap with the same
+        origin, resolution, outside and map_of whose cell at squared cell distance d2 from the nearest obstacle of its map
+        (a cell >= lethal; off the grid too when outside >= lethal) is the larger of the cell and table[d2] for
+        d2 < len(table), the cell itself otherwise.  table: float32 [n] on the map's device, 1 <= n <= 65536
+        (inflation_table)."""
+        dev = self.cells.device
+        assert (table.is_cuda and table.device == dev and table.is_contiguous() and table.dtype == torch.float32 and table.dim() == 1
+                and 1 <= table.numel() <= 65536), "table: float32 [n] contiguous tensor on the map's device, 1 <= n <= 65536"
+        lib = _cabi.load()
+        cells = torch.empty_like(self.cells)
+        work = torch.empty((lib.rk_plan_inflate_work_bytes(self.n_maps, self.width, self.height) + 3) // 4, dtype=torch.int32, device=dev)
+        spec = _cabi.PlanInflate()
+        spec.d_table, spec.n_table, spec.lethal = table.data_ptr(), table.numel(), float(lethal)
+        di = _dev_index(dev)
+        _cabi.check(lib.rk_set_device(di))
+        mp = self.struct(0.0)
+        _cabi.check(lib.rk_plan_inflate(C.byref(mp), C.byref(spec), cells.data_ptr(), work.data_ptr(),
+                                        C.c_void_p(torch.cuda.current_stream(di).cuda_stream)))
+        return CostMap(cells, (self.x0, self.y0), self.resolution, outside=self.outside, map_of=self.map_of)
+
+
+def inflation_table(resolution, inscribed, radius, scaling=0.0, peak=1.0, lethal=float("inf"), device="cuda:0"):
+    """The ROS-style inflation profile for CostMap.inflate: float32 [n] on `device`, entry d2 the cost at d = sqrt(d2) *
+    resolution metres (float64) from the nearest obstacle: `lethal` where d <= inscribed, peak * exp(-scaling * (d -
+    inscribed)) beyond, and the table ends at the last d2 whose d <= radius (at most 255 cells).  The comparisons are in
+    float64, so a radius or inscribed radius that is an exact multiple of the resolution may fall just short of it.
+
+    inscribed: the body's radius (for a body that is not round, its circumscribed radius: plan rollouts hold the heading,
+    so a disc footprint is the right model) plus 0.4 * P mm for the distance covered between two checkpoints P ticks
+    apart.  Make the lethal value at least the `lethal` of cost_to_go, so that the inflated wall blocks its paths."""
+    resolution, inscribed, radius = float(resolution), float(inscribed), float(radius)
+    assert 0.0 < resolution < float("inf"), "resolution: metres per cell, finite and > 0"
+    d = torch.arange(65537, dtype=torch.float64).sqrt() * resolution
+    n = int((d <= radius).sum())
+    assert 1 <= n <= 65536, "radius: >= 0 and at most 255 cells"
+    d = d[:n]
+    v = torch.where(d <= inscribed, torch.full_like(d, float(lethal)), float(peak) * torch.exp(-float(scaling) * (d - inscribed)))
+    return v.to(torch.float32).to(device)
 
 
 class CostToGo:

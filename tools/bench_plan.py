@@ -45,10 +45,17 @@ of shelving that opens toward the robot, its goal straight behind the U's bottom
 the map and with or without each robot's cost-to-go field over its 20-cell lane, and reports the share of robots within
 0.1 m of their goals.
 
+With --inflate the run also times rk_plan_inflate (CostMap.inflate) on 1 and 16 maps of the --map world's 800 x 800
+random walls at table radii of 4, 10 and 40 cells (CUDA events around a batch of calls; median over --reps), against the
+bytes a separable transform moves (16 per cell); then it plays the narrow-gap scenario of tests/plan_inflate_ref.py at
+size (R lanes, each with a gap narrower than the body straight ahead and wide gaps on the lane boundaries, --inflate-steps
+steps under argmin and CEM, each robot with its lane's cost-to-go field) on the raw walls and on the inflated map, and
+reports the share of robots whose 0.15 m body ever overlapped a wall cell and the share within 0.1 m of the goal.
+
     python tools/bench_plan.py [--R 4096] [--S 256] [--n-seg 8] [--seg-len 125] [--reps 10] [--out FILE]
                                [--obstacles 1,8 --check-period 125,25,10] [--cem 4:8 --cem-steps 8 --lam 1e-3]
                                [--moving 1:125,8:25] [--fleet 8 --fleet-steps 60] [--map 800:125,800:25,800:5]
-                               [--field 800:16] [--parent-lib path/to/librobotick_b200.so]
+                               [--field 800:16] [--inflate] [--parent-lib path/to/librobotick_b200.so]
 """
 import ctypes as C
 import argparse
@@ -66,7 +73,7 @@ import torch  # noqa: E402
 
 import roboken_fmskf_robot_controller_b200 as rk  # noqa: E402
 from roboken_fmskf_robot_controller_b200 import _cabi, layout, streams  # noqa: E402
-from roboken_fmskf_robot_controller_b200.planner import CostMap, CostToGo, VehiclePlanner, fleet_peers  # noqa: E402
+from roboken_fmskf_robot_controller_b200.planner import CostMap, CostToGo, VehiclePlanner, fleet_peers, inflation_table  # noqa: E402
 from roboken_fmskf_robot_controller_b200.vehicle import VehicleBatch  # noqa: E402
 
 
@@ -362,6 +369,104 @@ def field_bench(a, dev, pl, src, goal, cells_n, G, parent, iters, elite):
     return out
 
 
+# The narrow-gap scenario of tests/plan_inflate_ref.py: 0.15 m body; the inflated map is +inf within 0.225 m of a wall cell
+# (body, 10 mm between checkpoints, 65 mm for the grid) with a thin soft tail out to 0.3 m
+NARROW_BODY, NARROW_INSCRIBED, NARROW_RADIUS, NARROW_SCALING, NARROW_PEAK = 0.15, 0.225, 0.3, 20.0, 1e-4
+
+
+def narrow_gap_walls(R, cell=0.05):
+    """Raw walls bool [H, W] of R lanes x in [r - 0.5, r + 0.5), y in [-1, 1): a 0.1 m band across y = 0 with a 0.2 m gap on
+    the lane's line and a 0.6 m gap centred on each lane boundary; origin (-0.5, -1.0)."""
+    W, H = 20 * R, 40
+    ix = np.arange(W) % 20
+    gap = ((ix >= 8) & (ix < 12)) | (ix < 6) | (ix >= 14)
+    yc = -1.0 + (np.arange(H) + 0.5) * cell
+    return (np.abs(yc) < 0.05)[:, None] & ~gap[None, :]
+
+
+def clearance_overlap(pos, wall_t, origin, body, cell=0.05):
+    """bool [R]: whether some position float32 [T, R, 2] (device) lies closer than `body` to a wall cell's square (the
+    cells within 4 of the position's own are searched: 0.2 m > body)."""
+    H, W = wall_t.shape
+    p = pos.double()
+    ix = torch.floor((p[..., 0] - origin[0]) / cell).long()
+    iy = torch.floor((p[..., 1] - origin[1]) / cell).long()
+    hit = torch.zeros(pos.shape[1], dtype=torch.bool, device=pos.device)
+    for dy in range(-4, 5):
+        for dx in range(-4, 5):
+            cx, cy = ix + dx, iy + dy
+            ok = (cx >= 0) & (cx < W) & (cy >= 0) & (cy < H)
+            isw = ok & wall_t[cy.clamp(0, H - 1), cx.clamp(0, W - 1)]
+            lx, ly = origin[0] + cx * cell, origin[1] + cy * cell
+            ddx = torch.clamp(torch.maximum(lx - p[..., 0], p[..., 0] - (lx + cell)), min=0.0)
+            ddy = torch.clamp(torch.maximum(ly - p[..., 1], p[..., 1] - (ly + cell)), min=0.0)
+            hit |= (isw & (torch.hypot(ddx, ddy) < body)).any(dim=0)
+    return hit
+
+
+def inflate_bench(a, dev, iters, elite):
+    """--inflate: rk_plan_inflate's time on the random-wall world, and the narrow-gap scenario at size."""
+    out = {"timing": []}
+    rng = np.random.default_rng(31)
+    grids = np.stack([random_walls(800, rng) for _ in range(16)])
+    batch = 20  # calls per timed window: one call on one map takes microseconds
+    for n_maps in (1, 16):
+        cm = CostMap(torch.from_numpy(grids[:n_maps].copy()).to(dev), (-20.0, -20.0), 0.05)
+        for rc in (4, 10, 40):
+            table = inflation_table(0.05, 0.2, rc * 0.05 + 1e-9, scaling=3.0, device=dev)
+            cm.inflate(table, lethal=1.0)
+            torch.cuda.synchronize()
+            ts = [timed(lambda: [cm.inflate(table, lethal=1.0) for _ in range(batch)]) / batch for _ in range(a.reps)]
+            cells = n_maps * 800 * 800
+            ms = float(np.median(ts))
+            out["timing"].append({"maps": n_maps, "cells": cells, "radius_cells": rc, "n_table": table.numel(), "us_median": round(ms * 1e3, 2),
+                                  "us_min_max": [round(float(np.min(ts)) * 1e3, 2), round(float(np.max(ts)) * 1e3, 2)],
+                                  "model_bytes": 16 * cells, "model_GB_per_s": round(16 * cells / (ms * 1e-3) / 1e9, 1)})
+    out["timing_note"] = ("model_bytes: 16 per cell (cells read twice, a 2-byte column distance written and read, the output written); "
+                          "the 16 maps' 164 MB would take about 21 us at the 7.7 TB/s HBM data-sheet rate; the working set stays in L2 "
+                          "across the repeated calls")
+    R, n_seg, seg_len, P = a.R, a.n_seg, a.seg_len, 25
+    wall = narrow_gap_walls(R)
+    origin = (-0.5, -1.0)
+    raw = CostMap(torch.from_numpy(wall.astype(np.float32)).to(dev), origin, 0.05)
+    inflated = raw.inflate(inflation_table(0.05, NARROW_INSCRIBED, NARROW_RADIUS, NARROW_SCALING, NARROW_PEAK, device=dev), lethal=1.0)
+    wall_t = torch.from_numpy(wall).to(dev)
+    starts = np.stack([np.arange(R, dtype=np.float64), np.full(R, -0.40)], axis=1).astype(np.float32)
+    goals = np.stack([np.arange(R, dtype=np.float64), np.full(R, 0.40)], axis=1).astype(np.float32)
+    ref = torch.from_numpy(np.ascontiguousarray(np.broadcast_to(goals, (n_seg, R, 2)))).to(dev)
+    aos = np.zeros((R, layout.VS_WORDS), dtype=np.uint32)
+    aos[:, layout.VS_POS_X], aos[:, layout.VS_POS_Y] = starts[:, 0].view(np.uint32), starts[:, 1].view(np.uint32)
+    offs = np.stack([np.arange(R) * 20, np.zeros(R, np.int64)], axis=1).astype(np.int32)
+    sc = {"robots": R, "steps": a.inflate_steps, "check_period": P, "w_map": 1e4, "w_field": 10.0, "body_m": NARROW_BODY,
+          "inscribed_m": NARROW_INSCRIBED, "radius_m": NARROW_RADIUS, "scaling": NARROW_SCALING, "peak": NARROW_PEAK}
+    for use in (False, True):
+        cm = inflated if use else raw
+        ctg = cm.cost_to_go(goals, size=(cm.height, 20), offsets=offs, lethal=1.0, field_of=torch.arange(R, dtype=torch.int32, device=dev))
+        for mode in ("argmin", "cem"):
+            S = a.S if mode == "argmin" else a.S // iters
+            pl = VehiclePlanner(R, S, n_seg, seg_len, dev, sigma=(250.0, 250.0, 0.2), seed=0xA11)
+            vb = VehicleBatch(R, dev)
+            vb.load_state_soa(layout.aos_to_soa(aos))
+            tr = torch.empty((seg_len, _cabi.RK_VDT_TRACE_WORDS, R), dtype=torch.int32, device=dev)
+            hit = torch.zeros(R, dtype=torch.bool, device=dev)
+            kw = dict(check_period=P, costmap=cm, w_map=1e4, field=ctg, w_field=10.0)
+            for it in range(a.inflate_steps):
+                if mode == "argmin":
+                    pl.plan(vb, ref, 0.0, 1.0, 1e-9, lam=0.0, shift=0, seed=0xA11 + it, **kw)
+                else:
+                    pl.plan_cem(vb, ref, 0.0, 1.0, 1e-9, iters, elite, 0.0, (40.0, 40.0, 0.05), shift=0, seed=0xA11 + it, **kw)
+                vb.rollout(seg_len, sensor_mode=_cabi.RK_SENSOR_PLANT, cmd=pl.first_command(), seg_len=seg_len, trace=tr)
+                hit |= clearance_overlap(tr[:, :2].view(torch.float32).permute(0, 2, 1), wall_t, origin, NARROW_BODY)
+            st = layout.soa_to_aos(vb.state.cpu().numpy().view(np.uint32), R, layout.VS_WORDS)
+            pos = st[:, [layout.VS_POS_X, layout.VS_POS_Y]].view(np.float32)
+            d = np.hypot(pos[:, 0] - goals[:, 0], pos[:, 1] - goals[:, 1])
+            sc[f"{mode}_{'inflated' if use else 'raw'}"] = {
+                "S": S, "body_overlapped_wall_share": float(hit.float().mean()), "within_0.1m_share": float((d < 0.1).mean()),
+                "goal_dist_median_m": float(np.median(d)), "goal_dist_p90_m": float(np.quantile(d, 0.9))}
+    out["narrow_gap"] = sc
+    return out
+
+
 def wall_report(a, dev, iters, elite):
     """The wall scenario at size under argmin (S candidates) and CEM (iters rounds of S / iters), with and without the map:
     the share of robots that ever enter a wall cell and the distance to the goal after --map-steps steps."""
@@ -427,6 +532,8 @@ def main():
     ap.add_argument("--parent-lib", default=None, help="another build's library: time its rk_plan_rollout_moving side by side")
     ap.add_argument("--field", default=None, help="CELLS:G: time cost-to-go fields and play the wall and dead-end scenarios")
     ap.add_argument("--field-steps", type=int, default=60, help="planning steps of the dead-end scenario")
+    ap.add_argument("--inflate", action="store_true", help="time rk_plan_inflate and play the narrow-gap scenario")
+    ap.add_argument("--inflate-steps", type=int, default=60, help="planning steps of the narrow-gap scenario")
     a = ap.parse_args()
     moving = [tuple(int(v) for v in x.split(":")) for arg in a.moving for x in arg.split(",") if x]
     maps = [tuple(int(v) for v in x.split(":")) for arg in a.map for x in arg.split(",") if x]
@@ -703,7 +810,9 @@ def main():
     if a.field:
         cells_n, G = (int(v) for v in a.field.split(":"))
         res["field"] = field_bench(a, dev, pl, src, goal, cells_n, G, parent, *((cem_iters, cem_elite) if a.cem else (4, 8)))
-    if moving or a.fleet or maps or a.field:
+    if a.inflate:
+        res["inflate"] = inflate_bench(a, dev, *((cem_iters, cem_elite) if a.cem else (4, 8)))
+    if moving or a.fleet or maps or a.field or a.inflate:
         res["max_sm_clock"] = power_limit("clocks.max.sm")
     if a.fleet:
         res["fleet"] = fleet_report(a, a.fleet, dev)
